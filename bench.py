@@ -1,6 +1,7 @@
 """bench.py - headline benchmark of the M-GCN hot path on B200 (contract: see the task brief / DESIGN.md section 6).
 
     python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference] [--workload wn18rr|fb15k237|wikidata5m]
+                    [--dump-outputs DIR]
 
 Metric (BASELINE.json): edges/sec of the relation-aware graph convolution, forward + backward, where an "edge" is one
 directed edge of edge_index (2E per pass; SURVEY.md 8(d)).  ONE JSON line on stdout.
@@ -27,6 +28,8 @@ mode (N x the named shape).
                entity table sharded over the ranks, integer counts all-reduced, sharded == unsharded asserted in-run
 `--impl reference` times the reference's CPU implementation of the same two scopes (layer fwd+bwd = value, full training
 step = e2e) on a bounded sample of the same workload; rank 0 only.
+`--dump-outputs DIR` (N = 1) writes what the last timed layer step computed to DIR/<name>.npy (see dump_outputs), so that
+two builds can be compared output for output.  bench.py writes nothing into the source tree.
 """
 import argparse
 import json
@@ -41,6 +44,7 @@ import torch
 
 ROOT = os.path.dirname(os.path.abspath(__file__))
 sys.path.insert(0, ROOT)
+sys.dont_write_bytecode = True         # the source tree may be read-only; nothing is cached in it
 
 WORKLOADS = {
     # name: (N entities, R relations, E train triples, synthetic seed)        SURVEY.md 8(d)
@@ -338,7 +342,7 @@ def reference_cpu_legs(workload, steps, warmup, budget_s, want_step=True):
         return loss.item()
 
     def timed(fn, n_warm, n_steps, budget):
-        times, t_end = [], time.time() + budget
+        times, t_end = [], time.time() + (budget if budget is not None else float('inf'))
         for i in range(n_warm + n_steps):
             t0 = time.perf_counter()
             fn()
@@ -347,8 +351,11 @@ def reference_cpu_legs(workload, steps, warmup, budget_s, want_step=True):
             if len(times) >= 2 and time.time() > t_end:
                 break
         return times
+    # at least one untimed call per leg: the first one pays for first-touch allocation and thread-pool start-up, which
+    # would otherwise make the layer alone (timed first) look slower than the training step that contains it
+    warmup = max(1, warmup)
     lt = timed(layer, warmup, steps, budget_s)
-    st = timed(train_step, min(warmup, 1), steps, budget_s) if want_step else []
+    st = timed(train_step, warmup, steps, budget_s) if want_step else []
     return {'kind': 'reference' if ref is not None else 'port', 'cores': torch.get_num_threads(), 'N': N, 'R': R, 'E': E,
             'div': div, 'layer_s': float(np.mean(lt)), 'n_layer': len(lt),
             'step_s': float(np.mean(st)) if st else None, 'n_step': len(st)}
@@ -378,14 +385,15 @@ def run_reference(args, rank, world):
     if rank != 0:
         return
     workload = args.workload or 'wikidata5m'
-    legs = reference_cpu_legs(workload, args.steps, args.warmup, budget_s=45.0)
+    legs = reference_cpu_legs(workload, args.steps, args.warmup, budget_s=None)
     N, R, E, _ = WORKLOADS[workload]
     val = 2 * legs['E'] / legs['layer_s']
     e2e_val = 2 * legs['E'] / legs['step_s']
     base = cpu_baseline_entry(legs, workload)
     line = {
         'impl': 'reference', 'metric': 'edges/sec GCN fwd+bwd', 'value': val, 'unit': 'edges/s', 'n_gpus': args.gpus,
-        'steps': args.steps, 'warmup': args.warmup, 'ms_per_step': 1e3 * legs['layer_s'], 'higher_is_better': True,
+        'steps': args.steps, 'timed_steps': legs['n_layer'], 'warmup': max(1, args.warmup), 'ms_per_step': 1e3 * legs['layer_s'],
+        'higher_is_better': True,
         'scaling': 'strong' if (world > 1 and not os.environ.get('KGC_BENCH_WEAK')) else 'weak', 'vs_baseline': None,
         'dtype': 'f32', 'data': 'synthetic',
         'config': {'workload': workload + '_shape', 'N': N, 'R': R, 'E': E, 'd_in': D_IN, 'd_out': D_OUT, 'batch': BATCH,
@@ -624,14 +632,18 @@ def capture_and_time(case, args, dist, flush, clocks_index):
     L.LAUNCHES = 0
     case.step()
     launches_per_step = L.LAUNCHES
-    run_step = case.step
+    last = {}                                        # (all_ent, all_rel) of the latest step; a replay rewrites them in place
+
+    def run_step():
+        last.pop('out', None)                        # eager: do not hold the previous step's outputs through this one
+        last['out'] = case.step()
     if not args.no_graph:
         try:
             graph = torch.cuda.CUDAGraph()
             for t in case.leaves:
                 t.grad = None
             with torch.cuda.graph(graph):
-                case.step()
+                last['out'] = case.step()
             run_step = graph.replay
             launch_mode = 'cuda_graph'
         except Exception as exc:                      # pragma: no cover
@@ -644,12 +656,14 @@ def capture_and_time(case, args, dist, flush, clocks_index):
         dist.barrier()
     torch.cuda.synchronize()
     ev = [(torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)) for _ in range(args.steps)]
+    timed_steps = 0
     with ClockSampler(clocks_index) as clocks:
         for a, b in ev:
             flush()
             a.record()
             run_step()
             b.record()
+            timed_steps += 1
         torch.cuda.synchronize()
         if dist is not None:
             dist.barrier()
@@ -659,8 +673,8 @@ def capture_and_time(case, args, dist, flush, clocks_index):
         t = torch.tensor([total_ms], device=case.dev, dtype=torch.float64)
         dist.all_reduce(t, op=dist.ReduceOp.MAX)
         total_ms = float(t[0])
-    return {'total_ms': total_ms, 'launch_mode': launch_mode, 'launches_per_step': launches_per_step, 'clocks': clocks.summary(),
-            'graph': graph}
+    return {'total_ms': total_ms, 'timed_steps': timed_steps, 'launch_mode': launch_mode, 'launches_per_step': launches_per_step,
+            'clocks': clocks.summary(), 'graph': graph, 'outputs': last['out']}
 
 
 def kernel_rooflines(case, flush):
@@ -745,8 +759,32 @@ def kernel_rooflines(case, flush):
     return roof, out
 
 
-def bench_layer(k, orc, workload, dev, args, flush, with_roofline=True):
-    """value / parity / rooflines of one workload on ONE GPU."""
+DUMP_MAX_ROWS = 16384      # row sample of every output with more rows: ~29 MB in all at the Wikidata5M shape
+
+
+def dump_outputs(case, ent, rel, out_dir):
+    """What the last timed step handed its caller, as ``out_dir/<name>.npy`` (float32): the layer's outputs all_ent /
+    all_rel and the gradient of every input and parameter (d_x, d_ee, d_rel, d_<parameter>).  A tensor with more than
+    DUMP_MAX_ROWS rows is cut to that many rows, drawn by torch.randperm from a generator seeded with 0 (the same rows
+    for every tensor of the same height), in increasing row order.  The inputs are pure functions of the workload's
+    seeds, so two builds run with the same arguments can be compared array for array."""
+    os.makedirs(out_dir, exist_ok=True)
+    arrays = {'all_ent': ent, 'all_rel': rel, 'd_x': case.x.grad, 'd_ee': case.ee.grad, 'd_rel': case.rl.grad}
+    for name, prm in case.conv.named_parameters():
+        arrays['d_' + name.replace('.', '_')] = prm.grad
+    for name, t in arrays.items():
+        if t is None:
+            raise RuntimeError('--dump-outputs: the timed step produced no {}'.format(name))
+        t = t.detach()
+        if t.dim() > 0 and t.size(0) > DUMP_MAX_ROWS:
+            rows = torch.randperm(t.size(0), generator=torch.Generator().manual_seed(0))[:DUMP_MAX_ROWS].sort().values
+            t = t[rows.to(t.device)]
+        np.save(os.path.join(out_dir, name + '.npy'), t.to(torch.float32).cpu().numpy())
+    sys.stderr.write('--dump-outputs: {} arrays of the last timed step written to {}\n'.format(len(arrays), out_dir))
+
+
+def bench_layer(k, orc, workload, dev, args, flush, with_roofline=True, dump_dir=None):
+    """value / parity / rooflines of one workload on ONE GPU; ``dump_dir``: write the last timed step's outputs there."""
     case = LayerCase(k, orc, workload, dev)
     res = {'N': case.N, 'R': case.R, 'E': case.E, 'setup_s': case.setup_s}
     torch.cuda.synchronize()
@@ -761,10 +799,13 @@ def bench_layer(k, orc, workload, dev, args, flush, with_roofline=True):
             res['parity'] = {'ok': False, 'error': repr(exc)}
             torch.cuda.empty_cache()
     t = capture_and_time(case, args, None, flush, dev.index or 0)
-    ms = t['total_ms'] / args.steps
+    if dump_dir is not None:
+        dump_outputs(case, *t['outputs'], dump_dir)
+    t['outputs'] = None
+    ms = t['total_ms'] / t['timed_steps']
     fwd_b, bwd_b = algorithmic_bytes(case.N, case.R, case.E)
     _, peak, peak_src = measured_peaks()
-    res.update({'value': 2 * case.E / (ms * 1e-3), 'ms_per_step': ms, 'launch': t['launch_mode'],
+    res.update({'value': 2 * case.E / (ms * 1e-3), 'ms_per_step': ms, 'timed_steps': t['timed_steps'], 'launch': t['launch_mode'],
                 'launches_per_step': t['launches_per_step'], 'clocks': t['clocks'],
                 'step_hbm': {'algorithmic_bytes_fwd_bwd': fwd_b + bwd_b, 'achieved_gbs': (fwd_b + bwd_b) / (ms * 1e-3) / 1e9,
                              'frac_of_peak': (fwd_b + bwd_b) / (ms * 1e-3) / 1e9 / peak, 'peak_gbs': peak, 'peak_source': peak_src,
@@ -797,10 +838,11 @@ def run_ours(args, rank, world, local_rank):
             'warmup': max(3, args.warmup), 'higher_is_better': True, 'vs_baseline': None, 'dtype': 'f32', 'data': 'synthetic'}
     rc = 0
     if world == 1:
-        res, case = bench_layer(k, orc, workload, dev, args, flush)
+        res, case = bench_layer(k, orc, workload, dev, args, flush, dump_dir=args.dump_outputs)
         value, ms = res['value'], res['ms_per_step']
         N, E = case.N, case.E
-        line.update({'value': value, 'ms_per_step': ms, 'scaling': 'weak', 'gpu_launches': res['launches_per_step'] * args.steps,
+        line.update({'value': value, 'ms_per_step': ms, 'timed_steps': res['timed_steps'], 'scaling': 'weak',
+                     'gpu_launches': res['launches_per_step'] * res['timed_steps'],
                      'plan_build_s': res.get('plan_build_s'),
                      'clocks': res['clocks'], 'roofline': res.get('roofline'), 'kernels': res.get('kernels'),
                      'step_hbm': res['step_hbm'], 'parity': res.get('parity')})
@@ -834,7 +876,7 @@ def run_ours(args, rank, world, local_rank):
             if not parity['ok']:
                 rc = 3
         t = capture_and_time(case, args, dist, flush, local_rank)
-        ms = t['total_ms'] / args.steps
+        ms = t['total_ms'] / t['timed_steps']
         value = 2 * E / (ms * 1e-3)                      # E counts every rank's triples
         launch_mode = t['launch_mode']
         part = case.part
@@ -852,8 +894,8 @@ def run_ours(args, rank, world, local_rank):
                            'one-shot peer-memory kernel (K10)' if p2p is not None else 'NCCL'))
         if p2p is not None:
             p2p.check()
-        line.update({'value': value, 'ms_per_step': ms, 'scaling': 'weak' if weak else 'strong',
-                     'gpu_launches': t['launches_per_step'] * args.steps, 'clocks': t['clocks'], 'parity': parity,
+        line.update({'value': value, 'ms_per_step': ms, 'timed_steps': t['timed_steps'], 'scaling': 'weak' if weak else 'strong',
+                     'gpu_launches': t['launches_per_step'] * t['timed_steps'], 'clocks': t['clocks'], 'parity': parity,
                      'roofline': None, 'kernels': None,
                      'step_hbm': {'note': 'per-kernel rooflines are measured at N = 1 (same kernels on every rank)'}})
         if args.no_e2e:
@@ -1161,11 +1203,18 @@ def main():
     ap.add_argument('--no-e2e', action='store_true', help='profiling runs only: skip the end-to-end leg')
     ap.add_argument('--no-parity', action='store_true', help='profiling runs only: skip the parity check')
     ap.add_argument('--no-extras', action='store_true', help='N = 1: skip the WN18RR / FB15k-237 entries')
+    ap.add_argument('--dump-outputs', metavar='DIR', default=None,
+                    help='N = 1, --impl ours: write the outputs and gradients of the last timed layer step to DIR/<name>.npy '
+                         '(float32; tensors taller than {} rows as a seeded row sample)'.format(DUMP_MAX_ROWS))
     args = ap.parse_args()
-    guard_stdout()
     rank = int(os.environ.get('RANK', '0'))
     world = int(os.environ.get('WORLD_SIZE', '1'))
     local_rank = int(os.environ.get('LOCAL_RANK', '0'))
+    if args.steps < 1:
+        ap.error('--steps must be at least 1')
+    if args.dump_outputs is not None and (args.impl != 'ours' or world > 1):
+        ap.error('--dump-outputs needs --impl ours on one GPU (WORLD_SIZE=1)')
+    guard_stdout()
     if args.impl == 'reference':
         run_reference(args, rank, world)
     else:

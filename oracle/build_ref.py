@@ -1,14 +1,14 @@
-"""Build oracle/_ref/ from the reference where it lies.  TEST INFRASTRUCTURE ONLY.
+"""Build oracle/_ref/ from a checkout of the reference.  TEST INFRASTRUCTURE ONLY.
 
-    python oracle/build_ref.py            (also called by __graft_entry__.build())
+    KGC_REFERENCE_DIR=<checkout of weilonghu/KGC-GCN> python oracle/build_ref.py      (also called by __graft_entry__.build())
 
-The reference (weilonghu/KGC-GCN) is pure Python; its four modules are byte-compiled from /root/reference into
-``oracle/_ref/{model,data_loader,main,utils}.refbc`` (CPython bytecode: a BUILT artefact like a .so - git-ignored, it
-travels to the GPU box with the snapshot; no reference source is copied into the repository).  With ``oracle/shims`` on
-the path (stand-ins for the reference's absent third-party imports) they import unmodified, which is what
-``bench.py --impl reference`` times (cpu_baseline.kind = "reference") and what tests/test_oracle_golden.py cross-checks
-the port against when the directory is present.  /root/reference does not exist on the GPU box: there the prebuilt
-files are used as they are; when they are missing everything falls back to the pinned port (oracle/mgcn_oracle.py).
+The reference (weilonghu/KGC-GCN) is pure Python and is not part of this repository; its four modules are byte-compiled
+from $KGC_REFERENCE_DIR into ``oracle/_ref/{model,data_loader,main,utils}.refbc`` (CPython bytecode: a BUILT artefact like
+a .so - git-ignored; no reference source is copied into the repository).  With ``oracle/shims`` on the path (stand-ins
+for the reference's absent third-party imports) they import unmodified, which is what ``bench.py --impl reference`` times
+(cpu_baseline.kind = "reference") and what the tests that name the reference cross-check the port against.  Without
+KGC_REFERENCE_DIR nothing is built: bench.py falls back to the pinned port (oracle/mgcn_oracle.py), those tests skip, and
+the committed fixtures in tests/golden (written by oracle/make_golden.py from the reference) still pin the port.
 """
 import os
 import py_compile
@@ -21,9 +21,9 @@ EXT = '.refbc'                 # not '.pyc': snapshot tools commonly drop *.pyc
 
 
 def build_ref(ref_dir=None):
-    """-> list of written files ([] when the reference tree is absent)."""
-    ref_dir = ref_dir or os.environ.get('KGC_REFERENCE_DIR', '/root/reference')
-    if not all(os.path.exists(os.path.join(ref_dir, m + '.py')) for m in MODULES):
+    """-> list of written files ([] when no reference checkout is given or it lacks a module)."""
+    ref_dir = ref_dir or os.environ.get('KGC_REFERENCE_DIR')
+    if not ref_dir or not all(os.path.exists(os.path.join(ref_dir, m + '.py')) for m in MODULES):
         return []
     os.makedirs(OUT, exist_ok=True)
     written = []
@@ -71,4 +71,4 @@ def load_reference():
 
 
 if __name__ == '__main__':
-    print(build_ref() or 'reference tree not found: nothing built')
+    print(build_ref() or 'KGC_REFERENCE_DIR is not a reference checkout: nothing built')

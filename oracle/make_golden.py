@@ -1,7 +1,7 @@
 """Generate tests/golden/* by running the UNMODIFIED reference.  TEST INFRASTRUCTURE ONLY.
 
-Run in the authoring container only (needs /root/reference, which does not exist on the
-GPU box):   python oracle/make_golden.py
+Needs a checkout of the reference (weilonghu/KGC-GCN), which is not part of this repository:
+    KGC_REFERENCE_DIR=<checkout> python oracle/make_golden.py
 The reference modules are imported from where they lie through ``oracle/shims`` (four
 stand-ins for its absent third-party imports); nothing is copied.  The fixtures are small
 (< 2 MB in total), committed, and are what pins ``oracle/mgcn_oracle.py`` and the CUDA path.
@@ -16,7 +16,9 @@ import torch
 
 HERE = os.path.dirname(os.path.abspath(__file__))
 ROOT = os.path.dirname(HERE)
-REF = os.environ.get('KGC_REFERENCE_DIR', '/root/reference')
+REF = os.environ.get('KGC_REFERENCE_DIR')
+if not REF or not os.path.isfile(os.path.join(REF, 'model.py')):
+    sys.exit('oracle/make_golden.py runs the reference: set KGC_REFERENCE_DIR to a checkout of weilonghu/KGC-GCN')
 OUT = os.path.join(ROOT, 'tests', 'golden')
 
 sys.path.insert(0, os.path.join(HERE, 'shims'))

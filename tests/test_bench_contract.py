@@ -7,6 +7,8 @@ import os
 import subprocess
 import sys
 
+import pytest
+
 ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
 
 
@@ -42,6 +44,7 @@ def test_reference_arm_prints_one_contract_line():
     d = json.loads(lines[0])
     assert d['impl'] == 'reference' and d['metric'] == 'edges/sec GCN fwd+bwd' and d['unit'] == 'edges/s'
     assert d['n_gpus'] == 1 and d['steps'] == 1 and d['higher_is_better'] is True and d['gpu_launches'] == 0
+    assert d['timed_steps'] == 1 and d['e2e']['steps'] == 1
     # the default workload is the GPU arm's (Wikidata5M shape); the CPU runs a bounded sample of it and says which
     assert d['config']['workload'] == 'wikidata5m_shape' and 'divided by 64' in d['config']['sample']
     e_sample = 20614279 // 64
@@ -55,18 +58,18 @@ def test_reference_arm_prints_one_contract_line():
 
 
 def test_reference_bytecode_is_the_reference():
-    """oracle/_ref (built by oracle/build_ref.py from /root/reference when that tree exists) imports as the reference's own
-    modules; the port and the unmodified reference give the same layer outputs on a small graph (the golden fixtures pin
-    the same thing; this checks the artefact bench.py --impl reference actually runs)."""
+    """oracle/_ref (built by oracle/build_ref.py from the reference checkout KGC_REFERENCE_DIR names) imports as the
+    reference's own modules; the port and the unmodified reference give the same layer outputs on a small graph (the golden
+    fixtures pin the same thing; this checks the artefact bench.py --impl reference actually runs)."""
     import pytest
     import torch
     sys.path.insert(0, os.path.join(ROOT, 'oracle'))
     import build_ref
-    if os.path.isdir('/root/reference'):
+    if os.environ.get('KGC_REFERENCE_DIR'):
         assert build_ref.build_ref()
     ref = build_ref.load_reference()
     if ref is None:
-        pytest.skip('oracle/_ref was not built (no reference tree on this machine)')
+        pytest.skip('oracle/_ref was not built (set KGC_REFERENCE_DIR to a checkout of the reference)')
     import mgcn_oracle as orc
     ref_model = ref[0]
     N, R, E = 50, 3, 200
@@ -86,3 +89,14 @@ def test_reference_bytecode_is_the_reference():
 
 def test_reference_arm_other_ranks_exit_quietly():
     assert _run_reference({'RANK': '1', 'WORLD_SIZE': '2', 'LOCAL_RANK': '1'}) == []
+
+
+@pytest.mark.parametrize('extra', [['--steps', '0'], ['--impl', 'reference', '--dump-outputs', 'out'],
+                                   ['--dump-outputs', 'out', '--gpus', '2']])
+def test_bad_arguments_are_refused_before_any_work(extra, tmp_path):
+    """--steps below 1, and --dump-outputs where there is no single-GPU timed layer step to dump, end with a usage error."""
+    env = dict(os.environ, RANK='0', WORLD_SIZE='2' if '--gpus' in extra else '1')
+    p = subprocess.run([sys.executable, os.path.join(ROOT, 'bench.py')] + extra, stdout=subprocess.PIPE, stderr=subprocess.PIPE,
+                       text=True, timeout=120, env=env, cwd=str(tmp_path))
+    assert p.returncode == 2 and p.stdout == '' and 'error' in p.stderr
+    assert not os.path.exists(str(tmp_path / 'out'))

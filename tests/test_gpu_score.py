@@ -276,17 +276,38 @@ def test_filtered_rank_exact_mode(k):
     assert float(pes[1]) > float(mean[1]) > float(opt[1]) and float(pes[2]) < float(mean[2]) < float(opt[2])
 
 
+def _restated_evaluate(data_dir, sd, prm):
+    """evaluate() of main.py:80-135 on the valid split, restated by the oracle in float64 on the CPU (GCN + ConvE eval
+    forward, sigmoid scores, the reference's dense filtered rank on float32 scores, its sums and rounding) - the same
+    functions tests/test_oracle_golden.py holds to the reference's own predict() / evaluate() output stored in
+    tests/golden (toy_model.npz, toy_metrics.json, rank_case.npz).  ``sd``: a state dict with the reference's names."""
+    ds = orc.load_dataset(data_dir)
+    N = ds['num_entity']
+    g = orc.build_graph(ds['triples']['train'], N, ds['num_relation'])
+    sd = {kk: v.detach().cpu().double() for kk, v in sd.items() if v.is_floating_point()}
+    w = {kk[len('conv1.'):]: v for kk, v in sd.items() if kk.startswith('conv1.')}
+    dec = {kk[len('conv2.'):]: v for kk, v in sd.items() if kk.startswith('conv2.')}
+    ent, rel, _ = orc.conv_forward(sd['entity_embedding'], torch.from_numpy(g['edge_index']), torch.from_numpy(g['edge_attr'][0]),
+                                   sd['edge_embeddings'], sd['relation_embedding'], w, training=False)
+    sums = {}
+    for mode in ('tail', 'head'):
+        qs = ds['queries']['valid_' + mode]
+        trip = torch.tensor([q['triple'] for q in qs], dtype=torch.long)
+        sc = orc.score_tail(orc.conve_front(ent[trip[:, 0]], rel[trip[:, 1]], dec, prm.k_w, prm.k_h), ent, dec['bias'])
+        lab = torch.from_numpy(np.stack([orc.make_label(q['label'], N) for q in qs]))
+        sums[mode] = orc.metric_sums(orc.filtered_ranks_dense(sc.float(), lab, trip[:, 2]).numpy())
+    return g, orc.combine_metrics(sums['tail'], sums['head'])
+
+
 def test_predict_against_the_reference_at_realistic_size(k, tmp_path):
-    """The reference's OWN predict() / evaluate() (main.py:80-135, run on the CPU from oracle/_ref through oracle/shims)
-    against ours on a synthetic data set of realistic size (8,000 entities, 24,000 training triples, 400 validation
-    triples) written as text files both loaders read, with the same state dict: MR / MRR / hits@k of the exact mode
-    (precision='fp32') must equal the reference's to the 5 places evaluate() rounds to unless a rank sits on an fp32 tie;
-    the bf16 sweep is reported next to it.  Skipped when oracle/_ref was not built."""
+    """Our predict() / evaluate() on a synthetic data set of realistic size (8,000 entities, 24,000 training triples, 400
+    validation triples) written as text files, with a seeded state dict spread so that the scores are not at their xavier
+    init: MR / MRR / hits@k of the exact mode (precision='fp32') must equal, to the 5 places evaluate() rounds to unless a
+    rank sits on an fp32 tie, (a) the float64 restatement of the reference's evaluate() that the golden fixtures pin
+    (_restated_evaluate), and (b) when oracle/_ref is built (KGC_REFERENCE_DIR), the reference's OWN predict() / evaluate()
+    (main.py:80-135, run on the CPU through oracle/shims) on the same state dict.  The bf16 sweep is reported next to it."""
     import build_ref
     ref = build_ref.load_reference()
-    if ref is None:
-        pytest.skip('oracle/_ref not built')
-    ref_model, ref_dl, ref_main = ref
     N, R, E = 8000, 12, 24000
     tri = orc.synthetic_triples(N, R, E + 800, 21)
     root = tmp_path / 'data' / 'Synth'
@@ -299,29 +320,37 @@ def test_predict_against_the_reference_at_realistic_size(k, tmp_path):
     os.chdir(tmp_path)
     try:
         dl = k.DataLoader('Synth', prm)
-        rdl = ref_dl.DataLoader('Synth', prm)
+        rdl = ref[1].DataLoader('Synth', prm) if ref is not None else None
     finally:
         os.chdir(cwd)
-    assert dl.num_entity == rdl.num_entity and dl.num_edge == rdl.num_edge
     torch.manual_seed(3)
-    rm = ref_model.MGCN(rdl.num_entity, rdl.num_relation, rdl.num_edge, prm)
+    if ref is not None:
+        assert dl.num_entity == rdl.num_entity and dl.num_edge == rdl.num_edge
+        src = ref[0].MGCN(rdl.num_entity, rdl.num_relation, rdl.num_edge, prm)
+    else:
+        src = k.MGCN(dl.num_entity, dl.num_relation, dl.num_edge, prm)
     with torch.no_grad():                                    # spread the scores: a trained model is not at its xavier init
-        rm.conv2.bias.normal_(0, 0.5)
-        rm.entity_embedding.mul_(30.0)
-    rm.eval()
+        src.conv2.bias.normal_(0, 0.5)
+        src.entity_embedding.mul_(30.0)
+    src.eval()
     m = k.MGCN(dl.num_entity, dl.num_relation, dl.num_edge, prm)
-    m.load_state_dict(rm.state_dict(), strict=True)
+    m.load_state_dict(src.state_dict(), strict=True)
     m = m.cuda()
+    g, restated = _restated_evaluate(str(root), src.state_dict(), prm)
+    assert np.array_equal(g['edge_index'], dl.graph.edge_index.cpu().numpy())      # same entity / relation ids
     dl.graph.to('cuda')
-    prm_cpu = SimpleNamespace(**dict(vars(prm), device='cpu'))
-    torch.manual_seed(4)
-    ref_iters = rdl.get_data_loaders(128, 0, prm_cpu)
-    ref_ev = ref_main.evaluate(rm, ref_iters, rdl.graph, prm_cpu, 'valid')
+    compare = {'restated reference (float64 oracle)': restated}
+    if ref is not None:
+        prm_cpu = SimpleNamespace(**dict(vars(prm), device='cpu'))
+        torch.manual_seed(4)
+        compare['reference'] = ref[2].evaluate(src, rdl.get_data_loaders(128, 0, prm_cpu), rdl.graph, prm_cpu, 'valid')
     iters = dl.get_data_loaders(128, 0, prm)
     ours = {p_: k.evaluate(m, iters, dl.graph, prm, 'valid', precision=p_) for p_ in ('fp32', 'bf16')}
-    print('reference', ref_ev, 'fp32 mode', ours['fp32'], 'bf16 sweep', ours['bf16'])
-    # the GCN / ConvE front end run in fp32 on both sides with different summation orders (1e-6-level differences in the
-    # logits), so a handful of near-tied ranks may differ by one place: MR within 0.05%, MRR / hits within 2.5e-3 (1 of 800 queries = 1.25e-3)
-    for key, v in ref_ev.items():
-        tol = 5e-4 * abs(v) if key == 'mr' else 2.5e-3
-        assert abs(float(ours['fp32'][key]) - float(v)) <= tol, (key, ours['fp32'][key], v)
+    print(compare, 'fp32 mode', ours['fp32'], 'bf16 sweep', ours['bf16'])
+    # the GCN / ConvE front end run with different summation orders on both sides (1e-6-level differences in the logits),
+    # so a handful of near-tied ranks may differ by one place: MR within 0.05%, MRR / hits within 2.5e-3 (1 of 800 queries = 1.25e-3)
+    for what, want in compare.items():
+        assert set(want) == {'mr', 'mrr', 'hits@1', 'hits@3', 'hits@10'}, what
+        for key, v in want.items():
+            tol = 5e-4 * abs(v) if key == 'mr' else 2.5e-3
+            assert abs(float(ours['fp32'][key]) - float(v)) <= tol, (what, key, ours['fp32'][key], v)

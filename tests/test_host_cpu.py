@@ -463,8 +463,9 @@ def test_gather_segments_edge_cases():
 
 def test_checkpoint_interchanges_with_the_reference(tmp_path):
     """utils.save_checkpoint / load_checkpoint (reference utils.py:121-155): same files both ways - what ours writes the
-    reference's own loader reads (oracle/_ref, when built) and vice versa; best.ckpt follows is_best; the returned measure;
-    a missing file raises; last.ckpt is replaced atomically."""
+    reference's own loader reads (oracle/_ref, when built) and vice versa; a stored checkpoint of the same state still loads,
+    and both it and a fresh one load through the reference loader's own steps; best.ckpt follows is_best; the returned
+    measure; a missing file raises; last.ckpt is replaced atomically."""
     import sys
     import kgc_gcn_b200 as k
     sys.path.insert(0, os.path.join(ROOT, 'oracle'))
@@ -502,8 +503,29 @@ def test_checkpoint_interchanges_with_the_reference(tmp_path):
     same(m, o)
     with pytest.raises(FileNotFoundError):
         k.load_checkpoint(os.path.join(d, 'nope.ckpt'), m)
-    if ref is None:
-        pytest.skip('oracle/_ref not built (no /root/reference on this box): interchange with the reference not checked')
+
+    def close(m, o):                                  # same state, computed on another machine (last-bit differences)
+        for a, b in zip(m.state_dict().values(), model.state_dict().values()):
+            assert torch.allclose(a.float(), b.float(), rtol=1e-5, atol=1e-6)
+        sa, sb = o.state_dict()['state'], opt.state_dict()['state']
+        assert sa.keys() == sb.keys() and all(torch.allclose(sa[i]['exp_avg'], sb[i]['exp_avg'], rtol=1e-5, atol=1e-7) for i in sa)
+
+    # tests/golden/ckpt_linear_bn_adam.ckpt: this same state (epoch 3) as save_checkpoint wrote it when the file was stored -
+    # ours must keep reading it; and that file and the one written above load the way the reference's load_checkpoint
+    # reads a checkpoint (utils.py:139-155: torch.load, then load_state_dict of 'state_dict' and of 'optim_dict')
+    golden = os.path.join(ROOT, 'tests', 'golden', 'ckpt_linear_bn_adam.ckpt')
+    m, o = fresh()
+    assert k.load_checkpoint(golden, m, o) == {'mrr': 0.25}
+    close(m, o)
+    for path in (golden, os.path.join(d, 'best.ckpt')):
+        ckpt = torch.load(path, map_location='cpu')
+        m, o = fresh()
+        m.load_state_dict(ckpt['state_dict'])
+        o.load_state_dict(ckpt['optim_dict'])
+        assert ckpt['epoch'] == 3 and ckpt.get('measure') == {'mrr': 0.25}
+        close(m, o)
+    if ref is None:                                   # the reference's own utils.py: only where KGC_REFERENCE_DIR built it
+        return
     ref_utils = sys.modules['utils']
     m, o = fresh()
     assert ref_utils.load_checkpoint(os.path.join(d, 'best.ckpt'), m, o) == {'mrr': 0.25}     # ours -> reference
