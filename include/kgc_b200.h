@@ -493,6 +493,27 @@ int kgc_rank_finalize(const int32_t* count_gt, const int32_t* count_eq, const fl
                       const int64_t* filt_ptr, const int32_t* filt_idx, const int64_t* obj, int64_t b,
                       int32_t* ranks, int32_t* eq_out, double* sums13, void* stream);
 
+/* ---- K6k: filtered top-k entity prediction -------------------------------------------------------------
+ * For every query q, the k best ELIGIBLE entities: j in [0, n) not in q's exclusion list, ordered by (logit descending,
+ * entity id ascending), -0.0 equal to +0.0.  excl_ptr [b+1] int64 / excl_idx int32: the exclusion CSR, each row sorted
+ * ascending (duplicates allowed, ids outside [0, n) ignored); both NULL: no filter.  1 <= k <= 32.
+ * Output: top_s [b, k] logits, top_id [b, k], count [b] = number of real entries; rows with fewer than k eligible
+ * entities are padded with (-inf, -1).  Deterministic (no float atomics): repeated calls are bit-identical.
+ *   kgc_score_topk: the K6 sweep (same TMA / tcgen05 path and bf16 operands as kgc_score_rank and kgc_score_pairs, so
+ *     top_s[q, i] equals kgc_score_pairs of (q, top_id[q, i]) bit for bit) with a register-resident top-k epilogue; each
+ *     work item writes its partial list to the workspace, a merge kernel reduces them.  Items skip candidates below the
+ *     K-th score another item of the same query already found (integer max), which does not change the result.
+ *   kgc_topk_dense: the same selection over DENSE fp32 logits [b, ld] (kgc_score_1n_logits, exact mode); b <= 65,535.
+ * workspace: at least the matching *_workspace_bytes (0 for arguments the call rejects), device memory, 16-byte aligned. */
+size_t kgc_score_topk_workspace_bytes(int64_t b, int64_t n, int32_t kpad, int32_t k);
+int kgc_score_topk(const uint16_t* q_bf16, const uint16_t* e_bf16, int64_t b, int64_t n, int32_t kpad,
+                   const int64_t* excl_ptr, const int32_t* excl_idx, int32_t k, float* top_s, int32_t* top_id,
+                   int32_t* count, void* workspace, size_t workspace_bytes, void* stream);
+size_t kgc_topk_dense_workspace_bytes(int64_t b, int64_t n, int32_t k);
+int kgc_topk_dense(const float* logits, int64_t ld, int64_t n, int64_t b, const int64_t* excl_ptr,
+                   const int32_t* excl_idx, int32_t k, float* top_s, int32_t* top_id, int32_t* count,
+                   void* workspace, size_t workspace_bytes, void* stream);
+
 #if defined(__GNUC__)
 #pragma GCC visibility pop
 #endif

@@ -23,6 +23,10 @@
 // kgc_score_pairs runs the same MMA sequence on gathered (query row, entity row) pairs and returns the
 // diagonal: the target score thr[q] and the scores of the filtered positives come from the SAME
 // instruction path as the sweep, so the filter correction is bit-consistent.
+//
+// K6k (kgc_score_topk): the same sweep whose epilogue keeps each query's best K in {16, 32} (score, id) keys of a work
+// item, skipping its exclusion list; topk_merge_kernel reduces the per-item lists.  kgc_topk_dense makes the same
+// selection over dense fp32 logits (exact mode) with the same list, exclusion cursor, partial layout and merge.
 #include <cuda.h>
 
 #include <cstdlib>
@@ -223,7 +227,92 @@ struct ScoreParams {
   int32_t* count_eq;      // [B] or nullptr
   float* pair_out;        // pairs mode: [n_pairs]
   int64_t n_pairs;
+  const int64_t* excl_ptr;   // top-k mode: exclusion CSR [B + 1] / [nnz], ascending per row (nullptr: no filter)
+  const int32_t* excl_idx;
+  uint64_t* topk_part;       // top-k mode: [n_chunks, B, K] sorted keys of every work item
+  uint32_t* topk_floor;      // top-k mode: [B] order-preserving bits of the best K-th score a finished item found (0: none)
 };
+
+// ------------------------------------------------------------------------------------------------ top-k selection (K6k)
+// An entry is one 64-bit key: the score's order-preserving bits in the high word, ~id in the low word, so that ONE unsigned
+// compare orders by (score descending, id ascending).  -0.0 is mapped to +0.0 first (the float compares treat them as
+// equal).  The empty entry is the key of (-inf, id -1): its low word is 0, which no real id (< 2^31) produces.
+__device__ __forceinline__ uint64_t topk_key(float s, int32_t id) {
+  uint32_t u = __float_as_uint(s);
+  if (u == 0x80000000u) u = 0u;
+  const uint32_t ord = (u & 0x80000000u) ? ~u : (u | 0x80000000u);
+  return ((uint64_t)ord << 32) | (uint32_t)~id;
+}
+__device__ __forceinline__ float topk_key_score(uint64_t key) {
+  const uint32_t ord = (uint32_t)(key >> 32);
+  return __uint_as_float((ord & 0x80000000u) ? (ord & 0x7FFFFFFFu) : ~ord);
+}
+__device__ __forceinline__ int32_t topk_key_id(uint64_t key) { return (int32_t)~(uint32_t)key; }
+
+// Register-resident list of the K largest keys seen, sorted descending.  Every index is a compile-time constant after
+// unrolling: one dynamic index would move the whole list to local memory.
+template <int K>
+struct TopList {
+  uint64_t key[K];
+  float thr;              // insert test s > thr: max(score of key[K - 1], floor); -inf while the list is not full
+  float floor;            // candidates at or below it cannot reach the final top K (-inf: no bound known)
+
+  __device__ __forceinline__ void init(bool active) {
+#pragma unroll
+    for (int i = 0; i < K; ++i) key[i] = topk_key(__int_as_float(0xff800000), -1);
+    floor = __int_as_float(0xff800000);
+    thr = __int_as_float(active ? 0xff800000 : 0x7f800000);    // +inf: an inactive row never inserts
+  }
+  // c > key[K - 1]: compare-and-shift, the last entry falls off
+  __device__ __forceinline__ void insert(uint64_t c) {
+#pragma unroll
+    for (int i = K - 1; i > 0; --i) key[i] = c > key[i - 1] ? key[i - 1] : (c > key[i] ? c : key[i]);
+    key[0] = c > key[0] ? c : key[0];
+    thr = fmaxf(topk_key_score(key[K - 1]), floor);
+  }
+  // Another list of the same query already holds K real entries scoring >= s_K (its K-th): a candidate below s_K has K
+  // better keys elsewhere and cannot be in the final top K; one AT s_K still may (lower id), hence the next float down.
+  __device__ __forceinline__ void set_floor(uint32_t ord) {
+    if (ord == 0u) return;
+    floor = nextafterf(topk_key_score((uint64_t)ord << 32), __int_as_float(0xff800000));
+    thr = fmaxf(thr, floor);
+  }
+  __device__ __forceinline__ bool full() const { return (uint32_t)key[K - 1] != 0u; }
+};
+
+// Walks one row's ascending exclusion list alongside ascending candidate ids; ids outside the list's range and duplicates
+// are harmless.  Only candidates that beat the list's K-th entry ask, and most of them find nxt > id without a load.
+struct ExclCursor {
+  const int32_t* idx;
+  int64_t cur, end;
+  int32_t nxt;            // idx[cur], or INT_MAX past the end
+
+  __device__ __forceinline__ void init(const int64_t* ptr, const int32_t* idx_, int64_t q, int64_t first_id) {
+    idx = idx_;
+    cur = end = 0;
+    nxt = 0x7FFFFFFF;
+    if (ptr == nullptr) return;
+    int64_t lo = __ldg(ptr + q), hi = __ldg(ptr + q + 1);
+    end = hi;
+    while (lo < hi) {                                            // first entry >= first_id
+      const int64_t mid = (lo + hi) >> 1;
+      if ((int64_t)__ldg(idx + mid) < first_id) lo = mid + 1; else hi = mid;
+    }
+    cur = lo;
+    if (cur < end) nxt = __ldg(idx + cur);
+  }
+  __device__ __forceinline__ bool excluded(int32_t id) {
+    while (nxt < id) nxt = (++cur < end) ? __ldg(idx + cur) : 0x7FFFFFFF;
+    return nxt == id;
+  }
+};
+
+// The one selection step every top-k path uses: ids arrive ascending per list, so a candidate that only ties the K-th
+// entry loses to it (lower id first) and the strict float compare is the whole test on the common path.
+template <int K>
+__device__ __forceinline__ void topk_offer(TopList<K>& L, ExclCursor& X, float s, int32_t id) {
+  if (s > L.thr && !X.excluded(id)) L.insert(topk_key(s, id));
+}
 
 // kCluster: launched as clusters of TWO CTAs that sweep the same entity tiles for different query tiles.  Each CTA of the
 // pair fetches HALF of every B stage (64 entity rows) and the TMA multicasts it into both CTAs' shared memory: every byte
@@ -231,7 +320,10 @@ struct ScoreParams {
 // not bound by the 4.3 TB/s it pulls out of L2; opt-in.)  A stage's `full` barrier collects both halves (its own TMA and
 // the peer's), its `empty` barrier the retired MMAs of BOTH CTAs (tcgen05.commit multicast) - a slot is rewritten by the
 // peer's TMA as well.
-template <bool kPairs, bool kCountEq, bool kCluster>
+//
+// kTopK (K6k, 16 or 32): instead of counting, every epilogue thread keeps its query row's kTopK best (score, id) keys of the
+// work item in registers (TopList) and writes them to P.topk_part[chunk, q, :]; topk_merge_kernel reduces the chunks.
+template <bool kPairs, bool kCountEq, bool kCluster, int kTopK = 0>
 __global__ void __launch_bounds__(kThreads, 1)
 score_kernel(const __grid_constant__ CUtensorMap map_a, const __grid_constant__ CUtensorMap map_b,
              const __grid_constant__ CUtensorMap map_bh, const ScoreParams P) {
@@ -240,6 +332,7 @@ score_kernel(const __grid_constant__ CUtensorMap map_a, const __grid_constant__ 
   const int warp = threadIdx.x / 32, lane = threadIdx.x % 32;
   constexpr int kNumM = kPairs ? 1 : kMTiles;
   static_assert(!(kPairs && kCluster), "pairs mode runs single CTAs");
+  static_assert(kTopK == 0 || (!kPairs && !kCountEq && !kCluster), "top-k mode is a single-CTA sweep");
   const uint32_t cta_rank = kCluster ? cluster_ctarank() : 0u;
 
   if (warp == 0 && lane == 0) {
@@ -343,6 +436,74 @@ score_kernel(const __grid_constant__ CUtensorMap map_a, const __grid_constant__ 
           }
           if (++acc == kAccStages) { acc = 0; acc_phase ^= 1; }
         }
+      }
+    }
+  } else if (kTopK != 0 && warp >= kEpiWarp0) {
+    // ================================================================== top-k epilogue (TMEM -> registers -> sorted list)
+    // Single-buffered tcgen05.ld: the second 32-register buffer of the counting epilogue would not fit next to a K = 32
+    // list (64 registers) under the 168-register budget of 384 threads; the loads stay hidden behind the next tile's MMAs.
+    constexpr int K = kTopK > 0 ? kTopK : 1;
+    const int m = (warp - kEpiWarp0) / 4;
+    const int quarter = warp % 4;
+    const int row = quarter * 32 + lane;
+    int acc = 0;
+    uint32_t acc_phase = 0;
+    for (int item = blockIdx.x; item < P.n_items; item += gridDim.x) {
+      const int chunk = item / P.n_mp, mp = item % P.n_mp;
+      const int t0 = chunk * P.chunk_tiles;
+      const int t1 = min(t0 + P.chunk_tiles, P.n_tiles);
+      const int64_t q = (int64_t)(mp * kNumM + m) * kBlockM + row;
+      const bool active = q < P.n_queries;
+      TopList<K> L;
+      L.init(active);
+      // items of other entity chunks that already finished bound this query's K-th score from below: without that bound
+      // every item starts empty and pays ~K ln(entities / K) inserts per row, serialised over the warp's 32 rows
+      if (active) L.set_floor(*reinterpret_cast<volatile uint32_t*>(P.topk_floor + q));
+      ExclCursor X;
+      X.init(active ? P.excl_ptr : nullptr, P.excl_idx, q, (int64_t)t0 * kBlockN);
+      for (int t = t0; t < t1; ++t) {
+        mbar_wait(S.acc_full + acc, acc_phase);
+        tc_fence_after();
+        const uint32_t taddr = tmem_base + ((uint32_t)(quarter * 32) << 16) + acc * (kMTiles * kBlockN) + m * kBlockN;
+        const int valid = (int)min((int64_t)kBlockN, P.n_entities - (int64_t)t * kBlockN);
+#pragma unroll 1
+        for (int c = 0; c < kBlockN / 32; ++c) {
+          uint32_t v[32];
+          __syncwarp();                                        // tcgen05.ld is .aligned: the insert path diverges
+          tmem_ld32(taddr + c * 32, v);
+          tmem_ld_wait();
+          if (valid < kBlockN) {
+#pragma unroll
+            for (int j = 0; j < 32; ++j)                     // entity rows past N are zero-filled by TMA: never insert
+              if (c * 32 + j >= valid) v[j] = 0xff800000u;
+          }
+          // common path: the block's maximum against the K-th score (a tree: no 32-long dependent chain)
+          float mx[16];
+#pragma unroll
+          for (int j = 0; j < 16; ++j) mx[j] = fmaxf(__uint_as_float(v[j]), __uint_as_float(v[j + 16]));
+#pragma unroll
+          for (int w = 8; w > 0; w >>= 1)
+#pragma unroll
+            for (int j = 0; j < w; ++j) mx[j] = fmaxf(mx[j], mx[j + w]);
+          if (mx[0] > L.thr) {
+            const int32_t id0 = t * kBlockN + c * 32;
+#pragma unroll
+            for (int j = 0; j < 32; ++j) topk_offer(L, X, __uint_as_float(v[j]), id0 + j);
+          }
+        }
+        tc_fence_before();
+        __syncwarp();
+        if (lane == 0) mbar_arrive(S.acc_empty + acc);
+        if (++acc == kAccStages) { acc = 0; acc_phase ^= 1; }
+      }
+      if (active) {
+        uint4* dst = reinterpret_cast<uint4*>(P.topk_part + ((int64_t)chunk * P.n_queries + q) * K);
+#pragma unroll
+        for (int i = 0; i < K; i += 2)
+          dst[i / 2] = make_uint4((uint32_t)L.key[i], (uint32_t)(L.key[i] >> 32), (uint32_t)L.key[i + 1],
+                                  (uint32_t)(L.key[i + 1] >> 32));
+        // integer max: the merged result does not depend on which items saw the bound (every final entry survives it)
+        if (L.full()) atomicMax(P.topk_floor + q, (uint32_t)(L.key[K - 1] >> 32));
       }
     }
   } else if (warp >= kEpiWarp0 && (warp - kEpiWarp0) / 4 < kNumM) {
@@ -517,6 +678,75 @@ rank_count_dense_kernel(const float* __restrict__ z, int64_t ld, int64_t n, cons
   }
 }
 
+// Exact-mode top-k over DENSE fp32 logits: grid = (column chunks of kTopkDenseCols, queries).  Thread t offers columns
+// c0 + t, c0 + t + 256, ... (ascending ids) to its own TopList, then the block folds the 256 lists pairwise through shared
+// memory (each fold keeps the top K of two lists; keys are unique, so the result does not depend on the order) and writes
+// one list per chunk: the same [n_chunks, B, K] partials as the tcgen05 sweep, reduced by the same merge kernel.
+constexpr int kTopkDenseThreads = 256, kTopkDensePerThread = 64;
+constexpr int kTopkDenseCols = kTopkDenseThreads * kTopkDensePerThread;
+template <int K>
+__device__ __forceinline__ void topk_fold(TopList<K>& L, const uint64_t* list) {    // list: K keys, sorted descending
+  for (int i = 0; i < K; ++i) {
+    const uint64_t c = list[i];
+    if (!(c > L.key[K - 1])) break;
+    L.insert(c);
+  }
+}
+template <int K>
+__global__ void __launch_bounds__(kTopkDenseThreads)
+topk_dense_kernel(const float* __restrict__ z, int64_t ld, int64_t n, int64_t b, const int64_t* __restrict__ excl_ptr,
+                  const int32_t* __restrict__ excl_idx, uint64_t* __restrict__ part) {
+  const int64_t q = blockIdx.y;
+  const float* row = z + q * ld;
+  const int64_t c0 = (int64_t)blockIdx.x * kTopkDenseCols + threadIdx.x;
+  TopList<K> L;
+  L.init(true);
+  ExclCursor X;
+  X.init(excl_ptr, excl_idx, q, c0);
+#pragma unroll 4
+  for (int i = 0; i < kTopkDensePerThread; ++i) {
+    const int64_t c = c0 + (int64_t)i * kTopkDenseThreads;
+    if (c < n) topk_offer(L, X, __ldg(row + c), (int32_t)c);
+  }
+  __shared__ __align__(16) uint64_t sm[kTopkDenseThreads / 2 * K];
+  for (int half = kTopkDenseThreads / 2; half > 0; half >>= 1) {
+    __syncthreads();
+    if (threadIdx.x >= half && threadIdx.x < 2 * half) {
+#pragma unroll
+      for (int i = 0; i < K; ++i) sm[(threadIdx.x - half) * K + i] = L.key[i];
+    }
+    __syncthreads();
+    if (threadIdx.x < half) topk_fold(L, sm + threadIdx.x * K);
+  }
+  if (threadIdx.x == 0) {
+    uint64_t* dst = part + ((int64_t)blockIdx.x * b + q) * K;
+#pragma unroll
+    for (int i = 0; i < K; ++i) dst[i] = L.key[i];
+  }
+}
+
+// Final [k] per query from the [n_chunks, B, K] partial lists; one thread per query, chunks in order, keys unique ->
+// deterministic for any chunk count.  Output: scores (padding -inf), ids (padding -1), count of real entries.
+template <int K>
+__global__ void topk_merge_kernel(const uint64_t* __restrict__ part, int64_t n_chunks, int64_t b, int k,
+                                  float* __restrict__ top_s, int32_t* __restrict__ top_id, int32_t* __restrict__ count) {
+  const int64_t q = blockIdx.x * (int64_t)blockDim.x + threadIdx.x;
+  if (q >= b) return;
+  TopList<K> L;
+  L.init(true);
+  for (int64_t c = 0; c < n_chunks; ++c) topk_fold(L, part + (c * b + q) * K);
+  int cnt = 0;
+#pragma unroll
+  for (int i = 0; i < K; ++i) {
+    if (i < k) {
+      top_s[q * k + i] = topk_key_score(L.key[i]);
+      top_id[q * k + i] = topk_key_id(L.key[i]);
+      cnt += (uint32_t)L.key[i] != 0u ? 1 : 0;
+    }
+  }
+  count[q] = cnt;
+}
+
 // sums13 = {count, sum rank, sum 1/rank, hits@1..10}; one block, fixed order -> deterministic
 __global__ void rank_sums_kernel(const int32_t* __restrict__ ranks, int64_t b, double* __restrict__ sums13) {
   __shared__ double sm[13][256];
@@ -574,6 +804,57 @@ int make_map(CUtensorMap* map, const void* base, int64_t rows, int kpad, int box
 }
 
 inline int check_kpad(int kpad) { return (kpad < 16 || kpad % 16 != 0 || kpad > kMaxKBlocks * kBlockK) ? 1 : 0; }
+
+// Work items of the sweep: P.n_mp (query-tile pairs, set by the caller), n_tiles, chunk_tiles and n_items.  Entity
+// chunks: enough work items to balance 148 persistent CTAs, chunk small enough to stay in L2 (<= ~48 MB of bf16 rows) so
+// that the CTAs sweeping one chunk share its tiles.  kgc_score_rank, kgc_score_topk and its workspace size all use it.
+void plan_chunks(ScoreParams& P, int64_t n, int kpad) {
+  P.n_tiles = (int32_t)ceil_div(n, kBlockN);
+  const int64_t max_chunk_tiles = (int64_t)(48 << 20) / ((int64_t)kBlockN * kpad * 2);
+  int best_chunks = 1;
+  double best_cost = 1e30;
+  for (int c = 1; c <= 4096 && c <= P.n_tiles; ++c) {
+    const int64_t ct = ceil_div(P.n_tiles, c);
+    if (ct > max_chunk_tiles && c < P.n_tiles) continue;
+    const int64_t items = (int64_t)P.n_mp * c;
+    const int64_t waves = ceil_div(items, kNumSMs);
+    // cost ~ time of the slowest CTA: waves * (tiles per item + A-load overhead of ~2 tiles)
+    const double cost = (double)waves * (double)(ct + 2);
+    if (cost < best_cost) { best_cost = cost; best_chunks = c; }
+  }
+  P.chunk_tiles = (int32_t)ceil_div(P.n_tiles, best_chunks);
+  P.n_items = P.n_mp * (int32_t)ceil_div(P.n_tiles, P.chunk_tiles);
+}
+
+constexpr int kTopkMax = 32;              // the largest register list that fits the sweep's epilogue without spilling
+inline int topk_list_len(int k) { return k <= 16 ? 16 : 32; }
+
+// chunks of the top-k sweep for (b, n, kpad): the leading dimension of its partial lists
+int64_t topk_sweep_chunks(int64_t b, int64_t n, int kpad) {
+  ScoreParams P = {};
+  P.n_mp = (int32_t)ceil_div(b, kMTiles * kBlockM);
+  plan_chunks(P, n, kpad);
+  return ceil_div(P.n_tiles, P.chunk_tiles);
+}
+
+template <int K>
+int launch_topk_sweep(const CUtensorMap& ma, const CUtensorMap& mb, const ScoreParams& P, cudaStream_t st) {
+  auto kern = score_kernel<false, false, false, K>;
+  static SmemAttrCache attr;
+  KGC_CUDA_TRY(attr.ensure(kern, (size_t)kSmemBytes));
+  const int grid = P.n_items < kNumSMs ? P.n_items : kNumSMs;
+  kern<<<grid, kThreads, kSmemBytes, st>>>(ma, mb, mb, P);
+  KGC_LAUNCH_CHECK();
+  return 0;
+}
+
+template <int K>
+int launch_topk_merge(const uint64_t* part, int64_t n_chunks, int64_t b, int k, float* top_s, int32_t* top_id,
+                      int32_t* count, cudaStream_t st) {
+  topk_merge_kernel<K><<<(unsigned)ceil_div(b, 128), 128, 0, st>>>(part, n_chunks, b, k, top_s, top_id, count);
+  KGC_LAUNCH_CHECK();
+  return 0;
+}
 
 template <bool kPairs, bool kCountEq>
 int launch_score(const CUtensorMap& ma, const CUtensorMap& mb, const ScoreParams& P, cudaStream_t st) {
@@ -697,23 +978,7 @@ extern "C" int kgc_score_rank(const uint16_t* q_bf16, const uint16_t* e_bf16, in
   static const bool cluster_ok = [] { const char* e = getenv("KGC_SCORE_CLUSTER"); return e && e[0] == '1'; }();
   const bool cluster = cluster_ok && P.n_mp >= 2;
   if (cluster) P.n_mp = (P.n_mp + 1) & ~1;
-  P.n_tiles = (int32_t)ceil_div(n, kBlockN);
-  // entity chunks: enough work items to balance 148 persistent CTAs, chunk small enough to stay in L2
-  // (<= ~48 MB of bf16 rows) so that the CTAs sweeping one chunk share its tiles.
-  const int64_t max_chunk_tiles = (int64_t)(48 << 20) / ((int64_t)kBlockN * kpad * 2);
-  int best_chunks = 1;
-  double best_cost = 1e30;
-  for (int c = 1; c <= 4096 && c <= P.n_tiles; ++c) {
-    const int64_t ct = ceil_div(P.n_tiles, c);
-    if (ct > max_chunk_tiles && c < P.n_tiles) continue;
-    const int64_t items = (int64_t)P.n_mp * c;
-    const int64_t waves = ceil_div(items, kNumSMs);
-    // cost ~ time of the slowest CTA: waves * (tiles per item + A-load overhead of ~2 tiles)
-    const double cost = (double)waves * (double)(ct + 2);
-    if (cost < best_cost) { best_cost = cost; best_chunks = c; }
-  }
-  P.chunk_tiles = (int32_t)ceil_div(P.n_tiles, best_chunks);
-  P.n_items = P.n_mp * (int32_t)ceil_div(P.n_tiles, P.chunk_tiles);
+  plan_chunks(P, n, kpad);
   P.thr = thr;
   P.count_gt = count_gt;
   P.count_eq = count_eq;
@@ -725,6 +990,73 @@ extern "C" int kgc_score_rank(const uint16_t* q_bf16, const uint16_t* e_bf16, in
   }
   if (count_eq) return launch_score<false, true>(ma, mb, P, st);
   return launch_score<false, false>(ma, mb, P, st);
+}
+
+extern "C" size_t kgc_score_topk_workspace_bytes(int64_t b, int64_t n, int32_t kpad, int32_t k) {
+  if (b <= 0 || n <= 0 || check_kpad(kpad) || k < 1 || k > kTopkMax) return 0;
+  // [n_chunks, b, K] partial lists, then the [b] per-query score floors
+  return (size_t)topk_sweep_chunks(b, n, kpad) * (size_t)b * topk_list_len(k) * sizeof(uint64_t) + (size_t)b * sizeof(uint32_t);
+}
+
+extern "C" int kgc_score_topk(const uint16_t* q_bf16, const uint16_t* e_bf16, int64_t b, int64_t n, int32_t kpad,
+                              const int64_t* excl_ptr, const int32_t* excl_idx, int32_t k, float* top_s, int32_t* top_id,
+                              int32_t* count, void* workspace, size_t workspace_bytes, void* stream) {
+  KGC_REQUIRE(check_kpad(kpad) == 0, "kpad must be a multiple of 16 in [16, 256]");
+  KGC_REQUIRE(b > 0 && n > 0 && b < (int64_t(1) << 30) && n < (int64_t(1) << 31), "bad sizes");
+  KGC_REQUIRE(k >= 1 && k <= kTopkMax, "k must be in [1, 32]");
+  KGC_REQUIRE((excl_ptr == nullptr) == (excl_idx == nullptr), "excl_ptr and excl_idx go together");
+  KGC_REQUIRE(top_s && top_id && count, "null output");
+  KGC_REQUIRE(workspace && workspace_bytes >= kgc_score_topk_workspace_bytes(b, n, kpad, k), "workspace too small");
+  cudaStream_t st = as_stream(stream);
+  CUtensorMap ma, mb;
+  if (make_map(&ma, q_bf16, b, kpad) || make_map(&mb, e_bf16, n, kpad)) return 1;
+  ScoreParams P = {};
+  P.n_queries = b;
+  P.n_entities = n;
+  P.ksteps = kpad / kUmmaK;
+  P.n_kblocks = (kpad + kBlockK - 1) / kBlockK;
+  P.n_mp = (int32_t)ceil_div(b, kMTiles * kBlockM);
+  plan_chunks(P, n, kpad);
+  P.excl_ptr = excl_ptr;
+  P.excl_idx = excl_idx;
+  P.topk_part = static_cast<uint64_t*>(workspace);
+  const int64_t n_chunks = ceil_div(P.n_tiles, P.chunk_tiles);
+  P.topk_floor = reinterpret_cast<uint32_t*>(P.topk_part + n_chunks * b * topk_list_len(k));
+  KGC_CUDA_TRY(cudaMemsetAsync(P.topk_floor, 0, (size_t)b * sizeof(uint32_t), st));
+  if (topk_list_len(k) == 16) {
+    if (launch_topk_sweep<16>(ma, mb, P, st)) return 1;
+    return launch_topk_merge<16>(P.topk_part, n_chunks, b, k, top_s, top_id, count, st);
+  }
+  if (launch_topk_sweep<32>(ma, mb, P, st)) return 1;
+  return launch_topk_merge<32>(P.topk_part, n_chunks, b, k, top_s, top_id, count, st);
+}
+
+extern "C" size_t kgc_topk_dense_workspace_bytes(int64_t b, int64_t n, int32_t k) {
+  if (b <= 0 || n <= 0 || k < 1 || k > kTopkMax) return 0;
+  return (size_t)ceil_div(n, kTopkDenseCols) * (size_t)b * topk_list_len(k) * sizeof(uint64_t);
+}
+
+extern "C" int kgc_topk_dense(const float* logits, int64_t ld, int64_t n, int64_t b, const int64_t* excl_ptr,
+                              const int32_t* excl_idx, int32_t k, float* top_s, int32_t* top_id, int32_t* count,
+                              void* workspace, size_t workspace_bytes, void* stream) {
+  KGC_REQUIRE(logits && b > 0 && n > 0 && n < (int64_t(1) << 31) && ld >= n && b <= 65535,
+              "bad sizes (at most 65,535 queries per call)");
+  KGC_REQUIRE(k >= 1 && k <= kTopkMax, "k must be in [1, 32]");
+  KGC_REQUIRE((excl_ptr == nullptr) == (excl_idx == nullptr), "excl_ptr and excl_idx go together");
+  KGC_REQUIRE(top_s && top_id && count, "null output");
+  KGC_REQUIRE(workspace && workspace_bytes >= kgc_topk_dense_workspace_bytes(b, n, k), "workspace too small");
+  cudaStream_t st = as_stream(stream);
+  uint64_t* part = static_cast<uint64_t*>(workspace);
+  const int64_t n_chunks = ceil_div(n, kTopkDenseCols);
+  const dim3 grid((unsigned)n_chunks, (unsigned)b);
+  if (topk_list_len(k) == 16) {
+    topk_dense_kernel<16><<<grid, kTopkDenseThreads, 0, st>>>(logits, ld, n, b, excl_ptr, excl_idx, part);
+    KGC_LAUNCH_CHECK();
+    return launch_topk_merge<16>(part, n_chunks, b, k, top_s, top_id, count, st);
+  }
+  topk_dense_kernel<32><<<grid, kTopkDenseThreads, 0, st>>>(logits, ld, n, b, excl_ptr, excl_idx, part);
+  KGC_LAUNCH_CHECK();
+  return launch_topk_merge<32>(part, n_chunks, b, k, top_s, top_id, count, st);
 }
 
 extern "C" int kgc_rank_count_dense(const float* logits, int64_t ld, int64_t n_ent, int64_t b, const float* thr,

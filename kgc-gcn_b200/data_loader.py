@@ -347,6 +347,7 @@ class DataLoader(object):
             self.relation2id.update({name + '_reverse': i + n_rel for i, name in enumerate(native['relations'])})
             self.num_entity, self.num_relation = len(native['entities']), n_rel
             self.num_edge = int(native['train'].shape[0])
+            self._split_triples = {split: native[split] for split in ('train', 'valid', 'test')}
             self.triplets = LazyTriplets({k: native['q_' + k] for k in ('train', 'valid_tail', 'valid_head', 'test_tail',
                                                                           'test_head')})
             graph = self._build_graph(np.arange(self.num_entity, dtype=np.int64), native['train'], bi_direction=True)
@@ -392,6 +393,7 @@ class DataLoader(object):
                 known_train = OrderedDict((k, sorted(v)) for k, v in known.items())
         known_all = {k: sorted(v) for k, v in known.items()}
         self.num_edge = len(data['train'])
+        self._split_triples = {split: np.asarray(data[split], dtype=np.int64).reshape(-1, 3) for split in splits}
 
         # query lists (data_loader.py:98-111)
         trip = {'train': [{'triple': (s, r, -1), 'label': objs, 'sub_samp': 1} for (s, r), objs in known_train.items()]}
@@ -460,6 +462,37 @@ class DataLoader(object):
         data = GraphData(edge_index=sub[:2], edge_attr=sub[2:])
         data.entity, data.num_nodes = g.entity, g.num_nodes
         return data
+
+    def known_objects(self, src, rel):
+        """Exclusion CSR for arbitrary queries (src[q], rel[q], ?): (ptr [B+1] int64, idx int32) on the graph's device, row q
+        = the sorted objects o with (src[q], rel[q], o) in train, valid or test; a reverse relation r + R gives the subjects s
+        of (s, r, src[q]) (the reference's all-split filter, data_loader.py:80-96).  For ``MGCN.topk(..., exclude=...)``."""
+        if getattr(self, '_known', None) is None:
+            n_rel2 = 2 * self.num_relation
+            t = np.concatenate([self._split_triples[s] for s in ('train', 'valid', 'test')]).reshape(-1, 3)
+            keys = np.concatenate([t[:, 0] * n_rel2 + t[:, 1], t[:, 2] * n_rel2 + t[:, 1] + self.num_relation])
+            objs = np.concatenate([t[:, 2], t[:, 0]])
+            order = np.lexsort((objs, keys))
+            keys, objs = keys[order], objs[order]
+            if keys.size:
+                first = np.ones(keys.size, dtype=bool)
+                first[1:] = (keys[1:] != keys[:-1]) | (objs[1:] != objs[:-1])
+                keys, objs = keys[first], objs[first]
+            ukeys, start = np.unique(keys, return_index=True)
+            gptr = np.append(start, keys.size).astype(np.int64)
+            self._known = (ukeys, gptr, objs.astype(np.int32))
+        ukeys, gptr, gidx = self._known
+        src = np.asarray(src.cpu() if torch.is_tensor(src) else src, dtype=np.int64).reshape(-1)
+        rel = np.asarray(rel.cpu() if torch.is_tensor(rel) else rel, dtype=np.int64).reshape(-1)
+        q = src * (2 * self.num_relation) + rel
+        pos = np.minimum(np.searchsorted(ukeys, q), max(ukeys.size - 1, 0))
+        found = ukeys.size > 0
+        found = (ukeys[pos] == q) if found else np.zeros(q.shape, dtype=bool)
+        # unknown (s, r): an empty row, read from the empty group appended at the end
+        groups = np.where(found, pos, ukeys.size)
+        ptr, idx = _gather_segments(np.append(gptr, gptr[-1]), gidx, groups)
+        dev = self.graph.device
+        return torch.from_numpy(ptr).to(dev), torch.from_numpy(np.ascontiguousarray(idx, dtype=np.int32)).to(dev)
 
     def _queries(self, key):
         t = self.triplets

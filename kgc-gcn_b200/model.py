@@ -307,3 +307,13 @@ class MGCN(nn.Module):
         all_ent, all_rel = self.encode(data)
         xq = self.conv2.query(torch.index_select(all_ent, 0, src), torch.index_select(all_rel, 0, rel))
         return filtered_rank(xq, all_ent, self.conv2.bias, obj, filt_ptr, filt_idx, count_eq=count_eq)
+
+    def topk(self, src, rel, data, k=10, exclude=None, precision='bf16'):
+        """The k most likely objects of the queries (src, rel, ?) without materialising the [B, N] scores (K6k):
+        ``scoring.topk`` on the ConvE query.  ``exclude``: (ptr, idx) CSR of entities to leave out per query, e.g.
+        ``DataLoader.known_objects(src, rel)`` for the known facts; None keeps every entity."""
+        from .scoring import topk
+        all_ent, all_rel = self.encode(data)
+        xq = self.conv2.query(torch.index_select(all_ent, 0, src), torch.index_select(all_rel, 0, rel))
+        ptr, idx = exclude if exclude is not None else (None, None)
+        return topk(xq, all_ent, self.conv2.bias, k, ptr, idx, precision=precision)

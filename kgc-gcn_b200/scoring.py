@@ -296,6 +296,88 @@ def filtered_rank(xq, all_ent, bias, obj, filt_ptr, filt_idx, count_eq=False, ta
     return out
 
 
+TOPK_MAX = 32      # the largest list the fused sweep keeps in registers (K6k)
+
+
+def _check_exclusions(b, excl_ptr, excl_idx):
+    """Device copies of the exclusion CSR after checking its shape: ``ptr`` [b+1] non-decreasing within [0, nnz], every
+    row sorted ascending (what the kernels' forward cursor relies on).  (None, None) when no filter is given."""
+    if excl_ptr is None and excl_idx is None:
+        return None, None
+    if excl_ptr is None or excl_idx is None:
+        raise ValueError('excl_ptr and excl_idx go together')
+    ptr = _lib.require_cuda(excl_ptr, torch.int64, 'excl_ptr')
+    idx = _lib.require_cuda(excl_idx, torch.int32, 'excl_idx')
+    if ptr.dim() != 1 or int(ptr.numel()) != b + 1:
+        raise ValueError('excl_ptr must have B + 1 = {} entries, got {}'.format(b + 1, tuple(ptr.shape)))
+    nnz = int(idx.numel())
+    bad = (ptr[1:] < ptr[:-1]).any() | (ptr[0] < 0) | (ptr[-1] > nnz)
+    if nnz > 1:
+        # pair (p, p + 1) decreasing inside one row: rows end where the next one starts
+        dec = idx[1:] < idx[:-1]
+        cut = ptr[1:-1] - 1
+        dec[cut[(cut >= 0) & (cut < nnz - 1)]] = False
+        pos = torch.arange(nnz - 1, device=idx.device)
+        bad = bad | (dec & (pos >= ptr[0]) & (pos + 1 < ptr[-1])).any()
+    if bool(bad):
+        raise ValueError('malformed exclusion CSR: excl_ptr must be non-decreasing within [0, len(excl_idx)] and every '
+                         'row of excl_idx sorted ascending')
+    return (ptr, idx) if nnz > 0 else (None, None)
+
+
+def topk(xq, all_ent, bias, k, excl_ptr=None, excl_idx=None, table=None, precision='bf16'):
+    """The ``k`` best entities for every query row of ``xq`` [B, d] against ``all_ent`` [N, d] (+ ``bias`` [N]), leaving out
+    each query's exclusion list (the known positives: ``excl_ptr`` [B+1] int64 / ``excl_idx`` int32 CSR, rows sorted
+    ascending, e.g. ``DataLoader.known_objects``; None: no filter).
+
+    Order: logit descending, then entity id ascending (-0.0 == +0.0).  Returns {'scores': [B, k] float32 logits, 'ids':
+    [B, k] int64, 'count': [B] int32 real entries}; rows with fewer than k eligible entities are padded with (-inf, -1).
+    1 <= k <= 32.  Deterministic.
+
+    ``precision='bf16'`` (default): the fused tcgen05 sweep (K6k) on the bf16 entity table - ``table=`` reuses an
+    ``EntityTable`` - without writing the [B, N] logits; scores are bit-identical to ``pair_scores``.  ``precision='fp32'``:
+    the same selection over fp32-grade dense logits (3xTF32), 256 queries at a time, as in ``filtered_rank``'s exact mode."""
+    if isinstance(k, bool) or not isinstance(k, int) or not 1 <= k <= TOPK_MAX:
+        raise ValueError('k must be an integer in [1, {}], got {!r}'.format(TOPK_MAX, k))
+    if precision not in ('bf16', 'fp32'):
+        raise ValueError("precision must be 'bf16' or 'fp32'")
+    xq = _lib.require_cuda(xq.detach(), torch.float32, 'xq')
+    dev, b = xq.device, int(xq.shape[0])
+    ptr, idx = _check_exclusions(b, excl_ptr, excl_idx)
+    scores = torch.empty((b, k), dtype=torch.float32, device=dev)
+    ids = torch.empty((b, k), dtype=torch.int32, device=dev)
+    count = torch.empty((b,), dtype=torch.int32, device=dev)
+    p = _lib.ptr
+    if precision == 'bf16':
+        if table is None:
+            table = EntityTable(all_ent, bias)
+        if b > 0:
+            q_bf16 = pack_queries(xq)
+            ws_bytes = int(_lib.lib().kgc_score_topk_workspace_bytes(b, table.n, table.kpad, k))
+            ws = torch.empty((ws_bytes,), dtype=torch.uint8, device=dev)
+            _lib.call('kgc_score_topk', p(q_bf16), p(table.data), b, table.n, table.kpad, p(ptr), p(idx), k, p(scores),
+                      p(ids), p(count), p(ws), ws_bytes, _lib.stream())
+    else:
+        if all_ent is None:
+            raise ValueError("precision='fp32' takes the fp32 all_ent (and bias)")
+        ent = _lib.require_cuda(all_ent.detach(), torch.float32, 'all_ent')
+        n, d = int(ent.shape[0]), int(ent.shape[1])
+        bias = (torch.zeros((n,), dtype=torch.float32, device=dev) if bias is None
+                else _lib.require_cuda(bias.detach(), torch.float32, 'bias'))
+        if d % 4 != 0:       # the 3xTF32 scorer takes d % 4 == 0; zero columns leave every logit unchanged
+            pad = 4 - d % 4
+            xq = torch.nn.functional.pad(xq, (0, pad))
+            ent = torch.nn.functional.pad(ent, (0, pad))
+        ws_bytes = int(_lib.lib().kgc_topk_dense_workspace_bytes(min(b, B_TILE), n, k))
+        ws = torch.empty((ws_bytes,), dtype=torch.uint8, device=dev)
+        for i in range(0, b, B_TILE):
+            j = min(i + B_TILE, b)
+            z, ld = dense_logits(xq[i:j], ent, bias)
+            _lib.call('kgc_topk_dense', p(z), ld, n, j - i, p(ptr[i:]) if ptr is not None else None, p(idx), k,
+                      p(scores[i:j]), p(ids[i:j]), p(count[i:j]), p(ws), ws_bytes, _lib.stream())
+    return {'scores': scores, 'ids': ids.long(), 'count': count}
+
+
 def tie_adjusted_sums(ranks, count_eq, ties):
     """sums13 under a tie policy: 'optimistic' rank = 1 + gt (what kgc_rank_finalize gives), 'pessimistic' = 1 + gt + eq,
     'mean' = 1 + gt + eq / 2 (the expectation of the reference's arbitrary tie order, main.py:126)."""
