@@ -513,6 +513,14 @@ size_t kgc_topk_dense_workspace_bytes(int64_t b, int64_t n, int32_t k);
 int kgc_topk_dense(const float* logits, int64_t ld, int64_t n, int64_t b, const int64_t* excl_ptr,
                    const int32_t* excl_idx, int32_t k, float* top_s, int32_t* top_id, int32_t* count,
                    void* workspace, size_t workspace_bytes, void* stream);
+/* kgc_topk_merge: the k best entries of the union of n_lists finished results, e.g. one per entity shard.
+ * part_s [n_lists, b, k] float / part_id [n_lists, b, k] int32: each [k] row sorted as kgc_score_topk returns it
+ * (logit descending, id ascending), ids < 0 padding; ids must be disjoint across lists (shards own disjoint rows).
+ * Output as above: top_s / top_id [b, k] ordered by (logit descending, id ascending), -0.0 equal to +0.0, padded with
+ * (-inf, -1); count [b] real entries.  Keys are unique, so the result does not depend on the list order.
+ * n_lists >= 1, 0 < b < 2^31, 1 <= k <= 32.  One kernel, no workspace; deterministic. */
+int kgc_topk_merge(const float* part_s, const int32_t* part_id, int64_t n_lists, int64_t b, int32_t k,
+                   float* top_s, int32_t* top_id, int32_t* count, void* stream);
 
 #if defined(__GNUC__)
 #pragma GCC visibility pop

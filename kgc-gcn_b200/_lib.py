@@ -100,6 +100,7 @@ SIGNATURES = {
     'kgc_score_topk': (ctypes.c_int, [_vp, _vp, _i64, _i64, _i32, _vp, _vp, _i32, _vp, _vp, _vp, _vp, _sz, _vp]),
     'kgc_topk_dense_workspace_bytes': (_sz, [_i64, _i64, _i32]),
     'kgc_topk_dense': (ctypes.c_int, [_vp, _i64, _i64, _i64, _vp, _vp, _i32, _vp, _vp, _vp, _vp, _sz, _vp]),
+    'kgc_topk_merge': (ctypes.c_int, [_vp, _vp, _i64, _i64, _i32, _vp, _vp, _vp, _vp]),
 }
 
 

@@ -27,6 +27,7 @@
 // K6k (kgc_score_topk): the same sweep whose epilogue keeps each query's best K in {16, 32} (score, id) keys of a work
 // item, skipping its exclusion list; topk_merge_kernel reduces the per-item lists.  kgc_topk_dense makes the same
 // selection over dense fp32 logits (exact mode) with the same list, exclusion cursor, partial layout and merge.
+// kgc_topk_merge combines finished results of disjoint entity ranges (shards) with the same list and output loop.
 #include <cuda.h>
 
 #include <cstdlib>
@@ -684,13 +685,18 @@ rank_count_dense_kernel(const float* __restrict__ z, int64_t ld, int64_t n, cons
 // one list per chunk: the same [n_chunks, B, K] partials as the tcgen05 sweep, reduced by the same merge kernel.
 constexpr int kTopkDenseThreads = 256, kTopkDensePerThread = 64;
 constexpr int kTopkDenseCols = kTopkDenseThreads * kTopkDensePerThread;
-template <int K>
-__device__ __forceinline__ void topk_fold(TopList<K>& L, const uint64_t* list) {    // list: K keys, sorted descending
-  for (int i = 0; i < K; ++i) {
-    const uint64_t c = list[i];
+// Folds a list of `len` keys, sorted descending, into L: key(i) yields the i-th key.
+template <int K, class KeyAt>
+__device__ __forceinline__ void topk_fold_keys(TopList<K>& L, int len, KeyAt key) {
+  for (int i = 0; i < len; ++i) {
+    const uint64_t c = key(i);
     if (!(c > L.key[K - 1])) break;
     L.insert(c);
   }
+}
+template <int K>
+__device__ __forceinline__ void topk_fold(TopList<K>& L, const uint64_t* list) {    // list: K keys, sorted descending
+  topk_fold_keys(L, K, [list](int i) { return list[i]; });
 }
 template <int K>
 __global__ void __launch_bounds__(kTopkDenseThreads)
@@ -725,16 +731,10 @@ topk_dense_kernel(const float* __restrict__ z, int64_t ld, int64_t n, int64_t b,
   }
 }
 
-// Final [k] per query from the [n_chunks, B, K] partial lists; one thread per query, chunks in order, keys unique ->
-// deterministic for any chunk count.  Output: scores (padding -inf), ids (padding -1), count of real entries.
+// The first k entries of a finished list: scores (padding -inf), ids (padding -1), count of real entries.
 template <int K>
-__global__ void topk_merge_kernel(const uint64_t* __restrict__ part, int64_t n_chunks, int64_t b, int k,
-                                  float* __restrict__ top_s, int32_t* __restrict__ top_id, int32_t* __restrict__ count) {
-  const int64_t q = blockIdx.x * (int64_t)blockDim.x + threadIdx.x;
-  if (q >= b) return;
-  TopList<K> L;
-  L.init(true);
-  for (int64_t c = 0; c < n_chunks; ++c) topk_fold(L, part + (c * b + q) * K);
+__device__ __forceinline__ void topk_store(const TopList<K>& L, int64_t q, int k, float* __restrict__ top_s,
+                                           int32_t* __restrict__ top_id, int32_t* __restrict__ count) {
   int cnt = 0;
 #pragma unroll
   for (int i = 0; i < K; ++i) {
@@ -745,6 +745,41 @@ __global__ void topk_merge_kernel(const uint64_t* __restrict__ part, int64_t n_c
     }
   }
   count[q] = cnt;
+}
+
+// Final [k] per query from the [n_chunks, B, K] partial lists; one thread per query, chunks in order, keys unique ->
+// deterministic for any chunk count.  Output: scores (padding -inf), ids (padding -1), count of real entries.
+template <int K>
+__global__ void topk_merge_kernel(const uint64_t* __restrict__ part, int64_t n_chunks, int64_t b, int k,
+                                  float* __restrict__ top_s, int32_t* __restrict__ top_id, int32_t* __restrict__ count) {
+  const int64_t q = blockIdx.x * (int64_t)blockDim.x + threadIdx.x;
+  if (q >= b) return;
+  TopList<K> L;
+  L.init(true);
+  for (int64_t c = 0; c < n_chunks; ++c) topk_fold(L, part + (c * b + q) * K);
+  topk_store(L, q, k, top_s, top_id, count);
+}
+
+// Cross-shard merge (kgc_topk_merge): the same fold and output over n_lists finished [b, k] results (float scores, int32
+// ids, id < 0 padding), keys built as the lists are read.  Ids are disjoint across lists, so keys are unique and the
+// result does not depend on the list order.
+template <int K>
+__global__ void topk_merge_lists_kernel(const float* __restrict__ part_s, const int32_t* __restrict__ part_id,
+                                        int64_t n_lists, int64_t b, int k, float* __restrict__ top_s,
+                                        int32_t* __restrict__ top_id, int32_t* __restrict__ count) {
+  const int64_t q = blockIdx.x * (int64_t)blockDim.x + threadIdx.x;
+  if (q >= b) return;
+  TopList<K> L;
+  L.init(true);
+  for (int64_t l = 0; l < n_lists; ++l) {
+    const float* s = part_s + (l * b + q) * k;
+    const int32_t* id = part_id + (l * b + q) * k;
+    topk_fold_keys(L, k, [s, id](int i) {
+      const int32_t e = __ldg(id + i);
+      return e < 0 ? topk_key(__int_as_float(0xff800000), -1) : topk_key(__ldg(s + i), e);
+    });
+  }
+  topk_store(L, q, k, top_s, top_id, count);
 }
 
 // sums13 = {count, sum rank, sum 1/rank, hits@1..10}; one block, fixed order -> deterministic
@@ -1029,6 +1064,22 @@ extern "C" int kgc_score_topk(const uint16_t* q_bf16, const uint16_t* e_bf16, in
   }
   if (launch_topk_sweep<32>(ma, mb, P, st)) return 1;
   return launch_topk_merge<32>(P.topk_part, n_chunks, b, k, top_s, top_id, count, st);
+}
+
+extern "C" int kgc_topk_merge(const float* part_s, const int32_t* part_id, int64_t n_lists, int64_t b, int32_t k,
+                              float* top_s, int32_t* top_id, int32_t* count, void* stream) {
+  KGC_REQUIRE(n_lists >= 1 && b > 0 && b < (int64_t(1) << 31), "bad sizes (n_lists >= 1, 0 < b < 2^31)");
+  KGC_REQUIRE(k >= 1 && k <= kTopkMax, "k must be in [1, 32]");
+  KGC_REQUIRE(part_s && part_id, "null input");
+  KGC_REQUIRE(top_s && top_id && count, "null output");
+  cudaStream_t st = as_stream(stream);
+  const unsigned grid = (unsigned)ceil_div(b, 128);
+  if (topk_list_len(k) == 16)
+    topk_merge_lists_kernel<16><<<grid, 128, 0, st>>>(part_s, part_id, n_lists, b, k, top_s, top_id, count);
+  else
+    topk_merge_lists_kernel<32><<<grid, 128, 0, st>>>(part_s, part_id, n_lists, b, k, top_s, top_id, count);
+  KGC_LAUNCH_CHECK();
+  return 0;
 }
 
 extern "C" size_t kgc_topk_dense_workspace_bytes(int64_t b, int64_t n, int32_t k) {

@@ -308,12 +308,31 @@ class MGCN(nn.Module):
         xq = self.conv2.query(torch.index_select(all_ent, 0, src), torch.index_select(all_rel, 0, rel))
         return filtered_rank(xq, all_ent, self.conv2.bias, obj, filt_ptr, filt_idx, count_eq=count_eq)
 
-    def topk(self, src, rel, data, k=10, exclude=None, precision='bf16'):
+    def topk(self, src, rel, data, k=10, exclude=None, precision='bf16', table=None, n_offset=0, group=None):
         """The k most likely objects of the queries (src, rel, ?) without materialising the [B, N] scores (K6k):
         ``scoring.topk`` on the ConvE query.  ``exclude``: (ptr, idx) CSR of entities to leave out per query, e.g.
-        ``DataLoader.known_objects(src, rel)`` for the known facts; None keeps every entity."""
+        ``DataLoader.known_objects(src, rel)`` for the known facts; None keeps every entity.
+
+        Entity-sharded, as ``scoring.topk``: ``table`` is this rank's bf16 shard of the encoded entities, rows
+        ``n_offset .. n_offset + table.n`` (with precision='fp32' the same rows of the fp32 encoding are scored).  With a
+        ``group`` and no ``table``, the ranks split the entities into even ranges (rank r: rows r * ceil(N / world) ...).
+        Every rank of the group returns the unsharded answer."""
         from .scoring import topk
         all_ent, all_rel = self.encode(data)
         xq = self.conv2.query(torch.index_select(all_ent, 0, src), torch.index_select(all_rel, 0, rel))
         ptr, idx = exclude if exclude is not None else (None, None)
-        return topk(xq, all_ent, self.conv2.bias, k, ptr, idx, precision=precision)
+        ent, bias = all_ent, self.conv2.bias
+        if n_offset != 0 and table is None:
+            raise ValueError('n_offset names the first row of a table shard: pass table= as well')
+        if table is not None or group is not None:
+            if table is not None:
+                lo, hi = n_offset, n_offset + table.n
+            else:
+                import torch.distributed as dist
+                n, world = int(all_ent.shape[0]), dist.get_world_size(group)
+                per = -(-n // world)
+                lo = min(dist.get_rank(group) * per, n)
+                hi = min(lo + per, n)
+            n_offset = lo
+            ent, bias = all_ent[lo:hi], (bias[lo:hi] if bias is not None else None)
+        return topk(xq, ent, bias, k, ptr, idx, table=table, precision=precision, n_offset=n_offset, group=group)

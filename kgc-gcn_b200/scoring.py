@@ -325,7 +325,12 @@ def _check_exclusions(b, excl_ptr, excl_idx):
     return (ptr, idx) if nnz > 0 else (None, None)
 
 
-def topk(xq, all_ent, bias, k, excl_ptr=None, excl_idx=None, table=None, precision='bf16'):
+def _check_k(k):
+    if isinstance(k, bool) or not isinstance(k, int) or not 1 <= k <= TOPK_MAX:
+        raise ValueError('k must be an integer in [1, {}], got {!r}'.format(TOPK_MAX, k))
+
+
+def topk(xq, all_ent, bias, k, excl_ptr=None, excl_idx=None, table=None, precision='bf16', n_offset=0, group=None):
     """The ``k`` best entities for every query row of ``xq`` [B, d] against ``all_ent`` [N, d] (+ ``bias`` [N]), leaving out
     each query's exclusion list (the known positives: ``excl_ptr`` [B+1] int64 / ``excl_idx`` int32 CSR, rows sorted
     ascending, e.g. ``DataLoader.known_objects``; None: no filter).
@@ -336,14 +341,78 @@ def topk(xq, all_ent, bias, k, excl_ptr=None, excl_idx=None, table=None, precisi
 
     ``precision='bf16'`` (default): the fused tcgen05 sweep (K6k) on the bf16 entity table - ``table=`` reuses an
     ``EntityTable`` - without writing the [B, N] logits; scores are bit-identical to ``pair_scores``.  ``precision='fp32'``:
-    the same selection over fp32-grade dense logits (3xTF32), 256 queries at a time, as in ``filtered_rank``'s exact mode."""
-    if isinstance(k, bool) or not isinstance(k, int) or not 1 <= k <= TOPK_MAX:
-        raise ValueError('k must be an integer in [1, {}], got {!r}'.format(TOPK_MAX, k))
+    the same selection over fp32-grade dense logits (3xTF32), 256 queries at a time, as in ``filtered_rank``'s exact mode.
+
+    Entity-sharded use, as in ``filtered_rank``: the local rows (``table``, or ``all_ent`` / ``bias`` in fp32) are the
+    global entities ``n_offset .. n_offset + n``; the queries and the exclusion CSR are replicated and given in global ids.
+    Without ``group`` the result is this slice's top k in global ids (``merge_topk`` combines slices).  With the process
+    ``group`` every rank sweeps its rows, the [B, k] results are all-gathered and merged (``merge_topk``) on every rank:
+    every rank returns the answer of the unsharded call, bit for bit.  The ranks' row ranges must be disjoint and every
+    rank must pass the same B and k (checked: ValueError).  A rank may own no rows."""
+    _check_k(k)
     if precision not in ('bf16', 'fp32'):
         raise ValueError("precision must be 'bf16' or 'fp32'")
+    if isinstance(n_offset, bool) or not isinstance(n_offset, int) or n_offset < 0:
+        raise ValueError('n_offset must be a non-negative integer, got {!r}'.format(n_offset))
     xq = _lib.require_cuda(xq.detach(), torch.float32, 'xq')
     dev, b = xq.device, int(xq.shape[0])
     ptr, idx = _check_exclusions(b, excl_ptr, excl_idx)
+    if n_offset == 0 and group is None:
+        scores, ids, count = _topk_rows(xq, all_ent, bias, k, ptr, idx, table, precision)
+        return {'scores': scores, 'ids': ids.long(), 'count': count}
+    if precision == 'bf16' and table is not None:
+        n = table.n
+    elif all_ent is not None:
+        n = int(all_ent.shape[0])
+    else:
+        raise ValueError("topk takes this shard's rows: table= (bf16) or all_ent (fp32)")
+    if n_offset + n >= 2 ** 31:
+        raise ValueError('global entity ids must stay below 2^31 (n_offset + n = {})'.format(n_offset + n))
+    if group is not None:
+        _check_shards(dev, b, k, n_offset, n, group)
+    if n > 0 and b > 0:
+        if idx is not None:
+            # local ids: the shift keeps every row sorted; ids outside [0, n) match no row (clamped into int32 range)
+            idx = (idx.long() - n_offset).clamp_(-1, n).to(torch.int32)
+        scores, ids, count = _topk_rows(xq, all_ent, bias, k, ptr, idx, table, precision)
+        ids = torch.where(ids >= 0, ids + n_offset, ids)
+    else:                                  # no rows here: all padding, no launch (the kernels take n > 0 only)
+        scores = torch.full((b, k), -float('inf'), dtype=torch.float32, device=dev)
+        ids = torch.full((b, k), -1, dtype=torch.int32, device=dev)
+        count = torch.zeros((b,), dtype=torch.int32, device=dev)
+    if group is None:
+        return {'scores': scores, 'ids': ids.long(), 'count': count}
+    import torch.distributed as dist
+    world = dist.get_world_size(group)
+    all_s = torch.empty((world * b, k), dtype=torch.float32, device=dev)
+    all_i = torch.empty((world * b, k), dtype=torch.int32, device=dev)
+    dist.all_gather_into_tensor(all_s, scores, group=group)
+    dist.all_gather_into_tensor(all_i, ids, group=group)
+    return merge_topk(all_s.view(world, b, k), all_i.view(world, b, k))
+
+
+def _check_shards(dev, b, k, n_offset, n, group):
+    """One all-gather of (n_offset, n, B, k): every rank raises the same ValueError when the ranks disagree on B or k or
+    their row ranges overlap (overlapping shards would return an entity twice)."""
+    import torch.distributed as dist
+    world = dist.get_world_size(group)
+    meta = torch.tensor([n_offset, n, b, k], dtype=torch.int64, device=dev)
+    every = torch.empty((world, 4), dtype=torch.int64, device=dev)
+    dist.all_gather_into_tensor(every, meta, group=group)
+    every = every.tolist()
+    if any(r[2] != b or r[3] != k for r in every):
+        raise ValueError('topk with a group: every rank must pass the same B and k, got (B, k) = {}'.format(
+            [(r[2], r[3]) for r in every]))
+    spans = sorted((r[0], r[0] + r[1]) for r in every if r[1] > 0)
+    for (_, hi), (lo, _) in zip(spans, spans[1:]):
+        if lo < hi:
+            raise ValueError('topk with a group: the ranks\' row ranges overlap: {}'.format(
+                [(r[0], r[0] + r[1]) for r in every]))
+
+
+def _topk_rows(xq, all_ent, bias, k, ptr, idx, table, precision):
+    """(scores [B, k], ids [B, k] int32 local, count [B]) over the rows of ``table`` (bf16) or ``all_ent`` (fp32)."""
+    dev, b = xq.device, int(xq.shape[0])
     scores = torch.empty((b, k), dtype=torch.float32, device=dev)
     ids = torch.empty((b, k), dtype=torch.int32, device=dev)
     count = torch.empty((b,), dtype=torch.int32, device=dev)
@@ -375,7 +444,43 @@ def topk(xq, all_ent, bias, k, excl_ptr=None, excl_idx=None, table=None, precisi
             z, ld = dense_logits(xq[i:j], ent, bias)
             _lib.call('kgc_topk_dense', p(z), ld, n, j - i, p(ptr[i:]) if ptr is not None else None, p(idx), k,
                       p(scores[i:j]), p(ids[i:j]), p(count[i:j]), p(ws), ws_bytes, _lib.stream())
-    return {'scores': scores, 'ids': ids.long(), 'count': count}
+    return scores, ids, count
+
+
+def merge_topk(scores, ids, k=None):
+    """The ``k`` best entries of the union of S finished top-k results (``kgc_topk_merge``): ``scores`` [S, B, k_in] float32
+    and ``ids`` [S, B, k_in] int32 or int64 (< 0: padding), every row sorted as ``topk`` returns it, ids disjoint across
+    the S results - e.g. ``topk`` of disjoint entity ranges, one per shard or per slice of a table streamed through
+    ``topk(..., n_offset=lo)``.  ``k`` (default k_in, at most 32): a smaller k reads the first k entries of every row, a
+    larger one pads every row with (-inf, -1).  Returns the dict ``topk`` returns, ordered and padded the same way; the
+    result does not depend on the order of the S results.  With k <= k_in it equals ``topk`` over the union of the ranges."""
+    scores = _lib.require_cuda(scores.detach(), torch.float32, 'scores')
+    if not (torch.is_tensor(ids) and ids.is_cuda):
+        raise RuntimeError('ids must be a CUDA tensor: the M-GCN hot path runs on the GPU only (no CPU fallback)')
+    if scores.dim() != 3 or tuple(ids.shape) != tuple(scores.shape) or scores.shape[0] < 1 or scores.shape[2] < 1:
+        raise ValueError('scores and ids must both be [S, B, k] with S >= 1 and k >= 1, got {} and {}'.format(
+            tuple(scores.shape), tuple(ids.shape)))
+    if ids.dtype == torch.int64:
+        if ids.numel() and int(ids.max()) >= 2 ** 31:
+            raise ValueError('ids must be below 2^31')
+        ids = ids.clamp(min=-1).to(torch.int32)
+    ids = _lib.require_cuda(ids, torch.int32, 'ids')
+    n_lists, b, k_in = (int(v) for v in scores.shape)
+    k = k_in if k is None else k
+    _check_k(k)
+    if k < k_in:
+        scores, ids = scores[:, :, :k].contiguous(), ids[:, :, :k].contiguous()
+    elif k > k_in:
+        scores = torch.nn.functional.pad(scores, (0, k - k_in), value=-float('inf'))
+        ids = torch.nn.functional.pad(ids, (0, k - k_in), value=-1)
+    dev = scores.device
+    top_s = torch.empty((b, k), dtype=torch.float32, device=dev)
+    top_id = torch.empty((b, k), dtype=torch.int32, device=dev)
+    count = torch.empty((b,), dtype=torch.int32, device=dev)
+    if b > 0:
+        p = _lib.ptr
+        _lib.call('kgc_topk_merge', p(scores), p(ids), n_lists, b, k, p(top_s), p(top_id), p(count), _lib.stream())
+    return {'scores': top_s, 'ids': top_id.long(), 'count': count}
 
 
 def tie_adjusted_sums(ranks, count_eq, ties):
