@@ -304,6 +304,12 @@ int kgc_label_build(const int64_t* qid, int64_t B, const int64_t* triples, const
 int kgc_neg_sample(const int64_t* qid, int64_t B, const int64_t* ptr, const int32_t* idx, int64_t n_entity,
                    const uint32_t* draws, int32_t k, int32_t tries, int32_t* neg, void* stream);
 
+/* Positive sampler, the companion of kgc_neg_sample (extension): out[b, j] = idx[ptr[q] + ((draws[b, j] * len_q) >> 32)]
+ * with q = qid[b] and len_q = ptr[q + 1] - ptr[q] - sampling with replacement from the query's object list; -1 for a
+ * query without objects.  A pure function of the caller's uint32 draws [B, p]; out int32 [B, p]. */
+int kgc_pos_sample(const int64_t* qid, int64_t B, const int64_t* ptr, const int32_t* idx, const uint32_t* draws,
+                   int32_t p, int32_t* out, void* stream);
+
 /* Edge sampler, likewise an extension without a reference counterpart (the reference always convolves over the full
  * edge list built at data_loader.py:132-157).  m triples drawn with replacement, t_j = (draws[j] * n_triples) >> 32; the
  * sampled sub-graph keeps the reference's layout: columns 0..m-1 = in-half edges t_j, m..2m-1 = their reverses
@@ -521,6 +527,28 @@ int kgc_topk_dense(const float* logits, int64_t ld, int64_t n, int64_t b, const 
  * n_lists >= 1, 0 < b < 2^31, 1 <= k <= 32.  One kernel, no workspace; deterministic. */
 int kgc_topk_merge(const float* part_s, const int32_t* part_id, int64_t n_lists, int64_t b, int32_t k,
                    float* top_s, int32_t* top_id, int32_t* count, void* stream);
+
+/* K6s: sampled (1-vs-k) scoring fused with the BCE loss (extension: negative-sampled training).  Query b scores the C
+ * candidates cand[b, 0..C) (int32 [B, C]): the first n_pos carry the label pos, the rest add; an id outside [0, n_ent) is
+ * an empty slot (no loss, no gradient).  x [B, D] contiguous, ent [n_ent, D] with row pitch ld_ent, bias [n_ent];
+ * D % 4 == 0, D <= 256; x, ent, d_x 16-byte aligned.
+ * kgc_sampled_bce_fwd, in one pass: loss[0] = mean over the valid slots of ATen's BCE of p = sigmoid(<x[b], ent[c]> +
+ * bias[c]) (0 when no slot is valid), count[0] = the number of valid slots, g [B, C] = the logit gradient for a unit
+ * upstream gradient (0 on empty slots, formulas of kgc_bce_1n_bwd_logit_t with the valid-slot count as divisor) and
+ * d_x [B, D] = sum_c g[b, c] * ent[cand[b, c]] in slot order.  loss_partial: kgc_sampled_bce_fwd_blocks(B) doubles.
+ * kgc_sampled_bce_bwd_table: the dense table gradient for the upstream scalar *scale (device memory):
+ * d_ent[n] = sum over the slots s with cand[s] = n of g[s] * (*scale * x[b(s)]), d_bias[n] = *scale * sum g[s], in slot
+ * order; rows no slot names are zero (d_ent [n_ent, D] with row pitch ld_d).  The (entity, slot) pairs are
+ * stable-sorted by entity, no float atomics.  workspace: kgc_sampled_bce_bwd_table_workspace_bytes(B * C, n_ent) bytes.
+ * Both deterministic, no host synchronisation (graph-capturable). */
+int64_t kgc_sampled_bce_fwd_blocks(int64_t B);
+int kgc_sampled_bce_fwd(const float* x, int64_t B, int32_t D, const float* ent, int64_t n_ent, int64_t ld_ent,
+                        const float* bias, const int32_t* cand, int32_t C, int32_t n_pos, float pos, float add,
+                        float* g, float* d_x, int32_t* count, double* loss_partial, float* loss, void* stream);
+size_t kgc_sampled_bce_bwd_table_workspace_bytes(int64_t n_slots, int64_t n_ent);
+int kgc_sampled_bce_bwd_table(const float* x, int64_t B, int32_t D, const int32_t* cand, int32_t C, const float* g,
+                              const float* scale, int64_t n_ent, float* d_ent, int64_t ld_d, float* d_bias,
+                              void* workspace, size_t workspace_bytes, void* stream);
 
 #if defined(__GNUC__)
 #pragma GCC visibility pop

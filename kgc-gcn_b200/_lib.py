@@ -59,6 +59,7 @@ SIGNATURES = {
     'kgc_gemm_tn': (ctypes.c_int, [_vp, _i64, _vp, _i64, _i64, _i32, _i32, _vp, _vp, _sz, _vp]),
     'kgc_label_build': (ctypes.c_int, [_vp, _i64, _vp, _vp, _vp, _i64, _f32, _f32, _vp, _vp, _vp]),
     'kgc_neg_sample': (ctypes.c_int, [_vp, _i64, _vp, _vp, _i64, _vp, _i32, _i32, _vp, _vp]),
+    'kgc_pos_sample': (ctypes.c_int, [_vp, _i64, _vp, _vp, _vp, _i32, _vp, _vp]),
     'kgc_edge_sample': (ctypes.c_int, [_vp, _vp, _vp, _i64, _vp, _i64, _vp, _vp, _vp, _vp, _vp]),
     'kgc_bn2d_partials_bytes': (_sz, [_i32]),
     'kgc_bn2d_relu_drop_fwd': (ctypes.c_int, [_vp, _i64, _i32, _i32, _vp, _vp, _vp, _vp, _f32, _f32, _i32, _i32, _vp, _f32, _vp, _vp, _vp, _vp]),
@@ -101,6 +102,11 @@ SIGNATURES = {
     'kgc_topk_dense_workspace_bytes': (_sz, [_i64, _i64, _i32]),
     'kgc_topk_dense': (ctypes.c_int, [_vp, _i64, _i64, _i64, _vp, _vp, _i32, _vp, _vp, _vp, _vp, _sz, _vp]),
     'kgc_topk_merge': (ctypes.c_int, [_vp, _vp, _i64, _i64, _i32, _vp, _vp, _vp, _vp]),
+    'kgc_sampled_bce_fwd_blocks': (_i64, [_i64]),
+    'kgc_sampled_bce_fwd': (ctypes.c_int, [_vp, _i64, _i32, _vp, _i64, _i64, _vp, _vp, _i32, _i32, _f32, _f32, _vp, _vp, _vp, _vp,
+                                           _vp, _vp]),
+    'kgc_sampled_bce_bwd_table_workspace_bytes': (_sz, [_i64, _i64]),
+    'kgc_sampled_bce_bwd_table': (ctypes.c_int, [_vp, _i64, _i32, _vp, _i32, _vp, _vp, _i64, _vp, _i64, _vp, _vp, _sz, _vp]),
 }
 
 
@@ -122,7 +128,7 @@ def lib():
 
 
 LAUNCHES = 0     # kernels launched through the C ABI since import (bench.py reports it as gpu_launches)
-_KERNELS_PER_CALL = {'kgc_csr_build': 16, 'kgc_label_mask_build': 2, 'kgc_bce_1n_bwd_logit': 2, 'kgc_bce_1n_bwd_logit_t': 2, 'kgc_label_mask_t_build': 2, 'kgc_score_pairs': 3, 'kgc_rank_finalize': 2, 'kgc_score_topk': 2, 'kgc_topk_dense': 2, 'kgc_gemm_tn': 2, 'kgc_gemm_tn_tc': 2, 'kgc_gemm_tn_tc_batch': 2, 'kgc_gemm_tn_tc_batch_masked': 2}   # (kgc_p2p_allreduce: 1 or 3)
+_KERNELS_PER_CALL = {'kgc_csr_build': 16, 'kgc_label_mask_build': 2, 'kgc_bce_1n_bwd_logit': 2, 'kgc_bce_1n_bwd_logit_t': 2, 'kgc_label_mask_t_build': 2, 'kgc_score_pairs': 3, 'kgc_rank_finalize': 2, 'kgc_score_topk': 2, 'kgc_topk_dense': 2, 'kgc_sampled_bce_fwd': 4, 'kgc_sampled_bce_bwd_table': 7, 'kgc_gemm_tn': 2, 'kgc_gemm_tn_tc': 2, 'kgc_gemm_tn_tc_batch': 2, 'kgc_gemm_tn_tc_batch_masked': 2}   # (kgc_p2p_allreduce: 1 or 3)
 
 
 def call(name, *args):

@@ -145,14 +145,22 @@ def gemm_nt_splitk(a, bt, out):
     return out
 
 
+LINEAR_ROWS = 128       # rows of x per split-K forward / d_x launch (the kernels' Ma <= 128)
+LINEAR_DW_ROWS = 256    # rows of the d_W contraction per launch (K <= 256); partials added in chunk order
+
+
 class _LinearFn(torch.autograd.Function):
     """y = x @ W^T + b for a wide input (ConvE's fc, model.py:173: 39,200 -> 200) on the 3xTF32 tensor-core kernels:
-    split-K forward, transposed-operand kernels for d_W and d_x."""
+    split-K forward, transposed-operand kernels for d_W and d_x.  Any batch: the forward and d_x run tile by tile over 128
+    rows, d_W sums chunks of 256 rows in order (deterministic); up to 128 rows it is one launch each."""
 
     @staticmethod
     def forward(ctx, x, weight, bias):
         x_, w_ = x.detach(), weight.detach()
-        y = gemm_nt_splitk(x_, w_, torch.empty((x_.shape[0], w_.shape[0]), dtype=torch.float32, device=x.device))
+        B = x_.shape[0]
+        y = torch.empty((B, w_.shape[0]), dtype=torch.float32, device=x.device)
+        for i in range(0, B, LINEAR_ROWS):
+            gemm_nt_splitk(x_[i:i + LINEAR_ROWS], w_, y[i:i + LINEAR_ROWS])
         if bias is not None:
             y += bias.detach()
         ctx.save_for_backward(x_, w_)
@@ -164,10 +172,17 @@ class _LinearFn(torch.autograd.Function):
         x, w = ctx.saved_tensors
         dy = dy.contiguous()
         dx = dw = db = None
+        B = x.shape[0]
         if ctx.needs_input_grad[0]:
-            dx = gemm_nt_trans(w, dy.t(), torch.empty_like(x))          # d_x[B, F] = d_y @ W
+            dx = torch.empty_like(x)
+            for i in range(0, B, LINEAR_ROWS):                          # d_x[B, F] = d_y @ W
+                gemm_nt_trans(w, dy[i:i + LINEAR_ROWS].t(), dx[i:i + LINEAR_ROWS])
         if ctx.needs_input_grad[1]:
-            dw = gemm_nt_trans(x, dy, torch.empty_like(w))              # d_W[O, F] = d_y^T @ x
+            dw = gemm_nt_trans(x[:LINEAR_DW_ROWS], dy[:LINEAR_DW_ROWS], torch.empty_like(w))   # d_W[O, F] = d_y^T @ x
+            if B > LINEAR_DW_ROWS:
+                part = torch.empty_like(w)
+                for i in range(LINEAR_DW_ROWS, B, LINEAR_DW_ROWS):
+                    dw += gemm_nt_trans(x[i:i + LINEAR_DW_ROWS], dy[i:i + LINEAR_DW_ROWS], part)
         if ctx.has_bias and ctx.needs_input_grad[2]:
             db = dy.sum(0)
         return dx, dw, db
@@ -177,12 +192,13 @@ def linear_tc_supported(x, weight):
     B, F = x.shape
     O = weight.shape[0]
     return (x.is_cuda and x.dtype == torch.float32 and weight.dtype == torch.float32 and x.is_contiguous()
-            and weight.is_contiguous() and 0 < B <= 128 and O <= 224 and O % 4 == 0 and F % 32 == 0 and F >= 4096
+            and weight.is_contiguous() and B > 0 and O <= 224 and O % 4 == 0 and F % 32 == 0 and F >= 4096
             and x.data_ptr() % 16 == 0 and weight.data_ptr() % 16 == 0)
 
 
 def linear_tc(x, weight, bias=None):
-    """Differentiable y = x @ weight^T + bias on the tensor-core kernels (see linear_tc_supported for the shapes)."""
+    """Differentiable y = x @ weight^T + bias on the tensor-core kernels (see linear_tc_supported for the shapes); any
+    number of rows (tiles of 128)."""
     return _LinearFn.apply(x, weight, bias)
 
 

@@ -66,6 +66,18 @@ __global__ void neg_sample_kernel(const int64_t* __restrict__ qid, int64_t B, co
   neg[t] = out;
 }
 
+// Positive sampler (extension, companion of the negative sampler): slot j of query qid[b] is the
+// ((u * len) >> 32)-th entry of the query's object list - sampling with replacement; -1 for a query without objects.
+__global__ void pos_sample_kernel(const int64_t* __restrict__ qid, int64_t B, const int64_t* __restrict__ ptr,
+                                  const int32_t* __restrict__ idx, const uint32_t* __restrict__ draws, int p,
+                                  int32_t* __restrict__ out) {
+  const int64_t t = blockIdx.x * (int64_t)blockDim.x + threadIdx.x;
+  if (t >= B * p) return;
+  const int64_t q = qid[t / p];
+  const int64_t lo = ptr[q], len = ptr[q + 1] - lo;
+  out[t] = len > 0 ? idx[lo + (int64_t)(((uint64_t)draws[t] * (uint64_t)len) >> 32)] : -1;
+}
+
 // Edge sampler (extension, no reference counterpart): triple t_j = (draws[j] * E) >> 32 contributes its in-half edge t_j to
 // column j and its out-half edge t_j + E to column m + j of the sampled sub-graph - the layout MGCNConv expects (in half
 // first).  A pure function of the caller's draws (sampling with replacement).
@@ -124,6 +136,16 @@ extern "C" int kgc_neg_sample(const int64_t* qid, int64_t B, const int64_t* ptr,
   if (B == 0) return 0;
   neg_sample_kernel<<<(unsigned)ceil_div(B * k, kThreads), kThreads, 0, as_stream(stream)>>>(qid, B, ptr, idx, n_entity,
                                                                                          draws, k, tries, neg);
+  KGC_LAUNCH_CHECK();
+  return 0;
+}
+
+extern "C" int kgc_pos_sample(const int64_t* qid, int64_t B, const int64_t* ptr, const int32_t* idx, const uint32_t* draws,
+                              int32_t p, int32_t* out, void* stream) {
+  KGC_REQUIRE(B >= 0 && p > 0, "bad sizes");
+  if (B == 0) return 0;
+  KGC_REQUIRE(qid && ptr && idx && draws && out, "null buffer");
+  pos_sample_kernel<<<(unsigned)ceil_div(B * p, kThreads), kThreads, 0, as_stream(stream)>>>(qid, B, ptr, idx, draws, p, out);
   KGC_LAUNCH_CHECK();
   return 0;
 }

@@ -266,6 +266,31 @@ class KBDataset(object):
             _lib.call('kgc_neg_sample', p(qid), b, p(ptr), p(idx), self.num_entity, p(d32), int(k), int(tries), p(neg), _lib.stream())
         return neg
 
+    def positives(self, qid, p, draws=None, device='cuda', generator=None):
+        """GPU positive sampler, the companion of ``negatives``: ``p`` of each query's known objects, drawn with replacement
+        from its object list (the training queries are (s, r, -1): the objects come from the lists, not the triple) ->
+        int32 [B, p] on ``device``; -1 for a query without objects.  A pure function of ``draws`` (uint32 [B, p], slot =
+        list[(u * len) >> 32]); when omitted they come from torch's generator (``generator`` or the global one)."""
+        if isinstance(p, bool) or int(p) != p or p < 1:
+            raise ValueError('p must be a positive integer, got {!r}'.format(p))
+        device = torch.device(device)
+        if device.type != 'cuda':
+            raise RuntimeError('the positive sampler runs on the GPU only (no CPU fallback)')
+        _, ptr, idx = self.device_csr(device)
+        qid = torch.as_tensor(qid, dtype=torch.int64).to(device)
+        b = int(qid.numel())
+        if draws is None:
+            draws = torch.randint(0, 1 << 32, (b, int(p)), dtype=torch.int64, device=device, generator=generator)
+        draws = torch.as_tensor(draws).to(device)
+        if tuple(draws.shape) != (b, int(p)):
+            raise ValueError('draws must be [len(qid), p]')
+        d32 = _u32_bits(draws)
+        out = torch.empty((b, int(p)), dtype=torch.int32, device=device)
+        with torch.cuda.device(device):
+            _lib.call('kgc_pos_sample', _lib.ptr(qid), b, _lib.ptr(ptr), _lib.ptr(idx), _lib.ptr(d32), int(p), _lib.ptr(out),
+                      _lib.stream())
+        return out
+
     def sparse_batch(self, qid):
         """Host CSR slice for the fused scorer: (triple[B,3], filt_ptr[B+1] int64, filt_idx[nnz] int32), numpy."""
         qid = np.asarray(qid, dtype=np.int64)

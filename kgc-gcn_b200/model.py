@@ -168,7 +168,7 @@ class ConvE(nn.Module):
         if linear_tc_supported(x, self.fc.weight):
             x = linear_tc(x, self.fc.weight, self.fc.bias)
         else:
-            _lib.library_path('ConvE.fc', 'the tensor-core fc kernels take CUDA fp32, B <= 128, out <= 224, flat % 32 == 0, flat >= 4096')
+            _lib.library_path('ConvE.fc', 'the tensor-core fc kernels take CUDA fp32, out <= 224, flat % 32 == 0, flat >= 4096')
             x = self.fc(x)
         x = self.hidden_drop(x)
         return F.relu(self.bn2(x))
@@ -299,6 +299,27 @@ class MGCN(nn.Module):
                                'use loss(forward(...), label)')
         pos, add = dataset.label_values()
         return score_1n_bce(x, all_ent, self.conv2.bias, qid, ptr, idx, pos, add)
+
+    def loss_sampled(self, qid, dataset, data, k, n_pos=1, tries=4, draws=None, generator=None):
+        """Negative-sampled (1-vs-k) training loss for the training queries ``qid`` of ``dataset`` (a KBDataset): each query
+        scores ``n_pos`` of its known objects (``dataset.positives``) and ``k`` entities that are not (``dataset.negatives``,
+        ``tries`` draws per slot) - candidates [pos | neg] - through ``scoring.score_sampled_bce`` with the dataset's
+        ``label_values()``.  Unlike ``loss_sparse`` the cost of the scoring does not grow with N, so the batch can be large.
+        ``draws = (pos_draws [B, n_pos], neg_draws [B, k, tries])`` (uint32 values) makes the call a pure function of them;
+        otherwise they come from torch's generator (``generator`` or the global one), positives first."""
+        from .scoring import score_sampled_bce
+        dev = self.entity_embedding.device
+        triples, _, _ = dataset.device_csr(dev)
+        qid = torch.as_tensor(qid, dtype=torch.int64).to(dev, non_blocking=True)
+        pos_draws, neg_draws = draws if draws is not None else (None, None)
+        cand = torch.cat([dataset.positives(qid, n_pos, draws=pos_draws, device=dev, generator=generator),
+                          dataset.negatives(qid, k, draws=neg_draws, tries=tries, device=dev, generator=generator)], 1)
+        trip = torch.index_select(triples, 0, qid)
+        all_ent, all_rel = self.encode(data)
+        src_emb, all_ent = self._rows(all_ent, trip[:, 0])
+        x = self.conv2.query(src_emb, torch.index_select(all_rel, 0, trip[:, 1]))
+        pos, add = dataset.label_values()
+        return score_sampled_bce(x, all_ent, self.conv2.bias, cand, n_pos, pos, add)
 
     def rank(self, src, rel, obj, filt_ptr, filt_idx, data, count_eq=False):
         """Filtered rank of obj among all entities for the queries (src, rel) without materialising the

@@ -143,6 +143,84 @@ def score_1n_bce(x, all_ent, bias, qid, ptr, idx, pos=1.0, add=0.0):
     return total
 
 
+class _ScoreSampledBCE(torch.autograd.Function):
+    """loss = mean BCE of sigmoid(<x[b], all_ent[cand[b, c]]> + bias[cand[b, c]]) over the valid slots (K6s).  The forward
+    makes one pass that yields the loss, the logit gradient g [B, C] and d_x for a unit upstream gradient; the backward
+    scales d_x and builds the dense table gradient by sorting the (entity, slot) pairs (no float atomics)."""
+
+    @staticmethod
+    def forward(ctx, x, all_ent, bias, cand, n_pos, pos, add):
+        x = _lib.require_cuda(x.detach(), torch.float32, 'x')
+        ent = all_ent.detach()                           # rows may sit in a wider table: the kernel takes a row pitch
+        if ent.dtype != torch.float32:
+            raise TypeError('all_ent must be torch.float32, got {}'.format(ent.dtype))
+        if ent.stride(1) != 1 or ent.stride(0) % 4 != 0 or ent.data_ptr() % 16 != 0:
+            ent = ent.clone(memory_format=torch.contiguous_format)
+        bias_ = _lib.require_cuda(bias.detach(), torch.float32, 'bias')
+        cand = _lib.require_cuda(cand, torch.int32, 'cand')
+        B, D = int(x.shape[0]), int(x.shape[1])
+        C, N = int(cand.shape[1]), int(ent.shape[0])
+        dev, p = x.device, _lib.ptr
+        g = torch.empty((B, C), dtype=torch.float32, device=dev)
+        d_x = torch.empty((B, D), dtype=torch.float32, device=dev)
+        count = torch.empty((1,), dtype=torch.int32, device=dev)
+        partial = torch.empty((int(_lib.lib().kgc_sampled_bce_fwd_blocks(B)),), dtype=torch.float64, device=dev)
+        loss = torch.empty((1,), dtype=torch.float32, device=dev)
+        _lib.call('kgc_sampled_bce_fwd', p(x), B, D, p(ent), N, ent.stride(0), p(bias_), p(cand), C, int(n_pos), float(pos),
+                  float(add), p(g), p(d_x), p(count), p(partial), p(loss), _lib.stream())
+        ctx.save_for_backward(x, cand, g, d_x)
+        ctx.n_ent = N
+        return loss[0]
+
+    @staticmethod
+    def backward(ctx, d_loss):
+        x, cand, g, d_x = ctx.saved_tensors
+        B, D, C, N = int(x.shape[0]), int(x.shape[1]), int(cand.shape[1]), ctx.n_ent
+        d_ent = d_bias = None
+        if ctx.needs_input_grad[1] or ctx.needs_input_grad[2]:
+            dev, p = x.device, _lib.ptr
+            scale = d_loss.reshape(1).to(torch.float32).contiguous()
+            d_ent = torch.empty((N, D), dtype=torch.float32, device=dev)
+            d_bias = torch.empty((N,), dtype=torch.float32, device=dev)
+            ws_bytes = int(_lib.lib().kgc_sampled_bce_bwd_table_workspace_bytes(B * C, N))
+            ws = torch.empty((ws_bytes,), dtype=torch.uint8, device=dev)
+            _lib.call('kgc_sampled_bce_bwd_table', p(x), B, D, p(cand), C, p(g), p(scale), N, p(d_ent), D, p(d_bias), p(ws),
+                      ws_bytes, _lib.stream())
+        return (d_x * d_loss if ctx.needs_input_grad[0] else None, d_ent if ctx.needs_input_grad[1] else None,
+                d_bias if ctx.needs_input_grad[2] else None, None, None, None, None)
+
+
+def score_sampled_bce(x, all_ent, bias, cand, n_pos, pos=1.0, add=0.0):
+    """Negative-sampled (1-vs-k) BCE: query b of ``x`` [B, D] scores only its candidates ``cand`` [B, C] (int32 entity ids;
+    the first ``n_pos`` columns are positives with label ``pos``, the rest negatives with label ``add``, e.g.
+    ``KBDataset.label_values()``; -1 marks an empty slot, which adds neither loss nor gradient).  Returns the mean BCE of
+    sigmoid(<x[b], all_ent[c]> + bias[c]) over the valid slots (0 when there are none), differentiable in ``x``,
+    ``all_ent`` and ``bias``.  The cost is B x C gathered rows, independent of N.  D % 4 == 0, D <= 256; deterministic and graph-capturable."""
+    if x.dim() != 2 or all_ent.dim() != 2 or bias.dim() != 1 or cand.dim() != 2:
+        raise ValueError('score_sampled_bce takes x [B, D], all_ent [N, D], bias [N] and cand [B, C]')
+    B, D = int(x.shape[0]), int(x.shape[1])
+    N, C = int(all_ent.shape[0]), int(cand.shape[1])
+    if int(all_ent.shape[1]) != D or int(bias.shape[0]) != N or int(cand.shape[0]) != B:
+        raise ValueError('shape mismatch: x {}, all_ent {}, bias {}, cand {}'.format(
+            tuple(x.shape), tuple(all_ent.shape), tuple(bias.shape), tuple(cand.shape)))
+    if B < 1 or C < 1 or N < 1 or D < 4 or D > 256 or D % 4 != 0:
+        raise ValueError('score_sampled_bce needs B, C, N >= 1 and D % 4 == 0, D <= 256 (got B={}, C={}, N={}, D={})'.format(
+            B, C, N, D))
+    if isinstance(n_pos, bool) or int(n_pos) != n_pos or not 0 <= n_pos <= C:
+        raise ValueError('n_pos must be an integer in [0, C = {}], got {!r}'.format(C, n_pos))
+    if cand.dtype != torch.int32:
+        raise ValueError('cand must be torch.int32, got {}'.format(cand.dtype))
+    if B * C >= 2 ** 31 or N >= 2 ** 31 - 1:
+        raise ValueError('score_sampled_bce takes B * C < 2^31 slots and N < 2^31 - 1 entities')
+    for t, name in ((x, 'x'), (all_ent, 'all_ent'), (bias, 'bias'), (cand, 'cand')):
+        if not t.is_cuda:
+            raise RuntimeError('{} must be a CUDA tensor: the M-GCN hot path runs on the GPU only (no CPU fallback)'.format(name))
+    if not torch.cuda.is_current_stream_capturing() and bool((cand >= N).any()):
+        # (not checked while a CUDA graph is captured: the check reads back; the kernels treat such ids as empty slots)
+        raise ValueError('cand holds entity ids >= N = {}'.format(N))
+    return _ScoreSampledBCE.apply(x, all_ent, bias, cand, int(n_pos), pos, add)
+
+
 def score_kpad(d):
     kpad = int(_lib.lib().kgc_score_kpad(int(d)))
     if kpad < 0:

@@ -17,9 +17,20 @@ class GraphedTrainStep(object):
     clipping, or ``torch.optim.Adam(..., capturable=True)``); ``dataset`` is the KBDataset of the
     training queries; batches whose size differs from ``batch_size`` (the last one of an epoch) run eagerly.
     ``fused_loss=True`` (opt-in) trains through ``MGCN.loss_sparse``: the label stays a sparse list of positives and the
-    dense [B, N] label, its build and the BCE tensors drop out of the step (SURVEY.md 8(f) N1)."""
+    dense [B, N] label, its build and the BCE tensors drop out of the step (SURVEY.md 8(f) N1).
+    ``negatives=k`` trains the negative-sampled objective instead (``MGCN.loss_sampled``: ``n_pos`` positives and k
+    negatives per query, ``tries`` draws per negative): its cost does not grow with N, so ``batch_size`` can be in the
+    thousands.  Each step draws the samplers' uint32 inputs from ``generator`` (or torch's global one) into static device
+    buffers (``pos_draws`` [B, n_pos], ``neg_draws`` [B, k, tries]) before the replay; the graph itself holds no RNG, so
+    a replay equals the eager ``loss_sampled`` step on the same draws."""
 
-    def __init__(self, model, optimizer, graph, dataset, batch_size, clip_grad=1.0, warmup=3, fused_loss=False):
+    def __init__(self, model, optimizer, graph, dataset, batch_size, clip_grad=1.0, warmup=3, fused_loss=False,
+                 negatives=None, n_pos=1, tries=4, generator=None):
+        if negatives is not None:
+            if fused_loss:
+                raise ValueError('negatives= and fused_loss=True are two different objectives: pass one of them')
+            if int(negatives) < 1 or int(n_pos) < 1 or int(tries) < 1:
+                raise ValueError('negatives, n_pos and tries must be positive')
         self.model, self.opt, self.graph_data, self.ds = model, optimizer, graph, dataset
         self.clip, self.B = float(clip_grad), int(batch_size)
         dev = graph.edge_index.device
@@ -29,7 +40,14 @@ class GraphedTrainStep(object):
         self.params = [p for p in model.parameters() if p.requires_grad]
         self.trip = torch.zeros((self.B, 3), dtype=torch.int64, device=dev)
         self.fused_loss = bool(fused_loss)
-        self.label = None if self.fused_loss else torch.zeros((self.B, dataset.num_entity), dtype=torch.float32, device=dev)
+        self.negatives = None if negatives is None else int(negatives)
+        self.n_pos, self.tries, self.generator = int(n_pos), int(tries), generator
+        self.pos_draws = self.neg_draws = None
+        if self.negatives is not None:
+            self.pos_draws = torch.zeros((self.B, self.n_pos), dtype=torch.int64, device=dev)
+            self.neg_draws = torch.zeros((self.B, self.negatives, self.tries), dtype=torch.int64, device=dev)
+        self.label = None if (self.fused_loss or self.negatives is not None) else \
+            torch.zeros((self.B, dataset.num_entity), dtype=torch.float32, device=dev)
         self.qid = torch.zeros((self.B,), dtype=torch.int64, device=dev)
         self._opt_clips = bool(getattr(optimizer, 'param_groups', None)) and \
             all(g.get('max_norm') for g in optimizer.param_groups)
@@ -54,6 +72,10 @@ class GraphedTrainStep(object):
             self._pin_done.record()
         else:
             self.qid.copy_(host, non_blocking=True)
+        if self.negatives is not None:               # fresh sampler inputs, drawn outside the graph (positives first)
+            self.pos_draws.random_(0, 1 << 32, generator=self.generator)
+            self.neg_draws.random_(0, 1 << 32, generator=self.generator)
+            return
         if self.fused_loss:                           # the graph reads the triples and the positives through qid
             return
         triples, ptr, idx = self.ds.device_csr(self.dev)
@@ -62,8 +84,11 @@ class GraphedTrainStep(object):
         _lib.call('kgc_label_build', p(self.qid), self.B, p(triples), p(ptr), p(idx), self.ds.num_entity, pos, add,
                   p(self.trip), p(self.label), _lib.stream())
 
-    def _body(self, trip, label, qid=None):
-        if qid is not None:
+    def _body(self, trip, label, qid=None, draws=None):
+        if self.negatives is not None:
+            loss = self.model.loss_sampled(qid, self.ds, self.graph_data, self.negatives, n_pos=self.n_pos, tries=self.tries,
+                                           draws=draws, generator=self.generator)
+        elif qid is not None:
             loss = self.model.loss_sparse(qid, self.ds, self.graph_data)
         else:
             pred = self.model(trip[:, 0], trip[:, 1], self.graph_data)
@@ -100,7 +125,7 @@ class GraphedTrainStep(object):
         with torch.cuda.stream(side):
             for _ in range(max(self._warmup, 1)):
                 self.opt.zero_grad(set_to_none=True)
-                self._body(self.trip, self.label, self.qid if self.fused_loss else None)
+                self._body(self.trip, self.label, *self._graph_inputs())
         torch.cuda.current_stream().wait_stream(side)
         torch.cuda.synchronize()
         for g, lr in zip(self.opt.param_groups, saved_lr):
@@ -123,12 +148,18 @@ class GraphedTrainStep(object):
         self.cuda_graph = torch.cuda.CUDAGraph()
         self.opt.zero_grad(set_to_none=True)
         with torch.cuda.graph(self.cuda_graph):
-            self.loss = self._body(self.trip, self.label, self.qid if self.fused_loss else None)
+            self.loss = self._body(self.trip, self.label, *self._graph_inputs())
+
+    def _graph_inputs(self):
+        """(qid, draws) arguments of the captured body: the static buffers the objective reads."""
+        if self.negatives is not None:
+            return self.qid, (self.pos_draws, self.neg_draws)
+        return (self.qid if self.fused_loss else None), None
 
     def __call__(self, qid):
         if len(qid) != self.B:                       # ragged last batch: the eager path (same arithmetic)
             self.opt.zero_grad(set_to_none=True)
-            if self.fused_loss:
+            if self.fused_loss or self.negatives is not None:
                 return self._body(None, None, torch.as_tensor(qid, dtype=torch.int64).to(self.dev))
             trip, label = self.ds.build_batch(qid, self.dev)
             return self._body(trip, label)
