@@ -545,6 +545,21 @@ int64_t kgc_sampled_bce_fwd_blocks(int64_t B);
 int kgc_sampled_bce_fwd(const float* x, int64_t B, int32_t D, const float* ent, int64_t n_ent, int64_t ld_ent,
                         const float* bias, const int32_t* cand, int32_t C, int32_t n_pos, float pos, float add,
                         float* g, float* d_x, int32_t* count, double* loss_partial, float* loss, void* stream);
+/* kgc_sampled_adv_fwd: the same pass with self-adversarial negative weights (Sun et al. 2019, RotatE) at temperature
+ * alpha = `temperature` (finite, >= 0; 0 gives uniform weights).  With P_b / Q_b the valid positive / negative slots of
+ * query b, z its logits, l ATen's BCE term and w[b, j] = softmax over j in Q_b of (alpha z[b, j]) (a constant, no
+ * gradient through it):
+ *   loss[0] = 1/2 (1/Q+) sum_{b: P_b non-empty} (1/|P_b|) sum_{P_b} l(z, pos) + 1/2 (1/Q-) sum_{b: Q_b non-empty} sum_{Q_b} w l(z, add)
+ * (a half whose count is 0 adds 0).  counts[0] = Q+, counts[1] = Q- (the numbers of queries with a valid positive /
+ * negative slot).  g [B, C] = the logit gradient for a unit upstream gradient: c * (p - y) / max((1 - p) p, 1e-12) *
+ * p (1 - p) with c = 1 / (2 Q+ |P_b|) on a positive slot, w / (2 Q-) on a negative one, 0 on empty slots.  d_x [B, D] =
+ * sum_c g[b, c] * ent[cand[b, c]] (up to rounding: the negative part is summed online and rescaled as the running max
+ * of alpha z rises).  loss_partial: 2 * kgc_sampled_bce_fwd_blocks(B) doubles.  Every candidate row is read once.  The
+ * table gradient is kgc_sampled_bce_bwd_table on this g.  Deterministic, no host synchronisation (graph-capturable). */
+int kgc_sampled_adv_fwd(const float* x, int64_t B, int32_t D, const float* ent, int64_t n_ent, int64_t ld_ent,
+                        const float* bias, const int32_t* cand, int32_t C, int32_t n_pos, float pos, float add,
+                        float temperature, float* g, float* d_x, int32_t* counts, double* loss_partial, float* loss,
+                        void* stream);
 size_t kgc_sampled_bce_bwd_table_workspace_bytes(int64_t n_slots, int64_t n_ent);
 int kgc_sampled_bce_bwd_table(const float* x, int64_t B, int32_t D, const int32_t* cand, int32_t C, const float* g,
                               const float* scale, int64_t n_ent, float* d_ent, int64_t ld_d, float* d_bias,

@@ -300,14 +300,17 @@ class MGCN(nn.Module):
         pos, add = dataset.label_values()
         return score_1n_bce(x, all_ent, self.conv2.bias, qid, ptr, idx, pos, add)
 
-    def loss_sampled(self, qid, dataset, data, k, n_pos=1, tries=4, draws=None, generator=None):
+    def loss_sampled(self, qid, dataset, data, k, n_pos=1, tries=4, draws=None, generator=None, adversarial_temperature=None):
         """Negative-sampled (1-vs-k) training loss for the training queries ``qid`` of ``dataset`` (a KBDataset): each query
         scores ``n_pos`` of its known objects (``dataset.positives``) and ``k`` entities that are not (``dataset.negatives``,
         ``tries`` draws per slot) - candidates [pos | neg] - through ``scoring.score_sampled_bce`` with the dataset's
         ``label_values()``.  Unlike ``loss_sparse`` the cost of the scoring does not grow with N, so the batch can be large.
         ``draws = (pos_draws [B, n_pos], neg_draws [B, k, tries])`` (uint32 values) makes the call a pure function of them;
-        otherwise they come from torch's generator (``generator`` or the global one), positives first."""
-        from .scoring import score_sampled_bce
+        otherwise they come from torch's generator (``generator`` or the global one), positives first.
+        ``adversarial_temperature=alpha`` weights each query's negatives by softmax(alpha * logit) (self-adversarial
+        negative sampling, see ``scoring.score_sampled_bce``); None: the plain mean over the valid slots."""
+        from .scoring import check_adversarial_temperature, score_sampled_bce
+        check_adversarial_temperature(adversarial_temperature)
         dev = self.entity_embedding.device
         triples, _, _ = dataset.device_csr(dev)
         qid = torch.as_tensor(qid, dtype=torch.int64).to(dev, non_blocking=True)
@@ -319,7 +322,8 @@ class MGCN(nn.Module):
         src_emb, all_ent = self._rows(all_ent, trip[:, 0])
         x = self.conv2.query(src_emb, torch.index_select(all_rel, 0, trip[:, 1]))
         pos, add = dataset.label_values()
-        return score_sampled_bce(x, all_ent, self.conv2.bias, cand, n_pos, pos, add)
+        return score_sampled_bce(x, all_ent, self.conv2.bias, cand, n_pos, pos, add,
+                                 adversarial_temperature=adversarial_temperature)
 
     def rank(self, src, rel, obj, filt_ptr, filt_idx, data, count_eq=False):
         """Filtered rank of obj among all entities for the queries (src, rel) without materialising the

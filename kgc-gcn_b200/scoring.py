@@ -8,6 +8,9 @@ Tie semantics (SURVEY.md section 7): rank = 1 + count_gt on the LOGIT (sigmoid i
 in fp32, which manufactures ties the reference then breaks arbitrarily); count_eq is reported so that
 callers can check reference_rank in [1 + gt, 1 + gt + eq].
 """
+import math
+import numbers
+
 import torch
 
 from . import _lib
@@ -144,12 +147,13 @@ def score_1n_bce(x, all_ent, bias, qid, ptr, idx, pos=1.0, add=0.0):
 
 
 class _ScoreSampledBCE(torch.autograd.Function):
-    """loss = mean BCE of sigmoid(<x[b], all_ent[cand[b, c]]> + bias[cand[b, c]]) over the valid slots (K6s).  The forward
-    makes one pass that yields the loss, the logit gradient g [B, C] and d_x for a unit upstream gradient; the backward
-    scales d_x and builds the dense table gradient by sorting the (entity, slot) pairs (no float atomics)."""
+    """loss = mean BCE of sigmoid(<x[b], all_ent[cand[b, c]]> + bias[cand[b, c]]) over the valid slots (K6s), or with a
+    ``temperature`` the self-adversarial loss of ``score_sampled_bce``.  The forward makes one pass that yields the loss, the
+    logit gradient g [B, C] and d_x for a unit upstream gradient; the backward (shared by both objectives) scales d_x and
+    builds the dense table gradient by sorting the (entity, slot) pairs (no float atomics)."""
 
     @staticmethod
-    def forward(ctx, x, all_ent, bias, cand, n_pos, pos, add):
+    def forward(ctx, x, all_ent, bias, cand, n_pos, pos, add, temperature=None):
         x = _lib.require_cuda(x.detach(), torch.float32, 'x')
         ent = all_ent.detach()                           # rows may sit in a wider table: the kernel takes a row pitch
         if ent.dtype != torch.float32:
@@ -163,11 +167,18 @@ class _ScoreSampledBCE(torch.autograd.Function):
         dev, p = x.device, _lib.ptr
         g = torch.empty((B, C), dtype=torch.float32, device=dev)
         d_x = torch.empty((B, D), dtype=torch.float32, device=dev)
-        count = torch.empty((1,), dtype=torch.int32, device=dev)
-        partial = torch.empty((int(_lib.lib().kgc_sampled_bce_fwd_blocks(B)),), dtype=torch.float64, device=dev)
-        loss = torch.empty((1,), dtype=torch.float32, device=dev)
-        _lib.call('kgc_sampled_bce_fwd', p(x), B, D, p(ent), N, ent.stride(0), p(bias_), p(cand), C, int(n_pos), float(pos),
-                  float(add), p(g), p(d_x), p(count), p(partial), p(loss), _lib.stream())
+        if temperature is None:
+            count = torch.empty((1,), dtype=torch.int32, device=dev)
+            partial = torch.empty((int(_lib.lib().kgc_sampled_bce_fwd_blocks(B)),), dtype=torch.float64, device=dev)
+            loss = torch.empty((1,), dtype=torch.float32, device=dev)
+            _lib.call('kgc_sampled_bce_fwd', p(x), B, D, p(ent), N, ent.stride(0), p(bias_), p(cand), C, int(n_pos), float(pos),
+                      float(add), p(g), p(d_x), p(count), p(partial), p(loss), _lib.stream())
+        else:
+            counts = torch.empty((2,), dtype=torch.int32, device=dev)
+            partial = torch.empty((2 * int(_lib.lib().kgc_sampled_bce_fwd_blocks(B)),), dtype=torch.float64, device=dev)
+            loss = torch.empty((1,), dtype=torch.float32, device=dev)
+            _lib.call('kgc_sampled_adv_fwd', p(x), B, D, p(ent), N, ent.stride(0), p(bias_), p(cand), C, int(n_pos), float(pos),
+                      float(add), float(temperature), p(g), p(d_x), p(counts), p(partial), p(loss), _lib.stream())
         ctx.save_for_backward(x, cand, g, d_x)
         ctx.n_ent = N
         return loss[0]
@@ -187,15 +198,34 @@ class _ScoreSampledBCE(torch.autograd.Function):
             _lib.call('kgc_sampled_bce_bwd_table', p(x), B, D, p(cand), C, p(g), p(scale), N, p(d_ent), D, p(d_bias), p(ws),
                       ws_bytes, _lib.stream())
         return (d_x * d_loss if ctx.needs_input_grad[0] else None, d_ent if ctx.needs_input_grad[1] else None,
-                d_bias if ctx.needs_input_grad[2] else None, None, None, None, None)
+                d_bias if ctx.needs_input_grad[2] else None, None, None, None, None, None)
 
 
-def score_sampled_bce(x, all_ent, bias, cand, n_pos, pos=1.0, add=0.0):
+def check_adversarial_temperature(temperature):
+    """``temperature`` as a float: None stays None; anything but a finite real number >= 0 is a ValueError."""
+    if temperature is None:
+        return None
+    if isinstance(temperature, bool) or not isinstance(temperature, numbers.Real) or not math.isfinite(temperature) \
+            or temperature < 0:
+        raise ValueError('adversarial_temperature must be a finite number >= 0 (or None), got {!r}'.format(temperature))
+    return float(temperature)
+
+
+def score_sampled_bce(x, all_ent, bias, cand, n_pos, pos=1.0, add=0.0, adversarial_temperature=None):
     """Negative-sampled (1-vs-k) BCE: query b of ``x`` [B, D] scores only its candidates ``cand`` [B, C] (int32 entity ids;
     the first ``n_pos`` columns are positives with label ``pos``, the rest negatives with label ``add``, e.g.
     ``KBDataset.label_values()``; -1 marks an empty slot, which adds neither loss nor gradient).  Returns the mean BCE of
     sigmoid(<x[b], all_ent[c]> + bias[c]) over the valid slots (0 when there are none), differentiable in ``x``,
-    ``all_ent`` and ``bias``.  The cost is B x C gathered rows, independent of N.  D % 4 == 0, D <= 256; deterministic and graph-capturable."""
+    ``all_ent`` and ``bias``.  The cost is B x C gathered rows, independent of N.  D % 4 == 0, D <= 256; deterministic and graph-capturable.
+
+    ``adversarial_temperature=alpha`` (a finite number >= 0) selects self-adversarial negative sampling (Sun et al. 2019,
+    RotatE): query b's valid negatives are weighted by w = softmax(alpha * logit) over them, a constant (no gradient flows
+    through the weights), and the loss is 1/2 (mean over the queries with a valid positive of the mean BCE of its valid
+    positives) + 1/2 (mean over the queries with a valid negative of the w-weighted BCE sum of its valid negatives); a half
+    without such queries adds 0.  alpha = 0 weights a query's negatives uniformly; a large alpha approaches the hardest
+    negative.  Same single pass, same row traffic and the same backward as the plain objective.  None (default): the plain
+    mean over the valid slots."""
+    temperature = check_adversarial_temperature(adversarial_temperature)
     if x.dim() != 2 or all_ent.dim() != 2 or bias.dim() != 1 or cand.dim() != 2:
         raise ValueError('score_sampled_bce takes x [B, D], all_ent [N, D], bias [N] and cand [B, C]')
     B, D = int(x.shape[0]), int(x.shape[1])
@@ -218,7 +248,7 @@ def score_sampled_bce(x, all_ent, bias, cand, n_pos, pos=1.0, add=0.0):
     if not torch.cuda.is_current_stream_capturing() and bool((cand >= N).any()):
         # (not checked while a CUDA graph is captured: the check reads back; the kernels treat such ids as empty slots)
         raise ValueError('cand holds entity ids >= N = {}'.format(N))
-    return _ScoreSampledBCE.apply(x, all_ent, bias, cand, int(n_pos), pos, add)
+    return _ScoreSampledBCE.apply(x, all_ent, bias, cand, int(n_pos), pos, add, temperature)
 
 
 def score_kpad(d):

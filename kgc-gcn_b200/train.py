@@ -22,10 +22,16 @@ class GraphedTrainStep(object):
     negatives per query, ``tries`` draws per negative): its cost does not grow with N, so ``batch_size`` can be in the
     thousands.  Each step draws the samplers' uint32 inputs from ``generator`` (or torch's global one) into static device
     buffers (``pos_draws`` [B, n_pos], ``neg_draws`` [B, k, tries]) before the replay; the graph itself holds no RNG, so
-    a replay equals the eager ``loss_sampled`` step on the same draws."""
+    a replay equals the eager ``loss_sampled`` step on the same draws.  ``adversarial_temperature=alpha`` (with
+    ``negatives=k`` only) trains with self-adversarial negative weights (``MGCN.loss_sampled``); the graph holds alpha as
+    a constant."""
 
     def __init__(self, model, optimizer, graph, dataset, batch_size, clip_grad=1.0, warmup=3, fused_loss=False,
-                 negatives=None, n_pos=1, tries=4, generator=None):
+                 negatives=None, n_pos=1, tries=4, generator=None, adversarial_temperature=None):
+        from .scoring import check_adversarial_temperature
+        adversarial_temperature = check_adversarial_temperature(adversarial_temperature)
+        if adversarial_temperature is not None and negatives is None:
+            raise ValueError('adversarial_temperature weights the sampled negatives: it needs negatives=k')
         if negatives is not None:
             if fused_loss:
                 raise ValueError('negatives= and fused_loss=True are two different objectives: pass one of them')
@@ -42,6 +48,7 @@ class GraphedTrainStep(object):
         self.fused_loss = bool(fused_loss)
         self.negatives = None if negatives is None else int(negatives)
         self.n_pos, self.tries, self.generator = int(n_pos), int(tries), generator
+        self.adversarial_temperature = adversarial_temperature
         self.pos_draws = self.neg_draws = None
         if self.negatives is not None:
             self.pos_draws = torch.zeros((self.B, self.n_pos), dtype=torch.int64, device=dev)
@@ -87,7 +94,8 @@ class GraphedTrainStep(object):
     def _body(self, trip, label, qid=None, draws=None):
         if self.negatives is not None:
             loss = self.model.loss_sampled(qid, self.ds, self.graph_data, self.negatives, n_pos=self.n_pos, tries=self.tries,
-                                           draws=draws, generator=self.generator)
+                                           draws=draws, generator=self.generator,
+                                           adversarial_temperature=self.adversarial_temperature)
         elif qid is not None:
             loss = self.model.loss_sparse(qid, self.ds, self.graph_data)
         else:
