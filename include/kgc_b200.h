@@ -163,6 +163,17 @@ int32_t kgc_keep_pitch(void);
 int kgc_tail_fwd(const float* res3, const uint8_t* mask_in, const uint8_t* mask_out, const int64_t* seed, float drop_p,
                  float keep_scale, const float* bias, int64_t n_rows, int32_t Dout, float* pre, double* partials,
                  uint8_t* keep, void* stream);
+/* kgc_tail_fwd with compacted in / out planes (the layer's sparse halves): slot_h (NULL: plane h is read densely from
+ * res3) = int32 [n_rows], the row of node row r in rows_h [n_c, Dout], or -1 for a row without edges, which contributes
+ * exactly 0.  res3's plane h is not read when slot_h is given.  Same arithmetic order, dropout draws and keep flags. */
+int kgc_tail_fwd_rows(const float* res3, const int32_t* slot_in, const float* rows_in, const int32_t* slot_out,
+                      const float* rows_out, const uint8_t* mask_in, const uint8_t* mask_out, const int64_t* seed,
+                      float drop_p, float keep_scale, const float* bias, int64_t n_rows, int32_t Dout, float* pre,
+                      double* partials, uint8_t* keep, void* stream);
+/* dst[dst_rows[j]] = src[src_rows[j]] for j < n, rows of D floats (D, ld_src, ld_dst multiples of 4); a NULL row list is
+ * the identity.  Gathers the occupied rows of a plane into a compact block and scatters them back. */
+int kgc_rows_copy(const float* src, int64_t ld_src, const int32_t* src_rows, float* dst, int64_t ld_dst,
+                  const int32_t* dst_rows, int64_t n, int32_t D, void* stream);
 int kgc_colsum_finalize(const double* partials, int64_t n_blocks, int32_t Dout, double* sums, void* stream);
 int kgc_colstats_from_sums(const double* sums, int64_t n_rows, int32_t Dout, float eps, int32_t training,
                            const float* running_mean, const float* running_var, float* stats, void* stream);
@@ -196,6 +207,13 @@ int kgc_tail_bwd_apply(const float* g_ent, const float* pre, const float* stats,
                        const double* sums, int32_t training, int64_t n_rows, int64_t n_rows_global, int32_t Dout,
                        float* d_out, const uint8_t* keep, float keep_scale, float* d_res2, const uint8_t* out_keep,
                        float out_scale, void* stream);
+/* kgc_tail_bwd_apply with the in / out planes given separately (both or neither); slot_h != NULL: plane h is compacted
+ * (see kgc_tail_fwd_rows) and receives only the rows that have edges, at their compact row. */
+int kgc_tail_bwd_apply_rows(const float* g_ent, const float* pre, const float* stats, const float* gamma, const float* beta,
+                            const double* sums, int32_t training, int64_t n_rows, int64_t n_rows_global, int32_t Dout,
+                            float* d_out, const uint8_t* keep, float keep_scale, float* d_res_in, const int32_t* slot_in,
+                            float* d_res_out, const int32_t* slot_out, const uint8_t* out_keep, float out_scale,
+                            void* stream);
 
 /* ---- K0: parameter-side work of one layer step, batched --------------------------------------------------
  * kgc_conv_prep (forward): relp = cat(rels, loop_rel) (model.py:86); all_rel = relp @ w_rel (model.py:107, all
@@ -281,6 +299,11 @@ int kgc_gemm_nt_splitk(const float* A, int64_t lda, const float* Bt, int64_t ldb
 int kgc_gemm_tn_tc_batch(int32_t n_prob, const float* const* A, int64_t lda, const float* const* B, int64_t ldb,
                          int64_t M, int32_t Ka, int32_t Nb, float* const* C, void* workspace, size_t workspace_bytes,
                          void* stream);
+/* The same with rows[i] <= M rows in problem i (HOST array; a compacted plane of the layer).  The row slabs are those
+ * of M rows: a problem of M rows gets the bits of kgc_gemm_tn_tc_batch; the others sum the slabs their rows fill. */
+int kgc_gemm_tn_tc_batch_rows(int32_t n_prob, const float* const* A, int64_t lda, const float* const* B, int64_t ldb,
+                              const int64_t* rows, int64_t M, int32_t Ka, int32_t Nb, float* const* C, void* workspace,
+                              size_t workspace_bytes, void* stream);
 /* The same with the keep flags applied to the B operand (the upstream plane) while it is split: see
  * kgc_gemm_nt_batch_masked. */
 int kgc_gemm_tn_tc_batch_masked(int32_t n_prob, const float* const* A, int64_t lda, const float* const* B, int64_t ldb,

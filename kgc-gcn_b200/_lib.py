@@ -34,6 +34,8 @@ SIGNATURES = {
     'kgc_dropout_mask': (ctypes.c_int, [_vp, _i32, _f32, _i64, _vp, _vp]),
     'kgc_keep_pitch': (_i32, []),
     'kgc_tail_fwd': (ctypes.c_int, [_vp, _vp, _vp, _vp, _f32, _f32, _vp, _i64, _i32, _vp, _vp, _vp, _vp]),
+    'kgc_tail_fwd_rows': (ctypes.c_int, [_vp, _vp, _vp, _vp, _vp, _vp, _vp, _vp, _f32, _f32, _vp, _i64, _i32, _vp, _vp, _vp, _vp]),
+    'kgc_rows_copy': (ctypes.c_int, [_vp, _i64, _vp, _vp, _i64, _vp, _i64, _i32, _vp]),
     'kgc_colsum_finalize': (ctypes.c_int, [_vp, _i64, _i32, _vp, _vp]),
     'kgc_colstats_from_sums': (ctypes.c_int, [_vp, _i64, _i32, _f32, _i32, _vp, _vp, _vp, _vp]),
     'kgc_colstats_finalize': (ctypes.c_int, [_vp, _i64, _i64, _i32, _f32, _f32, _vp, _vp, _vp, _vp, _vp, _vp]),
@@ -41,6 +43,8 @@ SIGNATURES = {
     'kgc_tail_apply': (ctypes.c_int, [_vp, _vp, _vp, _vp, _i64, _i32, _vp, _vp, _f32, _vp, _vp]),
     'kgc_tail_bwd_reduce': (ctypes.c_int, [_vp, _vp, _vp, _vp, _vp, _i64, _i32, _vp, _vp, _f32, _vp]),
     'kgc_tail_bwd_apply': (ctypes.c_int, [_vp, _vp, _vp, _vp, _vp, _vp, _i32, _i64, _i64, _i32, _vp, _vp, _f32, _vp, _vp, _f32, _vp]),
+    'kgc_tail_bwd_apply_rows': (ctypes.c_int, [_vp, _vp, _vp, _vp, _vp, _vp, _i32, _i64, _i64, _i32, _vp, _vp, _f32, _vp, _vp, _vp,
+                                               _vp, _vp, _f32, _vp]),
     'kgc_gemm_packed_b_bytes': (_sz, [_i32, _i32]),
     'kgc_gemm_pack_b': (ctypes.c_int, [_vp, _i64, _i64, _i32, _i32, _vp, _vp]),
     'kgc_gemm_nt': (ctypes.c_int, [_vp, _i64, _i32, _i64, _vp, _i32, _vp, _i64, _vp]),
@@ -56,6 +60,7 @@ SIGNATURES = {
     'kgc_gemm_tn_tc_workspace_bytes': (_sz, [_i64, _i32, _i32]),
     'kgc_gemm_tn_tc': (ctypes.c_int, [_vp, _i64, _vp, _i64, _i64, _i32, _i32, _vp, _vp, _sz, _vp]),
     'kgc_gemm_tn_tc_batch': (ctypes.c_int, [_i32, _vp, _i64, _vp, _i64, _i64, _i32, _i32, _vp, _vp, _sz, _vp]),
+    'kgc_gemm_tn_tc_batch_rows': (ctypes.c_int, [_i32, _vp, _i64, _vp, _i64, _vp, _i64, _i32, _i32, _vp, _vp, _sz, _vp]),
     'kgc_gemm_tn': (ctypes.c_int, [_vp, _i64, _vp, _i64, _i64, _i32, _i32, _vp, _vp, _sz, _vp]),
     'kgc_label_build': (ctypes.c_int, [_vp, _i64, _vp, _vp, _vp, _i64, _f32, _f32, _vp, _vp, _vp]),
     'kgc_neg_sample': (ctypes.c_int, [_vp, _i64, _vp, _vp, _i64, _vp, _i32, _i32, _vp, _vp]),
@@ -130,7 +135,7 @@ def lib():
 
 
 LAUNCHES = 0     # kernels launched through the C ABI since import (bench.py reports it as gpu_launches)
-_KERNELS_PER_CALL = {'kgc_csr_build': 16, 'kgc_label_mask_build': 2, 'kgc_bce_1n_bwd_logit': 2, 'kgc_bce_1n_bwd_logit_t': 2, 'kgc_label_mask_t_build': 2, 'kgc_score_pairs': 3, 'kgc_rank_finalize': 2, 'kgc_score_topk': 2, 'kgc_topk_dense': 2, 'kgc_sampled_bce_fwd': 4, 'kgc_sampled_adv_fwd': 4, 'kgc_sampled_bce_bwd_table': 7, 'kgc_gemm_tn': 2, 'kgc_gemm_tn_tc': 2, 'kgc_gemm_tn_tc_batch': 2, 'kgc_gemm_tn_tc_batch_masked': 2}   # (kgc_p2p_allreduce: 1 or 3)
+_KERNELS_PER_CALL = {'kgc_csr_build': 16, 'kgc_label_mask_build': 2, 'kgc_bce_1n_bwd_logit': 2, 'kgc_bce_1n_bwd_logit_t': 2, 'kgc_label_mask_t_build': 2, 'kgc_score_pairs': 3, 'kgc_rank_finalize': 2, 'kgc_score_topk': 2, 'kgc_topk_dense': 2, 'kgc_sampled_bce_fwd': 4, 'kgc_sampled_adv_fwd': 4, 'kgc_sampled_bce_bwd_table': 7, 'kgc_gemm_tn': 2, 'kgc_gemm_tn_tc': 2, 'kgc_gemm_tn_tc_batch': 2, 'kgc_gemm_tn_tc_batch_rows': 2, 'kgc_gemm_tn_tc_batch_masked': 2}   # (kgc_p2p_allreduce: 1 or 3)
 
 
 def call(name, *args):

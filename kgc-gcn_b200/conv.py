@@ -110,6 +110,41 @@ def gemm_tn_batch(a_list, b_list, out_list, plan=None, keep=None, keep_scale=1.0
     return out_list
 
 
+def gemm_tn_batch_rows(a_list, b_list, out_list, rows, plan=None):
+    """gemm_tn_batch with rows[i] <= M leading rows of problem i (M = the operands' row count): one launch whose problems of
+    M rows get exactly the bits of gemm_tn_batch; a shorter problem (a compacted plane) sums only the slabs its rows fill."""
+    import ctypes
+    n = len(a_list)
+    M = max(a.shape[0] for a in a_list)
+    Ka, Nb = a_list[0].shape[1], b_list[0].shape[1]
+    lda, ldb = a_list[0].stride(0), b_list[0].stride(0)
+    ok = all(a.shape[1] == Ka and b.shape[1] == Nb and a.stride(1) == 1 and b.stride(1) == 1 and a.stride(0) == lda
+             and b.stride(0) == ldb and a.shape[0] >= r and b.shape[0] >= r and o.is_contiguous()
+             for a, b, o, r in zip(a_list, b_list, out_list, rows))
+    if not ok or max(rows) != M:
+        raise ValueError('gemm_tn_batch_rows needs operands of identical widths and strides and rows <= their heights')
+    if Ka > 128 or Nb > 224:                            # wide shapes: one gemm_tn per problem
+        for a, b, o, r in zip(a_list, b_list, out_list, rows):
+            if r:
+                gemm_tn(a[:r], b[:r], o, plan)
+            else:
+                o.zero_()
+        return out_list
+    nbytes = int(_lib.lib().kgc_gemm_tn_tc_workspace_bytes(M, Ka, Nb))
+    ws = plan.scratch('kgc_gemm_tn_tc_ws', (nbytes // 4,)) if plan is not None else \
+        torch.empty((nbytes // 4,), dtype=torch.float32, device=a_list[0].device)
+    arr = lambda ts: (ctypes.c_void_p * n)(*[t.data_ptr() for t in ts])       # noqa: E731
+    _lib.call('kgc_gemm_tn_tc_batch_rows', n, arr(a_list), lda, arr(b_list), ldb, (ctypes.c_int64 * n)(*rows), M, Ka, Nb,
+              arr(out_list), _lib.ptr(ws), nbytes, _lib.stream())
+    return out_list
+
+
+def rows_copy(src, src_rows, dst, dst_rows, n):
+    """dst[dst_rows[j]] = src[src_rows[j]] for j < n (row lists int32 or None = the identity; one launch, none for n = 0)."""
+    _lib.call('kgc_rows_copy', _lib.ptr(src), src.stride(0), _lib.ptr(src_rows), _lib.ptr(dst), dst.stride(0), _lib.ptr(dst_rows),
+              int(n), src.shape[1], _lib.stream())
+
+
 def _pack_b(b_kn):
     K, N = b_kn.shape
     nbytes = int(_lib.lib().kgc_gemm_packed_b_bytes(N, K))
@@ -393,11 +428,17 @@ class _ConvFn(torch.autograd.Function):
         if max(x_full.shape[0], 3 * n_dst, ee.shape[0]) * (D // 4) >= 1 << 32:      # K2/K3 use 32-bit float4 indices
             raise ValueError('kgc_gcn_b200: node / edge tables of 2^32 float4 elements or more are not supported')
         agg = torch.empty((2, n_dst, D), dtype=torch.float32, device=x.device)
+        agg_c, res_c = [None, None], [None, None]                   # compacted halves: [n_c, D] rows and their transforms
+        # one GPU: a half whose rows are mostly without edges (plan.compact_halves) runs its dense transform, its share of the
+        # tail and its weight gradient on its occupied rows only (plan.rows / plan.slot); its other rows are never read, so
+        # the aggregation does not zero-fill them
+        comp = plan.compact_halves(4 * Dout) if coll is None else (False, False)
 
         def level0(sp, out_final, carry):
             _lib.call('kgc_agg_fwd', p(x_full), p(rels_c), T - 1, p(ee), p(plan.rec_dst), p(sp.rowflags), p(sp.chunks), sp.n_rec,
                       p(out_final), p(carry), D, st())
-        plan.run_reduction(plan.fwd, level0, agg, D, tag='f')
+        plan.run_reduction(plan.fwd, level0, agg, D, tag='f',
+                           skip_prefill=[(h * n_dst, (h + 1) * n_dst) for h in (0, 1) if comp[h]])
         if gather is None:
             main.wait_stream(side)                                  # K0's operand packs are needed from here on
 
@@ -406,8 +447,22 @@ class _ConvFn(torch.autograd.Function):
         if gather is not None:
             coll.sum_hub_rows(agg, n_loc)
             gemm_nt_batch([agg[0, :Nl], agg[1, :Nl]], [packed_f[0], packed_f[1]], [res3[0], res3[1]])
-        else:                                                       # the three transforms of the step in one launch
+        elif not any(comp):                                         # the three transforms of the step in one launch
             gemm_nt_batch([agg[0], agg[1], x], [packed_f[0], packed_f[1], packed_f[2]], [res3[0], res3[1], res3[2]])
+        else:
+            # a compacted half: its occupied rows gathered into [n_c, D] and transformed on their own (a launch of n_c rows;
+            # sharing the batched launch would leave its CTAs idle), the dense planes in one launch
+            dense = [h for h in (0, 1) if not comp[h]]
+            for h in (0, 1):
+                if comp[h]:
+                    n_c = plan.n_c[h]
+                    agg_c[h] = torch.empty((max(n_c, 1), D), dtype=torch.float32, device=x.device)
+                    res_c[h] = plan.scratch('res_c%d' % h, (max(n_c, 1), Dout))
+                    if n_c:
+                        rows_copy(agg[h], plan.rows[h], agg_c[h], None, n_c)
+                        gemm_nt(agg_c[h][:n_c], None, res_c[h][:n_c], packed=packed_f[h])
+            gemm_nt_batch([agg[h] for h in dense] + [x], [packed_f[h] for h in dense] + [packed_f[2]],
+                          [res3[h] for h in dense] + [res3[2]])
 
         nb = int(_lib.lib().kgc_tail_num_blocks(Nl))
         partials = plan.scratch('colpart', (nb, 2, Dout), torch.float64)
@@ -419,8 +474,13 @@ class _ConvFn(torch.autograd.Function):
         # ONE upstream plane (no masked planes are written, nothing is regenerated)
         dropping = (mask_in is not None or seed is not None) and drop_p > 0.0
         keep = torch.empty((Nl, int(_lib.lib().kgc_keep_pitch())), dtype=torch.uint8, device=x.device) if dropping else None
-        _lib.call('kgc_tail_fwd', p(res3), p(mask_in), p(mask_out), p(seed), float(drop_p), float(keep_scale), p(bias),
-                  Nl, Dout, p(pre), p(partials), p(keep), st())
+        if any(comp):
+            _lib.call('kgc_tail_fwd_rows', p(res3), p(plan.slot[0]) if comp[0] else None, p(res_c[0]),
+                      p(plan.slot[1]) if comp[1] else None, p(res_c[1]), p(mask_in), p(mask_out), p(seed), float(drop_p),
+                      float(keep_scale), p(bias), Nl, Dout, p(pre), p(partials), p(keep), st())
+        else:
+            _lib.call('kgc_tail_fwd', p(res3), p(mask_in), p(mask_out), p(seed), float(drop_p), float(keep_scale), p(bias),
+                      Nl, Dout, p(pre), p(partials), p(keep), st())
         if training and coll is None:
             # one GPU: column sums -> batch statistics -> nn.BatchNorm1d's running-statistics bookkeeping in ONE launch
             # (bn_track = (momentum, num_batches_tracked) when the module tracks running statistics)
@@ -445,16 +505,17 @@ class _ConvFn(torch.autograd.Function):
         ctx.plan, ctx.training, ctx.keep_scale, ctx.has_bias, ctx.coll = plan, bool(training), float(keep_scale), \
             bias is not None, coll
         ctx.drop_p = float(drop_p)
+        ctx.comp = comp
         ctx.save_for_backward(x, x_full, relp, ee, w_in, w_out, w_loop, w_rel, loop_rel, loop_edge, gamma, beta, agg, pre,
-                              all_ent, stats, keep, packed_b, out_keep)
+                              all_ent, stats, keep, packed_b, out_keep, agg_c[0], agg_c[1])
         ctx.mark_non_differentiable(stats)
         return all_ent, all_rel, stats
 
     @staticmethod
     def backward(ctx, g_ent, g_rel, _g_stats):
         (x, x_full, relp, ee, w_in, w_out, w_loop, w_rel, loop_rel, loop_edge, gamma, beta, agg, pre, all_ent, stats, keep,
-         packed_b, out_keep) = ctx.saved_tensors
-        plan, coll = ctx.plan, ctx.coll
+         packed_b, out_keep, agg_c0, agg_c1) = ctx.saved_tensors
+        plan, coll, comp = ctx.plan, ctx.coll, ctx.comp
         Nl, D = x.shape
         n_global = Nl if coll is None else coll.n_global      # BatchNorm rows (real nodes of all ranks)
         n_hub = 0 if coll is None else coll.n_hub
@@ -487,12 +548,16 @@ class _ConvFn(torch.autograd.Function):
         # Wikidata5M shape 49.7 vs 50.5 ms, WN18RR 0.387 vs 0.400 ms - the operand splitters are the busier side of K4b /
         # K4c (+1.9 / +1.0 ms against -2.5 ms of tail traffic) - but FB15k-237 0.462 vs 0.411 ms: when the planes stay in
         # L2 the extra writes are what costs.  Default by size; KGC_TAIL_PLANES=1|3 overrides.
+        # A compacted half always takes the three-plane form: its upstream rows are written compact, [n_c, Dout].
         mode = os.environ.get('KGC_TAIL_PLANES', '')
         three = (3 * Nl * Dout * 4 > (48 << 20)) if mode not in ('1', '3') else mode == '3'
-        d_res2 = plan.scratch('d_res2', (2, Nl, Dout)) if three else None
-        _lib.call('kgc_tail_bwd_apply', p(g_ent), p(pre), p(stats), p(gamma), p(beta), p(sums), int(ctx.training), Nl,
-                  n_global, Dout, p(d_out), p(keep), ctx.keep_scale, p(d_res2), p(out_keep), ctx.out_scale, st())
-        ups = [d_res2[0], d_res2[1], d_out] if three else [d_out, d_out, d_out]
+        three = three or any(comp)
+        d_res = [(plan.scratch('d_res_c%d' % h, (max(plan.n_c[h], 1), Dout)) if comp[h] else plan.scratch('d_res2_%d' % h, (Nl, Dout)))
+                 if three else None for h in (0, 1)]
+        _lib.call('kgc_tail_bwd_apply_rows', p(g_ent), p(pre), p(stats), p(gamma), p(beta), p(sums), int(ctx.training), Nl,
+                  n_global, Dout, p(d_out), p(keep), ctx.keep_scale, p(d_res[0]), p(plan.slot[0]) if comp[0] else None,
+                  p(d_res[1]), p(plan.slot[1]) if comp[1] else None, p(out_keep), ctx.out_scale, st())
+        ups = [d_res[0], d_res[1], d_out] if three else [d_out, d_out, d_out]
         gkeep = None if three else keep
         d_beta, d_gamma = sums32[0], sums32[1]
 
@@ -506,16 +571,34 @@ class _ConvFn(torch.autograd.Function):
         main, side = torch.cuda.current_stream(), plan.side_stream()
         side.wait_stream(main)
         with torch.cuda.stream(side):
-            gemm_tn_batch([agg[0, :Nl], agg[1, :Nl], x], ups, [d_w_in, d_w_out, m_loop], plan,
-                          keep=gkeep, keep_scale=ctx.keep_scale)                                         # [D, Dout] each
+            if any(comp):                                       # a compacted half sums its n_c rows
+                agg_c = (agg_c0, agg_c1)
+                gemm_tn_batch_rows([agg_c[h] if comp[h] else agg[h, :Nl] for h in (0, 1)] + [x], ups,
+                                   [d_w_in, d_w_out, m_loop], [plan.n_c[h] if comp[h] else Nl for h in (0, 1)] + [Nl], plan)
+            else:
+                gemm_tn_batch([agg[0, :Nl], agg[1, :Nl], x], ups, [d_w_in, d_w_out, m_loop], plan,
+                              keep=gkeep, keep_scale=ctx.keep_scale)                                     # [D, Dout] each
             if ctx.has_bias:
                 torch.sum(d_out, 0, out=flat[3 * D * Dout + T * D:])
 
         # ---- d(agg) = d_res @ W^T on the tensor cores (3xTF32), main stream
         hybrid = coll is not None and coll.p2p is not None and coll.p2p.hybrid
         g3 = coll.p2p.g3_planes() if hybrid else plan.scratch('g3', (3, Nb, D))
-        gemm_nt_batch(ups, [packed_b[0], packed_b[1], packed_b[2]],
-                      [g3[0, :Nl], g3[1, :Nl], g3[2, :Nl]], keep=gkeep, keep_scale=ctx.keep_scale)
+        if not any(comp):
+            gemm_nt_batch(ups, [packed_b[0], packed_b[1], packed_b[2]],
+                          [g3[0, :Nl], g3[1, :Nl], g3[2, :Nl]], keep=gkeep, keep_scale=ctx.keep_scale)
+        else:
+            # a compacted half: d(agg) of its occupied rows, scattered into their rows of g3 (the only rows of that plane the
+            # aggregation backward reads: its edges' destinations)
+            dense = [h for h in (0, 1) if not comp[h]]
+            for h in (0, 1):
+                n_c = plan.n_c[h]
+                if comp[h] and n_c:
+                    g3_c = plan.scratch('g3_c%d' % h, (n_c, D))
+                    gemm_nt(d_res[h][:n_c], None, g3_c, packed=packed_b[h])
+                    rows_copy(g3_c, None, g3[h], plan.rows[h], n_c)
+            gemm_nt_batch([ups[h] for h in dense] + [d_out], [packed_b[h] for h in dense] + [packed_b[2]],
+                          [g3[h, :Nl] for h in dense] + [g3[2, :Nl]])
         if n_hub:
             coll.spread_hub_rows(g3, 2, n_loc)                       # the virtual rows see their hub's upstream gradient
         if hybrid:

@@ -786,6 +786,8 @@ struct GemmTnMaps {                              // per problem of a batched lau
 
 struct GemmTnParams {
   int64_t M;
+  int64_t m_prob[kMaxBatch];                     // rows of each problem (<= M; fewer for a compacted plane): slabs past them
+                                                 // have no CTA work and no partial
   int32_t n_prob, n_slabs;                       // CTA = (problem, row slab); partial[problem][slab][Ka][Nb]
   int32_t Ka, Nb, ga, gb, n_pad;                 // ga / gb = 32-column groups of A / B; n_pad = MMA N (multiple of 16)
   int32_t ga_full, gb_full;                      // groups that lie completely inside the operand (fetched by one 3-D TMA)
@@ -814,6 +816,10 @@ __device__ __forceinline__ uint64_t sw128_mn_desc(uint32_t smem_addr) {
 __global__ void __launch_bounds__(kThreadsG, 1)
 gemm_tn_tc_kernel(const __grid_constant__ GemmTnMaps maps, const GemmTnParams P) {
   extern __shared__ uint8_t smem_raw[];
+  const int prob = blockIdx.x % P.n_prob, slab = blockIdx.x / P.n_prob;
+  const int64_t Mp = prob == 0 ? P.m_prob[0] : (prob == 1 ? P.m_prob[1] : P.m_prob[2]);
+  const int64_t m0 = slab * P.rows_per_cta;
+  if (m0 >= Mp && Mp < P.M) return;                                // a slab past a shorter problem's rows: not reduced
   if (P.dbg != nullptr && threadIdx.x == 0) {                      // debug aid: launch-to-exit envelope over all CTAs (ns)
     long long g;
     asm volatile("mov.u64 %0, %globaltimer;" : "=l"(g));
@@ -856,14 +862,12 @@ gemm_tn_tc_kernel(const __grid_constant__ GemmTnMaps maps, const GemmTnParams P)
   const bool dbg_on = P.dbg != nullptr && blockIdx.x == 0;
   int dbg_n = 0;
 
-  const int prob = blockIdx.x % P.n_prob, slab = blockIdx.x / P.n_prob;
   const CUtensorMap* map_a = &maps.a[prob];
   const CUtensorMap* map_b = &maps.b[prob];
   const CUtensorMap* map_a3 = &maps.a3[prob];
   const CUtensorMap* map_b3 = &maps.b3[prob];
   const CUtensorMap* map_p = &maps.p[prob];
-  const int64_t m0 = slab * P.rows_per_cta;
-  const int64_t m1 = m0 + P.rows_per_cta < P.M ? m0 + P.rows_per_cta : P.M;
+  const int64_t m1 = m0 + P.rows_per_cta < Mp ? m0 + P.rows_per_cta : Mp;
   const int n_kb = m1 > m0 ? (int)((m1 - m0 + kTnRows - 1) / kTnRows) : 0;
 
   if (warp == 0) {
@@ -1078,22 +1082,26 @@ gemm_tn_tc_kernel(const __grid_constant__ GemmTnMaps maps, const GemmTnParams P)
 
 // C[e] = sum over the CTA partials in a FIXED order: 8 part-lanes per element, then their sums in lane order; the
 // partials (up to thousands at 4.6 M rows) are added in double precision and rounded once
-struct TnOut { float* c[kMaxBatch]; };
+struct TnOut {
+  float* c[kMaxBatch];
+  int32_t n_parts[kMaxBatch];                    // partials of each problem (its slabs; the stride is n_parts of the launch)
+};
 __global__ void __launch_bounds__(256)
 gemm_tn_partials_reduce(const float* __restrict__ partial_all, int n_parts, int n_elem, const TnOut outs) {
   __shared__ double sm[8][33];
   const float* partial = partial_all + (int64_t)blockIdx.y * n_parts * n_elem;      // blockIdx.y = problem of the batch
   float* C = blockIdx.y == 0 ? outs.c[0] : (blockIdx.y == 1 ? outs.c[1] : outs.c[2]);   // no runtime index into a parameter
+  const int n_parts_p = blockIdx.y == 0 ? outs.n_parts[0] : (blockIdx.y == 1 ? outs.n_parts[1] : outs.n_parts[2]);
   const int e = blockIdx.x * 32 + threadIdx.x;
   double s = 0.0;
   if (e < n_elem) {
     int g = threadIdx.y;
-    for (; g + 24 < n_parts; g += 32) {                      // four independent loads in flight, added in part order
+    for (; g + 24 < n_parts_p; g += 32) {                      // four independent loads in flight, added in part order
       const float v0 = partial[(int64_t)g * n_elem + e], v1 = partial[(int64_t)(g + 8) * n_elem + e];
       const float v2 = partial[(int64_t)(g + 16) * n_elem + e], v3 = partial[(int64_t)(g + 24) * n_elem + e];
       s += (double)v0; s += (double)v1; s += (double)v2; s += (double)v3;
     }
-    for (; g < n_parts; g += 8) s += (double)partial[(int64_t)g * n_elem + e];
+    for (; g < n_parts_p; g += 8) s += (double)partial[(int64_t)g * n_elem + e];
   }
   sm[threadIdx.y][threadIdx.x] = s;
   __syncthreads();
@@ -1321,9 +1329,12 @@ extern "C" size_t kgc_gemm_tn_tc_workspace_bytes(int64_t M, int32_t Ka, int32_t 
 }
 
 // C[Ka, Nb] = A[M, Ka]^T @ B[M, Nb] on the tensor cores (3xTF32).  Ka <= 128, Nb <= 224, multiples of 4.
+// m_prob (optional): rows of each problem, <= M.  The row slabs are those of M rows for every problem, so a problem of M rows
+// gets the same partials, in the same order, as in a launch where every problem has M rows.
 static int launch_gemm_tn_tc(int n_prob, const float* const* A, int64_t lda, const float* const* B, int64_t ldb, int64_t M,
                              int32_t Ka, int32_t Nb, float* const* C, void* workspace, size_t workspace_bytes, int32_t kmajor,
-                             void* stream, const uint8_t* keep = nullptr, int32_t keep_pitch = 0, float keep_scale = 1.f) {
+                             void* stream, const uint8_t* keep = nullptr, int32_t keep_pitch = 0, float keep_scale = 1.f,
+                             const int64_t* m_prob = nullptr) {
   KGC_REQUIRE(n_prob >= 1 && n_prob <= kMaxBatch, "1..3 problems per launch");
   KGC_REQUIRE(M > 0 && Ka > 0 && Nb > 0 && Ka <= 128 && Nb <= 224, "supported: Ka <= 128, Nb <= 224");
   KGC_REQUIRE(Nb % 4 == 0 && lda % 4 == 0 && ldb % 4 == 0 && (kmajor || Ka % 4 == 0), "dimensions and leading dimensions must be multiples of 4");
@@ -1338,6 +1349,13 @@ static int launch_gemm_tn_tc(int n_prob, const float* const* A, int64_t lda, con
   P.rows_per_cta = ceil_div(ceil_div(M, slabs), kTnRows) * kTnRows;     // slabs start on K-block boundaries
   slabs = (int)ceil_div(M, P.rows_per_cta);
   P.n_slabs = slabs;
+  TnOut outs;
+  for (int i = 0; i < kMaxBatch; ++i) {
+    const int64_t m = (m_prob != nullptr && i < n_prob) ? m_prob[i] : M;
+    KGC_REQUIRE(m >= 0 && m <= M, "rows of a problem must lie in [0, M]");
+    P.m_prob[i] = m;
+    outs.n_parts[i] = (int)ceil_div(m, P.rows_per_cta);
+  }
   P.partial = static_cast<float*>(workspace);
   P.dbg = g_gemm_dbg;
   KGC_REQUIRE(keep == nullptr || (!kmajor && keep_pitch >= 8 * P.gb), "keep flags: one byte per 4 columns of B, rows that cover the padded width");
@@ -1345,18 +1363,19 @@ static int launch_gemm_tn_tc(int n_prob, const float* const* A, int64_t lda, con
   P.ga_full = kmajor ? 0 : Ka / 32;
   P.gb_full = kmajor ? 0 : Nb / 32;
   GemmTnMaps maps;
-  TnOut outs;
   for (int i = 0; i < kMaxBatch; ++i) {
     const int j = i < n_prob ? i : 0;          // unused slots repeat problem 0 (never dereferenced)
     outs.c[i] = C[j];
+    // a problem without rows still gets valid maps (never read): one row of its operands
+    const int64_t Mi = P.m_prob[j] > 0 ? P.m_prob[j] : 1;
     if (kmajor) {      // A[Ka, M], Bt[Nb, M] with the contraction index M contiguous
-      if (make_map_f32(&maps.a[i], A[j], Ka, M, lda, kBM) || make_map_f32(&maps.b[i], B[j], Nb, M, ldb, P.n_pad)) return 1;
-    } else if (make_map_f32_mn(&maps.a[i], A[j], M, Ka, lda) || make_map_f32_mn(&maps.b[i], B[j], M, Nb, ldb)) {
+      if (make_map_f32(&maps.a[i], A[j], Ka, Mi, lda, kBM) || make_map_f32(&maps.b[i], B[j], Nb, Mi, ldb, P.n_pad)) return 1;
+    } else if (make_map_f32_mn(&maps.a[i], A[j], Mi, Ka, lda) || make_map_f32_mn(&maps.b[i], B[j], Mi, Nb, ldb)) {
       return 1;
     }
     maps.a3[i] = maps.a[i]; maps.b3[i] = maps.b[i];                      // placeholders when an operand has no complete group
-    if (P.ga_full > 0 && make_map_f32_mn_groups(&maps.a3[i], A[j], M, P.ga_full, lda)) return 1;
-    if (P.gb_full > 0 && make_map_f32_mn_groups(&maps.b3[i], B[j], M, P.gb_full, ldb)) return 1;
+    if (P.ga_full > 0 && make_map_f32_mn_groups(&maps.a3[i], A[j], Mi, P.ga_full, lda)) return 1;
+    if (P.gb_full > 0 && make_map_f32_mn_groups(&maps.b3[i], B[j], Mi, P.gb_full, ldb)) return 1;
     if (make_map_f32_parts(&maps.p[i], P.partial + (int64_t)j * slabs * Ka * Nb, slabs, Ka, Nb)) return 1;
   }
   const size_t stage = (size_t)(P.ga + P.gb) * kTnBox;
@@ -1382,6 +1401,14 @@ extern "C" int kgc_gemm_tn_tc_batch(int32_t n_prob, const float* const* A, int64
                                     size_t workspace_bytes, void* stream) {
   KGC_REQUIRE(A && B && C, "null pointer table");
   return launch_gemm_tn_tc(n_prob, A, lda, B, ldb, M, Ka, Nb, C, workspace, workspace_bytes, 0, stream);
+}
+
+// the same with rows[i] <= M rows for problem i (the layer's compacted planes): problems of M rows keep their bits
+extern "C" int kgc_gemm_tn_tc_batch_rows(int32_t n_prob, const float* const* A, int64_t lda, const float* const* B, int64_t ldb,
+                                         const int64_t* rows, int64_t M, int32_t Ka, int32_t Nb, float* const* C, void* workspace,
+                                         size_t workspace_bytes, void* stream) {
+  KGC_REQUIRE(A && B && C && rows, "null pointer table");
+  return launch_gemm_tn_tc(n_prob, A, lda, B, ldb, M, Ka, Nb, C, workspace, workspace_bytes, 0, stream, nullptr, 0, 1.f, rows);
 }
 
 extern "C" int kgc_gemm_tn_tc_batch_masked(int32_t n_prob, const float* const* A, int64_t lda, const float* const* B, int64_t ldb,

@@ -73,8 +73,21 @@ __device__ __forceinline__ void block_store_partials(double4 a, double4 b, int r
   }
 }
 
+// Compacted in / out planes (the layer's sparse halves): plane h holds only the rows with at least one edge, slot[h][r] =
+// the compact row of node row r or -1 (an empty row, whose value is exactly 0).  slot[h] == NULL: plane h is dense.
+struct PlaneRows {
+  const int32_t* slot[2];
+  const float4* rows[2];
+};
+__device__ __forceinline__ float4 plane_value(const float4* __restrict__ dense, const PlaneRows& pr, int h, int64_t r,
+                                              int64_t i, int c, int Do4) {
+  if (pr.slot[h] == nullptr) return __ldg(dense + i);
+  const int32_t s = __ldg(pr.slot[h] + r);
+  return s >= 0 ? __ldg(pr.rows[h] + (int64_t)s * Do4 + c) : make_float4(0.f, 0.f, 0.f, 0.f);
+}
+
 __global__ void __launch_bounds__(kThreads)
-tail_fwd_kernel(const float4* __restrict__ res3, const DropCfg drop, const float4* __restrict__ bias,
+tail_fwd_kernel(const float4* __restrict__ res3, const PlaneRows pr, const DropCfg drop, const float4* __restrict__ bias,
                 int64_t n_rows, int Do4, float4* __restrict__ pre, double* __restrict__ partials,
                 uint8_t* __restrict__ keep) {
   extern __shared__ double4 sm[];
@@ -87,7 +100,7 @@ tail_fwd_kernel(const float4* __restrict__ res3, const DropCfg drop, const float
     const float4 bv = bias ? __ldg(bias + c) : make_float4(0.f, 0.f, 0.f, 0.f);
     for (int64_t r = s.row_beg + rl; r < s.row_end; r += RL) {
       const int64_t i = r * Do4 + c;
-      float4 a = __ldg(res3 + i), b = __ldg(res3 + plane + i);
+      float4 a = plane_value(res3, pr, 0, r, i, c, Do4), b = plane_value(res3 + plane, pr, 1, r, i, c, Do4);
       const float4 l = __ldg(res3 + 2 * plane + i);
       uint32_t kb = 0;
       { const float4 m = drop_scale4(drop, 0, i); a.x *= m.x; a.y *= m.y; a.z *= m.z; a.w *= m.w; kb |= nibble(m); }
@@ -283,8 +296,9 @@ __global__ void __launch_bounds__(kThreads)
 tail_bwd_apply_kernel(const float4* __restrict__ g_ent, const float4* __restrict__ pre, const float4* __restrict__ stats,
                       const float4* __restrict__ gamma, const float4* __restrict__ beta, const double* __restrict__ sums,
                       int training, int64_t n_rows, int64_t n_rows_global, int Do4, float4* __restrict__ d_out,
-                      const uint8_t* __restrict__ keep, float keep_scale, float4* __restrict__ d_res2,
-                      const uint8_t* __restrict__ out_keep, float out_scale) {
+                      const uint8_t* __restrict__ keep, float keep_scale, float4* __restrict__ d_res_in,
+                      float4* __restrict__ d_res_out, const int32_t* __restrict__ slot_in,
+                      const int32_t* __restrict__ slot_out, const uint8_t* __restrict__ out_keep, float out_scale) {
   const int64_t n4 = n_rows * (int64_t)Do4;
   const int64_t i = blockIdx.x * (int64_t)kThreads + threadIdx.x;
   if (i >= n4) return;
@@ -316,16 +330,36 @@ tail_bwd_apply_kernel(const float4* __restrict__ g_ent, const float4* __restrict
   // their keep flags x 1 / (1 - p), applied by the GEMM kernels while they split the operand (tail_fwd's packed flags)
   const float4 third = make_float4(dp.x / 3.0f, dp.y / 3.0f, dp.z / 3.0f, dp.w / 3.0f);
   d_out[i] = third;
-  if (d_res2 != nullptr) {
+  if (d_res_in != nullptr) {
     // three-plane form: the dropped in / out planes are written here (tail_fwd's keep flags, nothing regenerated) and the
-    // GEMMs stream them as they are - their operand splitters are the busier side of those kernels
-    const uint32_t kb = keep != nullptr ? keep[(i / Do4) * kKeepPitch + c] : 0xFFu;
+    // GEMMs stream them as they are - their operand splitters are the busier side of those kernels.  A compacted plane
+    // (slot != NULL) receives only the rows that have edges, at their compact row
+    const int64_t r = i / Do4;
+    const uint32_t kb = keep != nullptr ? keep[r * kKeepPitch + c] : 0xFFu;
     const float s = keep != nullptr ? keep_scale : 1.f;
-    d_res2[i] = make_float4((kb & 1u) ? third.x * s : 0.f, (kb & 2u) ? third.y * s : 0.f, (kb & 4u) ? third.z * s : 0.f,
-                            (kb & 8u) ? third.w * s : 0.f);
-    d_res2[n4 + i] = make_float4((kb & 16u) ? third.x * s : 0.f, (kb & 32u) ? third.y * s : 0.f, (kb & 64u) ? third.z * s : 0.f,
-                                 (kb & 128u) ? third.w * s : 0.f);
+    const int64_t o_in = slot_in == nullptr ? i : (int64_t)__ldg(slot_in + r) * Do4 + c;
+    const int64_t o_out = slot_out == nullptr ? i : (int64_t)__ldg(slot_out + r) * Do4 + c;
+    if (o_in >= 0)
+      d_res_in[o_in] = make_float4((kb & 1u) ? third.x * s : 0.f, (kb & 2u) ? third.y * s : 0.f,
+                                   (kb & 4u) ? third.z * s : 0.f, (kb & 8u) ? third.w * s : 0.f);
+    if (o_out >= 0)
+      d_res_out[o_out] = make_float4((kb & 16u) ? third.x * s : 0.f, (kb & 32u) ? third.y * s : 0.f,
+                                     (kb & 64u) ? third.z * s : 0.f, (kb & 128u) ? third.w * s : 0.f);
   }
+}
+
+// dst[dst_rows[j]] = src[src_rows[j]] for j < n (rows of D floats; a NULL row list is the identity): the gather of the
+// occupied rows of an aggregation plane into its compact block, and the scatter of the compact upstream rows back
+__global__ void __launch_bounds__(kThreads)
+rows_copy_kernel(const float4* __restrict__ src, int64_t ld_src, const int32_t* __restrict__ src_rows, float4* __restrict__ dst,
+                 int64_t ld_dst, const int32_t* __restrict__ dst_rows, int64_t n4, int D4) {
+  const int64_t i = blockIdx.x * (int64_t)kThreads + threadIdx.x;
+  if (i >= n4) return;
+  const int64_t j = i / D4;
+  const int c = (int)(i % D4);
+  const int64_t rs = src_rows != nullptr ? (int64_t)__ldg(src_rows + j) : j;
+  const int64_t rd = dst_rows != nullptr ? (int64_t)__ldg(dst_rows + j) : j;
+  dst[rd * ld_dst + c] = __ldg(src + rs * ld_src + c);
 }
 
 inline int check_dout(int32_t Dout) { return (Dout <= 0 || Dout % 4 != 0 || Dout > 1024) ? 1 : 0; }
@@ -374,17 +408,44 @@ extern "C" int kgc_dropout_mask(const int64_t* seed, int32_t plane, float drop_p
 
 extern "C" int32_t kgc_keep_pitch() { return kKeepPitch; }
 
-extern "C" int kgc_tail_fwd(const float* res3, const uint8_t* mask_in, const uint8_t* mask_out, const int64_t* seed,
-                            float drop_p, float keep_scale, const float* bias, int64_t n_rows, int32_t Dout, float* pre,
-                            double* partials, uint8_t* keep, void* stream) {
+extern "C" int kgc_tail_fwd_rows(const float* res3, const int32_t* slot_in, const float* rows_in, const int32_t* slot_out,
+                                 const float* rows_out, const uint8_t* mask_in, const uint8_t* mask_out, const int64_t* seed,
+                                 float drop_p, float keep_scale, const float* bias, int64_t n_rows, int32_t Dout, float* pre,
+                                 double* partials, uint8_t* keep, void* stream) {
   KGC_REQUIRE(check_dout(Dout) == 0, "Dout must be a multiple of 4 and <= 1024");
   KGC_REQUIRE(keep == nullptr || Dout <= 4 * kKeepPitch, "packed keep flags need Dout <= 256");
   KGC_REQUIRE(n_rows > 0, "n_rows must be positive");
+  KGC_REQUIRE((slot_in == nullptr || rows_in != nullptr) && (slot_out == nullptr || rows_out != nullptr),
+              "a compacted plane needs its rows");
   const int Do4 = Dout / 4;
   const size_t smem = partial_smem(Do4);   // <= 16 KB
+  PlaneRows pr;
+  pr.slot[0] = slot_in;
+  pr.slot[1] = slot_out;
+  pr.rows[0] = (const float4*)rows_in;
+  pr.rows[1] = (const float4*)rows_out;
   tail_fwd_kernel<<<(unsigned)kgc_tail_num_blocks(n_rows), kThreads, smem, as_stream(stream)>>>(
-      (const float4*)res3, make_drop(mask_in, mask_out, seed, drop_p, keep_scale), (const float4*)bias, n_rows, Do4,
+      (const float4*)res3, pr, make_drop(mask_in, mask_out, seed, drop_p, keep_scale), (const float4*)bias, n_rows, Do4,
       (float4*)pre, partials, keep);
+  KGC_LAUNCH_CHECK();
+  return 0;
+}
+
+extern "C" int kgc_tail_fwd(const float* res3, const uint8_t* mask_in, const uint8_t* mask_out, const int64_t* seed,
+                            float drop_p, float keep_scale, const float* bias, int64_t n_rows, int32_t Dout, float* pre,
+                            double* partials, uint8_t* keep, void* stream) {
+  return kgc_tail_fwd_rows(res3, nullptr, nullptr, nullptr, nullptr, mask_in, mask_out, seed, drop_p, keep_scale, bias, n_rows,
+                           Dout, pre, partials, keep, stream);
+}
+
+extern "C" int kgc_rows_copy(const float* src, int64_t ld_src, const int32_t* src_rows, float* dst, int64_t ld_dst,
+                             const int32_t* dst_rows, int64_t n, int32_t D, void* stream) {
+  KGC_REQUIRE(D > 0 && D % 4 == 0 && ld_src % 4 == 0 && ld_dst % 4 == 0 && n >= 0, "rows of a multiple of 4 floats");
+  KGC_REQUIRE(n == 0 || (src != nullptr && dst != nullptr), "null buffer");
+  const int64_t n4 = n * (D / 4);
+  if (n4 == 0) return 0;
+  rows_copy_kernel<<<(unsigned)ceil_div(n4, kThreads), kThreads, 0, as_stream(stream)>>>(
+      (const float4*)src, ld_src / 4, src_rows, (float4*)dst, ld_dst / 4, dst_rows, n4, D / 4);
   KGC_LAUNCH_CHECK();
   return 0;
 }
@@ -463,16 +524,28 @@ extern "C" int kgc_tail_bwd_reduce(const float* g_ent, const float* pre, const f
   return 0;
 }
 
-extern "C" int kgc_tail_bwd_apply(const float* g_ent, const float* pre, const float* stats, const float* gamma,
-                                  const float* beta, const double* sums, int32_t training, int64_t n_rows,
-                                  int64_t n_rows_global, int32_t Dout, float* d_out, const uint8_t* keep, float keep_scale,
-                                  float* d_res2, const uint8_t* out_keep, float out_scale, void* stream) {
+extern "C" int kgc_tail_bwd_apply_rows(const float* g_ent, const float* pre, const float* stats, const float* gamma,
+                                       const float* beta, const double* sums, int32_t training, int64_t n_rows,
+                                       int64_t n_rows_global, int32_t Dout, float* d_out, const uint8_t* keep, float keep_scale,
+                                       float* d_res_in, const int32_t* slot_in, float* d_res_out, const int32_t* slot_out,
+                                       const uint8_t* out_keep, float out_scale, void* stream) {
   KGC_REQUIRE(check_dout(Dout) == 0, "Dout must be a multiple of 4 and <= 1024");
+  KGC_REQUIRE((d_res_in == nullptr) == (d_res_out == nullptr), "the in and out planes come together");
   const int Do4 = Dout / 4;
   const int64_t n4 = n_rows * Do4;
   tail_bwd_apply_kernel<<<(unsigned)ceil_div(n4, kThreads), kThreads, 0, as_stream(stream)>>>(
       (const float4*)g_ent, (const float4*)pre, (const float4*)stats, (const float4*)gamma, (const float4*)beta, sums,
-      training, n_rows, n_rows_global, Do4, (float4*)d_out, keep, keep_scale, (float4*)d_res2, out_keep, out_scale);
+      training, n_rows, n_rows_global, Do4, (float4*)d_out, keep, keep_scale, (float4*)d_res_in, (float4*)d_res_out, slot_in,
+      slot_out, out_keep, out_scale);
   KGC_LAUNCH_CHECK();
   return 0;
+}
+
+extern "C" int kgc_tail_bwd_apply(const float* g_ent, const float* pre, const float* stats, const float* gamma,
+                                  const float* beta, const double* sums, int32_t training, int64_t n_rows,
+                                  int64_t n_rows_global, int32_t Dout, float* d_out, const uint8_t* keep, float keep_scale,
+                                  float* d_res2, const uint8_t* out_keep, float out_scale, void* stream) {
+  return kgc_tail_bwd_apply_rows(g_ent, pre, stats, gamma, beta, sums, training, n_rows, n_rows_global, Dout, d_out, keep,
+                                 keep_scale, d_res2, nullptr, d_res2 != nullptr ? d_res2 + n_rows * Dout : nullptr, nullptr,
+                                 out_keep, out_scale, stream);
 }

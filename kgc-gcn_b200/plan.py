@@ -53,6 +53,16 @@ def build_levels(seg_beg, seg_end, seg_row, chunk0=CHUNK0, chunk1=CHUNK1):
         chunk = chunk1
 
 
+# Compacted halves of the single-GPU layer (conv._ConvFn): a half whose destination rows are mostly empty - a knowledge
+# graph's in half, whose rows are the objects of the training triples: 1.1 % of the rows at the Wikidata5M shape - runs its
+# dense transforms, tail and weight gradient on its occupied rows only.  A half is compacted when at most this share of its
+# rows has an edge ...
+COMPACT_MAX_OCCUPANCY = 0.5
+# ... and its [rows, Dout] plane is larger than L2 (126 MB): below that the planes are served from L2 and the two row copies
+# and the extra launches of the compact path are a larger share of what they save (tests/compact_planes_time.py times both
+# paths at the bench shapes)
+COMPACT_MIN_PLANE_BYTES = 128 << 20
+
 SMALL_ITEM = 16   # fix-up items with at most this many rows are summed by one 8-lane group instead of a whole block
 CHUNK_EDGES = 32  # KGC_CHUNK_EDGES: sorted records per streaming chunk (one warp)
 
@@ -281,6 +291,28 @@ class GraphPlan(object):
         self.bwd_src = StreamPlan(sp_s, n2, dev)
         self.bwd_rel = StreamPlan(sp_r, n2, dev)
         self._scratch = {}
+        # occupied destination rows of each half (single-GPU plans only): rows[h] int32 ascending, the rows with at least one
+        # record in half h; slot[h] int32 [Nd], the compact index of every row or -1; n_c[h] = their count (host int)
+        self.rows = self.slot = self.n_c = None
+        if n_dst_rows is None and deg is None and self.dst_offset == 0:
+            rp, rm = self.rowptr_dst.to(torch.int64), self.rowmid_dst.to(torch.int64)
+            self.rows, self.slot, self.n_c = [], [], []
+            for cnt in (rm - rp[:-1], rp[1:] - rm):
+                rows = torch.nonzero(cnt > 0).view(-1)
+                slot = torch.full((Nd,), -1, **i32)
+                slot[rows] = torch.arange(rows.numel(), **i32)
+                self.rows.append(rows.to(torch.int32))
+                self.slot.append(slot)
+                self.n_c.append(int(rows.numel()))
+
+    def compact_halves(self, row_bytes):
+        """(in, out): whether the single-GPU layer runs that half on its occupied rows, for planes of ``row_bytes`` per row
+        (see COMPACT_MAX_OCCUPANCY / COMPACT_MIN_PLANE_BYTES; the same rule for both halves)."""
+        if self.rows is None:
+            return (False, False)
+        Nd = self.num_dst_rows
+        large = Nd * row_bytes > COMPACT_MIN_PLANE_BYTES
+        return tuple(bool(large and n <= COMPACT_MAX_OCCUPANCY * Nd) for n in self.n_c)
 
     def side_stream(self):
         """A second stream of this device for work that is off the step's critical path (created once per plan)."""
@@ -306,13 +338,15 @@ class GraphPlan(object):
         self.run_reduction(self.bwd_rel, level0, part, D, tag=tag)
         _lib.call('kgc_block_sum', _lib.ptr(part), self.num_type_blocks, self.num_types * D, _lib.ptr(d_relp), _lib.stream())
 
-    def run_reduction(self, sp, level0, out_final, D, addend=None, tag=''):
+    def run_reduction(self, sp, level0, out_final, D, addend=None, tag='', skip_prefill=()):
         """Launch the streaming kernel through ``level0(sp, out_final, carry)``, fill the rows without records and
-        reduce the carry rows of chunk-spanning rows through kgc_rows_reduce (fixed order, deterministic)."""
+        reduce the carry rows of chunk-spanning rows through kgc_rows_reduce (fixed order, deterministic).
+        ``skip_prefill``: pre-filled row ranges the caller never reads (their rows without records stay unwritten)."""
         carry = self.scratch(tag + 'carry', (max(sp.n_carry, 1), D))
         if addend is None:
             for lo, hi in getattr(sp, 'prefill', ()):
-                out_final.view(-1, D)[lo:hi].zero_()
+                if (lo, hi) not in skip_prefill:
+                    out_final.view(-1, D)[lo:hi].zero_()
         elif getattr(sp, 'prefill', ()):
             raise ValueError('a pre-filled plan cannot take an addend')
         level0(sp, out_final, carry)
