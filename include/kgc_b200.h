@@ -31,7 +31,7 @@ extern "C" {
 #pragma GCC visibility push(default)   /* the library is built with -fvisibility=hidden */
 #endif
 
-#define KGC_ABI_VERSION 1
+#define KGC_ABI_VERSION 2
 
 /* Work item of a fix-up reduction level: rows [beg, end) of the carry / partial array are summed;
  * the result goes to row `out` of the final output (flags & 1) or of the partial buffer of this
@@ -460,26 +460,18 @@ int kgc_score_1n_bwd_logit(const float* d_pred, int64_t ld_dp, const float* pred
 /* ---- N1: training loss against SPARSE positives (SURVEY.md 8(f) row N1) ------------------------------------------
  * Replaces the dense label build (data_loader.py:34-43), its host-to-device copy (main.py:60), BCELoss (model.py:42-44,
  * main.py:62) and the loss's backward down to the logit gradient, for the batch's query ids and the query->objects CSR
- * that kgc_label_build takes.  kgc_label_mask_build: mask[b, w] (uint32 [B, kgc_label_mask_words(N)], zeroed here) gets
- * bit (j & 31) of word (j >> 5) set for every positive j of query qid[b]; triple_out as in kgc_label_build (may be NULL).
- * kgc_bce_1n_bwd_logit: with y[b, n] = pos where the bit is set, add elsewhere, and p = pred[b, n] (kgc_score_1n_fwd):
- *   loss[0]        = mean_{b,n} ((y - 1) * max(log1p(-p), -100) - y * max(log(p), -100))       (torch BCELoss, mean)
- *   d_logitT[n, b] = (p - y) / max((1 - p) p, 1e-12) / (B N) * p * (1 - p)   ([n_ent, ldt], columns [B, ldt) zeroed)
- *   d_bias[n]      = sum_b d_logitT[n, b]
- * i.e. the gradient of the loss for a unit upstream gradient, in the layout kgc_score_1n_bwd_logit produces.
- * loss_partial: double [kgc_label_mask_words(n_ent)] workspace; sums are formed in a fixed order (deterministic). */
-int64_t kgc_label_mask_words(int64_t n_entity);
-int kgc_label_mask_build(const int64_t* qid, int64_t B, const int64_t* triples, const int64_t* ptr, const int32_t* idx,
-                         int64_t n_entity, uint32_t* mask, int64_t* triple_out, void* stream);
-int kgc_bce_1n_bwd_logit(const float* pred, int64_t ld_p, const uint32_t* mask, int64_t n_ent, int32_t B, int32_t ldt,
-                         float pos, float add, float* d_logitT, float* d_bias, double* loss_partial, float* loss,
-                         void* stream);
-/* Entity-major form of the same three steps (round 2): kgc_score_1n_fwd_t stores predT[n, b] (rows of ldt >= B floats,
+ * that kgc_label_build takes.  kgc_score_1n_fwd_t stores predT[n, b] = sigmoid(logit) (rows of ldt >= B floats,
  * ldt % 4 == 0) - the scorer's natural orientation; kgc_label_mask_t_build keeps the positives as bits per ENTITY
- * (mask_t [n_entity, ceil(B / 32)] uint32, zeroed by the call); kgc_bce_1n_bwd_logit_t makes one row-wise pass that
- * OVERWRITES pred_t with the transposed logit gradient (pad columns [B, ldt) = 0), writes d_bias and the mean loss
- * (loss_partial: kgc_bce_1n_t_blocks(n_ent) doubles).  [B, N] row pitches of 4 N bytes made the batch-major kernels move
- * their 2.35 GB in 128-byte pieces, one per DRAM page (3.4 ms each at N = 4.6 M). */
+ * (mask_t [n_entity, ceil(B / 32)] uint32, zeroed by the call): bit (b & 31) of word (b >> 5) of row j is set for every
+ * positive j of query qid[b].  kgc_bce_1n_bwd_logit_t, with y[b, n] = pos where the bit is set, add elsewhere, and
+ * p = predT[n, b], makes one row-wise pass that OVERWRITES pred_t with the transposed logit gradient:
+ *   loss[0]        = mean_{b,n} ((y - 1) * max(log1p(-p), -100) - y * max(log(p), -100))       (torch BCELoss, mean)
+ *   predT[n, b]   <- (p - y) / max((1 - p) p, 1e-12) / (B N) * p * (1 - p)   (columns [B, ldt) zeroed)
+ *   d_bias[n]      = sum_b predT[n, b]
+ * i.e. the gradient of the loss for a unit upstream gradient, in the layout kgc_score_1n_bwd_logit produces.
+ * loss_partial: kgc_bce_1n_t_blocks(n_ent) doubles of workspace; sums are formed in a fixed order (deterministic).
+ * Entity-major because [B, N] row pitches of 4 N bytes made batch-major kernels move their 2.35 GB in 128-byte pieces,
+ * one per DRAM page (3.4 ms each at N = 4.6 M). */
 int kgc_score_1n_fwd_t(const float* ent, int64_t n_ent, int32_t D, int64_t ld_ent, const float* packed_x, int32_t B,
                        const float* bias, float* pred_t, int64_t ld_t, void* stream);
 int64_t kgc_bce_1n_t_blocks(int64_t n_ent);

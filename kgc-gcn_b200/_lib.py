@@ -88,9 +88,6 @@ SIGNATURES = {
     'kgc_score_1n_logits': (ctypes.c_int, [_vp, _i64, _i32, _i64, _vp, _i32, _vp, _vp, _i64, _vp]),
     'kgc_rank_count_dense': (ctypes.c_int, [_vp, _i64, _i64, _i64, _vp, _vp, _vp, _vp]),
     'kgc_score_1n_bwd_logit': (ctypes.c_int, [_vp, _i64, _vp, _i64, _i64, _i32, _i32, _vp, _vp, _vp]),
-    'kgc_label_mask_words': (_i64, [_i64]),
-    'kgc_label_mask_build': (ctypes.c_int, [_vp, _i64, _vp, _vp, _vp, _i64, _vp, _vp, _vp]),
-    'kgc_bce_1n_bwd_logit': (ctypes.c_int, [_vp, _i64, _vp, _i64, _i32, _i32, _f32, _f32, _vp, _vp, _vp, _vp, _vp]),
     'kgc_score_1n_fwd_t': (ctypes.c_int, [_vp, _i64, _i32, _i64, _vp, _i32, _vp, _vp, _i64, _vp]),
     'kgc_bce_1n_t_blocks': (_i64, [_i64]),
     'kgc_label_mask_t_build': (ctypes.c_int, [_vp, _i64, _vp, _vp, _i64, _vp, _vp]),
@@ -128,14 +125,14 @@ def lib():
         for name, (res, args) in SIGNATURES.items():
             fn = getattr(handle, name)       # AttributeError if the symbol is not exported
             fn.restype, fn.argtypes = res, args
-        if handle.kgc_abi_version() != 1:
+        if handle.kgc_abi_version() != 2:
             raise RuntimeError('libkgc_b200.so ABI version mismatch')
         _LIB = handle
     return _LIB
 
 
 LAUNCHES = 0     # kernels launched through the C ABI since import (bench.py reports it as gpu_launches)
-_KERNELS_PER_CALL = {'kgc_csr_build': 16, 'kgc_label_mask_build': 2, 'kgc_bce_1n_bwd_logit': 2, 'kgc_bce_1n_bwd_logit_t': 2, 'kgc_label_mask_t_build': 2, 'kgc_score_pairs': 3, 'kgc_rank_finalize': 2, 'kgc_score_topk': 2, 'kgc_topk_dense': 2, 'kgc_sampled_bce_fwd': 4, 'kgc_sampled_adv_fwd': 4, 'kgc_sampled_bce_bwd_table': 7, 'kgc_gemm_tn': 2, 'kgc_gemm_tn_tc': 2, 'kgc_gemm_tn_tc_batch': 2, 'kgc_gemm_tn_tc_batch_rows': 2, 'kgc_gemm_tn_tc_batch_masked': 2}   # (kgc_p2p_allreduce: 1 or 3)
+_KERNELS_PER_CALL = {'kgc_csr_build': 16, 'kgc_bce_1n_bwd_logit_t': 2, 'kgc_label_mask_t_build': 2, 'kgc_score_pairs': 3, 'kgc_rank_finalize': 2, 'kgc_score_topk': 2, 'kgc_topk_dense': 2, 'kgc_sampled_bce_fwd': 4, 'kgc_sampled_adv_fwd': 4, 'kgc_sampled_bce_bwd_table': 7, 'kgc_gemm_tn': 2, 'kgc_gemm_tn_tc': 2, 'kgc_gemm_tn_tc_batch': 2, 'kgc_gemm_tn_tc_batch_rows': 2, 'kgc_gemm_tn_tc_batch_masked': 2}   # (kgc_p2p_allreduce: 1 or 3)
 
 
 def call(name, *args):

@@ -15,13 +15,18 @@ Backward is hand-derived (SURVEY.md Appendix A) and runs K3 / K4-backward / K4b 
 ``forward_partitioned`` is the same layer on a partitioned graph (partition.py): one process per GPU, exchanges over
 NVLink peer memory (K10).
 """
-import os
-
 import torch
 import torch.nn as nn
 
 from . import _lib
 from .plan import get_plan
+
+# The backward's upstream planes of the in / out halves = d_out x keep flags x 1 / (1 - p): either written by the tail
+# kernel as two more planes, or applied by the GEMMs while they split the ONE plane.  Measured (graph-timed layer step,
+# B200): Wikidata5M shape 49.7 vs 50.5 ms, WN18RR 0.387 vs 0.400 ms - the operand splitters are the busier side of K4b /
+# K4c (+1.9 / +1.0 ms against -2.5 ms of tail traffic) - but FB15k-237 0.462 vs 0.411 ms: when the planes stay in L2 the
+# extra writes are what costs.  So the three planes are written when together they exceed this size.
+TAIL_MASKED_MAX_BYTES = 48 << 20
 
 
 def get_param(shape):
@@ -543,15 +548,9 @@ class _ConvFn(torch.autograd.Function):
             _lib.call('kgc_colsum_finalize', p(partials), nb, Dout, p(sums), st())
             coll.all_reduce(sums, 'bn_b')
             sums32 = sums.float()
-        # the in / out halves' upstream planes = d_out x keep flags x 1 / (1 - p): either written by the tail kernel as two
-        # more planes, or applied by the GEMMs while they split the ONE plane.  Measured (graph-timed layer step, B200):
-        # Wikidata5M shape 49.7 vs 50.5 ms, WN18RR 0.387 vs 0.400 ms - the operand splitters are the busier side of K4b /
-        # K4c (+1.9 / +1.0 ms against -2.5 ms of tail traffic) - but FB15k-237 0.462 vs 0.411 ms: when the planes stay in
-        # L2 the extra writes are what costs.  Default by size; KGC_TAIL_PLANES=1|3 overrides.
-        # A compacted half always takes the three-plane form: its upstream rows are written compact, [n_c, Dout].
-        mode = os.environ.get('KGC_TAIL_PLANES', '')
-        three = (3 * Nl * Dout * 4 > (48 << 20)) if mode not in ('1', '3') else mode == '3'
-        three = three or any(comp)
+        # the in / out halves' upstream planes: three planes or one masked plane by size (TAIL_MASKED_MAX_BYTES).  A
+        # compacted half always takes the three-plane form: its upstream rows are written compact, [n_c, Dout].
+        three = 3 * Nl * Dout * 4 > TAIL_MASKED_MAX_BYTES or any(comp)
         d_res = [(plan.scratch('d_res_c%d' % h, (max(plan.n_c[h], 1), Dout)) if comp[h] else plan.scratch('d_res2_%d' % h, (Nl, Dout)))
                  if three else None for h in (0, 1)]
         _lib.call('kgc_tail_bwd_apply_rows', p(g_ent), p(pre), p(stats), p(gamma), p(beta), p(sums), int(ctx.training), Nl,

@@ -35,7 +35,6 @@
 //     Relation rows staged in shared memory and grids balanced to equal chunks per warp changed nothing measurable.
 //     ncu of the kept kernel: DRAM 47%, L1TEX 62%, 19 resident warps per SM, long-scoreboard 9 cycles per issue - it is
 //     now memory-latency-bound; the torch copy of the same bytes, timed the same way, reaches 0.77-0.79.
-#include <cstdlib>
 
 #include "common.cuh"
 
@@ -235,15 +234,14 @@ agg_stream_kernel(const StreamArgs A) {
 // per-edge bounds checks; the stream's single partial chunk takes a plain loop), (ii) issues ALL row loads of a batch,
 // the relation row included, in the load phase, so the consume phase is pure arithmetic, (iii) forms addresses from
 // 32-bit float4 indices (one IMAD + one IMAD.WIDE per load), (iv) runs at 3-4 CTAs per SM with small batches.
-template <int MODE, int KU, int MINB, int UNR = kChunk>
+template <int MODE, int KU, int MINB>
 __global__ void __launch_bounds__(kThreads, MINB)
 agg_lean_kernel(const StreamArgs A) {
-  // UNR: edges of a chunk that are unrolled into straight-line code.  The d_x / d_ee pass has ~110 instructions per edge:
-  // unrolling all 32 makes a 56 KB loop body and ncu shows 6.5 stall cycles per issued instruction waiting for the
-  // instruction cache ("no instruction"; 0.4 in the two smaller kernels).  Measured with 2 x 16 and 4 x 8 edges
-  // (KGC_BWD_SRC_UNROLL): 11.69 / 11.63 / 11.60 ms at the Wikidata5M shape, 47.4 / 48.7 / 49.4 us at the WN18RR shape - the
-  // fetch stalls are not on the critical path of a DRAM-latency-bound kernel; the full unroll stays the default.
-  static_assert(kChunk % UNR == 0, "UNR must divide the chunk");
+  // Full unroll in every mode.  The d_x / d_ee pass has ~110 instructions per edge: unrolling all 32 makes a 56 KB loop
+  // body and ncu shows 6.5 stall cycles per issued instruction waiting for the instruction cache ("no instruction"; 0.4
+  // in the two smaller kernels).  Bodies of 32 / 16 / 8 edges (1, 2 or 4 trips per chunk) measured 11.69 / 11.63 /
+  // 11.60 ms at the Wikidata5M shape and 47.4 / 48.7 / 49.4 us at the WN18RR shape - the fetch stalls are not on the
+  // critical path of a DRAM-latency-bound kernel, so the partial unrolls were removed.
   static_assert(kChunk == 32, "one record per lane");
   constexpr bool kHasC = MODE != kFwd;        // third gathered operand
   constexpr bool kHasR = MODE != kBwdRel;     // relation row
@@ -352,17 +350,14 @@ agg_lean_kernel(const StreamArgs A) {
     const uint32_t last_mask = __ballot_sync(0xffffffffu, (flag & kLast) != 0) & valid;
     started_here = (__shfl_sync(0xffffffffu, flag, 0) & kFirst) != 0;
     if (cnt == kChunk) {
-#pragma unroll 1
-      for (int ob = 0; ob < kChunk; ob += UNR) {                   // one trip when UNR == kChunk
 #pragma unroll
-        for (int base = 0; base < UNR; base += KU) {
+      for (int base = 0; base < kChunk; base += KU) {
 #pragma unroll
-          for (int u = 0; u < KU; ++u)
-            if (base + u < UNR) issue(u, ob + base + u);
+        for (int u = 0; u < KU; ++u)
+          if (base + u < kChunk) issue(u, base + u);
 #pragma unroll
-          for (int u = 0; u < KU; ++u)
-            if (base + u < UNR) consume(u, ob + base + u, (last_mask >> (ob + base + u)) & 1u);
-        }
+        for (int u = 0; u < KU; ++u)
+          if (base + u < kChunk) consume(u, base + u, (last_mask >> (base + u)) & 1u);
       }
     } else {                                                     // the stream's last, partial chunk
       for (int e = 0; e < cnt; ++e) {
@@ -526,10 +521,7 @@ int launch_stream(const StreamArgs& A, cudaStream_t st) {
                 "tables of 2^32 float4 or more are not supported (32-bit float4 indices)");
     constexpr int minb = LeanCfg<MODE>::minb;
     if (blocks > (int64_t)minb * kNumSMs) blocks = (int64_t)minb * kNumSMs;   // persistent grid
-    static const int unroll = [] { const char* e = getenv("KGC_BWD_SRC_UNROLL"); return e ? atoi(e) : 32; }();   // measurement knob
-    if (MODE == kBwdSrc && unroll == 8) agg_lean_kernel<MODE, LeanCfg<MODE>::ku, minb, 8><<<(unsigned)blocks, kThreads, 0, st>>>(A);
-    else if (MODE == kBwdSrc && unroll == 16) agg_lean_kernel<MODE, LeanCfg<MODE>::ku, minb, 16><<<(unsigned)blocks, kThreads, 0, st>>>(A);
-    else agg_lean_kernel<MODE, LeanCfg<MODE>::ku, minb><<<(unsigned)blocks, kThreads, 0, st>>>(A);
+    agg_lean_kernel<MODE, LeanCfg<MODE>::ku, minb><<<(unsigned)blocks, kThreads, 0, st>>>(A);
   } else {
     if (blocks > 2 * kNumSMs) blocks = 2 * kNumSMs;               // persistent: 2 resident CTAs per SM (__launch_bounds__)
     agg_stream_kernel<MODE, 2><<<(unsigned)blocks, kThreads, 0, st>>>(A);

@@ -24,7 +24,6 @@
 //   warp 14     TMEM allocator (2 accumulator stages)
 #include <cuda.h>
 
-#include <cstdlib>
 #include "common.cuh"
 
 namespace kgc {
@@ -1285,20 +1284,11 @@ extern "C" int kgc_score_1n_fwd(const float* ent, int64_t n_ent, int32_t D, int6
 // reduce kernel.  Beyond one wave every extra CTA costs its set-up and epilogue (~4 us per 1.2 MB slab) and 80 KB of partial.
 constexpr int64_t kTnMaxSlabRows = 1024;
 
-static int64_t tn_max_slab_rows() {
-  static int64_t rows = 0;
-  if (rows == 0) {
-    const char* e = getenv("KGC_TN_SLAB_ROWS");            // measurement aid (profiles/r02_k4c_slabs.md)
-    rows = e != nullptr && atoll(e) >= 64 ? atoll(e) : kTnMaxSlabRows;
-  }
-  return rows;
-}
-
 static int64_t tn_slabs(int64_t M, int n_prob) {
   const int64_t per_wave = kNumSMs / n_prob > 0 ? kNumSMs / n_prob : 1;
   int64_t slabs = ceil_div(M, (int64_t)2 * kTnRows);        // at least two K blocks per CTA
   if (slabs > per_wave) slabs = per_wave;
-  const int64_t need = ceil_div(M, tn_max_slab_rows());
+  const int64_t need = ceil_div(M, kTnMaxSlabRows);
   if (slabs < need) slabs = ceil_div(need, per_wave) * per_wave;      // whole waves
   return slabs < 1 ? 1 : slabs;
 }

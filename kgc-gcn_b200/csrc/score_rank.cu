@@ -29,8 +29,6 @@
 // selection over dense fp32 logits (exact mode) with the same list, exclusion cursor, partial layout and merge.
 // kgc_topk_merge combines finished results of disjoint entity ranges (shards) with the same list and output loop.
 #include <cuda.h>
-
-#include <cstdlib>
 #include <cuda_bf16.h>
 
 #include "common.cuh"
@@ -107,24 +105,6 @@ __device__ __forceinline__ void tma_load_2d(void* smem_dst, const CUtensorMap* m
       "l"(reinterpret_cast<uint64_t>(map)), "r"(smem_u32(bar)), "r"(c0), "r"(c1)
       : "memory");
 }
-// the same load delivered to the same shared-memory offset (and the same mbarrier offset) of every CTA in cta_mask
-__device__ __forceinline__ void tma_load_2d_mc(void* smem_dst, const CUtensorMap* map, uint64_t* bar, int c0, int c1,
-                                               uint16_t cta_mask) {
-  asm volatile(
-      "cp.async.bulk.tensor.2d.shared::cluster.global.mbarrier::complete_tx::bytes.multicast::cluster [%0], [%1, {%4, %5}], "
-      "[%2], %3;" ::"r"(smem_u32(smem_dst)),
-      "l"(reinterpret_cast<uint64_t>(map)), "r"(smem_u32(bar)), "h"(cta_mask), "r"(c0), "r"(c1)
-      : "memory");
-}
-__device__ __forceinline__ uint32_t cluster_ctarank() {
-  uint32_t r;
-  asm volatile("mov.u32 %0, %%cluster_ctarank;" : "=r"(r));
-  return r;
-}
-__device__ __forceinline__ void cluster_sync_all() {          // every thread of every CTA of the cluster
-  asm volatile("barrier.cluster.arrive.release.aligned;\n"
-               "barrier.cluster.wait.acquire.aligned;" ::: "memory");
-}
 __device__ __forceinline__ void tma_prefetch_desc(const CUtensorMap* map) {
   asm volatile("prefetch.tensormap [%0];" ::"l"(reinterpret_cast<uint64_t>(map)) : "memory");
 }
@@ -151,13 +131,6 @@ __device__ __forceinline__ void umma_bf16(uint32_t tmem_d, uint64_t adesc, uint6
 // all tcgen05.mma issued so far by this thread arrive on the mbarrier when they complete
 __device__ __forceinline__ void umma_commit(uint64_t* bar) {
   asm volatile("tcgen05.commit.cta_group::1.mbarrier::arrive::one.shared::cluster.b64 [%0];" ::"r"(smem_u32(bar))
-               : "memory");
-}
-// the same arrival on the mbarrier at this offset in every CTA of cta_mask (the B stage is shared by a CTA pair)
-__device__ __forceinline__ void umma_commit_mc(uint64_t* bar, uint16_t cta_mask) {
-  asm volatile("tcgen05.commit.cta_group::1.mbarrier::arrive::one.shared::cluster.multicast::cluster.b64 [%0], %1;" ::"r"(
-                   smem_u32(bar)),
-               "h"(cta_mask)
                : "memory");
 }
 __device__ __forceinline__ void tmem_ld32(uint32_t taddr, uint32_t (&v)[32]) {
@@ -315,33 +288,23 @@ __device__ __forceinline__ void topk_offer(TopList<K>& L, ExclCursor& X, float s
   if (s > L.thr && !X.excluded(id)) L.insert(topk_key(s, id));
 }
 
-// kCluster: launched as clusters of TWO CTAs that sweep the same entity tiles for different query tiles.  Each CTA of the
-// pair fetches HALF of every B stage (64 entity rows) and the TMA multicasts it into both CTAs' shared memory: every byte
-// of the entity table crosses L2 -> SM once per 512 queries instead of once per 256.  (Measured: no gain - the sweep is
-// not bound by the 4.3 TB/s it pulls out of L2; opt-in.)  A stage's `full` barrier collects both halves (its own TMA and
-// the peer's), its `empty` barrier the retired MMAs of BOTH CTAs (tcgen05.commit multicast) - a slot is rewritten by the
-// peer's TMA as well.
-//
 // kTopK (K6k, 16 or 32): instead of counting, every epilogue thread keeps its query row's kTopK best (score, id) keys of the
 // work item in registers (TopList) and writes them to P.topk_part[chunk, q, :]; topk_merge_kernel reduces the chunks.
-template <bool kPairs, bool kCountEq, bool kCluster, int kTopK = 0>
+template <bool kPairs, bool kCountEq, int kTopK = 0>
 __global__ void __launch_bounds__(kThreads, 1)
-score_kernel(const __grid_constant__ CUtensorMap map_a, const __grid_constant__ CUtensorMap map_b,
-             const __grid_constant__ CUtensorMap map_bh, const ScoreParams P) {
+score_kernel(const __grid_constant__ CUtensorMap map_a, const __grid_constant__ CUtensorMap map_b, const ScoreParams P) {
   extern __shared__ uint8_t smem_raw[];
   const SharedLayout S = carve(smem_raw);
   const int warp = threadIdx.x / 32, lane = threadIdx.x % 32;
   constexpr int kNumM = kPairs ? 1 : kMTiles;
-  static_assert(!(kPairs && kCluster), "pairs mode runs single CTAs");
-  static_assert(kTopK == 0 || (!kPairs && !kCountEq && !kCluster), "top-k mode is a single-CTA sweep");
-  const uint32_t cta_rank = kCluster ? cluster_ctarank() : 0u;
+  static_assert(kTopK == 0 || (!kPairs && !kCountEq), "top-k mode is a sweep");
 
   if (warp == 0 && lane == 0) {
     tma_prefetch_desc(&map_a);
     tma_prefetch_desc(&map_b);
     for (int i = 0; i < kStagesB; ++i) {
       mbar_init(S.full + i, 1);
-      mbar_init(S.empty + i, kCluster ? 2 : 1);
+      mbar_init(S.empty + i, 1);
     }
     mbar_init(S.a_full, 1);
     mbar_init(S.a_empty, 1);
@@ -356,7 +319,6 @@ score_kernel(const __grid_constant__ CUtensorMap map_a, const __grid_constant__ 
   tc_fence_before();
   __syncthreads();
   tc_fence_after();
-  if (kCluster) cluster_sync_all();                            // the peer's barriers exist before anything targets them
   const uint32_t tmem_base = *S.tmem_slot;
 
   if (warp == 0) {
@@ -379,11 +341,7 @@ score_kernel(const __grid_constant__ CUtensorMap map_a, const __grid_constant__ 
           for (int kb = 0; kb < P.n_kblocks; ++kb) {
             mbar_wait(S.empty + stage, phase ^ 1);
             mbar_expect_tx(S.full + stage, kTileBytes);
-            if (kCluster)                                          // my half of the stage, into both CTAs
-              tma_load_2d_mc(S.b + stage * kTileBytes + cta_rank * (kTileBytes / 2), &map_bh, S.full + stage, kb * kBlockK,
-                             t * kBlockN + (int)cta_rank * (kBlockN / 2), (uint16_t)3);
-            else
-              tma_load_2d(S.b + stage * kTileBytes, &map_b, S.full + stage, kb * kBlockK, t * kBlockN);
+            tma_load_2d(S.b + stage * kTileBytes, &map_b, S.full + stage, kb * kBlockK, t * kBlockN);
             if (++stage == kStagesB) { stage = 0; phase ^= 1; }
           }
         }
@@ -425,8 +383,7 @@ score_kernel(const __grid_constant__ CUtensorMap map_a, const __grid_constant__ 
                   if (kNumM == 2) umma_bf16(d0 + kBlockN, adesc1 + 2 * k, bdesc + 2 * k, kInstrDesc, accum);
                 }
               }
-              if (kCluster) umma_commit_mc(S.empty + stage, (uint16_t)3);   // ... in BOTH CTAs: the slot is shared
-              else umma_commit(S.empty + stage);               // B stage is free once these MMAs retire
+              umma_commit(S.empty + stage);                    // B stage is free once these MMAs retire
               if (kb == P.n_kblocks - 1) {
                 umma_commit(S.acc_full + acc);                 // accumulators of this entity tile are complete
                 if (t == t1 - 1) umma_commit(S.a_empty);       // A tiles may be overwritten
@@ -575,7 +532,6 @@ score_kernel(const __grid_constant__ CUtensorMap map_a, const __grid_constant__ 
   }
   tc_fence_before();
   __syncthreads();
-  if (kCluster) cluster_sync_all();                            // no CTA leaves while the peer may still write or signal into it
   if (warp == 2) tmem_dealloc(tmem_base, kTmemCols);
 }
 
@@ -823,13 +779,13 @@ int get_encode_fn(EncodeTiledFn* out) {
 }
 
 // bf16 [rows, kpad] row-major -> boxes of 64 (K) x 128 (rows), 128-byte swizzle, zero fill out of bounds
-int make_map(CUtensorMap* map, const void* base, int64_t rows, int kpad, int box_rows = kBlockM) {
+int make_map(CUtensorMap* map, const void* base, int64_t rows, int kpad) {
   EncodeTiledFn enc;
   if (get_encode_fn(&enc)) return 1;
   KGC_REQUIRE((reinterpret_cast<uintptr_t>(base) & 15) == 0, "bf16 table must be 16-byte aligned");
   cuuint64_t dims[2] = {(cuuint64_t)kpad, (cuuint64_t)rows};
   cuuint64_t strides[1] = {(cuuint64_t)kpad * 2};
-  cuuint32_t box[2] = {(cuuint32_t)kBlockK, (cuuint32_t)box_rows};
+  cuuint32_t box[2] = {(cuuint32_t)kBlockK, (cuuint32_t)kBlockM};
   cuuint32_t estr[2] = {1, 1};
   CUresult r = enc(map, CU_TENSOR_MAP_DATA_TYPE_BFLOAT16, 2, const_cast<void*>(base), dims, strides, box, estr,
                    CU_TENSOR_MAP_INTERLEAVE_NONE, CU_TENSOR_MAP_SWIZZLE_128B, CU_TENSOR_MAP_L2_PROMOTION_L2_256B,
@@ -874,11 +830,11 @@ int64_t topk_sweep_chunks(int64_t b, int64_t n, int kpad) {
 
 template <int K>
 int launch_topk_sweep(const CUtensorMap& ma, const CUtensorMap& mb, const ScoreParams& P, cudaStream_t st) {
-  auto kern = score_kernel<false, false, false, K>;
+  auto kern = score_kernel<false, false, K>;
   static SmemAttrCache attr;
   KGC_CUDA_TRY(attr.ensure(kern, (size_t)kSmemBytes));
   const int grid = P.n_items < kNumSMs ? P.n_items : kNumSMs;
-  kern<<<grid, kThreads, kSmemBytes, st>>>(ma, mb, mb, P);
+  kern<<<grid, kThreads, kSmemBytes, st>>>(ma, mb, P);
   KGC_LAUNCH_CHECK();
   return 0;
 }
@@ -893,37 +849,12 @@ int launch_topk_merge(const uint64_t* part, int64_t n_chunks, int64_t b, int k, 
 
 template <bool kPairs, bool kCountEq>
 int launch_score(const CUtensorMap& ma, const CUtensorMap& mb, const ScoreParams& P, cudaStream_t st) {
-  auto kern = score_kernel<kPairs, kCountEq, false>;
+  auto kern = score_kernel<kPairs, kCountEq>;
   static SmemAttrCache attr;                           // one per <kPairs, kCountEq> instantiation
   KGC_CUDA_TRY(attr.ensure(kern, (size_t)kSmemBytes));
   const int grid = P.n_items < kNumSMs ? P.n_items : kNumSMs;
-  kern<<<grid, kThreads, kSmemBytes, st>>>(ma, mb, mb, P);
+  kern<<<grid, kThreads, kSmemBytes, st>>>(ma, mb, P);
   KGC_LAUNCH_CHECK();
-  return 0;
-}
-
-// sweep as clusters of two CTAs (see score_kernel): n_items and the grid are even, item 2i / 2i + 1 share an entity chunk
-template <bool kCountEq>
-int launch_score_pairs_of_ctas(const CUtensorMap& ma, const CUtensorMap& mb, const CUtensorMap& mbh, const ScoreParams& P,
-                               cudaStream_t st) {
-  auto kern = score_kernel<false, kCountEq, true>;
-  static SmemAttrCache attr;
-  KGC_CUDA_TRY(attr.ensure(kern, (size_t)kSmemBytes));
-  int grid = P.n_items < kNumSMs ? P.n_items : kNumSMs;
-  grid &= ~1;
-  cudaLaunchConfig_t cfg = {};
-  cfg.gridDim = dim3((unsigned)grid);
-  cfg.blockDim = dim3(kThreads);
-  cfg.dynamicSmemBytes = kSmemBytes;
-  cfg.stream = st;
-  cudaLaunchAttribute at[1];
-  at[0].id = cudaLaunchAttributeClusterDimension;
-  at[0].val.clusterDim.x = 2;
-  at[0].val.clusterDim.y = 1;
-  at[0].val.clusterDim.z = 1;
-  cfg.attrs = at;
-  cfg.numAttrs = 1;
-  KGC_CUDA_TRY(cudaLaunchKernelEx(&cfg, kern, ma, mb, mbh, P));
   return 0;
 }
 
@@ -1006,23 +937,10 @@ extern "C" int kgc_score_rank(const uint16_t* q_bf16, const uint16_t* e_bf16, in
   P.ksteps = kpad / kUmmaK;
   P.n_kblocks = (kpad + kBlockK - 1) / kBlockK;
   P.n_mp = (int32_t)ceil_div(b, kMTiles * kBlockM);
-  // CTA pairs that share their B stages (TMA multicast), KGC_SCORE_CLUSTER=1.  Built to test whether the sweep is bound by
-  // L2 -> SM traffic: it is not - 104.4 ms against 104.7 ms with single CTAs (65,536 x 4.59 M, B200 under its power cap) -
-  // so single CTAs stay the default.  The pair needs an even number of query-tile pairs (a padding pair has no valid
-  // query: its rows never count)
-  static const bool cluster_ok = [] { const char* e = getenv("KGC_SCORE_CLUSTER"); return e && e[0] == '1'; }();
-  const bool cluster = cluster_ok && P.n_mp >= 2;
-  if (cluster) P.n_mp = (P.n_mp + 1) & ~1;
   plan_chunks(P, n, kpad);
   P.thr = thr;
   P.count_gt = count_gt;
   P.count_eq = count_eq;
-  if (cluster) {
-    CUtensorMap mbh;
-    if (make_map(&mbh, e_bf16, n, kpad, kBlockN / 2)) return 1;
-    if (count_eq) return launch_score_pairs_of_ctas<true>(ma, mb, mbh, P, st);
-    return launch_score_pairs_of_ctas<false>(ma, mb, mbh, P, st);
-  }
   if (count_eq) return launch_score<false, true>(ma, mb, P, st);
   return launch_score<false, false>(ma, mb, P, st);
 }

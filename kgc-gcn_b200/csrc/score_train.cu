@@ -56,90 +56,20 @@ score_1n_bwd_logit_kernel(const float* __restrict__ d_pred, int64_t ld_dp, const
 
 // ---- N1 (SURVEY.md 8(f)): BCE against SPARSE positives fused with the backward through the sigmoid ----------------
 // The reference builds a dense multi-hot label [B, N] per batch (data_loader.py:34-43), copies it to the device and runs
-// BCELoss over it (model.py:42-44).  Here the label exists only as one bit per (query, entity): label_mask_kernel sets the
-// bits of the batch's positives (integer atomicOr: order-independent), and bce_1n_kernel walks pred once, producing the
-// summed loss AND the logit gradient (transposed, ready for the two gradient GEMMs) AND the bias gradient - the dense
-// label, the BCE forward and the BCE backward passes over [B, N] disappear.  Arithmetic follows ATen's kernels:
+// BCELoss over it (model.py:42-44).  Here the label exists only as one bit per (entity, query): label_mask_t_kernel sets the
+// bits of the batch's positives (integer atomicOr: order-independent), and bce_1n_t_kernel walks pred once, producing the
+// summed loss AND the logit gradient AND the bias gradient - the dense label, the BCE forward and the BCE backward passes
+// over [B, N] disappear.  Arithmetic follows ATen's kernels:
 //   loss term   = (y - 1) * max(log1p(-p), -100) - y * max(log(p), -100)
 //   d_pred      = (p - y) / max((1 - p) * p, 1e-12) * (1 / (B N))          (mean reduction, unit upstream)
 //   d_logit     = d_pred * p * (1 - p)                                     (as score_1n_bwd_logit_kernel)
 // with y = pos on the batch's positives and add elsewhere (the two values kgc_label_build writes).
-
-__global__ void __launch_bounds__(kThreadsST)
-label_mask_kernel(const int64_t* __restrict__ qid, const int64_t* __restrict__ triples, const int64_t* __restrict__ ptr,
-                  const int32_t* __restrict__ idx, int64_t n_entity, int64_t words, uint32_t* __restrict__ mask,
-                  int64_t* __restrict__ triple_out) {
-  const int64_t b = blockIdx.x;
-  const int64_t q = qid[b];
-  for (int64_t k = ptr[q] + threadIdx.x; k < ptr[q + 1]; k += kThreadsST) {
-    const int64_t j = idx[k];
-    if (j >= 0 && j < n_entity) atomicOr(mask + b * words + (j >> 5), 1u << (j & 31));
-  }
-  if (triple_out != nullptr && threadIdx.x < 3) triple_out[b * 3 + threadIdx.x] = triples[q * 3 + threadIdx.x];
-}
-
-__global__ void __launch_bounds__(kThreadsST)
-bce_1n_kernel(const float* __restrict__ pred, int64_t ld_p, const uint32_t* __restrict__ mask, int64_t words,
-              int64_t n_ent, int B, int ldt, float pos, float add, float inv_count, float* __restrict__ d_logitT,
-              float* __restrict__ d_bias, double* __restrict__ loss_partial) {
-  __shared__ float tile[32][33];
-  __shared__ double warp_loss[kThreadsST / 32];
-  const int lane = threadIdx.x % 32, warp = threadIdx.x / 32;      // 8 warps x 4 rows
-  const int64_t n0 = (int64_t)blockIdx.x * 32;                       // = bit 0 of mask word blockIdx.x of every row
-  float bias_acc[4] = {0.f, 0.f, 0.f, 0.f};
-  double loss = 0.0;
-  for (int b0 = 0; b0 < ldt; b0 += 32) {
-#pragma unroll
-    for (int i = 0; i < 4; ++i) {
-      const int b = b0 + warp * 4 + i;
-      const int64_t n = n0 + lane;
-      float g = 0.f;
-      if (b < B && n < n_ent) {
-        const float p = pred[(int64_t)b * ld_p + n];
-        const uint32_t w = __ldg(mask + (int64_t)b * words + blockIdx.x);      // one word per warp row: broadcast
-        const float y = ((w >> lane) & 1u) ? pos : add;
-        const float lp = fmaxf(logf(p), -100.f), l1p = fmaxf(log1pf(-p), -100.f);
-        loss += (double)((y - 1.f) * l1p - y * lp);
-        const float d_pred = (p - y) / fmaxf((1.f - p) * p, 1e-12f) * inv_count;
-        g = d_pred * p * (1.f - p);
-      }
-      tile[warp * 4 + i][lane] = g;
-    }
-    __syncthreads();
-#pragma unroll
-    for (int i = 0; i < 4; ++i) {
-      const int r = warp * 4 + i;                                   // entity n0 + r, query b0 + lane
-      const float g = tile[lane][r];
-      if (n0 + r < n_ent && b0 + lane < ldt) d_logitT[(n0 + r) * ldt + b0 + lane] = g;   // pad columns [B, ldt) get zeros
-      float s = g;
-#pragma unroll
-      for (int o = 16; o > 0; o >>= 1) s += __shfl_xor_sync(0xFFFFFFFFu, s, o);
-      bias_acc[i] += s;
-    }
-    __syncthreads();
-  }
-  if (lane == 0) {
-#pragma unroll
-    for (int i = 0; i < 4; ++i)
-      if (n0 + warp * 4 + i < n_ent) d_bias[n0 + warp * 4 + i] = bias_acc[i];
-  }
-  // the CTA's share of the summed loss: fixed shuffle tree per warp, warps added in order
-#pragma unroll
-  for (int o = 16; o > 0; o >>= 1) loss += __shfl_xor_sync(0xFFFFFFFFu, loss, o);
-  if (lane == 0) warp_loss[warp] = loss;
-  __syncthreads();
-  if (threadIdx.x == 0) {
-    double s = 0.0;
-    for (int w = 0; w < kThreadsST / 32; ++w) s += warp_loss[w];
-    loss_partial[blockIdx.x] = s;
-  }
-}
-
-// ---- the same, ENTITY-MAJOR (round 2).  pred [B, N] has rows 4 N bytes apart: the scorer's transposed TMA stores and this
-// kernel's reads touch it in 128-byte pieces, one per DRAM page - 3.4 ms each at N = 4.6 M (1.4-1.8 TB/s).  The fused-loss
-// path never has to hand out [B, N]: the scorer stores its natural orientation predT [N, ldt] (rows of 4 B bytes,
-// contiguous), the label bits are kept per entity (maskT [N, ceil(B / 32)]), and this kernel is a plain row-wise pass that
-// overwrites predT with the logit gradient IN PLACE - no transpose, no second [B, N]-sized buffer.
+//
+// Everything is ENTITY-MAJOR.  A batch-major pred [B, N] has rows 4 N bytes apart: the scorer's transposed TMA stores and a
+// loss kernel's reads touch it in 128-byte pieces, one per DRAM page - 3.4 ms each at N = 4.6 M (1.4-1.8 TB/s).  The
+// scorer instead stores its natural orientation predT [N, ldt] (rows of 4 B bytes, contiguous), the label bits are kept
+// per entity (maskT [N, ceil(B / 32)]), and bce_1n_t_kernel is a plain row-wise pass that overwrites predT with the logit
+// gradient IN PLACE - no transpose, no second [B, N]-sized buffer.
 __global__ void __launch_bounds__(kThreadsST)
 label_mask_t_kernel(const int64_t* __restrict__ qid, const int64_t* __restrict__ ptr, const int32_t* __restrict__ idx,
                     int64_t n_entity, int wb, uint32_t* __restrict__ mask_t) {
@@ -223,38 +153,6 @@ extern "C" int kgc_score_1n_bwd_logit(const float* d_pred, int64_t ld_dp, const 
   KGC_REQUIRE(d_pred && pred && d_logitT && d_bias, "null buffer");
   score_1n_bwd_logit_kernel<<<(unsigned)ceil_div(n_ent, 32), kThreadsST, 0, as_stream(stream)>>>(
       d_pred, ld_dp, pred, ld_p, n_ent, B, ldt, d_logitT, d_bias);
-  KGC_LAUNCH_CHECK();
-  return 0;
-}
-
-extern "C" int64_t kgc_label_mask_words(int64_t n_entity) { return n_entity > 0 ? ceil_div(n_entity, 32) : 0; }
-
-extern "C" int kgc_label_mask_build(const int64_t* qid, int64_t B, const int64_t* triples, const int64_t* ptr,
-                                    const int32_t* idx, int64_t n_entity, uint32_t* mask, int64_t* triple_out,
-                                    void* stream) {
-  KGC_REQUIRE(B >= 0 && n_entity > 0, "bad sizes");
-  if (B == 0) return 0;
-  KGC_REQUIRE(qid && ptr && idx && mask, "null buffer");
-  KGC_REQUIRE(triple_out == nullptr || triples != nullptr, "triple_out needs triples");
-  const int64_t words = kgc_label_mask_words(n_entity);
-  KGC_CUDA_TRY(cudaMemsetAsync(mask, 0, (size_t)(B * words) * sizeof(uint32_t), as_stream(stream)));
-  label_mask_kernel<<<(unsigned)B, kThreadsST, 0, as_stream(stream)>>>(qid, triples, ptr, idx, n_entity, words, mask,
-                                                                     triple_out);
-  KGC_LAUNCH_CHECK();
-  return 0;
-}
-
-extern "C" int kgc_bce_1n_bwd_logit(const float* pred, int64_t ld_p, const uint32_t* mask, int64_t n_ent, int32_t B,
-                                    int32_t ldt, float pos, float add, float* d_logitT, float* d_bias,
-                                    double* loss_partial, float* loss, void* stream) {
-  KGC_REQUIRE(n_ent > 0 && B > 0 && ldt >= B && ld_p >= n_ent, "bad sizes");
-  KGC_REQUIRE(pred && mask && d_logitT && d_bias && loss_partial && loss, "null buffer");
-  const int64_t words = kgc_label_mask_words(n_ent);               // = number of CTAs = number of loss partials
-  const double count = (double)B * (double)n_ent;
-  bce_1n_kernel<<<(unsigned)words, kThreadsST, 0, as_stream(stream)>>>(pred, ld_p, mask, words, n_ent, B, ldt, pos, add,
-                                                                     (float)(1.0 / count), d_logitT, d_bias, loss_partial);
-  KGC_LAUNCH_CHECK();
-  bce_1n_finalize_kernel<<<1, kThreadsST, 0, as_stream(stream)>>>(loss_partial, words, 1.0 / count, loss);
   KGC_LAUNCH_CHECK();
   return 0;
 }

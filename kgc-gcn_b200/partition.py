@@ -580,9 +580,8 @@ class _P2PContext(object):
             self.barrier()
         self.table[:n].copy_(x_local)
         self.barrier()
-        order = None if os.environ.get('KGC_HALO_ORDER', '1') == '0' else self.halo_order     # measurement knob
-        _lib.call('kgc_p2p_halo_gather', ctypes.c_void_p(self.table_ptrs), self.rank, _lib.ptr(self.halo_rows), _lib.ptr(order),
-                  self.halo_rows.numel(), self.block, self.D, _lib.stream())
+        _lib.call('kgc_p2p_halo_gather', ctypes.c_void_p(self.table_ptrs), self.rank, _lib.ptr(self.halo_rows),
+                  _lib.ptr(self.halo_order), self.halo_rows.numel(), self.block, self.D, _lib.stream())
         return self.table
 
     def reduce(self, addend, n_rows, out=None, channel=0):

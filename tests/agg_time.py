@@ -8,6 +8,6 @@ flush = bench.Flusher(dev)
 for wl in sys.argv[1:]:
     case = bench.LayerCase(k, orc, wl, dev)
     roof, out = bench.kernel_rooflines(case, flush)
-    print(wl, os.environ.get('KGC_BWD_SRC_UNROLL', 'default'), {n: round(v['ms'], 4) for n, v in out.items()}, {n: round(v['ms'], 4) for n, v in roof['passes'].items() if isinstance(v, dict)})
+    print(wl, {n: round(v['ms'], 4) for n, v in out.items()}, {n: round(v['ms'], 4) for n, v in roof['passes'].items() if isinstance(v, dict)})
     del case
     k.plan._PLAN_CACHE.clear(); torch.cuda.empty_cache()

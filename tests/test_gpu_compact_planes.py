@@ -25,7 +25,7 @@ def force(monkeypatch, k, mode):
     """'dense': no half compacted; 'sparse': the halves with at most half of their rows occupied; 'all': both halves."""
     monkeypatch.setattr(k.plan, 'COMPACT_MIN_PLANE_BYTES', -1)
     monkeypatch.setattr(k.plan, 'COMPACT_MAX_OCCUPANCY', {'dense': -1.0, 'sparse': 0.5, 'all': 1.0}[mode])
-    monkeypatch.setenv('KGC_TAIL_PLANES', '3')          # the compact path always writes three planes: compare like with like
+    monkeypatch.setattr(k.conv, 'TAIL_MASKED_MAX_BYTES', -1)   # the compact path always writes three planes: compare like with like
 
 
 def graph(kind, N=3000, R=7, E=9000, seed=61):
