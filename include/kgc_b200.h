@@ -31,7 +31,7 @@ extern "C" {
 #pragma GCC visibility push(default)   /* the library is built with -fvisibility=hidden */
 #endif
 
-#define KGC_ABI_VERSION 2
+#define KGC_ABI_VERSION 3
 
 /* Work item of a fix-up reduction level: rows [beg, end) of the carry / partial array are summed;
  * the result goes to row `out` of the final output (flags & 1) or of the partial buffer of this
@@ -150,8 +150,12 @@ int kgc_agg_bwd_rel(const float* x, const float* ee, const float* g3,
  *   kgc_tail_fwd           writes pre[n_rows,Dout] and per-block column partials (sum, sum of squares; fp64) and, when keep
  *                          is given (uint8 [n_rows, kgc_keep_pitch()], Dout <= 256), the keep flags it used: byte c of a
  *                          row = columns 4c..4c+3, low nibble = in half, high nibble = out half.  The backward GEMMs
- *                          apply them to ONE upstream plane while splitting it (kgc_gemm_nt_batch_masked,
- *                          kgc_gemm_tn_tc_batch_masked): no mask is regenerated, no masked plane is written.
+ *                          apply them to ONE upstream plane while splitting it (the keep argument of kgc_gemm_nt_batch
+ *                          and kgc_gemm_tn_tc_batch): no mask is regenerated, no masked plane is written.
+ *                          Compacted in / out planes (the layer's sparse halves): slot_h (NULL: plane h is read densely
+ *                          from res3) = int32 [n_rows], the row of node row r in rows_h [n_c, Dout], or -1 for a row
+ *                          without edges, which contributes exactly 0.  res3's plane h is not read when slot_h is given.
+ *                          Same arithmetic order, dropout draws and keep flags.
  *   kgc_colsum_finalize    reduces the partials in a fixed order into sums[2,Dout] (fp64).  A partitioned
  *                          graph all-reduces these 2*Dout doubles across ranks here (SURVEY.md 8(e)).
  *   kgc_colstats_from_sums stats[0]=mean, [1]=biased var, [2]=rstd=1/sqrt(var+eps) over n_rows (GLOBAL) rows
@@ -160,16 +164,10 @@ int kgc_agg_bwd_rel(const float* x, const float* ee, const float* g3,
 int64_t kgc_tail_num_blocks(int64_t n_rows);
 int kgc_dropout_mask(const int64_t* seed, int32_t plane, float drop_p, int64_t n_elem, uint8_t* mask, void* stream);
 int32_t kgc_keep_pitch(void);
-int kgc_tail_fwd(const float* res3, const uint8_t* mask_in, const uint8_t* mask_out, const int64_t* seed, float drop_p,
-                 float keep_scale, const float* bias, int64_t n_rows, int32_t Dout, float* pre, double* partials,
-                 uint8_t* keep, void* stream);
-/* kgc_tail_fwd with compacted in / out planes (the layer's sparse halves): slot_h (NULL: plane h is read densely from
- * res3) = int32 [n_rows], the row of node row r in rows_h [n_c, Dout], or -1 for a row without edges, which contributes
- * exactly 0.  res3's plane h is not read when slot_h is given.  Same arithmetic order, dropout draws and keep flags. */
-int kgc_tail_fwd_rows(const float* res3, const int32_t* slot_in, const float* rows_in, const int32_t* slot_out,
-                      const float* rows_out, const uint8_t* mask_in, const uint8_t* mask_out, const int64_t* seed,
-                      float drop_p, float keep_scale, const float* bias, int64_t n_rows, int32_t Dout, float* pre,
-                      double* partials, uint8_t* keep, void* stream);
+int kgc_tail_fwd(const float* res3, const int32_t* slot_in, const float* rows_in, const int32_t* slot_out,
+                 const float* rows_out, const uint8_t* mask_in, const uint8_t* mask_out, const int64_t* seed,
+                 float drop_p, float keep_scale, const float* bias, int64_t n_rows, int32_t Dout, float* pre,
+                 double* partials, uint8_t* keep, void* stream);
 /* dst[dst_rows[j]] = src[src_rows[j]] for j < n, rows of D floats (D, ld_src, ld_dst multiples of 4); a NULL row list is
  * the identity.  Gathers the occupied rows of a plane into a compact block and scatters them back. */
 int kgc_rows_copy(const float* src, int64_t ld_src, const int32_t* src_rows, float* dst, int64_t ld_dst,
@@ -197,27 +195,22 @@ int kgc_tail_apply(const float* pre, const float* stats, const float* gamma, con
  * sum dz (= d beta), sums[1] = sum dz*xhat (= d gamma), all-reduced by a partitioned caller; kgc_tail_bwd_apply:
  * d_out[n_rows,Dout] = d_pre / 3 (BatchNorm backward over n_rows_global rows when training) - ONE plane: the self-loop
  * transform's upstream gradient as it is, the in / out halves' after the keep flags x 1/(1-p): applied by the GEMMs
- * (d_res2 NULL), or written here as two more planes d_res2[2,n_rows,Dout] from kgc_tail_fwd's keep flags (keep NULL: no
- * dropout, both planes = d_out). */
+ * (d_res_in = d_res_out = NULL), or written here as two more planes d_res_in / d_res_out [n_rows,Dout] from
+ * kgc_tail_fwd's keep flags (keep NULL: no dropout, both planes = d_out; both planes or neither).  slot_h != NULL: plane h
+ * is compacted (see kgc_tail_fwd) and receives only the rows that have edges, at their compact row. */
 /* out_keep != NULL: the forward dropped its output (kgc_tail_apply): g_ent is taken x keep flag x out_scale = 1/(1-p). */
 int kgc_tail_bwd_reduce(const float* g_ent, const float* pre, const float* stats, const float* gamma, const float* beta,
                         int64_t n_rows, int32_t Dout, double* partials, const uint8_t* out_keep, float out_scale,
                         void* stream);
 int kgc_tail_bwd_apply(const float* g_ent, const float* pre, const float* stats, const float* gamma, const float* beta,
                        const double* sums, int32_t training, int64_t n_rows, int64_t n_rows_global, int32_t Dout,
-                       float* d_out, const uint8_t* keep, float keep_scale, float* d_res2, const uint8_t* out_keep,
-                       float out_scale, void* stream);
-/* kgc_tail_bwd_apply with the in / out planes given separately (both or neither); slot_h != NULL: plane h is compacted
- * (see kgc_tail_fwd_rows) and receives only the rows that have edges, at their compact row. */
-int kgc_tail_bwd_apply_rows(const float* g_ent, const float* pre, const float* stats, const float* gamma, const float* beta,
-                            const double* sums, int32_t training, int64_t n_rows, int64_t n_rows_global, int32_t Dout,
-                            float* d_out, const uint8_t* keep, float keep_scale, float* d_res_in, const int32_t* slot_in,
-                            float* d_res_out, const int32_t* slot_out, const uint8_t* out_keep, float out_scale,
-                            void* stream);
+                       float* d_out, const uint8_t* keep, float keep_scale, float* d_res_in, const int32_t* slot_in,
+                       float* d_res_out, const int32_t* slot_out, const uint8_t* out_keep, float out_scale,
+                       void* stream);
 
 /* ---- K0: parameter-side work of one layer step, batched --------------------------------------------------
  * kgc_conv_prep (forward): relp = cat(rels, loop_rel) (model.py:86); all_rel = relp @ w_rel (model.py:107, all
- * n_rels + 1 rows - the caller drops the last); and the hi / lo TF32 packs kgc_gemm_nt needs for the three
+ * n_rels + 1 rows - the caller drops the last); and the hi / lo TF32 packs kgc_gemm_nt_batch needs for the three
  * transforms of the step and of its backward: packed_fwd = 3 x pack(W_h as [K = D, N = Dout]), packed_bwd =
  * 4 x pack(W_h^T as [K = Dout, N = D]), h = in, out, loop, rel, each kgc_gemm_packed_b_bytes long, the self-loop weight
  * pre-scaled by loop_rel . loop_edge (model.py:92-94 folded: (x . lr . le) @ W = x @ diag(lr . le) W).
@@ -225,8 +218,8 @@ int kgc_tail_bwd_apply_rows(const float* g_ent, const float* pre, const float* s
  *   d_w_loop = diag(lr . le) m_loop;  d_v = rowsum(m_loop . w_loop);  d_loop_edge = d_v . lr;
  *   d_relp' = d_relp + [g_rel; 0] @ w_rel^T;  d_rels = d_relp'[:-1];  d_loop_rel = d_v . le + d_relp'[-1];
  *   d_w_rel = relp^T @ [g_rel; 0]   (g_rel may be NULL: no gradient reached all_rel).
- * rel_add (optional, [n_rels, D]): the caller already holds g_rel @ w_rel^T (kgc_gemm_nt with packed_bwd[3]) and has written
- * d_w_rel itself (kgc_gemm_tn_tc) - the two products over the relation rows then run on the tensor cores instead of
+ * rel_add (optional, [n_rels, D]): the caller already holds g_rel @ w_rel^T (kgc_gemm_nt_batch with packed_bwd[3]) and has
+ * written d_w_rel itself (kgc_gemm_tn_tc_batch) - the two products over the relation rows then run on the tensor cores instead of
  * this kernel's per-thread loops (0.29 ms at 1,644 relation rows).
  * Weights are contiguous [D, Dout]; D, Dout <= 256. */
 int kgc_conv_prep(const float* rels, int32_t n_rels, const float* loop_rel, const float* loop_edge, const float* w_in,
@@ -249,26 +242,23 @@ int kgc_conv_param_grads(const float* m_loop, const float* w_loop, const float* 
 size_t kgc_gemm_packed_b_bytes(int32_t N, int32_t K);
 int kgc_gemm_pack_b(const float* B, int64_t stride_k, int64_t stride_n, int32_t N, int32_t K, float* packed,
                     void* stream);
-int kgc_gemm_nt(const float* A, int64_t M, int32_t K, int64_t lda, const float* packed_b, int32_t N, float* C,
-                int64_t ldc, void* stream);
-/* n_prob (1..3) products of IDENTICAL shape in one launch (the in / out / self-loop transforms of a layer step):
- * A[i], packed_b[i], C[i] are HOST arrays of device pointers.  The CTAs are dealt to (problem, column tile) groups. */
+/* n_prob (1..3) products of IDENTICAL shape in one launch (one product: n_prob = 1; the in / out / self-loop transforms
+ * of a layer step: 3): A[i], packed_b[i], C[i] are HOST arrays of device pointers.  The CTAs are dealt to (problem, column
+ * tile) groups.
+ * keep (NULL: none) applies dropout to the streamed operand while it is split (backward of the layer tail, model.py:103):
+ * kgc_tail_fwd's packed keep flags (byte c of row m = columns 4c..4c+3, rows keep_pitch bytes apart; problem 0 reads the
+ * low nibble, problem 1 the high nibble, problem 2 takes the operand as it is); a kept element is multiplied by
+ * keep_scale, a dropped one is 0.  The three problems may (and in the layer do) stream the SAME plane A[0] = A[1] = A[2]. */
 int kgc_gemm_nt_batch(int32_t n_prob, const float* const* A, int64_t M, int32_t K, int64_t lda,
-                      const float* const* packed_b, int32_t N, float* const* C, int64_t ldc, void* stream);
-/* The same with dropout applied to the streamed operand while it is split (backward of the layer tail, model.py:103):
- * keep = kgc_tail_fwd's packed keep flags (byte c of row m = columns 4c..4c+3; problem 0 reads the low nibble, problem 1
- * the high nibble, problem 2 takes the operand as it is); a kept element is multiplied by keep_scale, a dropped one is 0.
- * The three problems may (and in the layer do) stream the SAME plane A[0] = A[1] = A[2]. */
-int kgc_gemm_nt_batch_masked(int32_t n_prob, const float* const* A, int64_t M, int32_t K, int64_t lda,
-                             const float* const* packed_b, int32_t N, float* const* C, int64_t ldc, const uint8_t* keep,
-                             int32_t keep_pitch, float keep_scale, void* stream);
+                      const float* const* packed_b, int32_t N, float* const* C, int64_t ldc, const uint8_t* keep,
+                      int32_t keep_pitch, float keep_scale, void* stream);
 /* Same kernel with the streamed operand AND the result transposed in memory (the long dimension M contiguous):
  *   Ct[n, m] = sum_k At[k, m] * Bt[n, k],  At: [K, M] row-major, pitch ldat;  Ct: [N, M] row-major, pitch ldct.
  * M % 32 == 0.  Used for the autograd of ConvE's fc layer (model.py:173): d_W[out, flat] = d_y^T @ x_flat and
  * d_x_flat[B, flat] = d_y @ W, where flat = 39,200 is the long dimension. */
 int kgc_gemm_nt_trans(const float* At, int64_t M, int32_t K, int64_t ldat, const float* packed_b, int32_t N,
                       float* Ct, int64_t ldct, void* stream);
-/* Debug aid: device buffer of 9 x 64 int64 that CTA 0 of the next kgc_gemm_nt / kgc_gemm_tn_tc launches fills with
+/* Debug aid: device buffer of 9 x 64 int64 that CTA 0 of the next kgc_gemm_nt_batch / kgc_gemm_tn_tc_batch launches fills with
  * clock64() stamps per warp role, row 8 = global-timer envelope (NULL switches it off; off by default). */
 void kgc_gemm_set_debug(long long* buf);
 
@@ -279,12 +269,8 @@ size_t kgc_gemm_tn_workspace_bytes(int64_t M, int32_t Ka, int32_t Nb);
 int kgc_gemm_tn(const float* A, int64_t lda, const float* B, int64_t ldb, int64_t M, int32_t Ka, int32_t Nb,
                 float* C, void* workspace, size_t workspace_bytes, void* stream);
 
-/* Same product on the tensor cores (3xTF32, fp32-grade): both operands are MN-major for the MMA (TMA boxes of
- * 32 columns x 32 rows, 128-byte swizzle), both are split hi / lo in shared memory, D[128 x Nb] stays in TMEM for the
- * CTA's row slab; per-CTA partials are added in CTA order.  Ka <= 128, Nb <= 224, multiples of 4. */
+/* Same product on the tensor cores (3xTF32, fp32-grade), see kgc_gemm_tn_tc_batch below. */
 size_t kgc_gemm_tn_tc_workspace_bytes(int64_t M, int32_t Ka, int32_t Nb);
-int kgc_gemm_tn_tc(const float* A, int64_t lda, const float* B, int64_t ldb, int64_t M, int32_t Ka, int32_t Nb,
-                   float* C, void* workspace, size_t workspace_bytes, void* stream);
 
 /* Split-K product of K-major operands with a LONG contraction (ConvE's fc forward, model.py:173: y[B, out] =
  * x_flat[B, flat] @ W[out, flat]^T, flat = 39,200):  C[Ma, Nb] = A[Ma, K] @ Bt[Nb, K]^T.  The K range is cut into
@@ -293,22 +279,21 @@ int kgc_gemm_tn_tc(const float* A, int64_t lda, const float* B, int64_t ldb, int
 int kgc_gemm_nt_splitk(const float* A, int64_t lda, const float* Bt, int64_t ldb, int64_t K, int32_t Ma, int32_t Nb,
                        float* C, void* workspace, size_t workspace_bytes, void* stream);
 
-/* n_prob (1..3) weight-gradient reductions of identical shape in one launch (d_W of the in / out / self-loop
- * transforms): HOST arrays of device pointers; the CTAs are dealt to (problem, row slab) pairs, so every CTA sweeps
- * a 3x longer slab than in three separate launches and three times fewer partials are added.  Same workspace size. */
+/* n_prob (1..3) weight-gradient reductions C[i] = A[i]^T @ B[i] of identical shape in one launch on the tensor cores
+ * (3xTF32, fp32-grade; one reduction: n_prob = 1; d_W of the in / out / self-loop transforms: 3).  Both operands are
+ * MN-major for the MMA (TMA boxes of 32 columns x 32 rows, 128-byte swizzle), both are split hi / lo in shared memory,
+ * D[128 x Nb] stays in TMEM for the CTA's row slab; per-CTA partials are added in CTA order.  Ka <= 128, Nb <= 224,
+ * multiples of 4.  A, B, C are HOST arrays of device pointers; the CTAs are dealt to (problem, row slab) pairs, so every
+ * CTA sweeps a 3x longer slab than in three separate launches and three times fewer partials are added.  Workspace:
+ * kgc_gemm_tn_tc_workspace_bytes(M, Ka, Nb) for any n_prob.
+ * rows (NULL: M for every problem) = HOST array of rows[i] <= M rows in problem i (a compacted plane of the layer).  The
+ * row slabs are those of M rows: a problem of M rows gets the bits it gets with rows = NULL; the others sum the slabs
+ * their rows fill.
+ * keep (NULL: none): the keep flags applied to the B operand (the upstream plane) while it is split, as in
+ * kgc_gemm_nt_batch. */
 int kgc_gemm_tn_tc_batch(int32_t n_prob, const float* const* A, int64_t lda, const float* const* B, int64_t ldb,
-                         int64_t M, int32_t Ka, int32_t Nb, float* const* C, void* workspace, size_t workspace_bytes,
-                         void* stream);
-/* The same with rows[i] <= M rows in problem i (HOST array; a compacted plane of the layer).  The row slabs are those
- * of M rows: a problem of M rows gets the bits of kgc_gemm_tn_tc_batch; the others sum the slabs their rows fill. */
-int kgc_gemm_tn_tc_batch_rows(int32_t n_prob, const float* const* A, int64_t lda, const float* const* B, int64_t ldb,
-                              const int64_t* rows, int64_t M, int32_t Ka, int32_t Nb, float* const* C, void* workspace,
-                              size_t workspace_bytes, void* stream);
-/* The same with the keep flags applied to the B operand (the upstream plane) while it is split: see
- * kgc_gemm_nt_batch_masked. */
-int kgc_gemm_tn_tc_batch_masked(int32_t n_prob, const float* const* A, int64_t lda, const float* const* B, int64_t ldb,
-                                int64_t M, int32_t Ka, int32_t Nb, float* const* C, void* workspace, size_t workspace_bytes,
-                                const uint8_t* keep, int32_t keep_pitch, float keep_scale, void* stream);
+                         const int64_t* rows, int64_t M, int32_t Ka, int32_t Nb, float* const* C, void* workspace,
+                         size_t workspace_bytes, const uint8_t* keep, int32_t keep_pitch, float keep_scale, void* stream);
 
 /* ---- K5: label / batch builder ---------------------------------------------------------------------
  * Replaces KBDataset.get_label + label smoothing + collate (data_loader.py:25-51): for the batch's
@@ -445,8 +430,8 @@ const char* kgc_ingest_name(const kgc_ingest_t* h, int32_t kind, int64_t id);
  * TMA-stores the block transposed:  pred[b, n] = sigmoid(X[b,:] . E[n,:] + bias[n]),  pred row pitch ld_pred
  * (a multiple of 4, >= n_ent; 16-byte aligned).  D <= 256, D % 4 == 0, B <= 1024.
  * Backward through the sigmoid: d_logitT[n, b] = d_pred[b, n] * pred[b, n] * (1 - pred[b, n]) written TRANSPOSED
- * ([n_ent, ldt], ldt >= B, columns [B, ldt) zeroed) so that d_X = kgc_gemm_tn_tc(d_logitT, E) and
- * d_E = kgc_gemm_nt(d_logitT, X) stream it row-major; d_bias[n] = sum_b d_logitT[n, b] in a fixed order. */
+ * ([n_ent, ldt], ldt >= B, columns [B, ldt) zeroed) so that d_X = kgc_gemm_tn_tc_batch(d_logitT, E) and
+ * d_E = kgc_gemm_nt_batch(d_logitT, X) stream it row-major; d_bias[n] = sum_b d_logitT[n, b] in a fixed order. */
 int kgc_score_1n_fwd(const float* ent, int64_t n_ent, int32_t D, int64_t ld_ent, const float* packed_x, int32_t B,
                      const float* bias, float* pred, int64_t ld_pred, void* stream);
 /* The same product without the sigmoid: logits[b, n] = X[b,:] . E[n,:] + bias[n] (fp32-grade).  Exact-mode evaluation

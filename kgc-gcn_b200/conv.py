@@ -15,6 +15,8 @@ Backward is hand-derived (SURVEY.md Appendix A) and runs K3 / K4-backward / K4b 
 ``forward_partitioned`` is the same layer on a partitioned graph (partition.py): one process per GPU, exchanges over
 NVLink peer memory (K10).
 """
+import ctypes
+
 import torch
 import torch.nn as nn
 
@@ -40,6 +42,30 @@ def _mm(a, b, out):
     return torch.mm(a, b, out=out)
 
 
+def _workspace(plan, name, nbytes, device):
+    """A float32 buffer of nbytes: the plan's scratch buffer ``name`` when there is a plan (the same memory on every step, as
+    a captured CUDA graph needs), else a new tensor."""
+    if plan is not None:
+        return plan.scratch(name, (nbytes // 4,))
+    return torch.empty((nbytes // 4,), dtype=torch.float32, device=device)
+
+
+def _ptr_array(ts):
+    return (ctypes.c_void_p * len(ts))(*[t.data_ptr() for t in ts])
+
+
+def _pack_b(b_kn, plan=None, name=None):
+    """The small operand of K4b, b_kn[K, N] (any strided view: a weight, its transpose, a query block), split into hi / lo
+    TF32 and packed by kgc_gemm_pack_b into a workspace buffer (see _workspace)."""
+    K, N = b_kn.shape
+    nbytes = int(_lib.lib().kgc_gemm_packed_b_bytes(N, K))
+    if nbytes == 0:
+        raise ValueError('unsupported small operand K={} N={} (K <= 256, N <= 1024)'.format(K, N))
+    packed = _workspace(plan, name, nbytes, b_kn.device)
+    _lib.call('kgc_gemm_pack_b', _lib.ptr(b_kn), b_kn.stride(0), b_kn.stride(1), N, K, _lib.ptr(packed), _lib.stream())
+    return packed
+
+
 def gemm_nt(a, b_kn, out, plan=None, tag='b', packed=None):
     """out[M, N] = a[M, K] @ b_kn[K, N] on the tensor cores with fp32-grade accuracy (K4b, 3xTF32).
     ``a`` and ``out`` are row-major (possibly row-strided views); ``b_kn`` is any strided [K, N] view of the small
@@ -48,18 +74,14 @@ def gemm_nt(a, b_kn, out, plan=None, tag='b', packed=None):
     N = out.shape[1]
     if a.stride(1) != 1 or out.stride(1) != 1:
         raise ValueError('gemm_nt needs unit inner strides')
-    p = _lib.ptr
-    if packed is None:                                  # ``packed``: the operand already split by kgc_conv_prep / kgc_gemm_pack_b
-        nbytes = int(_lib.lib().kgc_gemm_packed_b_bytes(N, K))
-        if nbytes == 0:
-            raise ValueError('gemm_nt: unsupported shape K={} N={}'.format(K, N))
-        packed = plan.scratch('gemm_pack_' + tag, (nbytes // 4,)) if plan is not None else \
-            torch.empty((nbytes // 4,), dtype=torch.float32, device=a.device)
-        _lib.call('kgc_gemm_pack_b', p(b_kn), b_kn.stride(0), b_kn.stride(1), N, K, p(packed), _lib.stream())
+    if packed is None:                                  # ``packed``: the operand already split by kgc_conv_prep / _pack_b
+        if tuple(b_kn.shape) != (K, N):
+            raise ValueError('gemm_nt: b_kn must be [K, N] = [{}, {}]'.format(K, N))
+        packed = _pack_b(b_kn, plan, 'gemm_pack_' + tag)
     # C is written by TMA stores: 16-byte aligned rows; an odd pitch goes through a padded buffer
     dst = out if (out.data_ptr() % 16 == 0 and out.stride(0) % 4 == 0) else \
         torch.empty((M, (N + 3) // 4 * 4), dtype=torch.float32, device=a.device)[:, :N]
-    _lib.call('kgc_gemm_nt', p(a), M, K, a.stride(0), p(packed), N, p(dst), dst.stride(0), _lib.stream())
+    gemm_nt_batch([a], [packed], [dst])
     if dst is not out:
         out.copy_(dst)
     return out
@@ -67,80 +89,56 @@ def gemm_nt(a, b_kn, out, plan=None, tag='b', packed=None):
 
 def gemm_nt_batch(a_list, packed_list, out_list, keep=None, keep_scale=1.0):
     """Up to three products out_i = a_i @ B_i of identical shape in ONE launch (K4b); ``packed_list`` holds the split small
-    operands (kgc_conv_prep / kgc_gemm_pack_b).  ``keep`` (uint8 [M, pitch], kgc_tail_fwd's packed keep flags): dropout of
-    the streamed operand while it is split - problem 0 by the low nibbles, problem 1 by the high nibbles, problem 2 as it is."""
-    import ctypes
-    n = len(a_list)
+    operands (kgc_conv_prep / _pack_b).  ``keep`` (uint8 [M, pitch], kgc_tail_fwd's packed keep flags): dropout of the
+    streamed operand while it is split - problem 0 by the low nibbles, problem 1 by the high nibbles, problem 2 as it is."""
     M, K = a_list[0].shape
     N = out_list[0].shape[1]
     lda, ldc = a_list[0].stride(0), out_list[0].stride(0)
     for a, o in zip(a_list, out_list):
         if a.shape != (M, K) or o.shape != (M, N) or a.stride() != (lda, 1) or o.stride() != (ldc, 1):
             raise ValueError('gemm_nt_batch needs operands of identical shape and strides')
-    arr = lambda ts: (ctypes.c_void_p * n)(*[t.data_ptr() for t in ts])       # noqa: E731
-    if keep is not None:
-        _lib.call('kgc_gemm_nt_batch_masked', n, arr(a_list), M, K, lda, arr(packed_list), N, arr(out_list), ldc,
-                  _lib.ptr(keep), keep.stride(0), float(keep_scale), _lib.stream())
-    else:
-        _lib.call('kgc_gemm_nt_batch', n, arr(a_list), M, K, lda, arr(packed_list), N, arr(out_list), ldc, _lib.stream())
+    _lib.call('kgc_gemm_nt_batch', len(a_list), _ptr_array(a_list), M, K, lda, _ptr_array(packed_list), N, _ptr_array(out_list),
+              ldc, _lib.ptr(keep), 0 if keep is None else keep.stride(0), float(keep_scale), _lib.stream())
     return out_list
 
 
-def gemm_tn_batch(a_list, b_list, out_list, plan=None, keep=None, keep_scale=1.0):
-    """Up to three weight-gradient reductions out_i = a_i^T @ b_i of identical shape in ONE launch (K4c on the tensor
-    cores; Ka <= 128, Nb <= 224 - wider shapes go through gemm_tn one by one)."""
-    import ctypes
+def _gemm_tn_tc(a_list, b_list, out_list, M, plan, rows=None, keep=None, keep_scale=1.0):
+    """One kgc_gemm_tn_tc_batch launch on operands the caller has checked."""
     n = len(a_list)
-    M, Ka = a_list[0].shape
-    Nb = b_list[0].shape[1]
-    lda, ldb = a_list[0].stride(0), b_list[0].stride(0)
-    same = all(a.shape == (M, Ka) and b.shape == (M, Nb) and a.stride() == (lda, 1) and b.stride() == (ldb, 1)
-               and o.is_contiguous() for a, b, o in zip(a_list, b_list, out_list))
-    if not same or Ka > 128 or Nb > 224:
-        if keep is not None:
-            raise ValueError('gemm_tn_batch: the masked form needs Ka <= 128, Nb <= 224 and operands of identical shape')
-        for a, b, o in zip(a_list, b_list, out_list):
-            gemm_tn(a, b, o, plan)
-        return out_list
+    Ka, Nb = a_list[0].shape[1], b_list[0].shape[1]
     nbytes = int(_lib.lib().kgc_gemm_tn_tc_workspace_bytes(M, Ka, Nb))
-    ws = plan.scratch('kgc_gemm_tn_tc_ws', (nbytes // 4,)) if plan is not None else \
-        torch.empty((nbytes // 4,), dtype=torch.float32, device=a_list[0].device)
-    arr = lambda ts: (ctypes.c_void_p * n)(*[t.data_ptr() for t in ts])       # noqa: E731
-    if keep is not None:
-        _lib.call('kgc_gemm_tn_tc_batch_masked', n, arr(a_list), lda, arr(b_list), ldb, M, Ka, Nb, arr(out_list), _lib.ptr(ws),
-                  nbytes, _lib.ptr(keep), keep.stride(0), float(keep_scale), _lib.stream())
-    else:
-        _lib.call('kgc_gemm_tn_tc_batch', n, arr(a_list), lda, arr(b_list), ldb, M, Ka, Nb, arr(out_list), _lib.ptr(ws), nbytes,
-                  _lib.stream())
-    return out_list
+    ws = _workspace(plan, 'kgc_gemm_tn_tc_ws', nbytes, a_list[0].device)
+    _lib.call('kgc_gemm_tn_tc_batch', n, _ptr_array(a_list), a_list[0].stride(0), _ptr_array(b_list), b_list[0].stride(0),
+              None if rows is None else (ctypes.c_int64 * n)(*rows), M, Ka, Nb, _ptr_array(out_list), _lib.ptr(ws), nbytes,
+              _lib.ptr(keep), 0 if keep is None else keep.stride(0), float(keep_scale), _lib.stream())
 
 
-def gemm_tn_batch_rows(a_list, b_list, out_list, rows, plan=None):
-    """gemm_tn_batch with rows[i] <= M leading rows of problem i (M = the operands' row count): one launch whose problems of
-    M rows get exactly the bits of gemm_tn_batch; a shorter problem (a compacted plane) sums only the slabs its rows fill."""
-    import ctypes
-    n = len(a_list)
+def gemm_tn_batch(a_list, b_list, out_list, plan=None, keep=None, keep_scale=1.0, rows=None):
+    """Up to three weight-gradient reductions out_i = a_i^T @ b_i of identical shape in ONE launch (K4c on the tensor
+    cores; Ka <= 128, Nb <= 224 - wider shapes go through gemm_tn one by one).  ``keep``: the b operands dropped while they
+    are split, as in gemm_nt_batch.  ``rows``: rows[i] <= M leading rows of problem i (M = the operands' row count): the
+    problems of M rows get exactly the bits they get without ``rows``; a shorter problem (a compacted plane) sums only the
+    slabs its rows fill."""
     M = max(a.shape[0] for a in a_list)
     Ka, Nb = a_list[0].shape[1], b_list[0].shape[1]
     lda, ldb = a_list[0].stride(0), b_list[0].stride(0)
-    ok = all(a.shape[1] == Ka and b.shape[1] == Nb and a.stride(1) == 1 and b.stride(1) == 1 and a.stride(0) == lda
-             and b.stride(0) == ldb and a.shape[0] >= r and b.shape[0] >= r and o.is_contiguous()
-             for a, b, o, r in zip(a_list, b_list, out_list, rows))
-    if not ok or max(rows) != M:
-        raise ValueError('gemm_tn_batch_rows needs operands of identical widths and strides and rows <= their heights')
-    if Ka > 128 or Nb > 224:                            # wide shapes: one gemm_tn per problem
-        for a, b, o, r in zip(a_list, b_list, out_list, rows):
+    fits = all(a.shape[1] == Ka and b.shape[1] == Nb and a.stride() == (lda, 1) and b.stride() == (ldb, 1) and o.is_contiguous()
+               for a, b, o in zip(a_list, b_list, out_list))
+    if rows is None:
+        fits = fits and all(a.shape[0] == M and b.shape[0] == M for a, b in zip(a_list, b_list))
+    elif not fits or max(rows) != M or any(a.shape[0] < r or b.shape[0] < r for a, b, r in zip(a_list, b_list, rows)):
+        raise ValueError('gemm_tn_batch with rows needs operands of identical widths and strides and rows <= their heights')
+    if not fits or Ka > 128 or Nb > 224:                # one gemm_tn per problem
+        if keep is not None:
+            raise ValueError('gemm_tn_batch: the masked form needs Ka <= 128, Nb <= 224 and operands of identical shape')
+        for i, (a, b, o) in enumerate(zip(a_list, b_list, out_list)):
+            r = a.shape[0] if rows is None else rows[i]
             if r:
                 gemm_tn(a[:r], b[:r], o, plan)
             else:
                 o.zero_()
         return out_list
-    nbytes = int(_lib.lib().kgc_gemm_tn_tc_workspace_bytes(M, Ka, Nb))
-    ws = plan.scratch('kgc_gemm_tn_tc_ws', (nbytes // 4,)) if plan is not None else \
-        torch.empty((nbytes // 4,), dtype=torch.float32, device=a_list[0].device)
-    arr = lambda ts: (ctypes.c_void_p * n)(*[t.data_ptr() for t in ts])       # noqa: E731
-    _lib.call('kgc_gemm_tn_tc_batch_rows', n, arr(a_list), lda, arr(b_list), ldb, (ctypes.c_int64 * n)(*rows), M, Ka, Nb,
-              arr(out_list), _lib.ptr(ws), nbytes, _lib.stream())
+    _gemm_tn_tc(a_list, b_list, out_list, M, plan, rows, keep, keep_scale)
     return out_list
 
 
@@ -148,16 +146,6 @@ def rows_copy(src, src_rows, dst, dst_rows, n):
     """dst[dst_rows[j]] = src[src_rows[j]] for j < n (row lists int32 or None = the identity; one launch, none for n = 0)."""
     _lib.call('kgc_rows_copy', _lib.ptr(src), src.stride(0), _lib.ptr(src_rows), _lib.ptr(dst), dst.stride(0), _lib.ptr(dst_rows),
               int(n), src.shape[1], _lib.stream())
-
-
-def _pack_b(b_kn):
-    K, N = b_kn.shape
-    nbytes = int(_lib.lib().kgc_gemm_packed_b_bytes(N, K))
-    if nbytes == 0:
-        raise ValueError('unsupported small operand K={} N={} (K <= 256, N <= 1024)'.format(K, N))
-    packed = torch.empty((nbytes // 4,), dtype=torch.float32, device=b_kn.device)
-    _lib.call('kgc_gemm_pack_b', _lib.ptr(b_kn), b_kn.stride(0), b_kn.stride(1), N, K, _lib.ptr(packed), _lib.stream())
-    return packed
 
 
 def gemm_nt_trans(a_t, b_kn, out_t):
@@ -252,15 +240,16 @@ def gemm_tn(a, b, out, plan=None, tensor_cores=True):
         raise ValueError('gemm_tn needs unit inner strides and a contiguous output')
     if Nb > 256:
         raise ValueError('gemm_tn supports Nb <= 256')
-    name = 'kgc_gemm_tn_tc' if (tensor_cores and Nb <= 224) else 'kgc_gemm_tn'
     for i0 in range(0, Ka, 128):                       # wider A: one call per block of 128 columns (= 128 contiguous rows of out)
         kb = min(128, Ka - i0)
         a_blk, out_blk = a[:, i0:i0 + kb], out[i0:i0 + kb]
-        nbytes = int(getattr(_lib.lib(), name + '_workspace_bytes')(M, kb, Nb))
-        ws = plan.scratch(name + '_ws', (nbytes // 4,)) if plan is not None else \
-            torch.empty((nbytes // 4,), dtype=torch.float32, device=a.device)
-        p = _lib.ptr
-        _lib.call(name, p(a_blk), a.stride(0), p(b), b.stride(0), M, kb, Nb, p(out_blk), p(ws), nbytes, _lib.stream())
+        if tensor_cores and Nb <= 224:
+            _gemm_tn_tc([a_blk], [b], [out_blk], M, plan)
+        else:
+            nbytes = int(_lib.lib().kgc_gemm_tn_workspace_bytes(M, kb, Nb))
+            ws = _workspace(plan, 'kgc_gemm_tn_ws', nbytes, a.device)
+            p = _lib.ptr
+            _lib.call('kgc_gemm_tn', p(a_blk), a.stride(0), p(b), b.stride(0), M, kb, Nb, p(out_blk), p(ws), nbytes, _lib.stream())
     return out
 
 
@@ -479,13 +468,9 @@ class _ConvFn(torch.autograd.Function):
         # ONE upstream plane (no masked planes are written, nothing is regenerated)
         dropping = (mask_in is not None or seed is not None) and drop_p > 0.0
         keep = torch.empty((Nl, int(_lib.lib().kgc_keep_pitch())), dtype=torch.uint8, device=x.device) if dropping else None
-        if any(comp):
-            _lib.call('kgc_tail_fwd_rows', p(res3), p(plan.slot[0]) if comp[0] else None, p(res_c[0]),
-                      p(plan.slot[1]) if comp[1] else None, p(res_c[1]), p(mask_in), p(mask_out), p(seed), float(drop_p),
-                      float(keep_scale), p(bias), Nl, Dout, p(pre), p(partials), p(keep), st())
-        else:
-            _lib.call('kgc_tail_fwd', p(res3), p(mask_in), p(mask_out), p(seed), float(drop_p), float(keep_scale), p(bias),
-                      Nl, Dout, p(pre), p(partials), p(keep), st())
+        _lib.call('kgc_tail_fwd', p(res3), p(plan.slot[0]) if comp[0] else None, p(res_c[0]), p(plan.slot[1]) if comp[1] else None,
+                  p(res_c[1]), p(mask_in), p(mask_out), p(seed), float(drop_p), float(keep_scale), p(bias), Nl, Dout, p(pre),
+                  p(partials), p(keep), st())
         if training and coll is None:
             # one GPU: column sums -> batch statistics -> nn.BatchNorm1d's running-statistics bookkeeping in ONE launch
             # (bn_track = (momentum, num_batches_tracked) when the module tracks running statistics)
@@ -553,7 +538,7 @@ class _ConvFn(torch.autograd.Function):
         three = 3 * Nl * Dout * 4 > TAIL_MASKED_MAX_BYTES or any(comp)
         d_res = [(plan.scratch('d_res_c%d' % h, (max(plan.n_c[h], 1), Dout)) if comp[h] else plan.scratch('d_res2_%d' % h, (Nl, Dout)))
                  if three else None for h in (0, 1)]
-        _lib.call('kgc_tail_bwd_apply_rows', p(g_ent), p(pre), p(stats), p(gamma), p(beta), p(sums), int(ctx.training), Nl,
+        _lib.call('kgc_tail_bwd_apply', p(g_ent), p(pre), p(stats), p(gamma), p(beta), p(sums), int(ctx.training), Nl,
                   n_global, Dout, p(d_out), p(keep), ctx.keep_scale, p(d_res[0]), p(plan.slot[0]) if comp[0] else None,
                   p(d_res[1]), p(plan.slot[1]) if comp[1] else None, p(out_keep), ctx.out_scale, st())
         ups = [d_res[0], d_res[1], d_out] if three else [d_out, d_out, d_out]
@@ -570,13 +555,10 @@ class _ConvFn(torch.autograd.Function):
         main, side = torch.cuda.current_stream(), plan.side_stream()
         side.wait_stream(main)
         with torch.cuda.stream(side):
-            if any(comp):                                       # a compacted half sums its n_c rows
-                agg_c = (agg_c0, agg_c1)
-                gemm_tn_batch_rows([agg_c[h] if comp[h] else agg[h, :Nl] for h in (0, 1)] + [x], ups,
-                                   [d_w_in, d_w_out, m_loop], [plan.n_c[h] if comp[h] else Nl for h in (0, 1)] + [Nl], plan)
-            else:
-                gemm_tn_batch([agg[0, :Nl], agg[1, :Nl], x], ups, [d_w_in, d_w_out, m_loop], plan,
-                              keep=gkeep, keep_scale=ctx.keep_scale)                                     # [D, Dout] each
+            agg_c = (agg_c0, agg_c1)                            # a compacted half sums its n_c rows
+            gemm_tn_batch([agg_c[h] if comp[h] else agg[h, :Nl] for h in (0, 1)] + [x], ups, [d_w_in, d_w_out, m_loop], plan,
+                          keep=gkeep, keep_scale=ctx.keep_scale,
+                          rows=[plan.n_c[h] if comp[h] else Nl for h in (0, 1)] + [Nl] if any(comp) else None)   # [D, Dout] each
             if ctx.has_bias:
                 torch.sum(d_out, 0, out=flat[3 * D * Dout + T * D:])
 

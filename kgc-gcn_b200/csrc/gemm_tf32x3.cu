@@ -22,9 +22,7 @@
 //   warp 1      one thread issues 3 tcgen05.mma (M = 128, N = NT, K = 8) per 8-wide k-step
 //   warps 10-13 epilogue: tcgen05.ld -> 32x32 transpose through shared memory -> coalesced 128-byte row segments of C
 //   warp 14     TMEM allocator (2 accumulator stages)
-#include <cuda.h>
-
-#include "common.cuh"
+#include "tcgen05.cuh"
 
 namespace kgc {
 namespace {
@@ -46,99 +44,6 @@ constexpr int kTmemColsG = 256;
 constexpr int kEpiBuf = 32 * 128;          // one epilogue buffer: a TMA-store box of 32 rows x 32 fp32 columns
 constexpr int kEpiStage = 4 * 2 * kEpiBuf; // 4 epilogue warps, double buffered (32 KB)
 
-__device__ __forceinline__ uint32_t s_u32(const void* p) { return (uint32_t)__cvta_generic_to_shared(p); }
-__device__ __forceinline__ void mb_init(uint64_t* bar, uint32_t count) {
-  asm volatile("mbarrier.init.shared::cta.b64 [%0], %1;" ::"r"(s_u32(bar)), "r"(count));
-}
-__device__ __forceinline__ void mb_expect_tx(uint64_t* bar, uint32_t bytes) {
-  asm volatile("mbarrier.arrive.expect_tx.shared::cta.b64 _, [%0], %1;" ::"r"(s_u32(bar)), "r"(bytes) : "memory");
-}
-__device__ __forceinline__ void mb_arrive(uint64_t* bar) {
-  asm volatile("mbarrier.arrive.shared::cta.b64 _, [%0];" ::"r"(s_u32(bar)) : "memory");
-}
-__device__ __forceinline__ void mb_wait(uint64_t* bar, uint32_t parity) {
-  asm volatile(
-      "{\n"
-      ".reg .pred P1;\n"
-      "LAB_WAIT:\n"
-      "mbarrier.try_wait.parity.shared::cta.b64 P1, [%0], %1;\n"
-      "@P1 bra DONE;\n"
-      "bra LAB_WAIT;\n"
-      "DONE:\n"
-      "}" ::"r"(s_u32(bar)),
-      "r"(parity)
-      : "memory");
-}
-__device__ __forceinline__ void tma_2d(void* smem_dst, const CUtensorMap* map, uint64_t* bar, int c0, int c1) {
-  asm volatile(
-      "cp.async.bulk.tensor.2d.shared::cluster.global.mbarrier::complete_tx::bytes [%0], [%1, {%3, %4}], [%2];" ::"r"(
-          s_u32(smem_dst)),
-      "l"(reinterpret_cast<uint64_t>(map)), "r"(s_u32(bar)), "r"(c0), "r"(c1)
-      : "memory");
-}
-__device__ __forceinline__ void tma_3d(void* smem_dst, const CUtensorMap* map, uint64_t* bar, int c0, int c1, int c2) {
-  asm volatile(
-      "cp.async.bulk.tensor.3d.shared::cluster.global.mbarrier::complete_tx::bytes [%0], [%1, {%3, %4, %5}], [%2];" ::"r"(
-          s_u32(smem_dst)),
-      "l"(reinterpret_cast<uint64_t>(map)), "r"(s_u32(bar)), "r"(c0), "r"(c1), "r"(c2)
-      : "memory");
-}
-__device__ __forceinline__ void tma_store_2d(const CUtensorMap* map, const void* smem_src, int c0, int c1) {
-  asm volatile("cp.async.bulk.tensor.2d.global.shared::cta.bulk_group [%0, {%2, %3}], [%1];" ::"l"(
-                   reinterpret_cast<uint64_t>(map)),
-               "r"(s_u32(smem_src)), "r"(c0), "r"(c1)
-               : "memory");
-}
-__device__ __forceinline__ void tma_store_3d(const CUtensorMap* map, const void* smem_src, int c0, int c1, int c2) {
-  asm volatile("cp.async.bulk.tensor.3d.global.shared::cta.bulk_group [%0, {%2, %3, %4}], [%1];" ::"l"(
-                   reinterpret_cast<uint64_t>(map)),
-               "r"(s_u32(smem_src)), "r"(c0), "r"(c1), "r"(c2)
-               : "memory");
-}
-__device__ __forceinline__ void umma_tf32(uint32_t tmem_d, uint64_t adesc, uint64_t bdesc, uint32_t idesc, uint32_t acc) {
-  asm volatile(
-      "{\n"
-      ".reg .pred p;\n"
-      "setp.ne.b32 p, %4, 0;\n"
-      "tcgen05.mma.cta_group::1.kind::tf32 [%0], %1, %2, %3, p;\n"
-      "}" ::"r"(tmem_d),
-      "l"(adesc), "l"(bdesc), "r"(idesc), "r"(acc)
-      : "memory");
-}
-// TS form: the A operand (128 rows x 8 TF32) is read from tensor memory, [lane 0.., column a_tmem..a_tmem+7]
-__device__ __forceinline__ void umma_tf32_ts(uint32_t tmem_d, uint32_t a_tmem, uint64_t bdesc, uint32_t idesc, uint32_t acc) {
-  asm volatile(
-      "{\n"
-      ".reg .pred p;\n"
-      "setp.ne.b32 p, %4, 0;\n"
-      "tcgen05.mma.cta_group::1.kind::tf32 [%0], [%1], %2, %3, p;\n"
-      "}" ::"r"(tmem_d),
-      "r"(a_tmem), "l"(bdesc), "r"(idesc), "r"(acc)
-      : "memory");
-}
-__device__ __forceinline__ void tmem_st16_g(uint32_t taddr, const uint32_t (&v)[16]) {
-  asm volatile(
-      "tcgen05.st.sync.aligned.32x32b.x16.b32 [%0], "
-      "{%1, %2, %3, %4, %5, %6, %7, %8, %9, %10, %11, %12, %13, %14, %15, %16};" ::"r"(taddr),
-      "r"(v[0]), "r"(v[1]), "r"(v[2]), "r"(v[3]), "r"(v[4]), "r"(v[5]), "r"(v[6]), "r"(v[7]), "r"(v[8]), "r"(v[9]),
-      "r"(v[10]), "r"(v[11]), "r"(v[12]), "r"(v[13]), "r"(v[14]), "r"(v[15])
-      : "memory");
-}
-// One lane of a fully converged warp (PTX elect.sync).  The surrounding code stays warp-uniform, so ptxas keeps the
-// shared-memory / instruction descriptors in UNIFORM registers; running the whole role under `if (lane == 0)` makes
-// them per-thread values and every tcgen05.mma then pays a chain of R2UR moves (~120 cycles per MMA, measured).
-__device__ __forceinline__ bool elect_one() {
-  uint32_t pred = 0;
-  asm volatile(
-      "{\n"
-      ".reg .b32 rx;\n"
-      ".reg .pred px;\n"
-      "elect.sync rx|px, 0xFFFFFFFF;\n"
-      "@px mov.s32 %0, 1;\n"
-      "}"
-      : "+r"(pred));
-  return pred != 0;
-}
 // Round to the nearest TF32 (10-bit mantissa, ties away from zero = cvt.rna.tf32.f32), result in fp32 bits.  Done with
 // two integer instructions: cvt.rna runs on the quarter-rate conversion pipe (16 lanes / clock / SM), which made the
 // splitter warps the bottleneck of both GEMM kernels (measured: ~512 cycles per 128 x 32 tile for the cvt alone).
@@ -146,29 +51,6 @@ __device__ __forceinline__ uint32_t tf32_rn(float v) { return (__float_as_uint(v
 __device__ __forceinline__ void split_tf32(uint32_t v, uint32_t& hi, uint32_t& lo) {
   hi = tf32_rn(__uint_as_float(v));
   lo = tf32_rn(__uint_as_float(v) - __uint_as_float(hi));
-}
-__device__ __forceinline__ void umma_commit_g(uint64_t* bar) {
-  asm volatile("tcgen05.commit.cta_group::1.mbarrier::arrive::one.shared::cluster.b64 [%0];" ::"r"(s_u32(bar)) : "memory");
-}
-__device__ __forceinline__ void tmem_ld32_g(uint32_t taddr, uint32_t (&v)[32]) {
-  asm volatile(
-      "tcgen05.ld.sync.aligned.32x32b.x32.b32 "
-      "{%0, %1, %2, %3, %4, %5, %6, %7, %8, %9, %10, %11, %12, %13, %14, %15, "
-      "%16, %17, %18, %19, %20, %21, %22, %23, %24, %25, %26, %27, %28, %29, %30, %31}, [%32];"
-      : "=r"(v[0]), "=r"(v[1]), "=r"(v[2]), "=r"(v[3]), "=r"(v[4]), "=r"(v[5]), "=r"(v[6]), "=r"(v[7]), "=r"(v[8]),
-        "=r"(v[9]), "=r"(v[10]), "=r"(v[11]), "=r"(v[12]), "=r"(v[13]), "=r"(v[14]), "=r"(v[15]), "=r"(v[16]),
-        "=r"(v[17]), "=r"(v[18]), "=r"(v[19]), "=r"(v[20]), "=r"(v[21]), "=r"(v[22]), "=r"(v[23]), "=r"(v[24]),
-        "=r"(v[25]), "=r"(v[26]), "=r"(v[27]), "=r"(v[28]), "=r"(v[29]), "=r"(v[30]), "=r"(v[31])
-      : "r"(taddr));
-}
-// K-major tile, 128-byte swizzle (rows of 32 fp32), 8-row atoms 1024 B apart
-__device__ __forceinline__ uint64_t sw128_desc(uint32_t smem_addr) {
-  uint64_t d = 0;
-  d |= (uint64_t)((smem_addr & 0x3FFFF) >> 4);
-  d |= (uint64_t)(1024 >> 4) << 32;
-  d |= (uint64_t)1 << 46;
-  d |= (uint64_t)2 << 61;
-  return d;
 }
 
 constexpr int kMaxBatch = 3;               // problems of one launch (same shapes, different operands): in / out / loop halves
@@ -225,30 +107,26 @@ gemm_tf32x3_kernel(const __grid_constant__ GemmMaps maps, const GemmParams P) {
   uint32_t* tmem_slot = reinterpret_cast<uint32_t*>(acc_empty + 2);
 
   if (warp == 0 && lane == 0) {
-    mb_init(b_full, 1);
+    mbar_init(b_full, 1);
     for (int i = 0; i < kStages; ++i) {
-      mb_init(raw_full + i, 1);
-      mb_init(raw_empty + i, kSplitWarps);
+      mbar_init(raw_full + i, 1);
+      mbar_init(raw_empty + i, kSplitWarps);
     }
     for (int i = 0; i < kAStages; ++i) {
-      mb_init(split_full + i, kSplitWarps);
-      mb_init(split_empty + i, 1);
+      mbar_init(split_full + i, kSplitWarps);
+      mbar_init(split_empty + i, 1);
     }
     for (int i = 0; i < 2; ++i) {
-      mb_init(acc_full + i, 1);
-      mb_init(acc_empty + i, 4);
+      mbar_init(acc_full + i, 1);
+      mbar_init(acc_empty + i, 4);
     }
-    asm volatile("fence.mbarrier_init.release.cluster;" ::: "memory");
-    asm volatile("fence.proxy.async.shared::cta;" ::: "memory");
+    fence_barrier_init();
+    fence_proxy_async();
   }
-  if (warp == 14) {
-    asm volatile("tcgen05.alloc.cta_group::1.sync.aligned.shared::cta.b32 [%0], %1;" ::"r"(s_u32(tmem_slot)), "r"(kTmemColsTS)
-                 : "memory");
-    asm volatile("tcgen05.relinquish_alloc_permit.cta_group::1.sync.aligned;" ::: "memory");
-  }
-  asm volatile("tcgen05.fence::before_thread_sync;" ::: "memory");
+  if (warp == 14) tmem_alloc(tmem_slot, kTmemColsTS);
+  tc_fence_before();
   __syncthreads();
-  asm volatile("tcgen05.fence::after_thread_sync;" ::: "memory");
+  tc_fence_after();
   const uint32_t tmem_base = *tmem_slot;
   const uint32_t tmem_a = tmem_base + kAccCols;                    // A stages: [kAStages][hi 32 columns | lo 32 columns]
   const bool dbg_on = P.dbg != nullptr && blockIdx.x == 0;
@@ -269,20 +147,20 @@ gemm_tf32x3_kernel(const __grid_constant__ GemmMaps maps, const GemmParams P) {
 
   if (warp == 0) {
     if (lane == 0) {
-      mb_expect_tx(b_full, 2u * P.n_kb * tile_b);
+      mbar_expect_tx(b_full, 2u * P.n_kb * tile_b);
       for (int kb = 0; kb < P.n_kb; ++kb) {
-        tma_2d(s_bhi + kb * tile_b_al, map_bhi, b_full, kb * kBK, nt * P.NT);
-        tma_2d(s_blo + kb * tile_b_al, map_blo, b_full, kb * kBK, nt * P.NT);
+        tma_load_2d(s_bhi + kb * tile_b_al, map_bhi, b_full, kb * kBK, nt * P.NT);
+        tma_load_2d(s_blo + kb * tile_b_al, map_blo, b_full, kb * kBK, nt * P.NT);
       }
       int stage = 0;
       uint32_t phase = 0;
       for (int mt = first; mt < P.n_mtiles; mt += step) {
         for (int kb = 0; kb < P.n_kb; ++kb) {
-          mb_wait(raw_empty + stage, phase ^ 1);
+          mbar_wait(raw_empty + stage, phase ^ 1);
           KGC_DBG(0);
-          mb_expect_tx(raw_full + stage, kTileA);
-          if (P.trans_a) tma_3d(s_a + stage * kTileA, map_a, raw_full + stage, 0, kb * kBK, mt * (kBM / 32));
-          else tma_2d(s_a + stage * kTileA, map_a, raw_full + stage, kb * kBK, mt * kBM);
+          mbar_expect_tx(raw_full + stage, kTileA);
+          if (P.trans_a) tma_load_3d(s_a + stage * kTileA, map_a, raw_full + stage, 0, kb * kBK, mt * (kBM / 32));
+          else tma_load_2d(s_a + stage * kTileA, map_a, raw_full + stage, kb * kBK, mt * kBM);
           if (++stage == kStages) { stage = 0; phase ^= 1; }
         }
       }
@@ -331,7 +209,7 @@ gemm_tf32x3_kernel(const __grid_constant__ GemmMaps maps, const GemmParams P) {
             if (kb == j) kw = kcur[j];
           if (prob == 1) kw >>= 4;
         }
-        mb_wait(raw_full + stage, phase);
+        mbar_wait(raw_full + stage, phase);
         if (warp == 2 && lane == 0) KGC_DBG(1);
         uint32_t h[16], l[16];
         if (P.trans_a) {
@@ -369,17 +247,17 @@ gemm_tf32x3_kernel(const __grid_constant__ GemmMaps maps, const GemmParams P) {
           }
         }
         __syncwarp();
-        if (lane == 0) mb_arrive(raw_empty + stage);               // the raw tile is in registers: hand the stage back to TMA
-        mb_wait(split_empty + ts, tphase ^ 1);                     // the MMAs that read this TMEM stage have retired
+        if (lane == 0) mbar_arrive(raw_empty + stage);               // the raw tile is in registers: hand the stage back to TMA
+        mbar_wait(split_empty + ts, tphase ^ 1);                     // the MMAs that read this TMEM stage have retired
         if (warp == 2 && lane == 0) KGC_DBG(2);
-        asm volatile("tcgen05.fence::after_thread_sync;" ::: "memory");
+        tc_fence_after();
         const uint32_t taddr = tmem_a + ((uint32_t)(quarter * 32) << 16) + ts * 64 + half * 16;
-        tmem_st16_g(taddr, h);
-        tmem_st16_g(taddr + 32, l);
-        asm volatile("tcgen05.wait::st.sync.aligned;" ::: "memory");
-        asm volatile("tcgen05.fence::before_thread_sync;" ::: "memory");
+        tmem_st16(taddr, h);
+        tmem_st16(taddr + 32, l);
+        tmem_st_wait();
+        tc_fence_before();
         __syncwarp();
-        if (lane == 0) mb_arrive(split_full + ts);
+        if (lane == 0) mbar_arrive(split_full + ts);
         if (warp == 2 && lane == 0) KGC_DBG(3);
         if (++stage == kStages) { stage = 0; phase ^= 1; }
         if (++ts == kAStages) { ts = 0; tphase ^= 1; }
@@ -391,20 +269,20 @@ gemm_tf32x3_kernel(const __grid_constant__ GemmMaps maps, const GemmParams P) {
       const uint32_t idesc = (1u << 4) | (2u << 7) | (2u << 10) | ((uint32_t)(P.NT >> 3) << 17) | ((uint32_t)(kBM >> 4) << 24);
       int ts = 0, acc = 0;
       uint32_t tphase = 0, acc_phase = 0;
-      mb_wait(b_full, 0);
-      asm volatile("tcgen05.fence::after_thread_sync;" ::: "memory");
+      mbar_wait(b_full, 0);
+      tc_fence_after();
       for (int mt = first; mt < P.n_mtiles; mt += step) {
-        mb_wait(acc_empty + acc, acc_phase ^ 1);
-        asm volatile("tcgen05.fence::after_thread_sync;" ::: "memory");
+        mbar_wait(acc_empty + acc, acc_phase ^ 1);
+        tc_fence_after();
         const uint32_t d_addr = tmem_base + acc * (kAccCols / 2);
         for (int kb = 0; kb < P.n_kb; ++kb) {
-          mb_wait(split_full + ts, tphase);
+          mbar_wait(split_full + ts, tphase);
           if (lane == 0) KGC_DBG(4);
-          asm volatile("tcgen05.fence::after_thread_sync;" ::: "memory");
+          tc_fence_after();
           const int nk = min(kBK / kUK, P.ksteps - kb * (kBK / kUK));
           const uint32_t a_hi = tmem_a + ts * 64, a_lo = a_hi + 32;            // TS mode: the A operand is read from TMEM
-          const uint64_t b_hi = sw128_desc(s_u32(s_bhi + kb * tile_b_al));
-          const uint64_t b_lo = sw128_desc(s_u32(s_blo + kb * tile_b_al));
+          const uint64_t b_hi = make_sw128_desc(smem_u32(s_bhi + kb * tile_b_al));
+          const uint64_t b_lo = make_sw128_desc(smem_u32(s_blo + kb * tile_b_al));
           if (elect_one()) {
             // straight-line issue (a runtime trip count makes the loop carry R2UR moves and ~20 uniform-datapath
             // instructions per step: measured on the K6 scorer, +6%)
@@ -416,8 +294,8 @@ gemm_tf32x3_kernel(const __grid_constant__ GemmMaps maps, const GemmParams P) {
                 umma_tf32_ts(d_addr, a_hi + 8 * k, b_hi + 2 * k, idesc, 1u);
               }
             }
-            umma_commit_g(split_empty + ts);
-            if (kb == P.n_kb - 1) umma_commit_g(acc_full + acc);
+            umma_commit(split_empty + ts);
+            if (kb == P.n_kb - 1) umma_commit(acc_full + acc);
           }
           __syncwarp();
           if (lane == 0) KGC_DBG(5);
@@ -439,22 +317,22 @@ gemm_tf32x3_kernel(const __grid_constant__ GemmMaps maps, const GemmParams P) {
     int acc = 0, buf = 0;
     uint32_t acc_phase = 0;
     for (int mt = first; mt < P.n_mtiles; mt += step) {
-      mb_wait(acc_full + acc, acc_phase);
+      mbar_wait(acc_full + acc, acc_phase);
       if (warp == 10 && lane == 0) KGC_DBG(6);
-      asm volatile("tcgen05.fence::after_thread_sync;" ::: "memory");
+      tc_fence_after();
       const int64_t m0 = (int64_t)mt * kBM + row_q;
       const uint32_t taddr = tmem_base + ((uint32_t)(quarter * 32) << 16) + acc * (kAccCols / 2);
       for (int c0 = 0; c0 < P.NT; c0 += 32) {
         uint32_t v[32];
-        tmem_ld32_g(taddr + c0, v);                                // columns past NT belong to the allocation: never stored
-        asm volatile("tcgen05.wait::ld.sync.aligned;" ::: "memory");
+        tmem_ld32(taddr + c0, v);                                // columns past NT belong to the allocation: never stored
+        tmem_ld_wait();
         if (c0 + 32 >= P.NT) {                                     // last read of this accumulator: give it back to the MMA warp
-          asm volatile("tcgen05.fence::before_thread_sync;" ::: "memory");
+          tc_fence_before();
           __syncwarp();
-          if (lane == 0) mb_arrive(acc_empty + acc);
+          if (lane == 0) mbar_arrive(acc_empty + acc);
         }
         // the TMA store that read this buffer two blocks ago must have drained it (bulk groups are per thread: lane 0)
-        if (lane == 0) asm volatile("cp.async.bulk.wait_group.read 1;" ::: "memory");
+        if (lane == 0) bulk_wait_group_read<1>();
         __syncwarp();
         uint8_t* bb = stg + buf * kEpiBuf;
         const bool wide = c0 + 32 <= P.NT;                         // 32-column box (128-byte rows), else the 16-column tail box
@@ -484,7 +362,7 @@ gemm_tf32x3_kernel(const __grid_constant__ GemmMaps maps, const GemmParams P) {
           for (int q = 0; q < 4; ++q)
             *reinterpret_cast<uint4*>(bx + ((q ^ sw) << 4)) = make_uint4(v[4 * q], v[4 * q + 1], v[4 * q + 2], v[4 * q + 3]);
         }
-        asm volatile("fence.proxy.async.shared::cta;" ::: "memory");
+        fence_proxy_async();
         __syncwarp();
         if (lane == 0) {
           const int col = nt * P.NT + c0;
@@ -492,16 +370,16 @@ gemm_tf32x3_kernel(const __grid_constant__ GemmMaps maps, const GemmParams P) {
             if (P.trans_c) tma_store_2d(wide ? map_c : map_c16, bb, (int)m0, col);     // Ct: inner coordinate = row of C
             else tma_store_2d(wide ? map_c : map_c16, bb, col, (int)m0);
           }
-          asm volatile("cp.async.bulk.commit_group;" ::: "memory");
+          bulk_commit_group();
         }
         buf ^= 1;
       }
       if (warp == 10 && lane == 0) KGC_DBG(7);
       if (++acc == 2) { acc = 0; acc_phase ^= 1; }
     }
-    if (lane == 0) asm volatile("cp.async.bulk.wait_group 0;" ::: "memory");   // all stores complete before the CTA exits
+    if (lane == 0) bulk_wait_group<0>();   // all stores complete before the CTA exits
   }
-  asm volatile("tcgen05.fence::before_thread_sync;" ::: "memory");
+  tc_fence_before();
   __syncthreads();
   if (P.dbg != nullptr && threadIdx.x == 0) {
     long long g;
@@ -509,9 +387,7 @@ gemm_tf32x3_kernel(const __grid_constant__ GemmMaps maps, const GemmParams P) {
     atomicMax(reinterpret_cast<long long*>(P.dbg) + 8 * 64 + 1, g);
     if (blockIdx.x == 0) { P.dbg[8 * 64 + 4] = g; P.dbg[8 * 64 + 5] = clock64(); }
   }
-  if (warp == 14) {
-    asm volatile("tcgen05.dealloc.cta_group::1.sync.aligned.b32 %0, %1;" ::"r"(tmem_base), "r"(kTmemColsTS) : "memory");
-  }
+  if (warp == 14) tmem_dealloc(tmem_base, kTmemColsTS);
 }
 
 // Bt_hi / Bt_lo [n_pad, k_pad] from B viewed as element (k, n) = B[k * sk + n * sn]; zero padded
@@ -675,55 +551,21 @@ __global__ void __launch_bounds__(256) conv_param_grads2_kernel(const ParamGradA
   }
 }
 
-typedef CUresult (*EncodeTiledFn)(CUtensorMap*, CUtensorMapDataType, cuuint32_t, void*, const cuuint64_t*, const cuuint64_t*,
-                                  const cuuint32_t*, const cuuint32_t*, CUtensorMapInterleave, CUtensorMapSwizzle,
-                                  CUtensorMapL2promotion, CUtensorMapFloatOOBfill);
-int encode_fn(EncodeTiledFn* out) {
-  ensure_thread_context();
-  static EncodeTiledFn cached = nullptr;
-  if (!cached) {
-    void* fn = nullptr;
-    cudaDriverEntryPointQueryResult qres;
-    KGC_CUDA_TRY(cudaGetDriverEntryPoint("cuTensorMapEncodeTiled", &fn, cudaEnableDefault, &qres));
-    KGC_REQUIRE(qres == cudaDriverEntryPointSuccess && fn != nullptr, "cuTensorMapEncodeTiled not available");
-    cached = reinterpret_cast<EncodeTiledFn>(fn);
-  }
-  *out = cached;
-  return 0;
-}
 // fp32 [rows, cols] with row pitch `pitch` floats -> boxes of 32 (K) x box_rows, 128-byte swizzle, zero fill
 int make_map_f32(CUtensorMap* map, const void* ptr, int64_t rows, int64_t cols, int64_t pitch, int box_rows,
                  CUtensorMapSwizzle swizzle = CU_TENSOR_MAP_SWIZZLE_128B, int box_cols = kBK) {
-  EncodeTiledFn enc;
-  if (encode_fn(&enc)) return 1;
-  KGC_REQUIRE((reinterpret_cast<uintptr_t>(ptr) & 15) == 0 && (pitch * 4) % 16 == 0, "operand must be 16-byte aligned with a 16-byte pitch");
-  cuuint64_t dims[2] = {(cuuint64_t)cols, (cuuint64_t)rows};
-  cuuint64_t strides[1] = {(cuuint64_t)pitch * 4};
-  cuuint32_t box[2] = {(cuuint32_t)box_cols, (cuuint32_t)box_rows};
-  cuuint32_t estr[2] = {1, 1};
-  CUresult r = enc(map, CU_TENSOR_MAP_DATA_TYPE_FLOAT32, 2, const_cast<void*>(ptr), dims, strides, box, estr,
-                   CU_TENSOR_MAP_INTERLEAVE_NONE, swizzle, CU_TENSOR_MAP_L2_PROMOTION_L2_256B,
-                   CU_TENSOR_MAP_FLOAT_OOB_FILL_NONE);
-  KGC_REQUIRE(r == CUDA_SUCCESS, "cuTensorMapEncodeTiled failed (" + std::to_string((int)r) + ")");
-  return 0;
+  const cuuint64_t dims[2] = {(cuuint64_t)cols, (cuuint64_t)rows}, strides[1] = {(cuuint64_t)pitch * 4};
+  const cuuint32_t box[2] = {(cuuint32_t)box_cols, (cuuint32_t)box_rows};
+  return encode_tiled(map, CU_TENSOR_MAP_DATA_TYPE_FLOAT32, 2, ptr, dims, strides, box, swizzle);
 }
 
 // 32-column groups of fp32 [rows, cols] fetched by ONE box: dims (32 columns, rows, groups), group stride 128 B;
 // the box takes 32 rows x box_groups groups and lands as [group][row][32 columns]
 int make_map_f32_groups(CUtensorMap* map, const void* ptr, int64_t rows, int groups, int64_t pitch, int box_groups,
                         CUtensorMapSwizzle swizzle) {
-  EncodeTiledFn enc;
-  if (encode_fn(&enc)) return 1;
-  KGC_REQUIRE((reinterpret_cast<uintptr_t>(ptr) & 15) == 0 && (pitch * 4) % 16 == 0, "operand must be 16-byte aligned with a 16-byte pitch");
-  cuuint64_t dims[3] = {32, (cuuint64_t)rows, (cuuint64_t)groups};
-  cuuint64_t strides[2] = {(cuuint64_t)pitch * 4, 128};
-  cuuint32_t box[3] = {32, 32, (cuuint32_t)box_groups};
-  cuuint32_t estr[3] = {1, 1, 1};
-  CUresult r = enc(map, CU_TENSOR_MAP_DATA_TYPE_FLOAT32, 3, const_cast<void*>(ptr), dims, strides, box, estr,
-                   CU_TENSOR_MAP_INTERLEAVE_NONE, swizzle, CU_TENSOR_MAP_L2_PROMOTION_L2_256B,
-                   CU_TENSOR_MAP_FLOAT_OOB_FILL_NONE);
-  KGC_REQUIRE(r == CUDA_SUCCESS, "cuTensorMapEncodeTiled (grouped operand) failed (" + std::to_string((int)r) + ")");
-  return 0;
+  const cuuint64_t dims[3] = {32, (cuuint64_t)rows, (cuuint64_t)groups}, strides[2] = {(cuuint64_t)pitch * 4, 128};
+  const cuuint32_t box[3] = {32, 32, (cuuint32_t)box_groups};
+  return encode_tiled(map, CU_TENSOR_MAP_DATA_TYPE_FLOAT32, 3, ptr, dims, strides, box, swizzle);
 }
 int make_map_f32_mn_groups(CUtensorMap* map, const void* ptr, int64_t rows, int groups, int64_t pitch) {
   return make_map_f32_groups(map, ptr, rows, groups, pitch, groups, CU_TENSOR_MAP_SWIZZLE_128B_ATOM_32B);
@@ -731,18 +573,10 @@ int make_map_f32_mn_groups(CUtensorMap* map, const void* ptr, int64_t rows, int 
 
 // partial sums [parts][rows][cols] fp32 -> boxes of 32 columns x 32 rows of one part, 128-byte swizzle (TMA stores clip)
 int make_map_f32_parts(CUtensorMap* map, const void* ptr, int64_t parts, int64_t rows, int64_t cols) {
-  EncodeTiledFn enc;
-  if (encode_fn(&enc)) return 1;
-  KGC_REQUIRE((reinterpret_cast<uintptr_t>(ptr) & 15) == 0 && cols % 4 == 0, "partials must be 16-byte aligned with a 16-byte pitch");
-  cuuint64_t dims[3] = {(cuuint64_t)cols, (cuuint64_t)rows, (cuuint64_t)parts};
-  cuuint64_t strides[2] = {(cuuint64_t)cols * 4, (cuuint64_t)rows * cols * 4};
-  cuuint32_t box[3] = {32, 32, 1};
-  cuuint32_t estr[3] = {1, 1, 1};
-  CUresult r = enc(map, CU_TENSOR_MAP_DATA_TYPE_FLOAT32, 3, const_cast<void*>(ptr), dims, strides, box, estr,
-                   CU_TENSOR_MAP_INTERLEAVE_NONE, CU_TENSOR_MAP_SWIZZLE_128B, CU_TENSOR_MAP_L2_PROMOTION_L2_256B,
-                   CU_TENSOR_MAP_FLOAT_OOB_FILL_NONE);
-  KGC_REQUIRE(r == CUDA_SUCCESS, "cuTensorMapEncodeTiled failed (" + std::to_string((int)r) + ")");
-  return 0;
+  const cuuint64_t dims[3] = {(cuuint64_t)cols, (cuuint64_t)rows, (cuuint64_t)parts};
+  const cuuint64_t strides[2] = {(cuuint64_t)cols * 4, (cuuint64_t)rows * cols * 4};
+  const cuuint32_t box[3] = {32, 32, 1};
+  return encode_tiled(map, CU_TENSOR_MAP_DATA_TYPE_FLOAT32, 3, ptr, dims, strides, box, CU_TENSOR_MAP_SWIZZLE_128B);
 }
 
 struct Tiling {
@@ -840,23 +674,19 @@ gemm_tn_tc_kernel(const __grid_constant__ GemmTnMaps maps, const GemmTnParams P)
 
   if (warp == 0 && lane == 0) {
     for (int i = 0; i < kTnStages; ++i) {
-      mb_init(raw_full + i, 1);
-      mb_init(split_full + i, kSplitWarps);
-      mb_init(empty + i, 1);
+      mbar_init(raw_full + i, 1);
+      mbar_init(split_full + i, kSplitWarps);
+      mbar_init(empty + i, 1);
     }
-    for (int i = 0; i < kTnLoStages; ++i) mb_init(lo_empty + i, 1);
-    mb_init(acc_full, 1);
-    asm volatile("fence.mbarrier_init.release.cluster;" ::: "memory");
-    asm volatile("fence.proxy.async.shared::cta;" ::: "memory");
+    for (int i = 0; i < kTnLoStages; ++i) mbar_init(lo_empty + i, 1);
+    mbar_init(acc_full, 1);
+    fence_barrier_init();
+    fence_proxy_async();
   }
-  if (warp == 14) {
-    asm volatile("tcgen05.alloc.cta_group::1.sync.aligned.shared::cta.b32 [%0], %1;" ::"r"(s_u32(tmem_slot)), "r"(kTmemColsG)
-                 : "memory");
-    asm volatile("tcgen05.relinquish_alloc_permit.cta_group::1.sync.aligned;" ::: "memory");
-  }
-  asm volatile("tcgen05.fence::before_thread_sync;" ::: "memory");
+  if (warp == 14) tmem_alloc(tmem_slot, kTmemColsG);
+  tc_fence_before();
   __syncthreads();
-  asm volatile("tcgen05.fence::after_thread_sync;" ::: "memory");
+  tc_fence_after();
   const uint32_t tmem_base = *tmem_slot;
   const bool dbg_on = P.dbg != nullptr && blockIdx.x == 0;
   int dbg_n = 0;
@@ -874,28 +704,28 @@ gemm_tn_tc_kernel(const __grid_constant__ GemmTnMaps maps, const GemmTnParams P)
       int stage = 0;
       uint32_t phase = 0;
       for (int kb = 0; kb < n_kb; ++kb) {
-        mb_wait(empty + stage, phase ^ 1);
+        mbar_wait(empty + stage, phase ^ 1);
         KGC_DBG(0);
         uint8_t* dst = s_raw + stage * stage_bytes;
         const int row = (int)(m0 + (int64_t)kb * kTnRows);
         if (P.kmajor) {
           // K-major operands A[Ka, K], Bt[Nb, K]: a K block is 32 contraction COLUMNS; A lands as 128 rows x 128 B,
           // Bt as n_pad rows x 128 B (128-byte swizzle), rows past Ka / Nb and columns past K zero-filled by TMA
-          mb_expect_tx(raw_full + stage, (uint32_t)(kTileA + P.n_pad * 128));
-          tma_2d(dst, map_a, raw_full + stage, row, 0);
-          tma_2d(dst + kTileA, map_b, raw_full + stage, row, 0);
+          mbar_expect_tx(raw_full + stage, (uint32_t)(kTileA + P.n_pad * 128));
+          tma_load_2d(dst, map_a, raw_full + stage, row, 0);
+          tma_load_2d(dst + kTileA, map_b, raw_full + stage, row, 0);
           if (++stage == kTnStages) { stage = 0; phase ^= 1; }
           continue;
         }
-        mb_expect_tx(raw_full + stage, (uint32_t)stage_bytes);
+        mbar_expect_tx(raw_full + stage, (uint32_t)stage_bytes);
         // rows past m1 belong to the next CTA's slab: they are masked out by the splitter (zeroed), rows past M are
         // zero-filled by TMA
         // one instruction fetches all the complete 32-column groups of an operand (a TMA issue costs ~170 cycles of the
         // producer thread); the ragged last group and the all-padding groups go through the zero-filling 2-D map
-        if (P.ga_full > 0) tma_3d(dst, map_a3, raw_full + stage, 0, row, 0);
-        for (int g = P.ga_full; g < P.ga; ++g) tma_2d(dst + g * kTnBox, map_a, raw_full + stage, g * 32, row);
-        if (P.gb_full > 0) tma_3d(dst + P.ga * kTnBox, map_b3, raw_full + stage, 0, row, 0);
-        for (int g = P.gb_full; g < P.gb; ++g) tma_2d(dst + (P.ga + g) * kTnBox, map_b, raw_full + stage, g * 32, row);
+        if (P.ga_full > 0) tma_load_3d(dst, map_a3, raw_full + stage, 0, row, 0);
+        for (int g = P.ga_full; g < P.ga; ++g) tma_load_2d(dst + g * kTnBox, map_a, raw_full + stage, g * 32, row);
+        if (P.gb_full > 0) tma_load_3d(dst + P.ga * kTnBox, map_b3, raw_full + stage, 0, row, 0);
+        for (int g = P.gb_full; g < P.gb; ++g) tma_load_2d(dst + (P.ga + g) * kTnBox, map_b, raw_full + stage, g * 32, row);
         if (++stage == kTnStages) { stage = 0; phase ^= 1; }
       }
     }
@@ -918,9 +748,9 @@ gemm_tn_tc_kernel(const __grid_constant__ GemmTnMaps maps, const GemmTnParams P)
         if (g < P.gb) nbn[g] = (uint32_t)__ldg(kp + g * 8);
     }
     for (int kb = 0; kb < n_kb; ++kb) {
-      mb_wait(raw_full + stage, phase);
+      mbar_wait(raw_full + stage, phase);
       if (t == 0) KGC_DBG(1);
-      mb_wait(lo_empty + ls, lphase ^ 1);
+      mbar_wait(lo_empty + ls, lphase ^ 1);
       if (t == 0) KGC_DBG(2);
       uint4* hi = reinterpret_cast<uint4*>(s_raw + stage * stage_bytes);
       uint4* lo = reinterpret_cast<uint4*>(s_lo + ls * stage_bytes);
@@ -977,9 +807,9 @@ gemm_tn_tc_kernel(const __grid_constant__ GemmTnMaps maps, const GemmTnParams P)
         hi[v] = h;
         lo[v] = l;
       }
-      asm volatile("fence.proxy.async.shared::cta;" ::: "memory");
+      fence_proxy_async();
       __syncwarp();
-      if (lane == 0) mb_arrive(split_full + stage);
+      if (lane == 0) mbar_arrive(split_full + stage);
       if (t == 0) KGC_DBG(3);
       if (++stage == kTnStages) { stage = 0; phase ^= 1; }
       if (++ls == kTnLoStages) { ls = 0; lphase ^= 1; }
@@ -991,24 +821,24 @@ gemm_tn_tc_kernel(const __grid_constant__ GemmTnMaps maps, const GemmTnParams P)
     int stage = 0, ls = 0;
     uint32_t phase = 0;
     for (int kb = 0; kb < n_kb; ++kb) {
-      mb_wait(split_full + stage, phase);
+      mbar_wait(split_full + stage, phase);
       if (lane == 0) KGC_DBG(4);
-      asm volatile("tcgen05.fence::after_thread_sync;" ::: "memory");
-      const uint32_t hi_a = s_u32(s_raw + stage * stage_bytes), hi_b = hi_a + P.ga * kTnBox;
-      const uint32_t lo_a = s_u32(s_lo + ls * stage_bytes), lo_b = lo_a + P.ga * kTnBox;
+      tc_fence_after();
+      const uint32_t hi_a = smem_u32(s_raw + stage * stage_bytes), hi_b = hi_a + P.ga * kTnBox;
+      const uint32_t lo_a = smem_u32(s_lo + ls * stage_bytes), lo_b = lo_a + P.ga * kTnBox;
       if (P.kmajor) {
         const uint32_t idesc_k = (1u << 4) | (2u << 7) | (2u << 10) | ((uint32_t)(P.n_pad >> 3) << 17) | ((uint32_t)(kBM >> 4) << 24);
-        const uint64_t a_hi = sw128_desc(hi_a), a_lo = sw128_desc(lo_a);
-        const uint64_t b_hi = sw128_desc(hi_a + kTileA), b_lo = sw128_desc(lo_a + kTileA);
+        const uint64_t a_hi = make_sw128_desc(hi_a), a_lo = make_sw128_desc(lo_a);
+        const uint64_t b_hi = make_sw128_desc(hi_a + kTileA), b_lo = make_sw128_desc(lo_a + kTileA);
         if (elect_one()) {
           for (int k = 0; k < kTnRows / kUK; ++k) {
             umma_tf32(tmem_base, a_lo + 2 * k, b_hi + 2 * k, idesc_k, (kb | k) != 0 ? 1u : 0u);
             umma_tf32(tmem_base, a_hi + 2 * k, b_lo + 2 * k, idesc_k, 1u);
             umma_tf32(tmem_base, a_hi + 2 * k, b_hi + 2 * k, idesc_k, 1u);
           }
-          umma_commit_g(empty + stage);
-          umma_commit_g(lo_empty + ls);
-          if (kb == n_kb - 1) umma_commit_g(acc_full);
+          umma_commit(empty + stage);
+          umma_commit(lo_empty + ls);
+          if (kb == n_kb - 1) umma_commit(acc_full);
         }
       } else if (elect_one()) {
         for (int k = 0; k < kTnRows / kUK; ++k) {                  // 8 node rows per MMA: the next 8-row K group is 1024 B on
@@ -1017,9 +847,9 @@ gemm_tn_tc_kernel(const __grid_constant__ GemmTnMaps maps, const GemmTnParams P)
           umma_tf32(tmem_base, sw128_mn_desc(hi_a + off), sw128_mn_desc(lo_b + off), idesc, 1u);
           umma_tf32(tmem_base, sw128_mn_desc(hi_a + off), sw128_mn_desc(hi_b + off), idesc, 1u);
         }
-        umma_commit_g(empty + stage);
-        umma_commit_g(lo_empty + ls);
-        if (kb == n_kb - 1) umma_commit_g(acc_full);
+        umma_commit(empty + stage);
+        umma_commit(lo_empty + ls);
+        if (kb == n_kb - 1) umma_commit(acc_full);
       }
       __syncwarp();
       if (lane == 0) KGC_DBG(5);
@@ -1034,17 +864,17 @@ gemm_tn_tc_kernel(const __grid_constant__ GemmTnMaps maps, const GemmTnParams P)
     const int i = quarter * 32 + lane;
     float* out = P.partial + (((int64_t)prob * P.n_slabs + slab) * P.Ka + i) * P.Nb;
     if (n_kb > 0) {
-      mb_wait(acc_full, 0);                                        // every MMA has retired: shared memory is free
+      mbar_wait(acc_full, 0);                                        // every MMA has retired: shared memory is free
       if (warp == 10 && lane == 0) KGC_DBG(6);
-      asm volatile("tcgen05.fence::after_thread_sync;" ::: "memory");
+      tc_fence_after();
       const uint32_t taddr = tmem_base + ((uint32_t)(quarter * 32) << 16);
       uint8_t* stg = s_raw + (warp - 10) * (2 * kEpiBuf);
       int buf = 0;
       for (int c0 = 0; c0 < P.n_pad; c0 += 32) {
         uint32_t v[32];
-        tmem_ld32_g(taddr + c0, v);
-        asm volatile("tcgen05.wait::ld.sync.aligned;" ::: "memory");
-        if (lane == 0) asm volatile("cp.async.bulk.wait_group.read 1;" ::: "memory");
+        tmem_ld32(taddr + c0, v);
+        tmem_ld_wait();
+        if (lane == 0) bulk_wait_group_read<1>();
         __syncwarp();
         uint8_t* bb = stg + buf * kEpiBuf;
         uint8_t* bx = bb + lane * 128;
@@ -1052,21 +882,21 @@ gemm_tn_tc_kernel(const __grid_constant__ GemmTnMaps maps, const GemmTnParams P)
 #pragma unroll
         for (int q = 0; q < 8; ++q)
           *reinterpret_cast<uint4*>(bx + ((q ^ sw) << 4)) = make_uint4(v[4 * q], v[4 * q + 1], v[4 * q + 2], v[4 * q + 3]);
-        asm volatile("fence.proxy.async.shared::cta;" ::: "memory");
+        fence_proxy_async();
         __syncwarp();
         if (lane == 0) {
           if (c0 < P.Nb && quarter * 32 < P.Ka) tma_store_3d(map_p, bb, c0, quarter * 32, slab);
-          asm volatile("cp.async.bulk.commit_group;" ::: "memory");
+          bulk_commit_group();
         }
         buf ^= 1;
       }
-      if (lane == 0) asm volatile("cp.async.bulk.wait_group 0;" ::: "memory");
+      if (lane == 0) bulk_wait_group<0>();
       if (warp == 10 && lane == 0) KGC_DBG(7);
     } else if (i < P.Ka) {
       for (int j = 0; j < P.Nb; ++j) out[j] = 0.f;
     }
   }
-  asm volatile("tcgen05.fence::before_thread_sync;" ::: "memory");
+  tc_fence_before();
   __syncthreads();
   if (P.dbg != nullptr && threadIdx.x == 0) {
     long long g;
@@ -1074,9 +904,7 @@ gemm_tn_tc_kernel(const __grid_constant__ GemmTnMaps maps, const GemmTnParams P)
     atomicMax(reinterpret_cast<long long*>(P.dbg) + 8 * 64 + 1, g);
     if (blockIdx.x == 0) { P.dbg[8 * 64 + 4] = g; P.dbg[8 * 64 + 5] = clock64(); }
   }
-  if (warp == 14) {
-    asm volatile("tcgen05.dealloc.cta_group::1.sync.aligned.b32 %0, %1;" ::"r"(tmem_base), "r"(kTmemColsG) : "memory");
-  }
+  if (warp == 14) tmem_dealloc(tmem_base, kTmemColsG);
 }
 
 // C[e] = sum over the CTA partials in a FIXED order: 8 part-lanes per element, then their sums in lane order; the
@@ -1244,26 +1072,16 @@ static int launch_gemm_nt(int n_prob, const float* const* A, int64_t M, int32_t 
   return 0;
 }
 
-extern "C" int kgc_gemm_nt(const float* A, int64_t M, int32_t K, int64_t lda, const float* packed_b, int32_t N, float* C,
-                           int64_t ldc, void* stream) {
-  return launch_gemm_nt(1, &A, M, K, lda, &packed_b, N, &C, ldc, nullptr, 0, 0, 0, stream);
-}
-
+// keep (optional): kgc_tail_fwd's keep flags, applied to the streamed operand of problems 0 and 1 while it is split
 extern "C" int kgc_gemm_nt_batch(int32_t n_prob, const float* const* A, int64_t M, int32_t K, int64_t lda,
-                                 const float* const* packed_b, int32_t N, float* const* C, int64_t ldc, void* stream) {
-  KGC_REQUIRE(A && packed_b && C, "null pointer table");
-  return launch_gemm_nt(n_prob, A, M, K, lda, packed_b, N, C, ldc, nullptr, 0, 0, 0, stream);
-}
-
-// Ct[N, M] = (A @ Bt^T)^T with A given transposed, At[K, M] row-major: the long dimension M is contiguous in BOTH the
-// streamed operand and the result (a [K, M] weight or activation matrix and a gradient of the same shape)
-extern "C" int kgc_gemm_nt_batch_masked(int32_t n_prob, const float* const* A, int64_t M, int32_t K, int64_t lda,
-                                        const float* const* packed_b, int32_t N, float* const* C, int64_t ldc,
-                                        const uint8_t* keep, int32_t keep_pitch, float keep_scale, void* stream) {
+                                 const float* const* packed_b, int32_t N, float* const* C, int64_t ldc, const uint8_t* keep,
+                                 int32_t keep_pitch, float keep_scale, void* stream) {
   KGC_REQUIRE(A && packed_b && C, "null pointer table");
   return launch_gemm_nt(n_prob, A, M, K, lda, packed_b, N, C, ldc, nullptr, 0, 0, 0, stream, keep, keep_pitch, keep_scale);
 }
 
+// Ct[N, M] = (A @ Bt^T)^T with A given transposed, At[K, M] row-major: the long dimension M is contiguous in BOTH the
+// streamed operand and the result (a [K, M] weight or activation matrix and a gradient of the same shape)
 extern "C" int kgc_gemm_nt_trans(const float* At, int64_t M, int32_t K, int64_t ldat, const float* packed_b, int32_t N,
                                  float* Ct, int64_t ldct, void* stream) {
   return launch_gemm_nt(1, &At, M, K, ldat, &packed_b, N, &Ct, ldct, nullptr, 0, 1, 1, stream);
@@ -1381,33 +1199,15 @@ static int launch_gemm_tn_tc(int n_prob, const float* const* A, int64_t lda, con
   return 0;
 }
 
-extern "C" int kgc_gemm_tn_tc(const float* A, int64_t lda, const float* B, int64_t ldb, int64_t M, int32_t Ka, int32_t Nb,
-                              float* C, void* workspace, size_t workspace_bytes, void* stream) {
-  return launch_gemm_tn_tc(1, &A, lda, &B, ldb, M, Ka, Nb, &C, workspace, workspace_bytes, 0, stream);
-}
-
+// rows (optional): rows[i] <= M rows of problem i (the layer's compacted planes): problems of M rows keep their bits.
+// keep (optional): the keep flags applied to the B operand while it is split (see kgc_gemm_nt_batch).
 extern "C" int kgc_gemm_tn_tc_batch(int32_t n_prob, const float* const* A, int64_t lda, const float* const* B, int64_t ldb,
-                                    int64_t M, int32_t Ka, int32_t Nb, float* const* C, void* workspace,
-                                    size_t workspace_bytes, void* stream) {
-  KGC_REQUIRE(A && B && C, "null pointer table");
-  return launch_gemm_tn_tc(n_prob, A, lda, B, ldb, M, Ka, Nb, C, workspace, workspace_bytes, 0, stream);
-}
-
-// the same with rows[i] <= M rows for problem i (the layer's compacted planes): problems of M rows keep their bits
-extern "C" int kgc_gemm_tn_tc_batch_rows(int32_t n_prob, const float* const* A, int64_t lda, const float* const* B, int64_t ldb,
-                                         const int64_t* rows, int64_t M, int32_t Ka, int32_t Nb, float* const* C, void* workspace,
-                                         size_t workspace_bytes, void* stream) {
-  KGC_REQUIRE(A && B && C && rows, "null pointer table");
-  return launch_gemm_tn_tc(n_prob, A, lda, B, ldb, M, Ka, Nb, C, workspace, workspace_bytes, 0, stream, nullptr, 0, 1.f, rows);
-}
-
-extern "C" int kgc_gemm_tn_tc_batch_masked(int32_t n_prob, const float* const* A, int64_t lda, const float* const* B, int64_t ldb,
-                                           int64_t M, int32_t Ka, int32_t Nb, float* const* C, void* workspace,
-                                           size_t workspace_bytes, const uint8_t* keep, int32_t keep_pitch, float keep_scale,
-                                           void* stream) {
+                                    const int64_t* rows, int64_t M, int32_t Ka, int32_t Nb, float* const* C, void* workspace,
+                                    size_t workspace_bytes, const uint8_t* keep, int32_t keep_pitch, float keep_scale,
+                                    void* stream) {
   KGC_REQUIRE(A && B && C, "null pointer table");
   return launch_gemm_tn_tc(n_prob, A, lda, B, ldb, M, Ka, Nb, C, workspace, workspace_bytes, 0, stream, keep, keep_pitch,
-                           keep_scale);
+                           keep_scale, rows);
 }
 
 // C[Ma, Nb] = A[Ma, K] @ Bt[Nb, K]^T with a LONG contraction (K >> Ma, Nb): the K range is cut into per-CTA slabs, both

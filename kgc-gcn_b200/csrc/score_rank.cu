@@ -28,10 +28,9 @@
 // item, skipping its exclusion list; topk_merge_kernel reduces the per-item lists.  kgc_topk_dense makes the same
 // selection over dense fp32 logits (exact mode) with the same list, exclusion cursor, partial layout and merge.
 // kgc_topk_merge combines finished results of disjoint entity ranges (shards) with the same list and output loop.
-#include <cuda.h>
 #include <cuda_bf16.h>
 
-#include "common.cuh"
+#include "tcgen05.cuh"
 
 namespace kgc {
 namespace {
@@ -53,109 +52,6 @@ constexpr int kSmemB = kStagesB * kTileBytes;                           //  96 K
 constexpr int kSmemBar = 256;
 constexpr int kSmemBytes = kSmemA + kSmemB + kSmemBar + 1024;           // + alignment slack
 
-// ------------------------------------------------------------------------------------------------ PTX wrappers
-__device__ __forceinline__ uint32_t smem_u32(const void* p) { return (uint32_t)__cvta_generic_to_shared(p); }
-
-__device__ __forceinline__ void mbar_init(uint64_t* bar, uint32_t count) {
-  asm volatile("mbarrier.init.shared::cta.b64 [%0], %1;" ::"r"(smem_u32(bar)), "r"(count));
-}
-__device__ __forceinline__ void mbar_expect_tx(uint64_t* bar, uint32_t bytes) {
-  asm volatile("mbarrier.arrive.expect_tx.shared::cta.b64 _, [%0], %1;" ::"r"(smem_u32(bar)), "r"(bytes) : "memory");
-}
-__device__ __forceinline__ void mbar_arrive(uint64_t* bar) {
-  asm volatile("mbarrier.arrive.shared::cta.b64 _, [%0];" ::"r"(smem_u32(bar)) : "memory");
-}
-__device__ __forceinline__ void mbar_wait(uint64_t* bar, uint32_t parity) {
-  asm volatile(
-      "{\n"
-      ".reg .pred P1;\n"
-      "LAB_WAIT:\n"
-      "mbarrier.try_wait.parity.shared::cta.b64 P1, [%0], %1;\n"
-      "@P1 bra DONE;\n"
-      "bra LAB_WAIT;\n"
-      "DONE:\n"
-      "}" ::"r"(smem_u32(bar)),
-      "r"(parity)
-      : "memory");
-}
-__device__ __forceinline__ void fence_barrier_init() { asm volatile("fence.mbarrier_init.release.cluster;" ::: "memory"); }
-__device__ __forceinline__ void fence_proxy_async() { asm volatile("fence.proxy.async.shared::cta;" ::: "memory"); }
-__device__ __forceinline__ void tc_fence_before() { asm volatile("tcgen05.fence::before_thread_sync;" ::: "memory"); }
-__device__ __forceinline__ void tc_fence_after() { asm volatile("tcgen05.fence::after_thread_sync;" ::: "memory"); }
-
-// One lane of a fully converged warp (PTX elect.sync).  The surrounding code stays warp-uniform, so ptxas keeps the
-// shared-memory / instruction descriptors in UNIFORM registers; running the whole role under `if (lane == 0)` makes
-// them per-thread values and every tcgen05.mma then pays a chain of R2UR moves (~120 cycles per MMA, measured).
-__device__ __forceinline__ bool elect_one() {
-  uint32_t pred = 0;
-  asm volatile(
-      "{\n"
-      ".reg .b32 rx;\n"
-      ".reg .pred px;\n"
-      "elect.sync rx|px, 0xFFFFFFFF;\n"
-      "@px mov.s32 %0, 1;\n"
-      "}"
-      : "+r"(pred));
-  return pred != 0;
-}
-__device__ __forceinline__ void tma_load_2d(void* smem_dst, const CUtensorMap* map, uint64_t* bar, int c0, int c1) {
-  asm volatile(
-      "cp.async.bulk.tensor.2d.shared::cluster.global.mbarrier::complete_tx::bytes [%0], [%1, {%3, %4}], [%2];" ::"r"(
-          smem_u32(smem_dst)),
-      "l"(reinterpret_cast<uint64_t>(map)), "r"(smem_u32(bar)), "r"(c0), "r"(c1)
-      : "memory");
-}
-__device__ __forceinline__ void tma_prefetch_desc(const CUtensorMap* map) {
-  asm volatile("prefetch.tensormap [%0];" ::"l"(reinterpret_cast<uint64_t>(map)) : "memory");
-}
-
-__device__ __forceinline__ void tmem_alloc(uint32_t* slot, uint32_t cols) {
-  asm volatile("tcgen05.alloc.cta_group::1.sync.aligned.shared::cta.b32 [%0], %1;" ::"r"(smem_u32(slot)), "r"(cols)
-               : "memory");
-  asm volatile("tcgen05.relinquish_alloc_permit.cta_group::1.sync.aligned;" ::: "memory");
-}
-__device__ __forceinline__ void tmem_dealloc(uint32_t taddr, uint32_t cols) {
-  asm volatile("tcgen05.dealloc.cta_group::1.sync.aligned.b32 %0, %1;" ::"r"(taddr), "r"(cols) : "memory");
-}
-// D[tmem] (+)= A[smem] * B[smem]^T, bf16 x bf16 -> fp32, issued by ONE thread for the CTA
-__device__ __forceinline__ void umma_bf16(uint32_t tmem_d, uint64_t adesc, uint64_t bdesc, uint32_t idesc, uint32_t acc) {
-  asm volatile(
-      "{\n"
-      ".reg .pred p;\n"
-      "setp.ne.b32 p, %4, 0;\n"
-      "tcgen05.mma.cta_group::1.kind::f16 [%0], %1, %2, %3, p;\n"
-      "}" ::"r"(tmem_d),
-      "l"(adesc), "l"(bdesc), "r"(idesc), "r"(acc)
-      : "memory");
-}
-// all tcgen05.mma issued so far by this thread arrive on the mbarrier when they complete
-__device__ __forceinline__ void umma_commit(uint64_t* bar) {
-  asm volatile("tcgen05.commit.cta_group::1.mbarrier::arrive::one.shared::cluster.b64 [%0];" ::"r"(smem_u32(bar))
-               : "memory");
-}
-__device__ __forceinline__ void tmem_ld32(uint32_t taddr, uint32_t (&v)[32]) {
-  asm volatile(
-      "tcgen05.ld.sync.aligned.32x32b.x32.b32 "
-      "{%0, %1, %2, %3, %4, %5, %6, %7, %8, %9, %10, %11, %12, %13, %14, %15, "
-      "%16, %17, %18, %19, %20, %21, %22, %23, %24, %25, %26, %27, %28, %29, %30, %31}, [%32];"
-      : "=r"(v[0]), "=r"(v[1]), "=r"(v[2]), "=r"(v[3]), "=r"(v[4]), "=r"(v[5]), "=r"(v[6]), "=r"(v[7]), "=r"(v[8]),
-        "=r"(v[9]), "=r"(v[10]), "=r"(v[11]), "=r"(v[12]), "=r"(v[13]), "=r"(v[14]), "=r"(v[15]), "=r"(v[16]),
-        "=r"(v[17]), "=r"(v[18]), "=r"(v[19]), "=r"(v[20]), "=r"(v[21]), "=r"(v[22]), "=r"(v[23]), "=r"(v[24]),
-        "=r"(v[25]), "=r"(v[26]), "=r"(v[27]), "=r"(v[28]), "=r"(v[29]), "=r"(v[30]), "=r"(v[31])
-      : "r"(taddr));
-}
-__device__ __forceinline__ void tmem_ld_wait() { asm volatile("tcgen05.wait::ld.sync.aligned;" ::: "memory"); }
-
-// Shared-memory matrix descriptor: K-major tile, 128-byte swizzle, rows of 128 B, 8-row atoms 1024 B apart.
-__device__ __forceinline__ uint64_t make_sw128_desc(uint32_t smem_addr) {
-  uint64_t d = 0;
-  d |= (uint64_t)((smem_addr & 0x3FFFF) >> 4);     // start address  [0,14)
-  d |= (uint64_t)0 << 16;                          // leading byte offset (unused for swizzled K-major)
-  d |= (uint64_t)(1024 >> 4) << 32;                // stride byte offset [32,46): 8 rows * 128 B
-  d |= (uint64_t)1 << 46;                          // descriptor version (sm_100)
-  d |= (uint64_t)2 << 61;                          // layout type: SWIZZLE_128B
-  return d;
-}
 // Instruction descriptor, kind::f16: D = f32, A = B = bf16, both K-major, N >> 3 at [17,23), M >> 4 at [24,29)
 constexpr uint32_t kInstrDesc = (1u << 4) | (1u << 7) | (1u << 10) | ((uint32_t)(kBlockN >> 3) << 17) |
                                 ((uint32_t)(kBlockM >> 4) << 24);
@@ -760,38 +656,11 @@ __global__ void rank_sums_kernel(const int32_t* __restrict__ ranks, int64_t b, d
 }
 
 // ------------------------------------------------------------------------------------------------ host helpers
-typedef CUresult (*EncodeTiledFn)(CUtensorMap*, CUtensorMapDataType, cuuint32_t, void*, const cuuint64_t*, const cuuint64_t*,
-                                  const cuuint32_t*, const cuuint32_t*, CUtensorMapInterleave, CUtensorMapSwizzle,
-                                  CUtensorMapL2promotion, CUtensorMapFloatOOBfill);
-
-int get_encode_fn(EncodeTiledFn* out) {
-  ensure_thread_context();
-  static EncodeTiledFn cached = nullptr;
-  if (!cached) {
-    void* fn = nullptr;
-    cudaDriverEntryPointQueryResult qres;
-    KGC_CUDA_TRY(cudaGetDriverEntryPoint("cuTensorMapEncodeTiled", &fn, cudaEnableDefault, &qres));
-    KGC_REQUIRE(qres == cudaDriverEntryPointSuccess && fn != nullptr, "cuTensorMapEncodeTiled not available");
-    cached = reinterpret_cast<EncodeTiledFn>(fn);
-  }
-  *out = cached;
-  return 0;
-}
-
 // bf16 [rows, kpad] row-major -> boxes of 64 (K) x 128 (rows), 128-byte swizzle, zero fill out of bounds
 int make_map(CUtensorMap* map, const void* base, int64_t rows, int kpad) {
-  EncodeTiledFn enc;
-  if (get_encode_fn(&enc)) return 1;
-  KGC_REQUIRE((reinterpret_cast<uintptr_t>(base) & 15) == 0, "bf16 table must be 16-byte aligned");
-  cuuint64_t dims[2] = {(cuuint64_t)kpad, (cuuint64_t)rows};
-  cuuint64_t strides[1] = {(cuuint64_t)kpad * 2};
-  cuuint32_t box[2] = {(cuuint32_t)kBlockK, (cuuint32_t)kBlockM};
-  cuuint32_t estr[2] = {1, 1};
-  CUresult r = enc(map, CU_TENSOR_MAP_DATA_TYPE_BFLOAT16, 2, const_cast<void*>(base), dims, strides, box, estr,
-                   CU_TENSOR_MAP_INTERLEAVE_NONE, CU_TENSOR_MAP_SWIZZLE_128B, CU_TENSOR_MAP_L2_PROMOTION_L2_256B,
-                   CU_TENSOR_MAP_FLOAT_OOB_FILL_NONE);
-  KGC_REQUIRE(r == CUDA_SUCCESS, "cuTensorMapEncodeTiled failed (" + std::to_string((int)r) + ")");
-  return 0;
+  const cuuint64_t dims[2] = {(cuuint64_t)kpad, (cuuint64_t)rows}, strides[1] = {(cuuint64_t)kpad * 2};
+  const cuuint32_t box[2] = {(cuuint32_t)kBlockK, (cuuint32_t)kBlockM};
+  return encode_tiled(map, CU_TENSOR_MAP_DATA_TYPE_BFLOAT16, 2, base, dims, strides, box, CU_TENSOR_MAP_SWIZZLE_128B);
 }
 
 inline int check_kpad(int kpad) { return (kpad < 16 || kpad % 16 != 0 || kpad > kMaxKBlocks * kBlockK) ? 1 : 0; }

@@ -408,10 +408,10 @@ extern "C" int kgc_dropout_mask(const int64_t* seed, int32_t plane, float drop_p
 
 extern "C" int32_t kgc_keep_pitch() { return kKeepPitch; }
 
-extern "C" int kgc_tail_fwd_rows(const float* res3, const int32_t* slot_in, const float* rows_in, const int32_t* slot_out,
-                                 const float* rows_out, const uint8_t* mask_in, const uint8_t* mask_out, const int64_t* seed,
-                                 float drop_p, float keep_scale, const float* bias, int64_t n_rows, int32_t Dout, float* pre,
-                                 double* partials, uint8_t* keep, void* stream) {
+extern "C" int kgc_tail_fwd(const float* res3, const int32_t* slot_in, const float* rows_in, const int32_t* slot_out,
+                            const float* rows_out, const uint8_t* mask_in, const uint8_t* mask_out, const int64_t* seed,
+                            float drop_p, float keep_scale, const float* bias, int64_t n_rows, int32_t Dout, float* pre,
+                            double* partials, uint8_t* keep, void* stream) {
   KGC_REQUIRE(check_dout(Dout) == 0, "Dout must be a multiple of 4 and <= 1024");
   KGC_REQUIRE(keep == nullptr || Dout <= 4 * kKeepPitch, "packed keep flags need Dout <= 256");
   KGC_REQUIRE(n_rows > 0, "n_rows must be positive");
@@ -429,13 +429,6 @@ extern "C" int kgc_tail_fwd_rows(const float* res3, const int32_t* slot_in, cons
       (float4*)pre, partials, keep);
   KGC_LAUNCH_CHECK();
   return 0;
-}
-
-extern "C" int kgc_tail_fwd(const float* res3, const uint8_t* mask_in, const uint8_t* mask_out, const int64_t* seed,
-                            float drop_p, float keep_scale, const float* bias, int64_t n_rows, int32_t Dout, float* pre,
-                            double* partials, uint8_t* keep, void* stream) {
-  return kgc_tail_fwd_rows(res3, nullptr, nullptr, nullptr, nullptr, mask_in, mask_out, seed, drop_p, keep_scale, bias, n_rows,
-                           Dout, pre, partials, keep, stream);
 }
 
 extern "C" int kgc_rows_copy(const float* src, int64_t ld_src, const int32_t* src_rows, float* dst, int64_t ld_dst,
@@ -524,11 +517,11 @@ extern "C" int kgc_tail_bwd_reduce(const float* g_ent, const float* pre, const f
   return 0;
 }
 
-extern "C" int kgc_tail_bwd_apply_rows(const float* g_ent, const float* pre, const float* stats, const float* gamma,
-                                       const float* beta, const double* sums, int32_t training, int64_t n_rows,
-                                       int64_t n_rows_global, int32_t Dout, float* d_out, const uint8_t* keep, float keep_scale,
-                                       float* d_res_in, const int32_t* slot_in, float* d_res_out, const int32_t* slot_out,
-                                       const uint8_t* out_keep, float out_scale, void* stream) {
+extern "C" int kgc_tail_bwd_apply(const float* g_ent, const float* pre, const float* stats, const float* gamma,
+                                  const float* beta, const double* sums, int32_t training, int64_t n_rows,
+                                  int64_t n_rows_global, int32_t Dout, float* d_out, const uint8_t* keep, float keep_scale,
+                                  float* d_res_in, const int32_t* slot_in, float* d_res_out, const int32_t* slot_out,
+                                  const uint8_t* out_keep, float out_scale, void* stream) {
   KGC_REQUIRE(check_dout(Dout) == 0, "Dout must be a multiple of 4 and <= 1024");
   KGC_REQUIRE((d_res_in == nullptr) == (d_res_out == nullptr), "the in and out planes come together");
   const int Do4 = Dout / 4;
@@ -539,13 +532,4 @@ extern "C" int kgc_tail_bwd_apply_rows(const float* g_ent, const float* pre, con
       slot_out, out_keep, out_scale);
   KGC_LAUNCH_CHECK();
   return 0;
-}
-
-extern "C" int kgc_tail_bwd_apply(const float* g_ent, const float* pre, const float* stats, const float* gamma,
-                                  const float* beta, const double* sums, int32_t training, int64_t n_rows,
-                                  int64_t n_rows_global, int32_t Dout, float* d_out, const uint8_t* keep, float keep_scale,
-                                  float* d_res2, const uint8_t* out_keep, float out_scale, void* stream) {
-  return kgc_tail_bwd_apply_rows(g_ent, pre, stats, gamma, beta, sums, training, n_rows, n_rows_global, Dout, d_out, keep,
-                                 keep_scale, d_res2, nullptr, d_res2 != nullptr ? d_res2 + n_rows * Dout : nullptr, nullptr,
-                                 out_keep, out_scale, stream);
 }

@@ -14,6 +14,7 @@ import numbers
 import torch
 
 from . import _lib
+from .conv import _pack_b
 
 
 class _Score1N(torch.autograd.Function):
@@ -22,7 +23,6 @@ class _Score1N(torch.autograd.Function):
 
     @staticmethod
     def forward(ctx, x, all_ent, bias):
-        from .conv import gemm_nt  # noqa: F401  (same packing routine)
         x = _lib.require_cuda(x.detach(), torch.float32, 'x')
         ent = _lib.require_cuda(all_ent.detach(), torch.float32, 'all_ent')
         bias_ = _lib.require_cuda(bias.detach(), torch.float32, 'bias')
@@ -30,10 +30,8 @@ class _Score1N(torch.autograd.Function):
         N = int(ent.shape[0])
         ldp = (N + 3) // 4 * 4
         p = _lib.ptr
-        nbytes = int(_lib.lib().kgc_gemm_packed_b_bytes(B, D))
-        packed = torch.empty((nbytes // 4,), dtype=torch.float32, device=x.device)
+        packed = _pack_b(x.t())                         # the queries are the small operand: [K = D, N = B]
         buf = torch.empty((B, ldp), dtype=torch.float32, device=x.device)
-        _lib.call('kgc_gemm_pack_b', p(x), x.stride(1), x.stride(0), B, D, p(packed), _lib.stream())
         _lib.call('kgc_score_1n_fwd', p(ent), N, D, ent.stride(0), p(packed), B, p(bias_), p(buf), ldp, _lib.stream())
         pred = buf[:, :N]
         ctx.save_for_backward(x, ent, pred)
@@ -100,12 +98,11 @@ class _Score1NBCE(torch.autograd.Function):
             raise ValueError('qid has {} entries for {} queries'.format(int(qid.numel()), B))
         ldt = (B + 3) // 4 * 4
         p, dev = _lib.ptr, x.device
-        packed = torch.empty((int(_lib.lib().kgc_gemm_packed_b_bytes(B, D)) // 4,), dtype=torch.float32, device=dev)
+        packed = _pack_b(x.t())
         # entity-major throughout: the scorer stores predT [N, ldt] (its natural orientation), the positives are bits per
         # entity, and the loss pass overwrites predT with the logit gradient in place (the [N, ldt] operand of both
         # gradient GEMMs) - no [B, N]-pitched buffer, no transpose
         d_logit_t = torch.empty((N, ldt), dtype=torch.float32, device=dev)
-        _lib.call('kgc_gemm_pack_b', p(x), x.stride(1), x.stride(0), B, D, p(packed), _lib.stream())
         _lib.call('kgc_score_1n_fwd_t', p(ent), N, D, ent.stride(0), p(packed), B, p(bias_), p(d_logit_t), ldt, _lib.stream())
         mask_t = torch.empty((N, (B + 31) // 32), dtype=torch.int32, device=dev)          # uint32 bits; zeroed by the call
         _lib.call('kgc_label_mask_t_build', p(qid), B, p(ptr), p(idx), N, p(mask_t), _lib.stream())
@@ -304,9 +301,8 @@ def dense_logits(xq, all_ent, bias):
         raise ValueError('dense_logits: at most {} queries per call, Dout <= 224, Dout % 4 == 0'.format(B_TILE))
     ldp = (N + 3) // 4 * 4
     p = _lib.ptr
-    packed = torch.empty((int(_lib.lib().kgc_gemm_packed_b_bytes(B, D)) // 4,), dtype=torch.float32, device=xq.device)
+    packed = _pack_b(xq.t())
     buf = torch.empty((B, ldp), dtype=torch.float32, device=xq.device)
-    _lib.call('kgc_gemm_pack_b', p(xq), xq.stride(1), xq.stride(0), B, D, p(packed), _lib.stream())
     _lib.call('kgc_score_1n_logits', p(ent), N, D, ent.stride(0), p(packed), B, p(bias), p(buf), ldp, _lib.stream())
     return buf, ldp
 

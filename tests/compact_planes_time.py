@@ -82,14 +82,11 @@ def kernel_times(case, reps, flush):
     del ids
 
     def tail_fwd(rows_on):
-        if rows_on:
-            L.call('kgc_tail_fwd_rows', p(res3), p(slot), p(res_c), None, None, None, None, p(seed), 0.1, scale, None, N, Do,
-                   p(pre), p(partials), p(keep), st())
-        else:
-            L.call('kgc_tail_fwd', p(res3), None, None, p(seed), 0.1, scale, None, N, Do, p(pre), p(partials), p(keep), st())
+        L.call('kgc_tail_fwd', p(res3), p(slot) if rows_on else None, p(res_c) if rows_on else None, None, None, None, None,
+               p(seed), 0.1, scale, None, N, Do, p(pre), p(partials), p(keep), st())
 
     def tail_bwd(rows_on):
-        L.call('kgc_tail_bwd_apply_rows', p(g_ent), p(pre), p(stats), p(gamma), p(beta), p(sums), 1, N, N, Do, p(d_out), p(keep),
+        L.call('kgc_tail_bwd_apply', p(g_ent), p(pre), p(stats), p(gamma), p(beta), p(sums), 1, N, N, Do, p(d_out), p(keep),
                scale, p(d_res_c if rows_on else d_res2[0]), p(slot) if rows_on else None, p(d_res2[1]), None, None, 1.0, st())
 
     out = {'N': N, 'n_c_in': n_c, 'D': D, 'Dout': Do}
@@ -108,8 +105,8 @@ def kernel_times(case, reps, flush):
         ('compact_batch2', lambda: conv_mod.gemm_nt_batch([d_res2[1], d_out], pb[1:], [g3[1], g3[2]]))], reps, flush)
     out['k4c'] = timed([
         ('dense_batch3', lambda: conv_mod.gemm_tn_batch([agg[0], agg[1], x], [d_res2[0], d_res2[1], d_out], [dw[0], dw[1], dw[2]])),
-        ('compact_rows', lambda: conv_mod.gemm_tn_batch_rows([agg_c, agg[1], x], [d_res_c, d_res2[1], d_out], [dw[0], dw[1], dw[2]],
-                                                             [n_c, N, N]))], reps, flush)
+        ('compact_rows', lambda: conv_mod.gemm_tn_batch([agg_c, agg[1], x], [d_res_c, d_res2[1], d_out], [dw[0], dw[1], dw[2]],
+                                                        rows=[n_c, N, N]))], reps, flush)
     for key in ('k4b_fwd', 'k4b_bwd'):
         v = out[key]
         v['compact_total_ms'] = round(sum(t['ms'] for n_, t in v.items() if n_.startswith('compact')), 4)

@@ -630,7 +630,8 @@ def test_linear_tc_fc_layer(k, B, F, O):
 
 
 def test_gemm_batches_match_single_launches(k):
-    """The batched K4b / K4c launches give bit-identical K4b results and fp32-accurate, deterministic K4c results."""
+    """The batched K4b / K4c launches give bit-identical K4b results and fp32-accurate, deterministic K4c results; K4c with
+    rows = M for every problem gives the bits of the launch without rows."""
     from kgc_gcn_b200.conv import gemm_nt_batch, gemm_tn_batch, _pack_b
     g = torch.Generator().manual_seed(5)
     M, K, N = 5000, 100, 200
@@ -648,10 +649,13 @@ def test_gemm_batches_match_single_launches(k):
         gemm_tn_batch(a[:n], b[:n], outs)
         outs2 = [torch.empty((K, N), device='cuda') for _ in range(n)]
         gemm_tn_batch(a[:n], b[:n], outs2)
+        outs3 = [torch.empty((K, N), device='cuda') for _ in range(n)]
+        gemm_tn_batch(a[:n], b[:n], outs3, rows=[M] * n)        # every problem of full height: the bits of rows=None
         for i in range(n):
             truth = a[i].double().t() @ b[i].double()
             assert float((outs[i].double() - truth).abs().max()) / float(truth.abs().max()) <= 3e-6
             assert torch.equal(outs[i], outs2[i])
+            assert torch.equal(outs[i], outs3[i])
 
 
 @pytest.mark.parametrize('workload', ['wn18rr', 'fb15k237', 'wikidata5m'])
