@@ -534,7 +534,7 @@ int kgc_topk_merge(const float* part_s, const int32_t* part_id, int64_t n_lists,
  * D % 4 == 0, D <= 256; x, ent, d_x 16-byte aligned.
  * kgc_sampled_bce_fwd, in one pass: loss[0] = mean over the valid slots of ATen's BCE of p = sigmoid(<x[b], ent[c]> +
  * bias[c]) (0 when no slot is valid), count[0] = the number of valid slots, g [B, C] = the logit gradient for a unit
- * upstream gradient (0 on empty slots, formulas of kgc_bce_1n_bwd_logit_t with the valid-slot count as divisor) and
+ * upstream gradient (0 on empty slots, kgc_bce_1n_bwd_logit_t's formulas, csrc/bce.cuh, with the valid-slot count as divisor) and
  * d_x [B, D] = sum_c g[b, c] * ent[cand[b, c]] in slot order.  loss_partial: kgc_sampled_bce_fwd_blocks(B) doubles.
  * kgc_sampled_bce_bwd_table: the dense table gradient for the upstream scalar *scale (device memory):
  * d_ent[n] = sum over the slots s with cand[s] = n of g[s] * (*scale * x[b(s)]), d_bias[n] = *scale * sum g[s], in slot

@@ -3,14 +3,12 @@
 // the rest negatives (label add); an id outside [0, N) is an empty slot (no loss, no gradient).  The cost is B x C
 // gathered rows, independent of N, so the batch can grow far beyond what the 1-N objective's [N, B] tiles allow.
 //
-// Forward (one pass): logit = <x[b], E[cand]> + bias[cand] in fp32 (per-lane FMA over the lane's float4 columns, then a
-// fixed xor-shuffle tree: every lane ends with the same bits), p = sigmoid, then ATen's BCE formulas as
-// kgc_bce_1n_bwd_logit_t (score_train.cu) with the VALID-slot count as the mean's divisor:
-//   loss term = (y - 1) * max(log1p(-p), -100) - y * max(log(p), -100)
-//   g         = (p - y) / max((1 - p) p, 1e-12) * (1 / count) * p (1 - p)            (unit upstream gradient)
-// and, while the candidate row is still in registers, d_x[b] += g * E[cand] in slot order.  A warp owns one query: the x
-// row lives in registers, a candidate row is one coalesced request of 4 D bytes (800 at D = 200), and the rows of a batch
-// of kRowsInFlight slots are all loaded before the first is consumed (the lesson of agg_lean_kernel, DESIGN section 4).
+// Forward (one pass): logit = <x[b], E[cand]> + bias[cand] in fp32 (warp_dot), p = sigmoid, then ATen's BCE as
+// kgc_bce_1n_bwd_logit_t (bce.cuh) with the VALID-slot count as the mean's divisor: g = bce_logit_grad(p, y, 1 / count)
+// (unit upstream gradient) and, while the candidate row is still in registers, d_x[b] += g * E[cand] in slot order.  A
+// warp owns one query: the x row lives in registers, a candidate row is one coalesced request of 4 D bytes (800 at
+// D = 200), and the rows of a batch of kRowsInFlight slots are all loaded before the first is consumed (the lesson of
+// agg_lean_kernel, DESIGN section 4).
 //
 // Table backward: d_E[n] = sum over the slots s with cand[s] = n of g[s] * (scale x[b(s)]) and d_bias[n] = scale sum g[s],
 // dense [N, D] / [N] with zeros elsewhere (the encoder's backward takes a dense upstream).  Duplicate candidates are the
@@ -24,6 +22,7 @@
 
 #include <cub/device/device_radix_sort.cuh>
 
+#include "bce.cuh"
 #include "common.cuh"
 
 namespace kgc {
@@ -43,6 +42,23 @@ __device__ __forceinline__ void fma4(float s, const float4& a, float4& acc) {
   acc.y = fmaf(s, a.y, acc.y);
   acc.z = fmaf(s, a.z, acc.z);
   acc.w = fmaf(s, a.w, acc.w);
+}
+
+// <x, r> in fp32: a per-lane FMA chain over the lane's float4 columns, then a fixed xor-shuffle tree (every lane ends
+// with the same bits)
+template <int NV>
+__device__ __forceinline__ float warp_dot(const float4 (&xr)[NV], const float4 (&r)[NV]) {
+  float s = 0.f;
+#pragma unroll
+  for (int v = 0; v < NV; ++v) {
+    s = fmaf(xr[v].x, r[v].x, s);
+    s = fmaf(xr[v].y, r[v].y, s);
+    s = fmaf(xr[v].z, r[v].z, s);
+    s = fmaf(xr[v].w, r[v].w, s);
+  }
+#pragma unroll
+  for (int o = 16; o > 0; o >>= 1) s += __shfl_xor_sync(kFull, s, o);
+  return s;
 }
 
 // number of valid slots (integer sum: the order of the atomics does not matter)
@@ -100,25 +116,14 @@ sampled_bce_fwd_kernel(const float* __restrict__ x, int64_t B, int D4, const flo
       float g_mine = 0.f;
 #pragma unroll
       for (int u = 0; u < kRowsInFlight; ++u) {
-        float s = 0.f;
-#pragma unroll
-        for (int v = 0; v < NV; ++v) {
-          s = fmaf(xr[v].x, r[u][v].x, s);
-          s = fmaf(xr[v].y, r[u][v].y, s);
-          s = fmaf(xr[v].z, r[u][v].z, s);
-          s = fmaf(xr[v].w, r[u][v].w, s);
-        }
-#pragma unroll
-        for (int o = 16; o > 0; o >>= 1) s += __shfl_xor_sync(kFull, s, o);
+        const float s = warp_dot(xr, r[u]);
         float g = 0.f;
         if (e[u] >= 0) {
           const float z = s + bi[u];
           const float p = 1.f / (1.f + expf(-z));                 // the 1-N scorer's epilogue sigmoid
           const float y = c0 + u < n_pos ? pos : add;
-          const float lp = fmaxf(logf(p), -100.f), l1p = fmaxf(log1pf(-p), -100.f);
-          loss += (double)((y - 1.f) * l1p - y * lp);
-          const float d_pred = (p - y) / fmaxf((1.f - p) * p, 1e-12f) * inv_count;
-          g = d_pred * p * (1.f - p);
+          loss += (double)bce_loss_term(p, y);
+          g = bce_logit_grad(p, y, inv_count);
 #pragma unroll
           for (int v = 0; v < NV; ++v) fma4(g, r[u][v], acc[v]);
         }
@@ -132,13 +137,8 @@ sampled_bce_fwd_kernel(const float* __restrict__ x, int64_t B, int D4, const flo
       if (c4 < D4) *reinterpret_cast<float4*>(d_x + b * 4 * D4 + 4 * c4) = acc[v];
     }
   }
-  if (lane == 0) warp_loss[warp] = loss;
-  __syncthreads();
-  if (threadIdx.x == 0) {
-    double s = 0.0;
-    for (int w = 0; w < kWarpsSS; ++w) s += warp_loss[w];
-    loss_partial[blockIdx.x] = s;
-  }
+  const double s = cta_sum(loss, warp_loss, lane, warp);
+  if (threadIdx.x == 0) loss_partial[blockIdx.x] = s;
 }
 
 // mean over the valid slots: one CTA adds the per-CTA partials in a fixed order (0 when no slot is valid)
@@ -146,15 +146,8 @@ __global__ void __launch_bounds__(kThreadsSS)
 sampled_bce_finalize_kernel(const double* __restrict__ partial, int64_t n_partial, const int32_t* __restrict__ count,
                             float* __restrict__ loss) {
   __shared__ double sh[kThreadsSS];
-  double s = 0.0;
-  for (int64_t i = threadIdx.x; i < n_partial; i += kThreadsSS) s += partial[i];
-  sh[threadIdx.x] = s;
-  __syncthreads();
-  for (int o = kThreadsSS / 2; o > 0; o >>= 1) {
-    if ((int)threadIdx.x < o) sh[threadIdx.x] += sh[threadIdx.x + o];
-    __syncthreads();
-  }
-  if (threadIdx.x == 0) loss[0] = *count > 0 ? (float)(sh[0] / (double)*count) : 0.f;
+  const double s = cta_sum_partials(partial, n_partial, sh);
+  if (threadIdx.x == 0) loss[0] = *count > 0 ? (float)(s / (double)*count) : 0.f;
 }
 
 // Self-adversarial variant (RotatE's negative weighting).  Q+ / Q- = the queries with at least one valid positive /
@@ -172,11 +165,6 @@ count_adv_kernel(const int32_t* __restrict__ cand, int64_t B, int C, int n_pos, 
   }
   if (lane == 0 && qp != 0) atomicAdd(counts, qp);
   if (lane == 0 && qn != 0) atomicAdd(counts + 1, qn);
-}
-
-// ATen's BCE gradient factor of one slot with the coefficient c applied as kgc_bce_1n_bwd_logit_t applies 1 / count
-__device__ __forceinline__ float bce_logit_grad(float p, float y, float c) {
-  return (p - y) / fmaxf((1.f - p) * p, 1e-12f) * c * p * (1.f - p);
 }
 
 // The loss of sampled_bce_fwd_kernel with the negatives of query b weighted by w = softmax over its valid negative slots
@@ -237,17 +225,7 @@ sampled_adv_fwd_kernel(const float* __restrict__ x, int64_t B, int D4, const flo
       float m_new = m;
 #pragma unroll
       for (int u = 0; u < kRowsInFlight; ++u) {
-        float s = 0.f;
-#pragma unroll
-        for (int v = 0; v < NV; ++v) {
-          s = fmaf(xr[v].x, r[u][v].x, s);
-          s = fmaf(xr[v].y, r[u][v].y, s);
-          s = fmaf(xr[v].z, r[u][v].z, s);
-          s = fmaf(xr[v].w, r[u][v].w, s);
-        }
-#pragma unroll
-        for (int o = 16; o > 0; o >>= 1) s += __shfl_xor_sync(kFull, s, o);
-        z[u] = s + bi[u];
+        z[u] = warp_dot(xr, r[u]) + bi[u];
         if (e[u] >= 0 && c0 + u >= n_pos) m_new = fmaxf(m_new, alpha * z[u]);
       }
       if (m_new > m) {                                           // rescale what was summed under the old max
@@ -292,8 +270,7 @@ sampled_adv_fwd_kernel(const float* __restrict__ x, int64_t B, int D4, const flo
         const float zc = gb[c];
         const float p = 1.f / (1.f + expf(-zc));
         const float y = c < n_pos ? pos : add;
-        const float lgp = fmaxf(logf(p), -100.f), l1p = fmaxf(log1pf(-p), -100.f);
-        const float term = (y - 1.f) * l1p - y * lgp;
+        const float term = bce_loss_term(p, y);
         if (c < n_pos) {
           lp += (double)term;
           gv = bce_logit_grad(p, y, cp);
@@ -305,11 +282,8 @@ sampled_adv_fwd_kernel(const float* __restrict__ x, int64_t B, int D4, const flo
       }
       gb[c] = gv;
     }
-#pragma unroll
-    for (int o = 16; o > 0; o >>= 1) {
-      lp += __shfl_xor_sync(kFull, lp, o);
-      ln += __shfl_xor_sync(kFull, ln, o);
-    }
+    lp = warp_sum(lp);
+    ln = warp_sum(ln);
     loss_p = n_p > 0 ? lp / (double)n_p : 0.0;
     loss_n = S > 0.f ? ln / (double)S : 0.0;
 #pragma unroll
@@ -322,15 +296,11 @@ sampled_adv_fwd_kernel(const float* __restrict__ x, int64_t B, int D4, const flo
       }
     }
   }
-  if (lane == 0) {
-    warp_loss[0][warp] = loss_p;
-    warp_loss[1][warp] = loss_n;
-  }
-  __syncthreads();
-  if (threadIdx.x < 2) {
-    double s = 0.0;
-    for (int w = 0; w < kWarpsSS; ++w) s += warp_loss[threadIdx.x][w];
-    loss_partial[threadIdx.x * gridDim.x + blockIdx.x] = s;
+  const double sp = cta_sum(loss_p, warp_loss[0], lane, warp);
+  const double sn = cta_sum(loss_n, warp_loss[1], lane, warp);
+  if (threadIdx.x == 0) {
+    loss_partial[blockIdx.x] = sp;
+    loss_partial[gridDim.x + blockIdx.x] = sn;
   }
 }
 
@@ -340,22 +310,11 @@ __global__ void __launch_bounds__(kThreadsSS)
 sampled_adv_finalize_kernel(const double* __restrict__ partial, int64_t n_partial, const int32_t* __restrict__ counts,
                             float* __restrict__ loss) {
   __shared__ double sh[2][kThreadsSS];
-  for (int h = 0; h < 2; ++h) {
-    double s = 0.0;
-    for (int64_t i = threadIdx.x; i < n_partial; i += kThreadsSS) s += partial[h * n_partial + i];
-    sh[h][threadIdx.x] = s;
-  }
-  __syncthreads();
-  for (int o = kThreadsSS / 2; o > 0; o >>= 1) {
-    if ((int)threadIdx.x < o) {
-      sh[0][threadIdx.x] += sh[0][threadIdx.x + o];
-      sh[1][threadIdx.x] += sh[1][threadIdx.x + o];
-    }
-    __syncthreads();
-  }
+  const double sp = cta_sum_partials(partial, n_partial, sh[0]);
+  const double sn = cta_sum_partials(partial + n_partial, n_partial, sh[1]);
   if (threadIdx.x == 0) {
-    const double lp = counts[0] > 0 ? sh[0][0] / (2.0 * (double)counts[0]) : 0.0;
-    const double ln = counts[1] > 0 ? sh[1][0] / (2.0 * (double)counts[1]) : 0.0;
+    const double lp = counts[0] > 0 ? sp / (2.0 * (double)counts[0]) : 0.0;
+    const double ln = counts[1] > 0 ? sn / (2.0 * (double)counts[1]) : 0.0;
     loss[0] = (float)(lp + ln);
   }
 }
@@ -458,6 +417,23 @@ bool shapes_ok(int64_t B, int32_t D, int32_t C, int64_t n_ent) {
          B * (int64_t)C < (int64_t{1} << 31);
 }
 
+// the requirements kgc_sampled_bce_fwd and kgc_sampled_adv_fwd share: the failed one's message, or nullptr
+const char* check_fwd_args(const float* x, int64_t B, int32_t D, const float* ent, int64_t n_ent, int64_t ld_ent,
+                           const float* bias, const int32_t* cand, int32_t C, int32_t n_pos, const float* g, const float* d_x,
+                           const int32_t* counts, const double* loss_partial, const float* loss) {
+  if (!shapes_ok(B, D, C, n_ent)) return "bad sizes (B, C > 0, B * C < 2^31, 0 < D <= 256, D % 4 == 0, 0 < N < 2^31 - 1)";
+  if (n_pos < 0 || n_pos > C) return "n_pos must lie in [0, C]";
+  if (ld_ent < D || ld_ent % 4 != 0) return "entity rows need ld_ent >= D and a 16-byte pitch";
+  if (!(x && ent && bias && cand && g && d_x && counts && loss_partial && loss)) return "null buffer";
+  if (((reinterpret_cast<uintptr_t>(x) | reinterpret_cast<uintptr_t>(ent) | reinterpret_cast<uintptr_t>(d_x)) & 15) != 0)
+    return "x, all_ent and d_x must be 16-byte aligned";
+  return nullptr;
+}
+
+// the instantiation of a row kernel for D = 4 * D4: one float4 column per lane up to D = 128, two up to 256
+template <typename Kernel>
+Kernel for_width(int D4, Kernel nv1, Kernel nv2) { return D4 <= 32 ? nv1 : nv2; }
+
 }  // namespace
 }  // namespace kgc
 
@@ -468,12 +444,8 @@ extern "C" int64_t kgc_sampled_bce_fwd_blocks(int64_t B) { return ceil_div(B > 0
 extern "C" int kgc_sampled_bce_fwd(const float* x, int64_t B, int32_t D, const float* ent, int64_t n_ent, int64_t ld_ent,
                                    const float* bias, const int32_t* cand, int32_t C, int32_t n_pos, float pos, float add,
                                    float* g, float* d_x, int32_t* count, double* loss_partial, float* loss, void* stream) {
-  KGC_REQUIRE(shapes_ok(B, D, C, n_ent), "bad sizes (B, C > 0, B * C < 2^31, 0 < D <= 256, D % 4 == 0, 0 < N < 2^31 - 1)");
-  KGC_REQUIRE(n_pos >= 0 && n_pos <= C, "n_pos must lie in [0, C]");
-  KGC_REQUIRE(ld_ent >= D && ld_ent % 4 == 0, "entity rows need ld_ent >= D and a 16-byte pitch");
-  KGC_REQUIRE(x && ent && bias && cand && g && d_x && count && loss_partial && loss, "null buffer");
-  KGC_REQUIRE(((reinterpret_cast<uintptr_t>(x) | reinterpret_cast<uintptr_t>(ent) | reinterpret_cast<uintptr_t>(d_x)) & 15) == 0,
-              "x, all_ent and d_x must be 16-byte aligned");
+  if (const char* err = check_fwd_args(x, B, D, ent, n_ent, ld_ent, bias, cand, C, n_pos, g, d_x, count, loss_partial, loss))
+    return fail(__func__, err);
   cudaStream_t s = as_stream(stream);
   const int64_t n_slots = B * C;
   KGC_CUDA_TRY(cudaMemsetAsync(count, 0, sizeof(int32_t), s));
@@ -482,12 +454,9 @@ extern "C" int kgc_sampled_bce_fwd(const float* x, int64_t B, int32_t D, const f
   KGC_LAUNCH_CHECK();
   const int64_t blocks = kgc_sampled_bce_fwd_blocks(B);
   const int D4 = D / 4;
-  if (D4 <= 32)
-    sampled_bce_fwd_kernel<1><<<(unsigned)blocks, kThreadsSS, 0, s>>>(x, B, D4, ent, ld_ent, n_ent, bias, cand, C, n_pos, pos,
-                                                                      add, count, g, d_x, loss_partial);
-  else
-    sampled_bce_fwd_kernel<2><<<(unsigned)blocks, kThreadsSS, 0, s>>>(x, B, D4, ent, ld_ent, n_ent, bias, cand, C, n_pos, pos,
-                                                                      add, count, g, d_x, loss_partial);
+  const auto fwd = for_width(D4, sampled_bce_fwd_kernel<1>, sampled_bce_fwd_kernel<2>);
+  fwd<<<(unsigned)blocks, kThreadsSS, 0, s>>>(x, B, D4, ent, ld_ent, n_ent, bias, cand, C, n_pos, pos, add, count, g, d_x,
+                                              loss_partial);
   KGC_LAUNCH_CHECK();
   sampled_bce_finalize_kernel<<<1, kThreadsSS, 0, s>>>(loss_partial, blocks, count, loss);
   KGC_LAUNCH_CHECK();
@@ -498,13 +467,9 @@ extern "C" int kgc_sampled_adv_fwd(const float* x, int64_t B, int32_t D, const f
                                    const float* bias, const int32_t* cand, int32_t C, int32_t n_pos, float pos, float add,
                                    float temperature, float* g, float* d_x, int32_t* counts, double* loss_partial, float* loss,
                                    void* stream) {
-  KGC_REQUIRE(shapes_ok(B, D, C, n_ent), "bad sizes (B, C > 0, B * C < 2^31, 0 < D <= 256, D % 4 == 0, 0 < N < 2^31 - 1)");
-  KGC_REQUIRE(n_pos >= 0 && n_pos <= C, "n_pos must lie in [0, C]");
-  KGC_REQUIRE(ld_ent >= D && ld_ent % 4 == 0, "entity rows need ld_ent >= D and a 16-byte pitch");
+  if (const char* err = check_fwd_args(x, B, D, ent, n_ent, ld_ent, bias, cand, C, n_pos, g, d_x, counts, loss_partial, loss))
+    return fail(__func__, err);
   KGC_REQUIRE(std::isfinite(temperature) && temperature >= 0.f, "the adversarial temperature must be finite and >= 0");
-  KGC_REQUIRE(x && ent && bias && cand && g && d_x && counts && loss_partial && loss, "null buffer");
-  KGC_REQUIRE(((reinterpret_cast<uintptr_t>(x) | reinterpret_cast<uintptr_t>(ent) | reinterpret_cast<uintptr_t>(d_x)) & 15) == 0,
-              "x, all_ent and d_x must be 16-byte aligned");
   cudaStream_t s = as_stream(stream);
   KGC_CUDA_TRY(cudaMemsetAsync(counts, 0, 2 * sizeof(int32_t), s));
   const int64_t blocks = kgc_sampled_bce_fwd_blocks(B);
@@ -512,12 +477,9 @@ extern "C" int kgc_sampled_adv_fwd(const float* x, int64_t B, int32_t D, const f
   count_adv_kernel<<<(unsigned)cblocks, kThreadsSS, 0, s>>>(cand, B, C, n_pos, n_ent, counts);
   KGC_LAUNCH_CHECK();
   const int D4 = D / 4;
-  if (D4 <= 32)
-    sampled_adv_fwd_kernel<1><<<(unsigned)blocks, kThreadsSS, 0, s>>>(x, B, D4, ent, ld_ent, n_ent, bias, cand, C, n_pos, pos,
-                                                                      add, temperature, counts, g, d_x, loss_partial);
-  else
-    sampled_adv_fwd_kernel<2><<<(unsigned)blocks, kThreadsSS, 0, s>>>(x, B, D4, ent, ld_ent, n_ent, bias, cand, C, n_pos, pos,
-                                                                      add, temperature, counts, g, d_x, loss_partial);
+  const auto fwd = for_width(D4, sampled_adv_fwd_kernel<1>, sampled_adv_fwd_kernel<2>);
+  fwd<<<(unsigned)blocks, kThreadsSS, 0, s>>>(x, B, D4, ent, ld_ent, n_ent, bias, cand, C, n_pos, pos, add, temperature, counts,
+                                              g, d_x, loss_partial);
   KGC_LAUNCH_CHECK();
   sampled_adv_finalize_kernel<<<1, kThreadsSS, 0, s>>>(loss_partial, blocks, counts, loss);
   KGC_LAUNCH_CHECK();
@@ -560,12 +522,8 @@ extern "C" int kgc_sampled_bce_bwd_table(const float* x, int64_t B, int32_t D, c
                                                key_bits(n_ent), s));
   const unsigned blocks = (unsigned)ceil_div(ceil_div(n_slots, 32), kWarpsSS);
   const int D4 = D / 4;
-  if (D4 <= 32)
-    table_grad_kernel<1><<<blocks, kThreadsSS, 0, s>>>(keys_out, slots_out, n_slots, n_ent, x, D4, C, g, scale, d_ent, ld_d,
-                                                       d_bias);
-  else
-    table_grad_kernel<2><<<blocks, kThreadsSS, 0, s>>>(keys_out, slots_out, n_slots, n_ent, x, D4, C, g, scale, d_ent, ld_d,
-                                                       d_bias);
+  const auto grad = for_width(D4, table_grad_kernel<1>, table_grad_kernel<2>);
+  grad<<<blocks, kThreadsSS, 0, s>>>(keys_out, slots_out, n_slots, n_ent, x, D4, C, g, scale, d_ent, ld_d, d_bias);
   KGC_LAUNCH_CHECK();
   return 0;
 }

@@ -8,6 +8,7 @@
 // One CTA owns 32 entities and walks the batch in tiles of 32 queries: coalesced 128-byte reads along n, a padded
 // shared-memory transpose, coalesced 128-byte writes along b.  The bias sum is a fixed shuffle tree per tile, tiles added
 // in order: deterministic, no atomics.
+#include "bce.cuh"
 #include "common.cuh"
 
 namespace kgc {
@@ -102,10 +103,8 @@ bce_1n_t_kernel(float* __restrict__ pred_t, const uint32_t* __restrict__ mask_t,
         if (4 * c + j < B) {
           const float p = e[j];
           const float y = ((w >> j) & 1u) ? pos : add;
-          const float lp = fmaxf(logf(p), -100.f), l1p = fmaxf(log1pf(-p), -100.f);
-          loss += (double)((y - 1.f) * l1p - y * lp);
-          const float d_pred = (p - y) / fmaxf((1.f - p) * p, 1e-12f) * inv_count;
-          g = d_pred * p * (1.f - p);
+          loss += (double)bce_loss_term(p, y);
+          g = bce_logit_grad(p, y, inv_count);
         }
         e[j] = g;                                                   // pad columns [B, ldt) get zeros
         bsum += g;
@@ -116,30 +115,16 @@ bce_1n_t_kernel(float* __restrict__ pred_t, const uint32_t* __restrict__ mask_t,
     for (int o = 16; o > 0; o >>= 1) bsum += __shfl_xor_sync(0xFFFFFFFFu, bsum, o);
     if (lane == 0) d_bias[n] = bsum;
   }
-#pragma unroll
-  for (int o = 16; o > 0; o >>= 1) loss += __shfl_xor_sync(0xFFFFFFFFu, loss, o);
-  if (lane == 0) warp_loss[warp] = loss;
-  __syncthreads();
-  if (threadIdx.x == 0) {
-    double s = 0.0;
-    for (int w = 0; w < kThreadsST / 32; ++w) s += warp_loss[w];
-    loss_partial[blockIdx.x] = s;
-  }
+  const double s = cta_sum(warp_sum(loss), warp_loss, lane, warp);
+  if (threadIdx.x == 0) loss_partial[blockIdx.x] = s;
 }
 
 // mean over B * N elements: one CTA adds the per-CTA partials in a fixed order (thread t takes t, t + 256, ...; then a tree)
 __global__ void __launch_bounds__(kThreadsST)
 bce_1n_finalize_kernel(const double* __restrict__ partial, int64_t n_partial, double inv_count, float* __restrict__ loss) {
   __shared__ double sh[kThreadsST];
-  double s = 0.0;
-  for (int64_t i = threadIdx.x; i < n_partial; i += kThreadsST) s += partial[i];
-  sh[threadIdx.x] = s;
-  __syncthreads();
-  for (int o = kThreadsST / 2; o > 0; o >>= 1) {
-    if ((int)threadIdx.x < o) sh[threadIdx.x] += sh[threadIdx.x + o];
-    __syncthreads();
-  }
-  if (threadIdx.x == 0) loss[0] = (float)(sh[0] * inv_count);
+  const double s = cta_sum_partials(partial, n_partial, sh);
+  if (threadIdx.x == 0) loss[0] = (float)(s * inv_count);
 }
 
 }  // namespace

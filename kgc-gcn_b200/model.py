@@ -281,19 +281,24 @@ class MGCN(nn.Module):
     def loss(self, pred, label):
         return self.loss_fn(pred, label)
 
+    def _train_queries(self, qid, triples, data):
+        """The training queries ``qid`` (rows of ``triples``) through the encoder and ConvE's front end: (qid on the device,
+        the query matrix x [B, Dout], the entity table to score, its gradient folded with the query rows' by _rows)."""
+        qid = torch.as_tensor(qid, dtype=torch.int64).to(triples.device, non_blocking=True)
+        trip = torch.index_select(triples, 0, qid)
+        all_ent, all_rel = self.encode(data)
+        src_emb, all_ent = self._rows(all_ent, trip[:, 0])
+        x = self.conv2.query(src_emb, torch.index_select(all_rel, 0, trip[:, 1]))
+        return qid, x, all_ent
+
     def loss_sparse(self, qid, dataset, data):
         """``loss(forward(src, rel, data), label)`` for the training queries ``qid`` of ``dataset`` (a KBDataset) without the
         dense [B, N] label or the BCE tensors (SURVEY.md 8(f) N1): src / rel are the queries' triples and the label is read
         as sparse positives from the dataset's CSR with its ``label_values()`` (label smoothing as data_loader.py:41-43).
         Same value and gradients as the dense route within fp32 rounding (tests/test_gpu_zz_loss.py)."""
         from .scoring import score_1n_bce, score_1n_supported
-        dev = self.entity_embedding.device
-        triples, ptr, idx = dataset.device_csr(dev)
-        qid = torch.as_tensor(qid, dtype=torch.int64).to(dev, non_blocking=True)
-        trip = torch.index_select(triples, 0, qid)
-        all_ent, all_rel = self.encode(data)
-        src_emb, all_ent = self._rows(all_ent, trip[:, 0])
-        x = self.conv2.query(src_emb, torch.index_select(all_rel, 0, trip[:, 1]))
+        triples, ptr, idx = dataset.device_csr(self.entity_embedding.device)
+        qid, x, all_ent = self._train_queries(qid, triples, data)
         if not score_1n_supported(x, all_ent):
             raise RuntimeError('loss_sparse: shape not taken by the tensor-core scorer (Dout <= 224, Dout % 4 == 0); '
                                'use loss(forward(...), label)')
@@ -315,12 +320,10 @@ class MGCN(nn.Module):
         triples, _, _ = dataset.device_csr(dev)
         qid = torch.as_tensor(qid, dtype=torch.int64).to(dev, non_blocking=True)
         pos_draws, neg_draws = draws if draws is not None else (None, None)
+        # drawn before encode, which may also draw from torch's generator: this order fixes the random stream
         cand = torch.cat([dataset.positives(qid, n_pos, draws=pos_draws, device=dev, generator=generator),
                           dataset.negatives(qid, k, draws=neg_draws, tries=tries, device=dev, generator=generator)], 1)
-        trip = torch.index_select(triples, 0, qid)
-        all_ent, all_rel = self.encode(data)
-        src_emb, all_ent = self._rows(all_ent, trip[:, 0])
-        x = self.conv2.query(src_emb, torch.index_select(all_rel, 0, trip[:, 1]))
+        _, x, all_ent = self._train_queries(qid, triples, data)
         pos, add = dataset.label_values()
         return score_sampled_bce(x, all_ent, self.conv2.bias, cand, n_pos, pos, add,
                                  adversarial_temperature=adversarial_temperature)

@@ -45,16 +45,17 @@ class GraphedTrainStep(object):
         self.dev = dev
         self.params = [p for p in model.parameters() if p.requires_grad]
         self.trip = torch.zeros((self.B, 3), dtype=torch.int64, device=dev)
-        self.fused_loss = bool(fused_loss)
+        # the objective: 'dense' (MGCN.loss on a dense label), 'sparse' (MGCN.loss_sparse) or 'sampled' (MGCN.loss_sampled)
+        self.objective = 'sampled' if negatives is not None else 'sparse' if fused_loss else 'dense'
         self.negatives = None if negatives is None else int(negatives)
         self.n_pos, self.tries, self.generator = int(n_pos), int(tries), generator
         self.adversarial_temperature = adversarial_temperature
-        self.pos_draws = self.neg_draws = None
-        if self.negatives is not None:
+        self.pos_draws = self.neg_draws = self.label = None
+        if self.objective == 'sampled':
             self.pos_draws = torch.zeros((self.B, self.n_pos), dtype=torch.int64, device=dev)
             self.neg_draws = torch.zeros((self.B, self.negatives, self.tries), dtype=torch.int64, device=dev)
-        self.label = None if (self.fused_loss or self.negatives is not None) else \
-            torch.zeros((self.B, dataset.num_entity), dtype=torch.float32, device=dev)
+        elif self.objective == 'dense':
+            self.label = torch.zeros((self.B, dataset.num_entity), dtype=torch.float32, device=dev)
         self.qid = torch.zeros((self.B,), dtype=torch.int64, device=dev)
         self._opt_clips = bool(getattr(optimizer, 'param_groups', None)) and \
             all(g.get('max_norm') for g in optimizer.param_groups)
@@ -79,11 +80,11 @@ class GraphedTrainStep(object):
             self._pin_done.record()
         else:
             self.qid.copy_(host, non_blocking=True)
-        if self.negatives is not None:               # fresh sampler inputs, drawn outside the graph (positives first)
+        if self.objective == 'sampled':              # fresh sampler inputs, drawn outside the graph (positives first)
             self.pos_draws.random_(0, 1 << 32, generator=self.generator)
             self.neg_draws.random_(0, 1 << 32, generator=self.generator)
             return
-        if self.fused_loss:                           # the graph reads the triples and the positives through qid
+        if self.objective == 'sparse':               # the graph reads the triples and the positives through qid
             return
         triples, ptr, idx = self.ds.device_csr(self.dev)
         pos, add = self.ds.label_values()
@@ -92,11 +93,11 @@ class GraphedTrainStep(object):
                   p(self.trip), p(self.label), _lib.stream())
 
     def _body(self, trip, label, qid=None, draws=None):
-        if self.negatives is not None:
+        if self.objective == 'sampled':
             loss = self.model.loss_sampled(qid, self.ds, self.graph_data, self.negatives, n_pos=self.n_pos, tries=self.tries,
                                            draws=draws, generator=self.generator,
                                            adversarial_temperature=self.adversarial_temperature)
-        elif qid is not None:
+        elif self.objective == 'sparse':
             loss = self.model.loss_sparse(qid, self.ds, self.graph_data)
         else:
             pred = self.model(trip[:, 0], trip[:, 1], self.graph_data)
@@ -160,14 +161,14 @@ class GraphedTrainStep(object):
 
     def _graph_inputs(self):
         """(qid, draws) arguments of the captured body: the static buffers the objective reads."""
-        if self.negatives is not None:
+        if self.objective == 'sampled':
             return self.qid, (self.pos_draws, self.neg_draws)
-        return (self.qid if self.fused_loss else None), None
+        return (self.qid if self.objective == 'sparse' else None), None
 
     def __call__(self, qid):
         if len(qid) != self.B:                       # ragged last batch: the eager path (same arithmetic)
             self.opt.zero_grad(set_to_none=True)
-            if self.fused_loss or self.negatives is not None:
+            if self.objective != 'dense':
                 return self._body(None, None, torch.as_tensor(qid, dtype=torch.int64).to(self.dev))
             trip, label = self.ds.build_batch(qid, self.dev)
             return self._body(trip, label)
