@@ -31,7 +31,7 @@ extern "C" {
 #pragma GCC visibility push(default)   /* the library is built with -fvisibility=hidden */
 #endif
 
-#define KGC_ABI_VERSION 3
+#define KGC_ABI_VERSION 4
 
 /* Work item of a fix-up reduction level: rows [beg, end) of the carry / partial array are summed;
  * the result goes to row `out` of the final output (flags & 1) or of the partial buffer of this
@@ -258,9 +258,6 @@ int kgc_gemm_nt_batch(int32_t n_prob, const float* const* A, int64_t M, int32_t 
  * d_x_flat[B, flat] = d_y @ W, where flat = 39,200 is the long dimension. */
 int kgc_gemm_nt_trans(const float* At, int64_t M, int32_t K, int64_t ldat, const float* packed_b, int32_t N,
                       float* Ct, int64_t ldct, void* stream);
-/* Debug aid: device buffer of 9 x 64 int64 that CTA 0 of the next kgc_gemm_nt_batch / kgc_gemm_tn_tc_batch launches fills with
- * clock64() stamps per warp role, row 8 = global-timer envelope (NULL switches it off; off by default). */
-void kgc_gemm_set_debug(long long* buf);
 
 /* ---- K4c: weight-gradient reductions  C[Ka,Nb] = A[M,Ka]^T @ B[M,Nb]  (autograd of model.py:116 w.r.t. W) ----
  * Plain fp32 FMAs; every CTA reduces a slab of rows into a register-resident Ka x Nb partial, partials are added

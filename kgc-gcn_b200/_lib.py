@@ -50,7 +50,6 @@ SIGNATURES = {
     'kgc_gemm_nt_batch': (ctypes.c_int, [_i32, _vp, _i64, _i32, _i64, _vp, _i32, _vp, _i64, _vp, _i32, _f32, _vp]),
     'kgc_gemm_nt_trans': (ctypes.c_int, [_vp, _i64, _i32, _i64, _vp, _i32, _vp, _i64, _vp]),
     'kgc_gemm_nt_splitk': (ctypes.c_int, [_vp, _i64, _vp, _i64, _i64, _i32, _i32, _vp, _vp, _sz, _vp]),
-    'kgc_gemm_set_debug': (None, [_vp]),
     'kgc_gemm_tn_workspace_bytes': (_sz, [_i64, _i32, _i32]),
     'kgc_gemm_tn_tc_workspace_bytes': (_sz, [_i64, _i32, _i32]),
     'kgc_gemm_tn_tc_batch': (ctypes.c_int, [_i32, _vp, _i64, _vp, _i64, _vp, _i64, _i32, _i32, _vp, _vp, _sz, _vp, _i32, _f32,
@@ -119,7 +118,7 @@ def lib():
         for name, (res, args) in SIGNATURES.items():
             fn = getattr(handle, name)       # AttributeError if the symbol is not exported
             fn.restype, fn.argtypes = res, args
-        if handle.kgc_abi_version() != 3:
+        if handle.kgc_abi_version() != 4:
             raise RuntimeError('libkgc_b200.so ABI version mismatch')
         _LIB = handle
     return _LIB

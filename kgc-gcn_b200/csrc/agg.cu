@@ -505,7 +505,7 @@ inline int check_dim(int32_t D, int* D4, int* NF) {
   }
 
 // Lean kernel configuration (edges per batch, CTAs per SM), measured on B200 at the WN18RR / FB15k-237 shapes
-// (tests/agg_variants.py history in profiles/r01_agg_variants.md): fwd 4 x 3, bwd_src 3 x 3, bwd_rel 4 x 3 - the largest
+// (history in profiles/r01_agg_variants.md): fwd 4 x 3, bwd_src 3 x 3, bwd_rel 4 x 3 - the largest
 // batches that fit 80 registers without spills; 2 CTAs x 8 edges and 4 CTAs x 2-3 edges were 10-20% slower.
 template <int MODE> struct LeanCfg { static constexpr int ku = 4, minb = 3; };
 template <> struct LeanCfg<kBwdSrc> { static constexpr int ku = 3, minb = 3; };

@@ -9,7 +9,7 @@
 //
 //   C[M, N] = A[M, K] @ Bt[N, K]^T        A row-major fp32 (streamed), Bt = the small operand, pre-split and packed
 //
-// Measured limits (round 1, tests/gemm_timeline.py + ncu): the kernel is bound by the SHARED-MEMORY port, not by the
+// Measured limits (round 1): the kernel is bound by the SHARED-MEMORY port, not by the
 // tensor pipe: SS-mode MMAs re-read the A tile three times per k-step, the splitter moves 3x the tile bytes and the
 // epilogue transposes through shared memory - about 600 KB of shared-memory traffic per 128 x 80 output tile
 // (~4,700 cycles at 128 B/cycle).  Next step: A_hi / A_lo in TMEM (tcgen05.st by the splitter, TS-mode MMA).
@@ -75,18 +75,11 @@ struct GemmParams {
   const uint8_t* keep;
   int32_t keep_pitch;
   float keep_scale;
-  long long* dbg;     // optional timeline of CTA 0: [role][event] clock64 stamps (debug aid)
 };
 
 __global__ void __launch_bounds__(kThreadsG, 1)
 gemm_tf32x3_kernel(const __grid_constant__ GemmMaps maps, const GemmParams P) {
   extern __shared__ uint8_t smem_raw[];
-  if (P.dbg != nullptr && threadIdx.x == 0) {                      // debug aid: launch-to-exit envelope over all CTAs (ns)
-    long long g;
-    asm volatile("mov.u64 %0, %globaltimer;" : "=l"(g));
-    atomicMin(reinterpret_cast<long long*>(P.dbg) + 8 * 64 + 0, g);
-    if (blockIdx.x == 0) { P.dbg[8 * 64 + 2] = g; P.dbg[8 * 64 + 3] = clock64(); }
-  }
   uint8_t* base = reinterpret_cast<uint8_t*>((reinterpret_cast<uintptr_t>(smem_raw) + 1023) & ~uintptr_t(1023));
   const int warp = threadIdx.x / 32, lane = threadIdx.x % 32;
   const int tile_b = P.NT * kBK * 4;                               // bytes of one Bt K-block tile (NT rows x 128 B)
@@ -129,9 +122,6 @@ gemm_tf32x3_kernel(const __grid_constant__ GemmMaps maps, const GemmParams P) {
   tc_fence_after();
   const uint32_t tmem_base = *tmem_slot;
   const uint32_t tmem_a = tmem_base + kAccCols;                    // A stages: [kAStages][hi 32 columns | lo 32 columns]
-  const bool dbg_on = P.dbg != nullptr && blockIdx.x == 0;
-  int dbg_n = 0;
-#define KGC_DBG(role) do { if (dbg_on && dbg_n < 64) P.dbg[(role) * 64 + dbg_n++] = clock64(); } while (0)
 
   // work: this CTA owns column tile nt of problem prob and the row tiles mt = first, first + step, ...
   const int groups = P.n_prob * P.n_ntiles;                        // host launches a multiple of groups CTAs
@@ -157,7 +147,6 @@ gemm_tf32x3_kernel(const __grid_constant__ GemmMaps maps, const GemmParams P) {
       for (int mt = first; mt < P.n_mtiles; mt += step) {
         for (int kb = 0; kb < P.n_kb; ++kb) {
           mbar_wait(raw_empty + stage, phase ^ 1);
-          KGC_DBG(0);
           mbar_expect_tx(raw_full + stage, kTileA);
           if (P.trans_a) tma_load_3d(s_a + stage * kTileA, map_a, raw_full + stage, 0, kb * kBK, mt * (kBM / 32));
           else tma_load_2d(s_a + stage * kTileA, map_a, raw_full + stage, kb * kBK, mt * kBM);
@@ -210,7 +199,6 @@ gemm_tf32x3_kernel(const __grid_constant__ GemmMaps maps, const GemmParams P) {
           if (prob == 1) kw >>= 4;
         }
         mbar_wait(raw_full + stage, phase);
-        if (warp == 2 && lane == 0) KGC_DBG(1);
         uint32_t h[16], l[16];
         if (P.trans_a) {
           // At tile: box (32 m, 32 k) per m group = quarter; this thread's row m = lane is a COLUMN of the box: k-th
@@ -249,7 +237,6 @@ gemm_tf32x3_kernel(const __grid_constant__ GemmMaps maps, const GemmParams P) {
         __syncwarp();
         if (lane == 0) mbar_arrive(raw_empty + stage);               // the raw tile is in registers: hand the stage back to TMA
         mbar_wait(split_empty + ts, tphase ^ 1);                     // the MMAs that read this TMEM stage have retired
-        if (warp == 2 && lane == 0) KGC_DBG(2);
         tc_fence_after();
         const uint32_t taddr = tmem_a + ((uint32_t)(quarter * 32) << 16) + ts * 64 + half * 16;
         tmem_st16(taddr, h);
@@ -258,7 +245,6 @@ gemm_tf32x3_kernel(const __grid_constant__ GemmMaps maps, const GemmParams P) {
         tc_fence_before();
         __syncwarp();
         if (lane == 0) mbar_arrive(split_full + ts);
-        if (warp == 2 && lane == 0) KGC_DBG(3);
         if (++stage == kStages) { stage = 0; phase ^= 1; }
         if (++ts == kAStages) { ts = 0; tphase ^= 1; }
       }
@@ -277,7 +263,6 @@ gemm_tf32x3_kernel(const __grid_constant__ GemmMaps maps, const GemmParams P) {
         const uint32_t d_addr = tmem_base + acc * (kAccCols / 2);
         for (int kb = 0; kb < P.n_kb; ++kb) {
           mbar_wait(split_full + ts, tphase);
-          if (lane == 0) KGC_DBG(4);
           tc_fence_after();
           const int nk = min(kBK / kUK, P.ksteps - kb * (kBK / kUK));
           const uint32_t a_hi = tmem_a + ts * 64, a_lo = a_hi + 32;            // TS mode: the A operand is read from TMEM
@@ -298,7 +283,6 @@ gemm_tf32x3_kernel(const __grid_constant__ GemmMaps maps, const GemmParams P) {
             if (kb == P.n_kb - 1) umma_commit(acc_full + acc);
           }
           __syncwarp();
-          if (lane == 0) KGC_DBG(5);
           if (++ts == kAStages) { ts = 0; tphase ^= 1; }
         }
         if (++acc == 2) { acc = 0; acc_phase ^= 1; }
@@ -318,7 +302,6 @@ gemm_tf32x3_kernel(const __grid_constant__ GemmMaps maps, const GemmParams P) {
     uint32_t acc_phase = 0;
     for (int mt = first; mt < P.n_mtiles; mt += step) {
       mbar_wait(acc_full + acc, acc_phase);
-      if (warp == 10 && lane == 0) KGC_DBG(6);
       tc_fence_after();
       const int64_t m0 = (int64_t)mt * kBM + row_q;
       const uint32_t taddr = tmem_base + ((uint32_t)(quarter * 32) << 16) + acc * (kAccCols / 2);
@@ -374,19 +357,12 @@ gemm_tf32x3_kernel(const __grid_constant__ GemmMaps maps, const GemmParams P) {
         }
         buf ^= 1;
       }
-      if (warp == 10 && lane == 0) KGC_DBG(7);
       if (++acc == 2) { acc = 0; acc_phase ^= 1; }
     }
     if (lane == 0) bulk_wait_group<0>();   // all stores complete before the CTA exits
   }
   tc_fence_before();
   __syncthreads();
-  if (P.dbg != nullptr && threadIdx.x == 0) {
-    long long g;
-    asm volatile("mov.u64 %0, %globaltimer;" : "=l"(g));
-    atomicMax(reinterpret_cast<long long*>(P.dbg) + 8 * 64 + 1, g);
-    if (blockIdx.x == 0) { P.dbg[8 * 64 + 4] = g; P.dbg[8 * 64 + 5] = clock64(); }
-  }
   if (warp == 14) tmem_dealloc(tmem_base, kTmemColsTS);
 }
 
@@ -630,7 +606,6 @@ struct GemmTnParams {
   const uint8_t* keep;                           // optional dropout of the B operand while it is split (see GemmParams::keep)
   int32_t keep_pitch;
   float keep_scale;
-  long long* dbg;                                // optional timeline of CTA 0 (debug aid, see kgc_gemm_set_debug)
 };
 
 // MN-major TF32 operands have ONE legal shared-memory layout on sm_100: 128-byte swizzle with 32-byte atoms
@@ -653,12 +628,6 @@ gemm_tn_tc_kernel(const __grid_constant__ GemmTnMaps maps, const GemmTnParams P)
   const int64_t Mp = prob == 0 ? P.m_prob[0] : (prob == 1 ? P.m_prob[1] : P.m_prob[2]);
   const int64_t m0 = slab * P.rows_per_cta;
   if (m0 >= Mp && Mp < P.M) return;                                // a slab past a shorter problem's rows: not reduced
-  if (P.dbg != nullptr && threadIdx.x == 0) {                      // debug aid: launch-to-exit envelope over all CTAs (ns)
-    long long g;
-    asm volatile("mov.u64 %0, %globaltimer;" : "=l"(g));
-    atomicMin(reinterpret_cast<long long*>(P.dbg) + 8 * 64 + 0, g);
-    if (blockIdx.x == 0) { P.dbg[8 * 64 + 2] = g; P.dbg[8 * 64 + 3] = clock64(); }
-  }
   uint8_t* base = reinterpret_cast<uint8_t*>((reinterpret_cast<uintptr_t>(smem_raw) + 1023) & ~uintptr_t(1023));
   const int warp = threadIdx.x / 32, lane = threadIdx.x % 32;
   const int stage_bytes = (P.ga + P.gb) * kTnBox;          // A boxes then B boxes
@@ -688,8 +657,6 @@ gemm_tn_tc_kernel(const __grid_constant__ GemmTnMaps maps, const GemmTnParams P)
   __syncthreads();
   tc_fence_after();
   const uint32_t tmem_base = *tmem_slot;
-  const bool dbg_on = P.dbg != nullptr && blockIdx.x == 0;
-  int dbg_n = 0;
 
   const CUtensorMap* map_a = &maps.a[prob];
   const CUtensorMap* map_b = &maps.b[prob];
@@ -705,7 +672,6 @@ gemm_tn_tc_kernel(const __grid_constant__ GemmTnMaps maps, const GemmTnParams P)
       uint32_t phase = 0;
       for (int kb = 0; kb < n_kb; ++kb) {
         mbar_wait(empty + stage, phase ^ 1);
-        KGC_DBG(0);
         uint8_t* dst = s_raw + stage * stage_bytes;
         const int row = (int)(m0 + (int64_t)kb * kTnRows);
         if (P.kmajor) {
@@ -749,9 +715,7 @@ gemm_tn_tc_kernel(const __grid_constant__ GemmTnMaps maps, const GemmTnParams P)
     }
     for (int kb = 0; kb < n_kb; ++kb) {
       mbar_wait(raw_full + stage, phase);
-      if (t == 0) KGC_DBG(1);
       mbar_wait(lo_empty + ls, lphase ^ 1);
-      if (t == 0) KGC_DBG(2);
       uint4* hi = reinterpret_cast<uint4*>(s_raw + stage * stage_bytes);
       uint4* lo = reinterpret_cast<uint4*>(s_lo + ls * stage_bytes);
       // rows of this K block that lie past the CTA's slab must not contribute: a 16-byte vector v of a box belongs to
@@ -810,7 +774,6 @@ gemm_tn_tc_kernel(const __grid_constant__ GemmTnMaps maps, const GemmTnParams P)
       fence_proxy_async();
       __syncwarp();
       if (lane == 0) mbar_arrive(split_full + stage);
-      if (t == 0) KGC_DBG(3);
       if (++stage == kTnStages) { stage = 0; phase ^= 1; }
       if (++ls == kTnLoStages) { ls = 0; lphase ^= 1; }
     }
@@ -822,7 +785,6 @@ gemm_tn_tc_kernel(const __grid_constant__ GemmTnMaps maps, const GemmTnParams P)
     uint32_t phase = 0;
     for (int kb = 0; kb < n_kb; ++kb) {
       mbar_wait(split_full + stage, phase);
-      if (lane == 0) KGC_DBG(4);
       tc_fence_after();
       const uint32_t hi_a = smem_u32(s_raw + stage * stage_bytes), hi_b = hi_a + P.ga * kTnBox;
       const uint32_t lo_a = smem_u32(s_lo + ls * stage_bytes), lo_b = lo_a + P.ga * kTnBox;
@@ -852,7 +814,6 @@ gemm_tn_tc_kernel(const __grid_constant__ GemmTnMaps maps, const GemmTnParams P)
         if (kb == n_kb - 1) umma_commit(acc_full);
       }
       __syncwarp();
-      if (lane == 0) KGC_DBG(5);
       if (++stage == kTnStages) { stage = 0; phase ^= 1; }
       if (++ls == kTnLoStages) ls = 0;
     }
@@ -865,7 +826,6 @@ gemm_tn_tc_kernel(const __grid_constant__ GemmTnMaps maps, const GemmTnParams P)
     float* out = P.partial + (((int64_t)prob * P.n_slabs + slab) * P.Ka + i) * P.Nb;
     if (n_kb > 0) {
       mbar_wait(acc_full, 0);                                        // every MMA has retired: shared memory is free
-      if (warp == 10 && lane == 0) KGC_DBG(6);
       tc_fence_after();
       const uint32_t taddr = tmem_base + ((uint32_t)(quarter * 32) << 16);
       uint8_t* stg = s_raw + (warp - 10) * (2 * kEpiBuf);
@@ -891,19 +851,12 @@ gemm_tn_tc_kernel(const __grid_constant__ GemmTnMaps maps, const GemmTnParams P)
         buf ^= 1;
       }
       if (lane == 0) bulk_wait_group<0>();
-      if (warp == 10 && lane == 0) KGC_DBG(7);
     } else if (i < P.Ka) {
       for (int j = 0; j < P.Nb; ++j) out[j] = 0.f;
     }
   }
   tc_fence_before();
   __syncthreads();
-  if (P.dbg != nullptr && threadIdx.x == 0) {
-    long long g;
-    asm volatile("mov.u64 %0, %globaltimer;" : "=l"(g));
-    atomicMax(reinterpret_cast<long long*>(P.dbg) + 8 * 64 + 1, g);
-    if (blockIdx.x == 0) { P.dbg[8 * 64 + 4] = g; P.dbg[8 * 64 + 5] = clock64(); }
-  }
   if (warp == 14) tmem_dealloc(tmem_base, kTmemColsG);
 }
 
@@ -949,8 +902,6 @@ int make_map_f32_mn(CUtensorMap* map, const void* ptr, int64_t rows, int64_t col
 }  // namespace kgc
 
 using namespace kgc;
-
-static long long* g_gemm_dbg = nullptr;
 
 extern "C" int kgc_conv_prep(const float* rels, int32_t n_rels, const float* loop_rel, const float* loop_edge, const float* w_in,
                              const float* w_out, const float* w_loop, const float* w_rel, int32_t D, int32_t Dout, float* relp,
@@ -1010,8 +961,6 @@ extern "C" int kgc_gemm_pack_b(const float* B, int64_t stride_k, int64_t stride_
   return 0;
 }
 
-extern "C" void kgc_gemm_set_debug(long long* buf) { g_gemm_dbg = buf; }   // device buffer of 9 * 64 int64, or NULL
-
 // C_i[M, N] = f(A_i[M, K] @ Bt_i^T + row_bias) (trans_c = 0) or Ct_i[N, M] = the same, stored transposed (trans_c = 1),
 // i < n_prob problems of identical shape in ONE launch: the CTAs are dealt to (problem, column tile) groups, so a batch
 // fills the 148 SMs with whole row-tile rounds where a single N x 100 x 200 product leaves a 14% tail
@@ -1049,7 +998,7 @@ static int launch_gemm_nt(int n_prob, const float* const* A, int64_t M, int32_t 
   P.M = M; P.N = N; P.K = K; P.n_prob = n_prob;
   P.n_kb = t.n_kb; P.ksteps = t.ksteps; P.NT = t.NT; P.n_ntiles = t.n_ntiles;
   P.n_mtiles = (int32_t)ceil_div(M, kBM);
-  P.C = C[0]; P.ldc = ldc; P.row_bias = row_bias; P.act = act; P.trans_c = trans_c; P.trans_a = trans_a; P.dbg = g_gemm_dbg;
+  P.C = C[0]; P.ldc = ldc; P.row_bias = row_bias; P.act = act; P.trans_c = trans_c; P.trans_a = trans_a;
   KGC_REQUIRE(keep == nullptr || (!trans_a && keep_pitch % 16 == 0 && keep_pitch >= 8 * kMaxKB && (reinterpret_cast<uintptr_t>(keep) & 15) == 0),
               "keep flags: one byte per 4 columns, 16-byte aligned rows of at least 64 bytes");
   P.keep = keep; P.keep_pitch = keep_pitch; P.keep_scale = keep_scale;
@@ -1165,7 +1114,6 @@ static int launch_gemm_tn_tc(int n_prob, const float* const* A, int64_t lda, con
     outs.n_parts[i] = (int)ceil_div(m, P.rows_per_cta);
   }
   P.partial = static_cast<float*>(workspace);
-  P.dbg = g_gemm_dbg;
   KGC_REQUIRE(keep == nullptr || (!kmajor && keep_pitch >= 8 * P.gb), "keep flags: one byte per 4 columns of B, rows that cover the padded width");
   P.keep = keep; P.keep_pitch = keep_pitch; P.keep_scale = keep_scale;
   P.ga_full = kmajor ? 0 : Ka / 32;

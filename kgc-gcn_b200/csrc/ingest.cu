@@ -14,7 +14,6 @@
 #include <string.h>
 
 #include <algorithm>
-#include <chrono>
 #include <string>
 #include <vector>
 
@@ -217,19 +216,7 @@ int for_each_line(const std::string& text, std::string* err, Fn fn) {
   return 0;
 }
 
-struct PhaseTimer {               // KGC_INGEST_TIMING=1: wall time per phase on stderr
-  bool on = getenv("KGC_INGEST_TIMING") != nullptr;
-  std::chrono::steady_clock::time_point t = std::chrono::steady_clock::now();
-  void lap(const char* what) {
-    if (!on) return;
-    const auto now = std::chrono::steady_clock::now();
-    fprintf(stderr, "[kgc_ingest] %-28s %8.1f ms\n", what, std::chrono::duration<double, std::milli>(now - t).count());
-    t = now;
-  }
-};
-
 int ingest(const std::string& dir, kgc_ingest* h) {
-  PhaseTimer timer;
   static const char* kNames[3] = {"train.txt", "valid.txt", "test.txt"};
   std::string text[3];
   for (int s = 0; s < 3; ++s)
@@ -237,7 +224,6 @@ int ingest(const std::string& dir, kgc_ingest* h) {
       h->error = "cannot read " + dir + "/" + kNames[s];
       return 3;
     }
-  timer.lap("read files");
   // ---- pass 1: ids in first-appearance order over the lower-cased tokens, and with them the triples.  The reference looks
   // the tokens up a second time AS WRITTEN (data_loader.py:83-85) in the lower-cased vocabulary: a token without an ASCII
   // upper-case letter is its own lower-cased form (found, same id), any other token cannot be in the vocabulary (KeyError) -
@@ -275,7 +261,6 @@ int ingest(const std::string& dir, kgc_ingest* h) {
     while (done < seen) resolve(&win[3 * (done++ % kWindow)]);
     tri.shrink_to_fit();
   }
-  timer.lap("pass 1 (vocabulary, ids)");
   const int64_t R = (int64_t)h->rel_names.size();
   for (const auto& name : h->rel_names)
     if (name.size() >= 8 && name.compare(name.size() - 8, 8, "_reverse") == 0) {
@@ -320,7 +305,6 @@ int ingest(const std::string& dir, kgc_ingest* h) {
       n_train_pairs = pair_g.size();
     }
   }
-  timer.lap("pass 2 (ids, groups)");
   const size_t n_groups = gid.n;
   std::vector<uint64_t> group_key(n_groups);
   for (const KeyTable::Slot& sl : gid.slots)
@@ -355,14 +339,12 @@ int ingest(const std::string& dir, kgc_ingest* h) {
       c.triples[3 * g + 2] = -1;
     }
   }
-  timer.lap("train query set");
   // ---- valid / test queries: the objects of ALL splits; a group is sorted the first time a query needs it and shared
   // by every later query (a hub group is referenced by thousands of queries)
   std::vector<int64_t> all_ptr, all_len;
   std::vector<int32_t> all_val;
   bucket(pair_g.size(), n_groups, &all_ptr, &all_val);
   all_len.assign(n_groups, -1);
-  timer.lap("all-split buckets");
   auto all_objs = [&](int64_t a, int64_t r, const int32_t** b) -> int64_t {
     const int32_t g = gid.find(((uint64_t)a << 32) | (uint64_t)r);
     int32_t* lo = all_val.data() + all_ptr[g];
@@ -395,7 +377,6 @@ int ingest(const std::string& dir, kgc_ingest* h) {
       }
     }
   }
-  timer.lap("valid / test query sets");
   return 0;
 }
 

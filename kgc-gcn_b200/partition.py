@@ -17,8 +17,6 @@ Two ways of choosing the owners:
     n_hub rows of a block are the virtual rows), so the range machinery (K1 with dst_offset, all-gather, reduce-scatter)
     is used unchanged.
 """
-import os
-
 import numpy as np
 import torch
 
@@ -431,9 +429,8 @@ class GraphPartition(object):
         elif balance == 'hybrid':
             # an edge lives with its lower-degree endpoint (partition_edges_hybrid): remote rows are few; they are read as
             # sources AND written as destinations (partial aggregates the owners add up), one compact numbering for both.
-            # On a CUDA device the partition itself is computed there (same integers; KGC_PARTITION_HOST=1: numpy)
-            on_dev = self.device.type == 'cuda' and os.environ.get('KGC_PARTITION_HOST', '0') in ('', '0')
-            if on_dev:
+            # On a CUDA device the partition itself is computed there (the same integers as the numpy version)
+            if self.device.type == 'cuda':
                 ei_d = (edge_index if torch.is_tensor(edge_index) else torch.from_numpy(np.asarray(edge_index))).to(self.device)
                 et_d = (edge_type if torch.is_tensor(edge_type) else torch.from_numpy(np.asarray(edge_type))).to(self.device)
                 info = partition_edges_hybrid_device(ei_d, et_d, num_nodes, world, rank)

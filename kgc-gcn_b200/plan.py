@@ -4,8 +4,6 @@ deterministic segmented reductions of K2/K3.
 The plan is built once per graph (the reference re-derives degrees, norms and gather/scatter
 indices on every step: model.py:96-101) and cached on the identity of the edge tensors.
 """
-import os
-
 import numpy as np
 import torch
 
@@ -236,10 +234,9 @@ class GraphPlan(object):
         self.perm_dst, self.perm_src, self.perm_type = (torch.empty((n2,), **i32) for _ in range(3))
         self.rowptr_dst, self.rowptr_src = torch.empty((Nd + 1,), **i32), torch.empty((N + 1,), **i32)
         # the d_rel pass blocked by subject row (kgc_csr_build): node tables far beyond L2 only.  65,536 rows = 26 MB of x
-        # + 26 MB of g per block at D = 100; KGC_TYPE_BLOCK_ROWS overrides (0 = plain type sort)
+        # + 26 MB of g per block at D = 100; type_block_rows overrides (0 = plain type sort)
         if type_block_rows is None:
-            env = os.environ.get('KGC_TYPE_BLOCK_ROWS', '')
-            type_block_rows = int(env) if env else (TYPE_BLOCK_ROWS if N >= 4 * TYPE_BLOCK_ROWS else 0)
+            type_block_rows = TYPE_BLOCK_ROWS if N >= 4 * TYPE_BLOCK_ROWS else 0
         self.type_block_rows = int(type_block_rows)
         Tr = int(_lib.lib().kgc_csr_type_rows(N, T, self.type_block_rows))
         self.num_type_rows, self.num_type_blocks = Tr, Tr // T
@@ -260,33 +257,20 @@ class GraphPlan(object):
                   p(self.perm_type), p(self.rowptr_type), p(self.rec_type), self.type_block_rows, p(ws), ws_bytes, _lib.stream())
         del ws
         # ---- reduction plans: the per-record / per-chunk tables are built on the device from the row pointers
-        # (KGC_PLAN_HOST=1: the numpy restatement, kept as the tested reference of the same tables)
-        if os.environ.get('KGC_PLAN_HOST', '0') not in ('', '0'):
-            rp_dst = self.rowptr_dst.cpu().numpy().astype(np.int64)
-            rm_dst = self.rowmid_dst.cpu().numpy().astype(np.int64)
-            rp_src = self.rowptr_src.cpu().numpy().astype(np.int64)
-            rp_typ = self.rowptr_type.cpu().numpy().astype(np.int64)
-            # forward: records of dst row i = [rowptr[i], rowmid[i]) (in half, output row i) then [rowmid[i], rowptr[i+1])
-            # (out half, output row Nd + i): 2 * Nd segments in record order
-            fb = np.stack([rp_dst[:-1], rm_dst], 1).reshape(-1)
-            fe = np.stack([rm_dst, rp_dst[1:]], 1).reshape(-1)
-            drows = np.arange(Nd, dtype=np.int64)
-            fr = np.stack([drows, drows + Nd], 1).reshape(-1)
-            sp_f = build_stream_plan(fb, fe, fr, n2)
-            sp_s = build_stream_plan(rp_src[:-1], rp_src[1:], np.arange(N, dtype=np.int64), n2)
-            sp_r = build_stream_plan(rp_typ[:-1], rp_typ[1:], np.arange(Tr, dtype=np.int64), n2)
-        else:
-            rp, rm = self.rowptr_dst, self.rowmid_dst
-            drows = torch.arange(Nd, dtype=torch.int32, device=dev)
-            fb = torch.stack([rp[:-1], rm], 1).reshape(-1).contiguous()
-            fe = torch.stack([rm, rp[1:]], 1).reshape(-1).contiguous()
-            fr = torch.stack([drows, drows + Nd], 1).reshape(-1).contiguous()
-            sp_f = build_stream_plan_device(fb, fe, fr, n2)
-            del fb, fe, fr
-            sp_s = build_stream_plan_device(self.rowptr_src[:-1].contiguous(), self.rowptr_src[1:].contiguous(),
-                                            torch.arange(N, dtype=torch.int32, device=dev), n2)
-            sp_r = build_stream_plan_device(self.rowptr_type[:-1].contiguous(), self.rowptr_type[1:].contiguous(),
-                                            torch.arange(Tr, dtype=torch.int32, device=dev), n2)
+        # (build_stream_plan is the numpy restatement of the same tables, the tested reference)
+        # forward: records of dst row i = [rowptr[i], rowmid[i]) (in half, output row i) then [rowmid[i], rowptr[i+1])
+        # (out half, output row Nd + i): 2 * Nd segments in record order
+        rp, rm = self.rowptr_dst, self.rowmid_dst
+        drows = torch.arange(Nd, dtype=torch.int32, device=dev)
+        fb = torch.stack([rp[:-1], rm], 1).reshape(-1).contiguous()
+        fe = torch.stack([rm, rp[1:]], 1).reshape(-1).contiguous()
+        fr = torch.stack([drows, drows + Nd], 1).reshape(-1).contiguous()
+        sp_f = build_stream_plan_device(fb, fe, fr, n2)
+        del fb, fe, fr
+        sp_s = build_stream_plan_device(self.rowptr_src[:-1].contiguous(), self.rowptr_src[1:].contiguous(),
+                                        torch.arange(N, dtype=torch.int32, device=dev), n2)
+        sp_r = build_stream_plan_device(self.rowptr_type[:-1].contiguous(), self.rowptr_type[1:].contiguous(),
+                                        torch.arange(Tr, dtype=torch.int32, device=dev), n2)
         self.fwd = StreamPlan(sp_f, n2, dev, prefill_ranges=[(0, Nd), (Nd, 2 * Nd)])     # per plane; no addend in the forward
         self.bwd_src = StreamPlan(sp_s, n2, dev)
         self.bwd_rel = StreamPlan(sp_r, n2, dev)

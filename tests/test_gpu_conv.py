@@ -223,12 +223,12 @@ def test_hybrid_partition_on_device(k):
                 assert np.array_equal(np.asarray(a[key]), np.asarray(got)), (world, rank, key)
 
 
-def test_stream_plan_on_device(k, monkeypatch):
+def test_stream_plan_on_device(k):
     """kgc_stream_plan_flags + the device-side slot numbering (plan.build_stream_plan_device) against the numpy
     restatement (plan.build_stream_plan): rowflags, chunk carry slots, carry count, empty rows and fix-up levels bit for
-    bit - random segment sets with empty segments, rows spanning many chunks, a partial last chunk; then whole GraphPlans
-    built both ways."""
-    from kgc_gcn_b200.plan import build_stream_plan, build_stream_plan_device
+    bit - random segment sets with empty segments, rows spanning many chunks, a partial last chunk; then the three
+    schedules of a whole GraphPlan against the numpy schedules of its row pointers."""
+    from kgc_gcn_b200.plan import StreamPlan, build_stream_plan, build_stream_plan_device
     rng = np.random.default_rng(21)
     for trial in range(6):
         n_seg = int(rng.integers(1, 400))
@@ -257,12 +257,21 @@ def test_stream_plan_on_device(k, monkeypatch):
     tri = orc.synthetic_triples(N, R, E, 5)
     g = orc.build_graph(tri, N, R)
     ei, et = torch.from_numpy(g['edge_index']).cuda(), torch.from_numpy(g['edge_attr'][0]).cuda()
-    plans = {}
-    for host in ('1', '0'):
-        monkeypatch.setenv('KGC_PLAN_HOST', host)
-        plans[host] = k.GraphPlan(ei, et, N, 2 * R + 1, type_block_rows=512)
+    plan = k.GraphPlan(ei, et, N, 2 * R + 1, type_block_rows=512)
+    rp_dst, rm_dst, rp_src, rp_typ = (t.cpu().numpy().astype(np.int64)
+                                      for t in (plan.rowptr_dst, plan.rowmid_dst, plan.rowptr_src, plan.rowptr_type))
+    Nd, n2, dev = plan.num_dst_rows, plan.num_edges2, plan.device
+    # forward: records [rowptr[i], rowmid[i]) reduce into row i (in half), [rowmid[i], rowptr[i+1]) into row Nd + i (out half)
+    drows = np.arange(Nd, dtype=np.int64)
+    fb = np.stack([rp_dst[:-1], rm_dst], 1).reshape(-1)
+    fe = np.stack([rm_dst, rp_dst[1:]], 1).reshape(-1)
+    fr = np.stack([drows, drows + Nd], 1).reshape(-1)
+    host = {'fwd': StreamPlan(build_stream_plan(fb, fe, fr, n2), n2, dev, prefill_ranges=[(0, Nd), (Nd, 2 * Nd)]),
+            'bwd_src': StreamPlan(build_stream_plan(rp_src[:-1], rp_src[1:], np.arange(N, dtype=np.int64), n2), n2, dev),
+            'bwd_rel': StreamPlan(build_stream_plan(rp_typ[:-1], rp_typ[1:], np.arange(plan.num_type_rows, dtype=np.int64),
+                                                    n2), n2, dev)}
     for name in ('fwd', 'bwd_src', 'bwd_rel'):
-        a, b = getattr(plans['1'], name), getattr(plans['0'], name)
+        a, b = host[name], getattr(plan, name)
         assert torch.equal(a.rowflags, b.rowflags) and torch.equal(a.chunks, b.chunks) and a.n_carry == b.n_carry
         assert len(a.levels) == len(b.levels) and a.prefill == b.prefill
         for la, lb in zip(a.levels, b.levels):
@@ -296,15 +305,17 @@ def test_type_sort_blocked_by_subject(k, monkeypatch):
         np.testing.assert_array_equal(perm_t.cpu().numpy(), orc.stable_csr(key, N)[0])
     z, _ = synth_case(2000, 5, 12000, 100, 200, 43)
     res = {}
-    for br in ('0', '128'):
-        monkeypatch.setenv('KGC_TYPE_BLOCK_ROWS', br)
+    # N = 2,000 rows: the default block of 65,536 rows leaves the type sort plain (N < 4 blocks), 128 rows block it
+    for br in (k.plan.TYPE_BLOCK_ROWS, 128):
+        monkeypatch.setattr(k.plan, 'TYPE_BLOCK_ROWS', br)
         k.plan._PLAN_CACHE.clear()
         _, ent, rel, grads = run_case(k, z)
         res[br] = (ent, rel, grads)
     k.plan._PLAN_CACHE.clear()
-    assert torch.equal(res['0'][0], res['128'][0]) and torch.equal(res['0'][1], res['128'][1])
-    for name in res['0'][2]:
-        a, b = res['0'][2][name], res['128'][2][name]
+    plain, blocked = res.values()
+    assert torch.equal(plain[0], blocked[0]) and torch.equal(plain[1], blocked[1])
+    for name in plain[2]:
+        a, b = plain[2][name], blocked[2][name]
         if torch.equal(a, b):
             continue
         assert name in ('rels', 'w.loop_rel'), name

@@ -271,8 +271,8 @@ def test_product_never_imports_oracle():
             assert 'mgcn_oracle' not in src and 'oracle' not in re.findall(r'^\s*(?:from|import)\s+(\w+)', src, re.M), fn
 
 
-def test_c_abi_v3_exports_every_declared_symbol():
-    """libkgc_b200.so loads, reports ABI version 3 and exports every function include/kgc_b200.h declares (no compute calls
+def test_c_abi_v4_exports_every_declared_symbol():
+    """libkgc_b200.so loads, reports ABI version 4 and exports every function include/kgc_b200.h declares (no compute calls
     here)."""
     import kgc_gcn_b200 as k
     hdr = open(os.path.join(ROOT, 'include', 'kgc_b200.h')).read()
@@ -283,7 +283,7 @@ def test_c_abi_v3_exports_every_declared_symbol():
     for name in sorted(declared):
         assert hasattr(h, name), 'missing export ' + name
     assert declared == set(k._lib.SIGNATURES), declared ^ set(k._lib.SIGNATURES)
-    assert k._lib.lib().kgc_abi_version() == 3
+    assert k._lib.lib().kgc_abi_version() == 4
 
 
 def test_cpu_tensors_fail_loudly():
