@@ -29,6 +29,8 @@ from .plan import get_plan
 # K4c (+1.9 / +1.0 ms against -2.5 ms of tail traffic) - but FB15k-237 0.462 vs 0.411 ms: when the planes stay in L2 the
 # extra writes are what costs.  So the three planes are written when together they exceed this size.
 TAIL_MASKED_MAX_BYTES = 48 << 20
+# ... and whenever the layer is wider than the masked K4c launch (gemm_tn_batch with keep flags) takes: d_in <= 128, d_out <= 224.
+GEMM_TN_TC_MAX_KA, GEMM_TN_TC_MAX_NB = 128, 224
 
 
 def get_param(shape):
@@ -128,7 +130,7 @@ def gemm_tn_batch(a_list, b_list, out_list, plan=None, keep=None, keep_scale=1.0
         fits = fits and all(a.shape[0] == M and b.shape[0] == M for a, b in zip(a_list, b_list))
     elif not fits or max(rows) != M or any(a.shape[0] < r or b.shape[0] < r for a, b, r in zip(a_list, b_list, rows)):
         raise ValueError('gemm_tn_batch with rows needs operands of identical widths and strides and rows <= their heights')
-    if not fits or Ka > 128 or Nb > 224:                # one gemm_tn per problem
+    if not fits or Ka > GEMM_TN_TC_MAX_KA or Nb > GEMM_TN_TC_MAX_NB:    # one gemm_tn per problem
         if keep is not None:
             raise ValueError('gemm_tn_batch: the masked form needs Ka <= 128, Nb <= 224 and operands of identical shape')
         for i, (a, b, o) in enumerate(zip(a_list, b_list, out_list)):
@@ -533,9 +535,9 @@ class _ConvFn(torch.autograd.Function):
             _lib.call('kgc_colsum_finalize', p(partials), nb, Dout, p(sums), st())
             coll.all_reduce(sums, 'bn_b')
             sums32 = sums.float()
-        # the in / out halves' upstream planes: three planes or one masked plane by size (TAIL_MASKED_MAX_BYTES).  A
-        # compacted half always takes the three-plane form: its upstream rows are written compact, [n_c, Dout].
-        three = 3 * Nl * Dout * 4 > TAIL_MASKED_MAX_BYTES or any(comp)
+        # the in / out halves' upstream planes: three planes or one masked plane by size and width (TAIL_MASKED_MAX_BYTES,
+        # GEMM_TN_TC_MAX_*).  A compacted half always takes the three-plane form: its upstream rows are written compact, [n_c, Dout].
+        three = 3 * Nl * Dout * 4 > TAIL_MASKED_MAX_BYTES or D > GEMM_TN_TC_MAX_KA or Dout > GEMM_TN_TC_MAX_NB or any(comp)
         d_res = [(plan.scratch('d_res_c%d' % h, (max(plan.n_c[h], 1), Dout)) if comp[h] else plan.scratch('d_res2_%d' % h, (Nl, Dout)))
                  if three else None for h in (0, 1)]
         _lib.call('kgc_tail_bwd_apply', p(g_ent), p(pre), p(stats), p(gamma), p(beta), p(sums), int(ctx.training), Nl,

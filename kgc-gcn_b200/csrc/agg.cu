@@ -7,34 +7,22 @@
 //   res      = agg @ W                                                   (dense GEMM, host side)
 //
 // Streaming design: the sorted edge records are cut into CHUNKS of 32 consecutive records, one warp per chunk whatever
-// the row boundaries (every warp has the same amount of work, no per-row launch overhead); lane l owns float4 column l
-// of a row, so a 400-byte row is one fully coalesced 25-lane request; a row that lies inside one chunk is written
-// straight to the output; the (at most two) rows a chunk shares with its neighbours go to CARRY rows, which
-// kgc_rows_reduce adds in a fixed order.  No float atomics anywhere: results are bit-reproducible run to run.
+// the row boundaries (every warp has the same amount of work, no per-row launch overhead); lane l owns float4 columns
+// l and l + 32 of a row (the second only for D > 128), so a 400-byte row is one fully coalesced 25-lane request; a row
+// that lies inside one chunk is written straight to the output; the (at most two) rows a chunk shares with its
+// neighbours go to CARRY rows, which kgc_rows_reduce adds in a fixed order.  No float atomics anywhere: results are
+// bit-reproducible run to run.
 //
-// Two kernels implement it.  agg_lean_kernel (D <= 128, the product path at the reference's D = 100) and
-// agg_stream_kernel (the earlier version, kept for 128 < D <= 256: two float4 columns per lane).
-//
-// History of the measurements that shaped agg_lean_kernel (profiles/r01_agg_variants.md has every number):
-//   * agg_stream_kernel reached 0.53 / 0.53 / 0.47 of the measured HBM peak (fwd / bwd_src / bwd_rel, WN18RR shape) and
-//     looked latency-bound: every unit below 45% busy, same time for sequential and for random row order
-//     (tests/gather_probe.py), no gain from more loads in flight.  Rejected on the way: per-row bulk async copies
-//     (UBLKCP, 0.2-0.3 - the copy engine retires ~one 400-byte request per 30 cycles per SM), a per-warp cp.async ring
-//     (0.29 / 0.37 / 0.23), double-buffered register batches (no change), L2 prefetch of the next chunk (worse), records
-//     broadcast from shared memory (spills), one-warp CTAs, dynamic chunk claiming (same).
-//   * ncu source-level sampling then showed WHY: 75 warp instructions per edge, only 28% of the stall samples on the first
-//     use of a loaded row, the other 72% spread evenly over ~700 SASS instructions (fixed-latency waits, shuffles, branch
-//     bookkeeping, per-edge bounds checks, 64-bit address arithmetic) at 3.5 warps per scheduler.  The kernel was bound by
-//     the serial instruction latency of each warp, not by memory.
-//   * a continuous register ring (edge e + P issued as soon as edge e is consumed) cut the instruction count to 47 per
-//     edge but ran SLOWER (45 / 88 / 63 us): a warp has six scoreboard slots, the load being waited for shares its slot
-//     with loads issued after it, and the ring degenerates (long-scoreboard stall 3 -> 12 cycles per issue).  Batches -
-//     all loads of kU edges, then all their arithmetic - are the structure the scoreboards reward.
-//   * agg_lean_kernel: 42 instructions per edge, batches of 3-4 edges at 3 CTAs per SM (80 registers, no spills):
-//     35.8 / 64.6 / 39.9 us -> 26.6 / 47.1 / 28.8 us = 0.70 / 0.73 / 0.65 of the measured peak, bit-identical outputs.
-//     Relation rows staged in shared memory and grids balanced to equal chunks per warp changed nothing measurable.
-//     ncu of the kept kernel: DRAM 47%, L1TEX 62%, 19 resident warps per SM, long-scoreboard 9 cycles per issue - it is
-//     now memory-latency-bound; the torch copy of the same bytes, timed the same way, reaches 0.77-0.79.
+// Why agg_kernel looks as it does (profiles/r01_agg_variants.md has the measurements and the rejected variants):
+//   * the kernel is bound by the latency of each warp's serial instruction stream and of its row loads, not by DRAM
+//     bandwidth.  So it keeps instructions per edge low: the 32 edges of a full chunk are fully unrolled (shuffle lanes
+//     and batch slots are compile-time, no per-edge bounds checks) and addresses are 32-bit float4 indices (one IMAD +
+//     one IMAD.WIDE per load; the launcher checks that every table fits).
+//   * loads go in BATCHES: all row loads of KU edges, then all their arithmetic.  A warp has six scoreboard slots; a
+//     continuous ring of loads (edge e + P issued as soon as edge e is consumed) shares them between the load being waited
+//     for and the loads behind it and ran slower than batches despite fewer instructions.
+//   * batches are as large as fit the register budget of 3 CTAs per SM (one column per lane) or 2 (two columns) without
+//     spills: more resident warps hide more load latency than longer batches.
 
 #include "common.cuh"
 
@@ -84,159 +72,12 @@ struct StreamArgs {
   int64_t max_rows;           // known bound on the row indices of g3 / outputs (guard of the 32-bit float4 indices)
 };
 
-// agg_stream_kernel (128 < D <= 256).  One warp walks one chunk of kChunk (= 32) sorted records.  Lane l first loads record cb + l (one coalesced
-// 512-byte + 128-byte request for the whole chunk); every edge's record is then broadcast with warp shuffles,
-// so all gather addresses of the chunk are known after a single memory round trip.  kU edges are in flight per
-// trip: phase 1 issues their DRAM / L2 row loads (edge embedding + the gathered operand), phase 2 consumes them
-// in record order with the L1-resident operands (relation row, and the source row in the backward pass).
-template <int MODE> struct Unroll { static constexpr int value = 8; };
-template <> struct Unroll<kBwdRel> { static constexpr int value = 4; };      // three DRAM/L2 operands per edge
-template <> struct Unroll<kBwdSrc> { static constexpr int value = 6; };      // ee, g[dst] and x[src] per edge
-
-template <int MODE, int NF>
-__global__ void __launch_bounds__(kThreads, 2)
-agg_stream_kernel(const StreamArgs A) {
-  constexpr int kU = Unroll<MODE>::value;
-  static_assert(kChunk == 32, "one record per lane");
-  // PERSISTENT warps: the grid fills the GPU once (2 CTAs per SM) and every warp walks chunks w, w + W, w + 2W, ...
-  // (W = warps of the grid), fetching the records of its next chunk while it processes the current one.  One warp per
-  // chunk with a one-shot grid paid a record round trip per chunk with nothing else in flight (fwd 37.4 -> 34.9 us).
-  // Claiming chunks dynamically from an atomic work counter instead of the static stride measured the same (35.2 us).
-  const int lane = threadIdx.x % 32;
-  const int64_t n_chunks = (A.n_rec + kChunk - 1) / kChunk;
-  const int64_t stride = (int64_t)gridDim.x * kWarpsPerBlock;
-  int64_t chunk = blockIdx.x * (int64_t)kWarpsPerBlock + threadIdx.x / 32;
-  if (chunk >= n_chunks) return;
-  const int D4 = A.D4;
-  bool active[NF];
-#pragma unroll
-  for (int f = 0; f < NF; ++f) active[f] = lane + f * 32 < D4;
-  auto rec_index = [&](int64_t ch) {
-    const int64_t b = ch * kChunk;
-    const int n = (int)(b + kChunk < A.n_rec ? kChunk : A.n_rec - b);
-    return b + (lane < n ? lane : n - 1);
-  };
-  int2 slots_n = __ldg(reinterpret_cast<const int2*>(A.chunks + chunk));
-  int4 myrec_n = ld_rec(A.rec + rec_index(chunk));
-  uint32_t myflag_n = __ldg(A.rowflags + rec_index(chunk));
- while (chunk < n_chunks) {
-  const int64_t next = chunk + stride;
-  const int64_t cb = chunk * kChunk;
-  const int cnt = (int)(cb + kChunk < A.n_rec ? kChunk : A.n_rec - cb);
-  const int2 slots = slots_n;
-  const int4 myrec = myrec_n;
-  const uint32_t myflag = myflag_n;
-  if (next < n_chunks) {                                         // records of the next chunk: in flight during this one
-    slots_n = __ldg(reinterpret_cast<const int2*>(A.chunks + next));
-    myrec_n = ld_rec(A.rec + rec_index(next));
-    myflag_n = __ldg(A.rowflags + rec_index(next));
-  }
-
-  float4 acc[NF];
-#pragma unroll
-  for (int f = 0; f < NF; ++f) acc[f] = make_float4(0.f, 0.f, 0.f, 0.f);
-  bool started_here = (__shfl_sync(0xffffffffu, myflag, 0) & kFirst) != 0;
-  bool open_row = false;
-
-  for (int base = 0; base < cnt; base += kU) {
-    float4 va[kU][NF], vb[kU][NF], vc[kU][MODE == kFwd ? 1 : NF];
-    // ---- phase 1: the long-latency row loads of kU edges
-#pragma unroll
-    for (int u = 0; u < kU; ++u) {
-      const int e = base + u < cnt ? base + u : cnt - 1;          // clamped: a duplicate load, never consumed
-      const uint32_t eid = (uint32_t)__shfl_sync(0xffffffffu, myrec.x, e);
-      const uint32_t ra = (uint32_t)__shfl_sync(0xffffffffu, myrec.y, e);
-      const uint32_t rb = (uint32_t)__shfl_sync(0xffffffffu, myrec.z, e);
-      const uint32_t erow = __shfl_sync(0xffffffffu, myflag, e) & kRowMask;
-#pragma unroll
-      for (int f = 0; f < NF; ++f) {
-        const int c = lane + f * 32;
-        if (active[f]) {
-          va[u][f] = ld_stream(A.ee + (uint64_t)eid * D4 + c);
-          if (MODE == kFwd) {
-            vb[u][f] = __ldg(A.x + (uint64_t)ra * D4 + c);
-          } else if (MODE == kBwdSrc) {
-            vb[u][f] = __ldg(A.g3 + ((int)eid >= A.n_edges_in ? A.plane : 0) + (uint64_t)ra * D4 + c);
-            vc[u][f] = __ldg(A.x + (uint64_t)erow * D4 + c);                 // x[src]: one miss per row, then L1
-          } else {
-            vb[u][f] = __ldg(A.g3 + ((int)eid >= A.n_edges_in ? A.plane : 0) + (uint64_t)rb * D4 + c);
-            vc[u][f] = __ldg(A.x + (uint64_t)ra * D4 + c);
-          }
-        }
-      }
-    }
-    // ---- phase 2: consume in record order
-#pragma unroll
-    for (int u = 0; u < kU; ++u) {
-      if (base + u < cnt) {                                      // warp-uniform
-        const int e = base + u;
-        const uint32_t flags = __shfl_sync(0xffffffffu, myflag, e);
-        const float nrm = __int_as_float(__shfl_sync(0xffffffffu, myrec.w, e));
-        const int64_t row = flags & kRowMask;
-        // shuffles stay outside the lane predicate: every lane of the warp must take part
-        const uint32_t rb = (uint32_t)__shfl_sync(0xffffffffu, myrec.z, e);
-        const uint32_t eid = (uint32_t)__shfl_sync(0xffffffffu, myrec.x, e);
-        (void)rb; (void)eid;
-        if (flags & kFirst) {
-#pragma unroll
-          for (int f = 0; f < NF; ++f) acc[f] = make_float4(0.f, 0.f, 0.f, 0.f);
-          started_here = true;
-        }
-        open_row = true;
-#pragma unroll
-        for (int f = 0; f < NF; ++f) {
-          const int c = lane + f * 32;
-          if (active[f]) {
-            if (MODE == kFwd) {
-              add4(acc[f], mul3s(nrm, vb[u][f], __ldg(A.rel + (uint64_t)rb * D4 + c), va[u][f]));
-            } else if (MODE == kBwdSrc) {
-              const float4 pe = scale4(nrm, mul4(vb[u][f], __ldg(A.rel + (uint64_t)rb * D4 + c)));   // norm * g[dst] * rel
-              st_stream(A.d_ee + (uint64_t)eid * D4 + c, mul4(pe, vc[u][f]));                           // * x[src]
-              add4(acc[f], mul4(pe, va[u][f]));
-            } else {
-              add4(acc[f], mul3s(nrm, vb[u][f], vc[u][f], va[u][f]));                                   // norm * g * x * ee
-            }
-          }
-        }
-        if (flags & kLast) {                                     // the row ends here
-          float4* out = started_here ? A.out_final + row * D4 : A.carry + (int64_t)slots.x * D4;
-#pragma unroll
-          for (int f = 0; f < NF; ++f) {
-            const int c = lane + f * 32;
-            if (active[f]) {
-              float4 v = acc[f];
-              if (MODE == kBwdSrc && started_here && A.addend != nullptr) add4(v, __ldg(A.addend + row * D4 + c));
-              out[c] = v;
-            }
-          }
-          open_row = false;
-        }
-      }
-    }
-  }
-  if (open_row) {                                                // the row continues in the next chunk
-    float4* out = A.carry + (int64_t)slots.y * D4;
-#pragma unroll
-    for (int f = 0; f < NF; ++f) {
-      const int c = lane + f * 32;
-      if (active[f]) out[c] = acc[f];
-    }
-  }
-  chunk = next;
- }   // persistent chunk loop
-}
-
-// ---------------------------------------------------------------------------------------------- lean variant
-// Same chunks / carry protocol / arithmetic as agg_stream_kernel.  ncu of that kernel (profiles/r01_ncu_agg_lean.md):
-// 75 warp instructions per edge, 72% of the stall samples spread evenly over them (fixed-latency waits, shuffles,
-// branch bookkeeping) and only 28% on the first use of a loaded row - instruction-latency-bound at 14 warps per SM.
-// This version (i) fully unrolls the 32 edges of a FULL chunk (shuffle lanes and batch slots are compile-time, no
-// per-edge bounds checks; the stream's single partial chunk takes a plain loop), (ii) issues ALL row loads of a batch,
-// the relation row included, in the load phase, so the consume phase is pure arithmetic, (iii) forms addresses from
-// 32-bit float4 indices (one IMAD + one IMAD.WIDE per load), (iv) runs at 3-4 CTAs per SM with small batches.
-template <int MODE, int KU, int MINB>
+// One warp walks one chunk of kChunk (= 32) sorted records.  Lane l first loads record cb + l (one coalesced request for
+// the whole chunk); every edge's record is then broadcast with warp shuffles, so all gather addresses of the chunk are
+// known after a single memory round trip.  NC = float4 columns per lane (1: D <= 128, 2: D <= 256).
+template <int MODE, int KU, int MINB, int NC>
 __global__ void __launch_bounds__(kThreads, MINB)
-agg_lean_kernel(const StreamArgs A) {
+agg_kernel(const StreamArgs A) {
   // Full unroll in every mode.  The d_x / d_ee pass has ~110 instructions per edge: unrolling all 32 makes a 56 KB loop
   // body and ncu shows 6.5 stall cycles per issued instruction waiting for the instruction cache ("no instruction"; 0.4
   // in the two smaller kernels).  Bodies of 32 / 16 / 8 edges (1, 2 or 4 trips per chunk) measured 11.69 / 11.63 /
@@ -246,14 +87,16 @@ agg_lean_kernel(const StreamArgs A) {
   constexpr bool kHasC = MODE != kFwd;        // third gathered operand
   constexpr bool kHasR = MODE != kBwdRel;     // relation row
   const int lane = threadIdx.x % 32;
+  // PERSISTENT warps: the grid fills the GPU once and every warp walks chunks w, w + W, w + 2W, ... (W = warps of the
+  // grid), fetching the records of its next chunk while it processes the current one
   const int warp = __shfl_sync(0xffffffffu, (int)threadIdx.x / 32, 0);          // warp-uniform for the compiler
   const int64_t n_chunks = (A.n_rec + kChunk - 1) / kChunk;
   const int64_t stride = (int64_t)gridDim.x * kWarpsPerBlock;
   int64_t chunk = blockIdx.x * (int64_t)kWarpsPerBlock + warp;
   if (chunk >= n_chunks) return;
   const uint32_t D4 = (uint32_t)A.D4;
-  const bool act = lane < (int)D4;
-  const uint32_t c = act ? lane : 0;
+  auto active = [&](int f) { return lane + 32 * f < (int)D4; };                  // column f of this lane exists
+  auto col = [&](int f) -> uint32_t { return active(f) ? lane + 32 * f : 0; };
   const float4* __restrict__ ee = A.ee;
   const float4* __restrict__ xs = A.x;
   const float4* __restrict__ rel = A.rel;
@@ -269,39 +112,49 @@ agg_lean_kernel(const StreamArgs A) {
   int4 rec_n = ld_rec(A.rec + rec_index(chunk));
   uint32_t flag_n = __ldg(A.rowflags + rec_index(chunk));
 
-  float4 va[KU], vb[KU], vc[kHasC ? KU : 1], vr[kHasR ? KU : 1];
+  float4 va[KU][NC], vb[KU][NC], vc[kHasC ? KU : 1][NC], vr[kHasR ? KU : 1][NC];
   int4 rec;
   uint32_t flag;
-  float4 acc;
+  float4 acc[NC];
   bool started_here;
   int2 slots;
   float4* const out_final = A.out_final;
   float4* const carry = A.carry;
   float4* const d_ee = A.d_ee;
   const float4* const addend = A.addend;
+  // the relation row and every gathered row of edge e into batch slot u
   auto issue = [&](int u, int e) {
     const uint32_t eid = (uint32_t)__shfl_sync(0xffffffffu, rec.x, e);
     const uint32_t ra = (uint32_t)__shfl_sync(0xffffffffu, rec.y, e);
     const uint32_t rb = (uint32_t)__shfl_sync(0xffffffffu, rec.z, e);
     if (MODE == kFwd) {
-      if (act) {
-        va[u] = ld_stream(ee + (eid * D4 + c));
-        vb[u] = __ldg(xs + (ra * D4 + c));
-        vr[kHasR ? u : 0] = __ldg(rel + (rb * D4 + c));
+#pragma unroll
+      for (int f = 0; f < NC; ++f) {
+        if (active(f)) {
+          va[u][f] = ld_stream(ee + (eid * D4 + col(f)));
+          vb[u][f] = __ldg(xs + (ra * D4 + col(f)));
+          vr[kHasR ? u : 0][f] = __ldg(rel + (rb * D4 + col(f)));
+        }
       }
     } else if (MODE == kBwdSrc) {
       const uint32_t erow = __shfl_sync(0xffffffffu, flag, e) & kRowMask;
-      if (act) {
-        va[u] = ld_stream(ee + (eid * D4 + c));
-        vb[u] = __ldg(g3 + ((eid >= n_in ? plane : 0u) + ra * D4 + c));
-        vc[kHasC ? u : 0] = __ldg(xs + (erow * D4 + c));
-        vr[kHasR ? u : 0] = __ldg(rel + (rb * D4 + c));
+#pragma unroll
+      for (int f = 0; f < NC; ++f) {
+        if (active(f)) {
+          va[u][f] = ld_stream(ee + (eid * D4 + col(f)));
+          vb[u][f] = __ldg(g3 + ((eid >= n_in ? plane : 0u) + ra * D4 + col(f)));
+          vc[kHasC ? u : 0][f] = __ldg(xs + (erow * D4 + col(f)));
+          vr[kHasR ? u : 0][f] = __ldg(rel + (rb * D4 + col(f)));
+        }
       }
     } else {
-      if (act) {
-        va[u] = ld_stream(ee + (eid * D4 + c));
-        vb[u] = __ldg(g3 + ((eid >= n_in ? plane : 0u) + rb * D4 + c));
-        vc[kHasC ? u : 0] = __ldg(xs + (ra * D4 + c));
+#pragma unroll
+      for (int f = 0; f < NC; ++f) {
+        if (active(f)) {
+          va[u][f] = ld_stream(ee + (eid * D4 + col(f)));
+          vb[u][f] = __ldg(g3 + ((eid >= n_in ? plane : 0u) + rb * D4 + col(f)));
+          vc[kHasC ? u : 0][f] = __ldg(xs + (ra * D4 + col(f)));
+        }
       }
     }
   };
@@ -309,26 +162,33 @@ agg_lean_kernel(const StreamArgs A) {
   // here and no per-edge "first" test is needed)
   auto consume = [&](int u, int e, bool last) {
     const float nrm = __int_as_float(__shfl_sync(0xffffffffu, rec.w, e));
-    const float4 rv = vr[kHasR ? u : 0];
     if (MODE == kFwd) {
-      add4(acc, mul3s(nrm, vb[u], rv, va[u]));
+#pragma unroll
+      for (int f = 0; f < NC; ++f) add4(acc[f], mul3s(nrm, vb[u][f], vr[kHasR ? u : 0][f], va[u][f]));
     } else if (MODE == kBwdSrc) {
       const uint32_t eid = (uint32_t)__shfl_sync(0xffffffffu, rec.x, e);
-      const float4 pe = scale4(nrm, mul4(vb[u], rv));
-      if (act) st_stream(d_ee + (eid * D4 + c), mul4(pe, vc[kHasC ? u : 0]));
-      add4(acc, mul4(pe, va[u]));
+#pragma unroll
+      for (int f = 0; f < NC; ++f) {
+        const float4 pe = scale4(nrm, mul4(vb[u][f], vr[kHasR ? u : 0][f]));
+        if (active(f)) st_stream(d_ee + (eid * D4 + col(f)), mul4(pe, vc[kHasC ? u : 0][f]));
+        add4(acc[f], mul4(pe, va[u][f]));
+      }
     } else {
-      add4(acc, mul3s(nrm, vb[u], vc[kHasC ? u : 0], va[u]));
+#pragma unroll
+      for (int f = 0; f < NC; ++f) add4(acc[f], mul3s(nrm, vb[u][f], vc[kHasC ? u : 0][f], va[u][f]));
     }
     if (last) {
       const uint32_t row = __shfl_sync(0xffffffffu, flag, e) & kRowMask;
-      float4* out = started_here ? out_final + (row * D4 + c) : carry + ((uint32_t)slots.x * D4 + c);
-      if (act) {
-        float4 v = acc;
-        if (MODE == kBwdSrc && started_here && addend != nullptr) add4(v, __ldg(addend + (row * D4 + c)));
-        *out = v;
+#pragma unroll
+      for (int f = 0; f < NC; ++f) {
+        float4* out = started_here ? out_final + (row * D4 + col(f)) : carry + ((uint32_t)slots.x * D4 + col(f));
+        if (active(f)) {
+          float4 v = acc[f];
+          if (MODE == kBwdSrc && started_here && addend != nullptr) add4(v, __ldg(addend + (row * D4 + col(f))));
+          *out = v;
+        }
+        acc[f] = make_float4(0.f, 0.f, 0.f, 0.f);
       }
-      acc = make_float4(0.f, 0.f, 0.f, 0.f);
       started_here = true;
     }
   };
@@ -345,7 +205,8 @@ agg_lean_kernel(const StreamArgs A) {
       rec_n = ld_rec(A.rec + rec_index(next));
       flag_n = __ldg(A.rowflags + rec_index(next));
     }
-    acc = make_float4(0.f, 0.f, 0.f, 0.f);
+#pragma unroll
+    for (int f = 0; f < NC; ++f) acc[f] = make_float4(0.f, 0.f, 0.f, 0.f);
     const uint32_t valid = cnt == kChunk ? 0xffffffffu : ((1u << cnt) - 1u);
     const uint32_t last_mask = __ballot_sync(0xffffffffu, (flag & kLast) != 0) & valid;
     started_here = (__shfl_sync(0xffffffffu, flag, 0) & kFirst) != 0;
@@ -366,7 +227,9 @@ agg_lean_kernel(const StreamArgs A) {
       }
     }
     if (!((last_mask >> (cnt - 1)) & 1u)) {                      // the row continues in the next chunk
-      if (act) carry[(uint32_t)slots.y * D4 + c] = acc;
+#pragma unroll
+      for (int f = 0; f < NC; ++f)
+        if (active(f)) carry[(uint32_t)slots.y * D4 + col(f)] = acc[f];
     }
     chunk = next;
   }
@@ -504,28 +367,30 @@ inline int check_dim(int32_t D, int* D4, int* NF) {
     default: { constexpr int NF = 8; __VA_ARGS__; } break; \
   }
 
-// Lean kernel configuration (edges per batch, CTAs per SM), measured on B200 at the WN18RR / FB15k-237 shapes
-// (history in profiles/r01_agg_variants.md): fwd 4 x 3, bwd_src 3 x 3, bwd_rel 4 x 3 - the largest
-// batches that fit 80 registers without spills; 2 CTAs x 8 edges and 4 CTAs x 2-3 edges were 10-20% slower.
-template <int MODE> struct LeanCfg { static constexpr int ku = 4, minb = 3; };
-template <> struct LeanCfg<kBwdSrc> { static constexpr int ku = 3, minb = 3; };
+// agg_kernel configuration: edges per batch (kAggKU[NC - 1][MODE]) and CTAs per SM, the largest batches that compile
+// without spills.  One column per lane (measured on B200 at the WN18RR / FB15k-237 shapes, profiles/r01_agg_variants.md):
+// fwd 4, bwd_src 3, bwd_rel 4 edges at 3 CTAs (80 registers); 2 CTAs x 8 edges and 4 CTAs x 2-3 edges were 10-20% slower.
+// Two columns per lane: fwd 4, bwd_src 2, bwd_rel 3 edges at 2 CTAs (128 registers; profiles/r12_one_agg_kernel_ptxas_sass.md).
+constexpr int kAggKU[2][3] = {{4, 3, 4}, {4, 2, 3}};
+
+template <int MODE, int NC>
+void launch_agg(const StreamArgs& A, int64_t blocks, cudaStream_t st) {
+  constexpr int minb = NC == 1 ? 3 : 2;
+  if (blocks > (int64_t)minb * kNumSMs) blocks = (int64_t)minb * kNumSMs;   // persistent grid
+  agg_kernel<MODE, kAggKU[NC - 1][MODE], minb, NC><<<(unsigned)blocks, kThreads, 0, st>>>(A);
+}
 
 template <int MODE>
 int launch_stream(const StreamArgs& A, cudaStream_t st) {
   if (A.n_rec == 0) return 0;
-  const int64_t n_chunks = ceil_div(A.n_rec, kChunk);
-  int64_t blocks = ceil_div(n_chunks, kWarpsPerBlock);
-  if (A.D4 <= 32) {                                               // D <= 128: one float4 column per lane
-    // 32-bit float4 indices: edge ids are < n_rec, node / output rows < max_rows (the host checks the node table)
-    KGC_REQUIRE((uint64_t)A.n_rec * A.D4 < (1ull << 32) && (uint64_t)A.max_rows * A.D4 < (1ull << 32),
-                "tables of 2^32 float4 or more are not supported (32-bit float4 indices)");
-    constexpr int minb = LeanCfg<MODE>::minb;
-    if (blocks > (int64_t)minb * kNumSMs) blocks = (int64_t)minb * kNumSMs;   // persistent grid
-    agg_lean_kernel<MODE, LeanCfg<MODE>::ku, minb><<<(unsigned)blocks, kThreads, 0, st>>>(A);
-  } else {
-    if (blocks > 2 * kNumSMs) blocks = 2 * kNumSMs;               // persistent: 2 resident CTAs per SM (__launch_bounds__)
-    agg_stream_kernel<MODE, 2><<<(unsigned)blocks, kThreads, 0, st>>>(A);
-  }
+  // 32-bit float4 indices: edge ids are < n_rec, node / output rows < max_rows (the host checks the node table)
+  KGC_REQUIRE((uint64_t)A.n_rec * A.D4 < (1ull << 32) && (uint64_t)A.max_rows * A.D4 < (1ull << 32),
+              "tables of 2^32 float4 or more are not supported (32-bit float4 indices)");
+  const int64_t blocks = ceil_div(ceil_div(A.n_rec, kChunk), kWarpsPerBlock);
+  if (A.D4 <= 32)                                                 // D <= 128: one float4 column per lane
+    launch_agg<MODE, 1>(A, blocks, st);
+  else
+    launch_agg<MODE, 2>(A, blocks, st);
   KGC_LAUNCH_CHECK();
   return 0;
 }

@@ -8,7 +8,7 @@
 // (unit upstream gradient) and, while the candidate row is still in registers, d_x[b] += g * E[cand] in slot order.  A
 // warp owns one query: the x row lives in registers, a candidate row is one coalesced request of 4 D bytes (800 at
 // D = 200), and the rows of a batch of kRowsInFlight slots are all loaded before the first is consumed (the lesson of
-// agg_lean_kernel, DESIGN section 4).
+// agg_kernel, DESIGN section 4).
 //
 // Table backward: d_E[n] = sum over the slots s with cand[s] = n of g[s] * (scale x[b(s)]) and d_bias[n] = scale sum g[s],
 // dense [N, D] / [N] with zeros elsewhere (the encoder's backward takes a dense upstream).  Duplicate candidates are the

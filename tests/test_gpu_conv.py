@@ -110,10 +110,12 @@ def synth_case(N, R, E, d_in, d_out, seed):
     return z, p
 
 
-@pytest.mark.parametrize('shape', [(3000, 7, 9000, 100, 200, 31), (500, 40, 4000, 36, 24, 32), (64, 2, 70000, 8, 12, 33)])
+@pytest.mark.parametrize('shape', [(3000, 7, 9000, 100, 200, 31), (500, 40, 4000, 36, 24, 32), (64, 2, 70000, 8, 12, 33),
+                                   (3000, 7, 9000, 200, 232, 34), (64, 2, 150000, 256, 24, 35)])
 def test_conv_vs_oracle_f64(k, shape):
     """Mid-size synthetic graphs with Zipf hubs (multi-level reductions: one dst row holds ~44% of the edges)
-    against the oracle evaluated in float64 on the same inputs."""
+    against the oracle evaluated in float64 on the same inputs.  d_in = 200 / 256: the aggregation's lanes own a partial /
+    full second float4 column; d_out = 232: wider than the batched weight-gradient GEMM."""
     N, R, E, d_in, d_out, seed = shape
     z, p = synth_case(N, R, E, d_in, d_out, seed)
     dt = torch.float64
@@ -495,8 +497,19 @@ def test_gemm_tn_weight_gradient(k, M, Ka, Nb):
 def test_in_kernel_dropout_matches_its_own_masks(k):
     """K4 Philox dropout: a training step with the in-kernel generator equals, bit for bit, the same step with the
     masks that generator produces injected explicitly; the keep rate is 1 - p; seeds change every step."""
-    z, _ = synth_case(1500, 4, 6000, 100, 200, 61)
-    d_in, d_out, R = 100, 200, 4
+    check_in_kernel_dropout(k, 100, 200)
+
+
+@pytest.mark.parametrize('d_in,d_out', [(200, 200), (100, 256)])
+def test_in_kernel_dropout_wide_layers(k, d_in, d_out):
+    """The same for layers wider than the masked weight-gradient GEMM takes (d_in <= 128, d_out <= 224): their backward
+    writes the three upstream planes."""
+    check_in_kernel_dropout(k, d_in, d_out)
+
+
+def check_in_kernel_dropout(k, d_in, d_out):
+    z, _ = synth_case(1500, 4, 6000, d_in, d_out, 61)
+    R = 4
     conv = make_conv(k, z, d_in, d_out, R, 0.1).train()
     torch.manual_seed(7)
     dev = 'cuda'
