@@ -139,6 +139,34 @@ int kgc_agg_bwd_rel(const float* x, const float* ee, const float* g3,
                     int64_t n_dst_rows, int64_t n_edges_in,
                     float* drel_final, float* carry, int32_t D, void* stream);
 
+/* ---- K3, factorized by (row, type) group (single GPU; kgc_gcn_b200/plan.py GroupedPlan) -------------------------------
+ * A knowledge graph's objects are hubs that see each relation type many times, so a sum over edges that carries a factor
+ * rel[type] can be regrouped: sum_e rel[t_e] (.) y_e = sum_groups rel[t] (.) (sum over the group's edges of y_e).  The
+ * grouped forward stream (kgc_agg_fwd on GroupedPlan records, whose in-half records carry the index of a row of ones)
+ * writes P[g] = sum_{e in g} norm_e x[src_e] (.) ee[e] per (dst, type) group of the in half.
+ *
+ * kgc_agg_bwd_src_grouped: the d_x / d_ee pass over the grouped src-sorted records.  rowflags hold the OUTPUT row of each
+ * record: its source row j for an in-half record (as kgc_agg_bwd_src) or n_dst_rows + g for an out-half record of group g
+ * (its (src, type) run); xrow[p] = the source row of record p.
+ *   d_ee[e]              = norm_e * g3[half_e][a_e] (.) rel[b_e] (.) x[xrow_e]      (bit-identical to kgc_agg_bwd_src)
+ *   out[j]               = sum over the in-half records of row j of that product with ee[e] in place of x (+ loop_addend[j])
+ *   out[n_dst_rows + g]  = sum_{e in g} norm_e * g3[1][a_e] (.) ee[e]              (Q: no relation factor)
+ * loop_addend must have n_dst_rows + n_groups rows whose group rows are zero (the fix-up levels add it on every final row).
+ *
+ * kgc_group_reduce: first level of a deterministic reduction over groups.  Item k (items[k] = beg, end, out, flags as for
+ * kgc_rows_reduce, end - beg <= 32) computes
+ *   s = sum over i in [beg, end), ascending, of mult[mrow[i]] (.) part[prow ? prow[i] : i]
+ * and writes it to out_final[out] (flags & 1; plus the row's previous value when accumulate != 0) or to out_part[out].
+ * Longer segments continue on kgc_rows_reduce levels (addend = out_final itself to accumulate). */
+int kgc_agg_bwd_src_grouped(const float* x, const float* rel, int64_t n_types, const float* ee, const float* g3,
+                            const kgc_edge_rec_t* rec, const uint32_t* rowflags, const uint32_t* xrow,
+                            const kgc_chunk_t* chunks, int64_t n_rec, int64_t n_dst_rows, int64_t n_edges_in,
+                            int64_t n_groups, const float* loop_addend, float* d_ee, float* out_final, float* carry,
+                            int32_t D, void* stream);
+int kgc_group_reduce(const float* part, const int32_t* prow, const float* mult, const int32_t* mrow,
+                     const kgc_item_t* items, int64_t n_items, float* out_final, float* out_part, int32_t accumulate,
+                     int32_t D, void* stream);
+
 /* ---- K4: layer tail ------------------------------------------------------------------------------
  * Replaces model.py:103-106: out = (drop(in_res) + drop(out_res) + loop_res) / 3 [+ bias];
  * BatchNorm1d over the node rows; tanh.  res3 is [3,n_rows,Dout] (in, out, loop planes).

@@ -30,6 +30,9 @@ SIGNATURES = {
     'kgc_rows_reduce': (ctypes.c_int, [_vp, _vp, _i64, _i64, _vp, _vp, _vp, _i32, _vp]),
     'kgc_agg_bwd_src': (ctypes.c_int, [_vp, _vp, _i64, _vp, _vp, _vp, _vp, _vp, _i64, _i64, _i64, _vp, _vp, _vp, _vp, _i32, _vp]),
     'kgc_agg_bwd_rel': (ctypes.c_int, [_vp, _vp, _vp, _vp, _vp, _vp, _i64, _i64, _i64, _vp, _vp, _i32, _vp]),
+    'kgc_agg_bwd_src_grouped': (ctypes.c_int, [_vp, _vp, _i64, _vp, _vp, _vp, _vp, _vp, _vp, _i64, _i64, _i64, _i64, _vp, _vp, _vp,
+                                               _vp, _i32, _vp]),
+    'kgc_group_reduce': (ctypes.c_int, [_vp, _vp, _vp, _vp, _vp, _i64, _vp, _vp, _i32, _i32, _vp]),
     'kgc_tail_num_blocks': (_i64, [_i64]),
     'kgc_dropout_mask': (ctypes.c_int, [_vp, _i32, _f32, _i64, _vp, _vp]),
     'kgc_keep_pitch': (_i32, []),

@@ -423,18 +423,37 @@ class _ConvFn(torch.autograd.Function):
             gather.wait()
         if max(x_full.shape[0], 3 * n_dst, ee.shape[0]) * (D // 4) >= 1 << 32:      # K2/K3 use 32-bit float4 indices
             raise ValueError('kgc_gcn_b200: node / edge tables of 2^32 float4 elements or more are not supported')
-        agg = torch.empty((2, n_dst, D), dtype=torch.float32, device=x.device)
         agg_c, res_c = [None, None], [None, None]                   # compacted halves: [n_c, D] rows and their transforms
         # one GPU: a half whose rows are mostly without edges (plan.compact_halves) runs its dense transform, its share of the
         # tail and its weight gradient on its occupied rows only (plan.rows / plan.slot); its other rows are never read, so
         # the aggregation does not zero-fill them
         comp = plan.compact_halves(4 * Dout) if coll is None else (False, False)
+        # one GPU, hub-heavy graph (plan.grouped, GroupedPlan): the in half is aggregated per (object, type) group into the
+        # rows P behind the two planes, without the relation factor (its records name a row of ones), and agg_in = sum_t
+        # rel[t] (.) P[o, t] follows; the backward reuses P for d_rel
+        grp = plan.grouped if coll is None else None
+        agg_all = torch.empty((2 * n_dst + (grp.n_in if grp is not None else 0), D), dtype=torch.float32, device=x.device)
+        agg = agg_all[:2 * n_dst].view(2, n_dst, D)
+        if grp is None:
+            def level0(sp, out_final, carry):
+                _lib.call('kgc_agg_fwd', p(x_full), p(rels_c), T - 1, p(ee), p(plan.rec_dst), p(sp.rowflags), p(sp.chunks),
+                          sp.n_rec, p(out_final), p(carry), D, st())
+            plan.run_reduction(plan.fwd, level0, agg, D, tag='f',
+                               skip_prefill=[(h * n_dst, (h + 1) * n_dst) for h in (0, 1) if comp[h]])
+        else:
+            rel_f = torch.cat([rels_c, rels_c.new_ones((1, D))], 0)      # row T - 1 = grp.ones_row
 
-        def level0(sp, out_final, carry):
-            _lib.call('kgc_agg_fwd', p(x_full), p(rels_c), T - 1, p(ee), p(plan.rec_dst), p(sp.rowflags), p(sp.chunks), sp.n_rec,
-                      p(out_final), p(carry), D, st())
-        plan.run_reduction(plan.fwd, level0, agg, D, tag='f',
-                           skip_prefill=[(h * n_dst, (h + 1) * n_dst) for h in (0, 1) if comp[h]])
+            def level0(sp, out_final, carry):
+                _lib.call('kgc_agg_fwd', p(x_full), p(rel_f), T, p(ee), p(grp.rec_f), p(sp.rowflags), p(sp.chunks), sp.n_rec,
+                          p(out_final), p(carry), D, st())
+            plan.run_reduction(grp.fwd, level0, agg_all, D, tag='fg', skip_prefill=[(n_dst, 2 * n_dst)] if comp[1] else ())
+            P = agg_all[2 * n_dst:]
+            if comp[0]:                                             # agg_in straight into the compacted rows
+                agg_c[0] = torch.empty((max(plan.n_c[0], 1), D), dtype=torch.float32, device=x.device)
+                grp.agg_in_c.run(plan, P, rels_c, agg_c[0], D, tag='gi')
+            else:
+                agg[0].zero_()
+                grp.agg_in.run(plan, P, rels_c, agg[0], D, tag='gi')
         if gather is None:
             main.wait_stream(side)                                  # K0's operand packs are needed from here on
 
@@ -452,10 +471,12 @@ class _ConvFn(torch.autograd.Function):
             for h in (0, 1):
                 if comp[h]:
                     n_c = plan.n_c[h]
-                    agg_c[h] = torch.empty((max(n_c, 1), D), dtype=torch.float32, device=x.device)
                     res_c[h] = plan.scratch('res_c%d' % h, (max(n_c, 1), Dout))
+                    if agg_c[h] is None:
+                        agg_c[h] = torch.empty((max(n_c, 1), D), dtype=torch.float32, device=x.device)
+                        if n_c:
+                            rows_copy(agg[h], plan.rows[h], agg_c[h], None, n_c)
                     if n_c:
-                        rows_copy(agg[h], plan.rows[h], agg_c[h], None, n_c)
                         gemm_nt(agg_c[h][:n_c], None, res_c[h][:n_c], packed=packed_f[h])
             gemm_nt_batch([agg[h] for h in dense] + [x], [packed_f[h] for h in dense] + [packed_f[2]],
                           [res3[h] for h in dense] + [res3[2]])
@@ -497,17 +518,18 @@ class _ConvFn(torch.autograd.Function):
         ctx.plan, ctx.training, ctx.keep_scale, ctx.has_bias, ctx.coll = plan, bool(training), float(keep_scale), \
             bias is not None, coll
         ctx.drop_p = float(drop_p)
-        ctx.comp = comp
-        ctx.save_for_backward(x, x_full, relp, ee, w_in, w_out, w_loop, w_rel, loop_rel, loop_edge, gamma, beta, agg, pre,
+        ctx.comp, ctx.grp = comp, grp
+        ctx.save_for_backward(x, x_full, relp, ee, w_in, w_out, w_loop, w_rel, loop_rel, loop_edge, gamma, beta, agg_all, pre,
                               all_ent, stats, keep, packed_b, out_keep, agg_c[0], agg_c[1])
         ctx.mark_non_differentiable(stats)
         return all_ent, all_rel, stats
 
     @staticmethod
     def backward(ctx, g_ent, g_rel, _g_stats):
-        (x, x_full, relp, ee, w_in, w_out, w_loop, w_rel, loop_rel, loop_edge, gamma, beta, agg, pre, all_ent, stats, keep,
+        (x, x_full, relp, ee, w_in, w_out, w_loop, w_rel, loop_rel, loop_edge, gamma, beta, agg_all, pre, all_ent, stats, keep,
          packed_b, out_keep, agg_c0, agg_c1) = ctx.saved_tensors
-        plan, coll, comp = ctx.plan, ctx.coll, ctx.comp
+        plan, coll, comp, grp = ctx.plan, ctx.coll, ctx.comp, ctx.grp
+        agg = agg_all[:2 * plan.num_dst_rows].view(2, plan.num_dst_rows, -1)
         Nl, D = x.shape
         n_global = Nl if coll is None else coll.n_global      # BatchNorm rows (real nodes of all ranks)
         n_hub = 0 if coll is None else coll.n_hub
@@ -566,7 +588,13 @@ class _ConvFn(torch.autograd.Function):
 
         # ---- d(agg) = d_res @ W^T on the tensor cores (3xTF32), main stream
         hybrid = coll is not None and coll.p2p is not None and coll.p2p.hybrid
-        g3 = coll.p2p.g3_planes() if hybrid else plan.scratch('g3', (3, Nb, D))
+        if grp is None:
+            g3 = coll.p2p.g3_planes() if hybrid else plan.scratch('g3', (3, Nb, D))
+        else:
+            # the grouped d_x pass takes the self-loop plane as addend on its node rows and the zero rows behind it on its
+            # group rows (never written after allocation)
+            g3_all = plan.scratch('g3grp', (3 * Nb + grp.n_out, D), zeros=True)
+            g3 = g3_all[:3 * Nb].view(3, Nb, D)
         if not any(comp):
             gemm_nt_batch(ups, [packed_b[0], packed_b[1], packed_b[2]],
                           [g3[0, :Nl], g3[1, :Nl], g3[2, :Nl]], keep=gkeep, keep_scale=ctx.keep_scale)
@@ -588,17 +616,35 @@ class _ConvFn(torch.autograd.Function):
             coll.p2p.gather_g()                                      # K10: upstream rows of the remote destinations, from their owners
         # ---- K3: d_x (+ self-loop term) and d_ee over src-sorted rows, d_rel over type-sorted rows
         p2p = None if coll is None else coll.p2p
-        d_x_full = p2p.partial if (p2p is not None and not hybrid) else torch.empty((plan.num_nodes, D), dtype=torch.float32, device=dev)
         d_ee = torch.empty_like(ee)
-        # self-loop term: added by the aggregation itself when its output rows are final (one GPU; hybrid cut: the remote rows
-        # of plane 2 are zero), otherwise by the owner-side reduction
-        loop_addend = g3[2] if (coll is None or hybrid) else None
+        if grp is not None:
+            # d_x / d_ee over the grouped src stream: d_x of the in-half records and the out-half group rows Q behind it; then
+            # d_x += rel (.) Q and d_rel from the group rows - no second pass over the edge table
+            dxq = torch.empty((plan.num_nodes + grp.n_out, D), dtype=torch.float32, device=dev)
+            d_x_full, Q = dxq[:plan.num_nodes], dxq[plan.num_nodes:]
+            addend_g = g3_all[2 * Nb:]
 
-        def level0_src(sp, out_final, carry):
-            _lib.call('kgc_agg_bwd_src', p(x_full), p(relp), relp.shape[0], p(ee), p(g3), p(plan.rec_src), p(sp.rowflags), p(sp.chunks),
-                      sp.n_rec, plan.num_dst_rows, plan.num_edges_in, p(loop_addend), p(d_ee), p(out_final), p(carry),
-                      D, st())
-        plan.run_reduction(plan.bwd_src, level0_src, d_x_full, D, addend=loop_addend, tag='s')
+            def level0_src(sp, out_final, carry):
+                _lib.call('kgc_agg_bwd_src_grouped', p(x_full), p(relp), T, p(ee), p(g3), p(grp.rec_s), p(sp.rowflags),
+                          p(grp.xrow_s), p(sp.chunks), sp.n_rec, plan.num_dst_rows, plan.num_edges_in, grp.n_out, p(addend_g),
+                          p(d_ee), p(out_final), p(carry), D, st())
+            plan.run_reduction(grp.src, level0_src, dxq, D, addend=addend_g, tag='sg')
+            grp.dx.run(plan, Q, relp, d_x_full, D, accumulate=True, tag='gx')
+            P = agg_all[2 * plan.num_dst_rows:]
+            grp.drel_in.run(plan, P, g3[0], d_relp, D, tag='gri')
+            grp.drel_out.run(plan, Q, x_full, d_relp, D, accumulate=True, tag='gro')
+        else:
+            d_x_full = p2p.partial if (p2p is not None and not hybrid) else torch.empty((plan.num_nodes, D), dtype=torch.float32,
+                                                                                        device=dev)
+            # self-loop term: added by the aggregation itself when its output rows are final (one GPU; hybrid cut: the remote
+            # rows of plane 2 are zero), otherwise by the owner-side reduction
+            loop_addend = g3[2] if (coll is None or hybrid) else None
+
+            def level0_src(sp, out_final, carry):
+                _lib.call('kgc_agg_bwd_src', p(x_full), p(relp), relp.shape[0], p(ee), p(g3), p(plan.rec_src), p(sp.rowflags),
+                          p(sp.chunks), sp.n_rec, plan.num_dst_rows, plan.num_edges_in, p(loop_addend), p(d_ee), p(out_final),
+                          p(carry), D, st())
+            plan.run_reduction(plan.bwd_src, level0_src, d_x_full, D, addend=loop_addend, tag='s')
         scatter = None
         if hybrid:
             # K10 on the exchange stream: partial rows of the remote sources to symmetric memory, barrier (own channel), the
@@ -621,10 +667,11 @@ class _ConvFn(torch.autograd.Function):
         if coll is not None and p2p is None and not compact:   # source-row gradients go back to their owners while the d_rel pass runs
             d_x, scatter = coll.reduce_scatter_rows(d_x_full, async_op=True)
 
-        def level0_rel(sp, out_final, carry):
-            _lib.call('kgc_agg_bwd_rel', p(x_full), p(ee), p(g3), p(plan.rec_type), p(sp.rowflags), p(sp.chunks), sp.n_rec,
-                      plan.num_dst_rows, plan.num_edges_in, p(out_final), p(carry), D, st())
-        plan.run_rel_reduction(level0_rel, d_relp, D)
+        if grp is None:
+            def level0_rel(sp, out_final, carry):
+                _lib.call('kgc_agg_bwd_rel', p(x_full), p(ee), p(g3), p(plan.rec_type), p(sp.rowflags), p(sp.chunks), sp.n_rec,
+                          plan.num_dst_rows, plan.num_edges_in, p(out_final), p(carry), D, st())
+            plan.run_rel_reduction(level0_rel, d_relp, D)
 
         main.wait_stream(side)                                        # the weight gradients are part of `flat`
         if coll is None:

@@ -51,7 +51,10 @@ __device__ __forceinline__ float4 scale4(float s, const float4& a) {
   return make_float4(s * a.x, s * a.y, s * a.z, s * a.w);
 }
 
-enum Mode { kFwd = 0, kBwdSrc = 1, kBwdRel = 2 };
+// kBwdSrcGrp: the d_x / d_ee pass over the GROUPED src-sorted stream (plan.GroupedPlan): a row's in-half records reduce
+// into its d_x row as in kBwdSrc, its out-half records are sorted by type and every (row, type) run reduces into a group
+// row (row >= n_dst_rows) WITHOUT the relation factor; kgc_group_reduce applies rel[type] once per group afterwards
+enum Mode { kFwd = 0, kBwdSrc = 1, kBwdRel = 2, kBwdSrcGrp = 3 };
 
 struct StreamArgs {
   const float4* x;            // node rows (global ids)
@@ -70,6 +73,7 @@ struct StreamArgs {
   int32_t n_edges_in;         // records with eid >= n_edges_in belong to the out half (bwd)
   int32_t D4;
   int64_t max_rows;           // known bound on the row indices of g3 / outputs (guard of the 32-bit float4 indices)
+  const uint32_t* xrow;       // bwd_src_grp: per sorted record its source row (the x row of d_ee; rowflags hold the output row)
 };
 
 // One warp walks one chunk of kChunk (= 32) sorted records.  Lane l first loads record cb + l (one coalesced request for
@@ -86,6 +90,8 @@ agg_kernel(const StreamArgs A) {
   static_assert(kChunk == 32, "one record per lane");
   constexpr bool kHasC = MODE != kFwd;        // third gathered operand
   constexpr bool kHasR = MODE != kBwdRel;     // relation row
+  constexpr bool kGrp = MODE == kBwdSrcGrp;
+  constexpr bool kSrc = MODE == kBwdSrc || kGrp;
   const int lane = threadIdx.x % 32;
   // PERSISTENT warps: the grid fills the GPU once and every warp walks chunks w, w + W, w + 2W, ... (W = warps of the
   // grid), fetching the records of its next chunk while it processes the current one
@@ -111,10 +117,11 @@ agg_kernel(const StreamArgs A) {
   int2 slots_n = __ldg(reinterpret_cast<const int2*>(A.chunks + chunk));
   int4 rec_n = ld_rec(A.rec + rec_index(chunk));
   uint32_t flag_n = __ldg(A.rowflags + rec_index(chunk));
+  uint32_t xrow_n = kGrp ? __ldg(A.xrow + rec_index(chunk)) : 0u;
 
   float4 va[KU][NC], vb[KU][NC], vc[kHasC ? KU : 1][NC], vr[kHasR ? KU : 1][NC];
   int4 rec;
-  uint32_t flag;
+  uint32_t flag, xrow = 0u;
   float4 acc[NC];
   bool started_here;
   int2 slots;
@@ -136,8 +143,8 @@ agg_kernel(const StreamArgs A) {
           vr[kHasR ? u : 0][f] = __ldg(rel + (rb * D4 + col(f)));
         }
       }
-    } else if (MODE == kBwdSrc) {
-      const uint32_t erow = __shfl_sync(0xffffffffu, flag, e) & kRowMask;
+    } else if (kSrc) {
+      const uint32_t erow = kGrp ? (uint32_t)__shfl_sync(0xffffffffu, xrow, e) : __shfl_sync(0xffffffffu, flag, e) & kRowMask;
 #pragma unroll
       for (int f = 0; f < NC; ++f) {
         if (active(f)) {
@@ -165,13 +172,16 @@ agg_kernel(const StreamArgs A) {
     if (MODE == kFwd) {
 #pragma unroll
       for (int f = 0; f < NC; ++f) add4(acc[f], mul3s(nrm, vb[u][f], vr[kHasR ? u : 0][f], va[u][f]));
-    } else if (MODE == kBwdSrc) {
+    } else if (kSrc) {
       const uint32_t eid = (uint32_t)__shfl_sync(0xffffffffu, rec.x, e);
 #pragma unroll
       for (int f = 0; f < NC; ++f) {
         const float4 pe = scale4(nrm, mul4(vb[u][f], vr[kHasR ? u : 0][f]));
         if (active(f)) st_stream(d_ee + (eid * D4 + col(f)), mul4(pe, vc[kHasC ? u : 0][f]));
-        add4(acc[f], mul4(pe, va[u][f]));
+        if (kGrp)                                                // a group record: norm * g (.) ee, rel applied per group
+          add4(acc[f], mul4(eid >= n_in ? scale4(nrm, vb[u][f]) : pe, va[u][f]));
+        else
+          add4(acc[f], mul4(pe, va[u][f]));
       }
     } else {
 #pragma unroll
@@ -185,6 +195,8 @@ agg_kernel(const StreamArgs A) {
         if (active(f)) {
           float4 v = acc[f];
           if (MODE == kBwdSrc && started_here && addend != nullptr) add4(v, __ldg(addend + (row * D4 + col(f))));
+          // the self-loop term belongs to the node rows only: group rows lie past plane = n_dst_rows * D4
+          if (kGrp && started_here && addend != nullptr && row * D4 < plane) add4(v, __ldg(addend + (row * D4 + col(f))));
           *out = v;
         }
         acc[f] = make_float4(0.f, 0.f, 0.f, 0.f);
@@ -200,10 +212,12 @@ agg_kernel(const StreamArgs A) {
     slots = slots_n;
     rec = rec_n;
     flag = flag_n;
+    xrow = xrow_n;
     if (next < n_chunks) {                                         // records of the next chunk: in flight during this one
       slots_n = __ldg(reinterpret_cast<const int2*>(A.chunks + next));
       rec_n = ld_rec(A.rec + rec_index(next));
       flag_n = __ldg(A.rowflags + rec_index(next));
+      if (kGrp) xrow_n = __ldg(A.xrow + rec_index(next));
     }
 #pragma unroll
     for (int f = 0; f < NC; ++f) acc[f] = make_float4(0.f, 0.f, 0.f, 0.f);
@@ -371,7 +385,8 @@ inline int check_dim(int32_t D, int* D4, int* NF) {
 // without spills.  One column per lane (measured on B200 at the WN18RR / FB15k-237 shapes, profiles/r01_agg_variants.md):
 // fwd 4, bwd_src 3, bwd_rel 4 edges at 3 CTAs (80 registers); 2 CTAs x 8 edges and 4 CTAs x 2-3 edges were 10-20% slower.
 // Two columns per lane: fwd 4, bwd_src 2, bwd_rel 3 edges at 2 CTAs (128 registers; profiles/r12_one_agg_kernel_ptxas_sass.md).
-constexpr int kAggKU[2][3] = {{4, 3, 4}, {4, 2, 3}};
+// bwd_src_grp: bwd_src's batches (profiles/r13_factorized_rel_ptxas_sass.md).
+constexpr int kAggKU[2][4] = {{4, 3, 4, 3}, {4, 2, 3, 2}};
 
 template <int MODE, int NC>
 void launch_agg(const StreamArgs& A, int64_t blocks, cudaStream_t st) {
@@ -393,6 +408,65 @@ int launch_stream(const StreamArgs& A, cudaStream_t st) {
     launch_agg<MODE, 2>(A, blocks, st);
   KGC_LAUNCH_CHECK();
   return 0;
+}
+
+// ------------------------------------------------------------------------------------------------ group reduce
+// First level of a group reduction (kgc_group_reduce): one warp per item of at most 32 entries, lane l owns float4 columns
+// l and l + 32 (NC = 2).  Entry i of the item adds mult[mrow[i]] (.) part[prow ? prow[i] : i]; the item's entry indices
+// are loaded once (one per lane) and broadcast by shuffles, rows are loaded kGrpKU entries at a time and added in entry
+// order.  Fixed order, no atomics.
+constexpr int kGrpKU = 4;
+
+template <int NC>
+__global__ void __launch_bounds__(kThreads)
+group_reduce_kernel(const float4* __restrict__ part, const int32_t* __restrict__ prow, const float4* __restrict__ mult,
+                    const int32_t* __restrict__ mrow, const kgc_item_t* __restrict__ items, int64_t n_items,
+                    float4* __restrict__ out_final, float4* __restrict__ out_part, int accumulate, int D4) {
+  const int64_t item = (blockIdx.x * (int64_t)blockDim.x + threadIdx.x) / 32;
+  const int lane = threadIdx.x % 32;
+  if (item >= n_items) return;
+  const int4 it = __ldg(reinterpret_cast<const int4*>(items + item));
+  const int n = it.y - it.x;                                     // <= 32 (the host builds level 0 with fan-in 32)
+  int my_p = 0, my_m = 0;
+  if (lane < n) {
+    my_p = prow != nullptr ? __ldg(prow + it.x + lane) : it.x + lane;
+    my_m = __ldg(mrow + it.x + lane);
+  }
+  float4 acc[NC];
+#pragma unroll
+  for (int f = 0; f < NC; ++f) acc[f] = make_float4(0.f, 0.f, 0.f, 0.f);
+  for (int e = 0; e < n; e += kGrpKU) {
+    float4 vp[kGrpKU][NC], vm[kGrpKU][NC];
+#pragma unroll
+    for (int u = 0; u < kGrpKU; ++u) {
+      const int64_t pr = __shfl_sync(0xffffffffu, my_p, (e + u) & 31);
+      const int64_t mr = __shfl_sync(0xffffffffu, my_m, (e + u) & 31);
+#pragma unroll
+      for (int f = 0; f < NC; ++f) {
+        const int c = lane + 32 * f;
+        if (e + u < n && c < D4) {
+          vp[u][f] = __ldg(part + pr * D4 + c);
+          vm[u][f] = __ldg(mult + mr * D4 + c);
+        }
+      }
+    }
+#pragma unroll
+    for (int u = 0; u < kGrpKU; ++u)
+#pragma unroll
+      for (int f = 0; f < NC; ++f)
+        if (e + u < n) add4(acc[f], mul4(vm[u][f], vp[u][f]));
+  }
+  const bool final_row = (it.w & 1) != 0;
+  float4* out = (final_row ? out_final : out_part) + (int64_t)it.z * D4;
+#pragma unroll
+  for (int f = 0; f < NC; ++f) {
+    const int c = lane + 32 * f;
+    if (c < D4) {
+      float4 v = acc[f];
+      if (final_row && accumulate) add4(v, out[c]);             // sum + old, the order of kgc_rows_reduce's addend
+      out[c] = v;
+    }
+  }
 }
 
 }  // namespace
@@ -482,6 +556,46 @@ extern "C" int kgc_rows_reduce(const float* part_in, const kgc_item_t* items, in
   KGC_DISPATCH_NF(nf, (rows_reduce_kernel<NF><<<grid, kRedThreads, 0, as_stream(stream)>>>(
                           (const float4*)part_in, items, n_items, n_large, (float4*)out_final, (float4*)out_part,
                           (const float4*)addend, D4)));
+  KGC_LAUNCH_CHECK();
+  return 0;
+}
+
+extern "C" int kgc_agg_bwd_src_grouped(const float* x, const float* rel, int64_t n_types, const float* ee, const float* g3,
+                                       const kgc_edge_rec_t* rec, const uint32_t* rowflags, const uint32_t* xrow,
+                                       const kgc_chunk_t* chunks, int64_t n_rec, int64_t n_dst_rows, int64_t n_edges_in,
+                                       int64_t n_groups, const float* loop_addend, float* d_ee, float* out_final, float* carry,
+                                       int32_t D, void* stream) {
+  int D4, nf;
+  KGC_REQUIRE(check_dim(D, &D4, &nf) == 0, "D must be a multiple of 4 and <= 256");
+  KGC_REQUIRE(n_groups >= 0 && (n_rec == 0 || xrow != nullptr), "bad arguments");
+  StreamArgs A = {};
+  (void)n_types;
+  A.max_rows = 3 * n_dst_rows + n_groups;
+  A.x = (const float4*)x; A.rel = (const float4*)rel; A.ee = (const float4*)ee; A.g3 = (const float4*)g3;
+  A.addend = (const float4*)loop_addend;
+  A.rec = rec; A.rowflags = rowflags; A.chunks = chunks; A.xrow = xrow;
+  A.out_final = (float4*)out_final; A.carry = (float4*)carry; A.d_ee = (float4*)d_ee;
+  A.n_rec = n_rec; A.plane = n_dst_rows * (int64_t)D4; A.n_edges_in = (int32_t)n_edges_in; A.D4 = D4;
+  return launch_stream<kBwdSrcGrp>(A, as_stream(stream));
+}
+
+extern "C" int kgc_group_reduce(const float* part, const int32_t* prow, const float* mult, const int32_t* mrow,
+                                const kgc_item_t* items, int64_t n_items, float* out_final, float* out_part,
+                                int32_t accumulate, int32_t D, void* stream) {
+  int D4, nf;
+  KGC_REQUIRE(check_dim(D, &D4, &nf) == 0, "D must be a multiple of 4 and <= 256");
+  KGC_REQUIRE(n_items >= 0, "bad arguments");
+  if (n_items == 0) return 0;
+  KGC_REQUIRE(items && out_final, "null buffer");             // mrow / mult / part are read only by non-empty items
+  const unsigned grid = (unsigned)ceil_div(n_items * 32, (int64_t)kThreads);
+  if (D4 <= 32)
+    group_reduce_kernel<1><<<grid, kThreads, 0, as_stream(stream)>>>((const float4*)part, prow, (const float4*)mult, mrow, items,
+                                                                      n_items, (float4*)out_final, (float4*)out_part,
+                                                                      accumulate, D4);
+  else
+    group_reduce_kernel<2><<<grid, kThreads, 0, as_stream(stream)>>>((const float4*)part, prow, (const float4*)mult, mrow, items,
+                                                                      n_items, (float4*)out_final, (float4*)out_part,
+                                                                      accumulate, D4);
   KGC_LAUNCH_CHECK();
   return 0;
 }

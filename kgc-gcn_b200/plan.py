@@ -61,8 +61,200 @@ COMPACT_MAX_OCCUPANCY = 0.5
 # paths at the bench shapes)
 COMPACT_MIN_PLANE_BYTES = 128 << 20
 
+# Relation gradient factorized by (object, type) group (GroupedPlan): the single-GPU layer takes the grouped streams when in
+# both halves the groups - (dst, type) pairs of the in half, (src, type) pairs of the out half - number at most this share of
+# the half's edges.  A knowledge graph's objects are hubs (Wikidata5M shape: 3.2 % of the in-half edges), so the d_rel pass,
+# a second full read of the edge-embedding table, becomes a reduction over group rows
+GROUP_MAX_SHARE = 0.25
+# ... and the graph has at least this many directed edges.  Below it the d_rel pass is served largely from L2 and the step is
+# bound by launches, which the grouped path adds (tests/factorized_rel_time.py on one B200: WN18RR shape, 173,670 edges,
+# 0.383 -> 0.416 ms; FB15k-237 shape, 544,230 edges, 0.413 -> 0.433 ms; Wikidata5M shape, 41.2 M edges, 41.1 -> 38.4 ms)
+GROUP_MIN_EDGES = 1 << 22
+GROUP_FAN_IN = 32  # entries per first-level item of kgc_group_reduce (one warp, one entry index per lane)
+
 SMALL_ITEM = 16   # fix-up items with at most this many rows are summed by one 8-lane group instead of a whole block
 CHUNK_EDGES = 32  # KGC_CHUNK_EDGES: sorted records per streaming chunk (one warp)
+
+
+def build_grouped_stream(rec_row, rec_grouped, rec_type, rowptr, n_types, plain_base, group_base):
+    """Host-side restatement (numpy) of one grouped stream of GroupedPlan.
+
+    The records of a row-sorted CSR (record p belongs to row rec_row[p]; row r holds [rowptr[r], rowptr[r+1])) are
+    re-sorted stably by (row, 0) for the records of the PLAIN half and (row, 1 + type) for those of the GROUPED half
+    (rec_grouped), so every row keeps its plain records first, in their order, followed by one run per (row, type) group.
+    Segments, in record order: one per row for its plain records (output row plain_base + row; empty when it has none) and one
+    per group (output row group_base + group id, ids in (row, type) order).  Returns dict with
+      order     [n_rec] int64   CSR position of every re-sorted record
+      seg_beg / seg_end / seg_row  int64   the segments (for build_stream_plan)
+      grp_row / grp_type           int64   row and type of every group"""
+    rec_row = np.asarray(rec_row, dtype=np.int64)
+    rowptr = np.asarray(rowptr, dtype=np.int64)
+    T1 = int(n_types) + 1
+    n_rec, n_rows = rec_row.shape[0], rowptr.shape[0] - 1
+    key = rec_row * T1 + np.where(np.asarray(rec_grouped, dtype=bool), np.asarray(rec_type, dtype=np.int64) + 1, 0)
+    order = np.argsort(key, kind='stable')
+    skey = key[order]
+    brk = np.flatnonzero(np.diff(skey)) + 1
+    beg = np.concatenate([np.zeros(min(n_rec, 1), dtype=np.int64), brk])
+    end = np.concatenate([brk, np.full(min(n_rec, 1), n_rec, dtype=np.int64)])
+    ukey = skey[beg]
+    is_grp = ukey % T1 != 0
+    row = np.where(is_grp, group_base + np.cumsum(is_grp) - 1, plain_base + ukey // T1)
+    has_plain = np.zeros(n_rows, dtype=bool)
+    has_plain[ukey[~is_grp] // T1] = True
+    miss = np.flatnonzero(~has_plain)                  # rows without plain records: an empty segment where their records begin
+    allkey = np.concatenate([ukey, miss * T1])
+    o = np.argsort(allkey, kind='stable')              # the keys are distinct
+    return {'order': order, 'seg_beg': np.concatenate([beg, rowptr[miss]])[o],
+            'seg_end': np.concatenate([end, rowptr[miss]])[o], 'seg_row': np.concatenate([row, plain_base + miss])[o],
+            'grp_row': ukey[is_grp] // T1, 'grp_type': ukey[is_grp] % T1 - 1}
+
+
+def build_grouped_stream_device(rec_row, rec_grouped, rec_type, rowptr, n_types, plain_base, group_base):
+    """build_grouped_stream with torch ops on the device (int64 CUDA tensors in, the same dict of int64 CUDA tensors out;
+    bit-identical, tests/test_gpu_factorized_rel.py)."""
+    dev = rec_row.device
+    T1 = int(n_types) + 1
+    n_rows = rowptr.numel() - 1
+    key = rec_row * T1 + torch.where(rec_grouped, rec_type + 1, torch.zeros_like(rec_type))
+    skey, order = torch.sort(key, stable=True)
+    del key
+    ukey, cnt = torch.unique_consecutive(skey, return_counts=True)
+    del skey
+    end = torch.cumsum(cnt, 0)
+    beg = end - cnt
+    is_grp = ukey % T1 != 0
+    row = torch.where(is_grp, group_base + torch.cumsum(is_grp, 0) - 1, plain_base + torch.div(ukey, T1, rounding_mode='floor'))
+    has_plain = torch.zeros((n_rows,), dtype=torch.bool, device=dev)
+    has_plain[torch.div(ukey[~is_grp], T1, rounding_mode='floor')] = True
+    miss = torch.nonzero(~has_plain).view(-1)
+    o = torch.argsort(torch.cat([ukey, miss * T1]))
+    rp = rowptr.to(torch.int64)
+    gk = ukey[is_grp]
+    return {'order': order, 'seg_beg': torch.cat([beg, rp[miss]])[o], 'seg_end': torch.cat([end, rp[miss]])[o],
+            'seg_row': torch.cat([row, plain_base + miss])[o], 'grp_row': torch.div(gk, T1, rounding_mode='floor'),
+            'grp_type': gk % T1 - 1}
+
+
+def group_segments(keys, n_out=None):
+    """Segments of a key-sorted group table: (beg, end, key) of every distinct key, or - n_out given - of every key in
+    [0, n_out) (empty segments for the keys without groups)."""
+    keys = np.asarray(keys, dtype=np.int64)
+    if n_out is None:
+        u, first = np.unique(keys, return_index=True)
+        return first, np.append(first[1:], keys.shape[0]), u
+    ptr = np.searchsorted(keys, np.arange(n_out + 1, dtype=np.int64))
+    return ptr[:-1], ptr[1:], np.arange(n_out, dtype=np.int64)
+
+
+def _fixup_levels(levels, device):
+    """Device copies of build_levels tables for kgc_rows_reduce: hub rows first (a block each), then the many small items
+    (an 8-lane group each).  [(items, n_items, n_part, n_large)]"""
+    out = []
+    for it, n_part in levels:
+        large = (it[:, 1] - it[:, 0]) > SMALL_ITEM
+        order = np.concatenate([np.nonzero(large)[0], np.nonzero(~large)[0]])
+        out.append((torch.from_numpy(np.ascontiguousarray(it[order])).to(device), int(it.shape[0]), n_part, int(large.sum())))
+    return out
+
+
+class GroupReduce(object):
+    """Schedule of one deterministic reduction over group rows (kgc_group_reduce + kgc_rows_reduce levels):
+    out[seg_row[s]] (= or +=) sum over i in [seg_beg[s], seg_end[s]), ascending, of mult[mrow[i]] (.) part[prow[i] or i]."""
+
+    def __init__(self, seg_beg, seg_end, seg_row, mrow, prow, device):
+        levels = build_levels(seg_beg, seg_end, seg_row, GROUP_FAN_IN, CHUNK1)
+        it0, self.n_part0 = levels[0]
+        assert (it0[:, 1] - it0[:, 0]).max(initial=0) <= GROUP_FAN_IN
+        self.items0, self.n_items0 = torch.from_numpy(np.ascontiguousarray(it0)).to(device), int(it0.shape[0])
+        self.levels = _fixup_levels(levels[1:], device)
+        self.mrow = torch.from_numpy(np.asarray(mrow, dtype=np.int32)).to(device)
+        self.prow = None if prow is None else torch.from_numpy(np.asarray(prow, dtype=np.int32)).to(device)
+
+    def run(self, plan, part, mult, out, D, accumulate=False, tag='g'):
+        p = _lib.ptr
+        prev = plan.scratch(tag + 'part0', (self.n_part0, D)) if self.n_part0 else None
+        _lib.call('kgc_group_reduce', p(part), p(self.prow), p(mult), p(self.mrow), p(self.items0), self.n_items0, p(out), p(prev),
+                  int(accumulate), D, _lib.stream())
+        for li, (items, n_items, n_part, n_large) in enumerate(self.levels):
+            nxt = plan.scratch('{}part{}'.format(tag, li + 1), (n_part, D)) if n_part else None
+            _lib.call('kgc_rows_reduce', p(prev), p(items), n_items, n_large, p(out), p(nxt), p(out) if accumulate else None, D,
+                      _lib.stream())
+            prev = nxt
+
+
+class GroupedPlan(object):
+    """The single-GPU layer's streams and group tables for the d_rel pass factorized by (object, type) group.
+
+    Edge e = s -> o of type t (in half; its reverse o -> s of type t + R is in the out half):
+      agg_in[o]    = sum_t rel[t] (.) P[o,t],   P[o,t] = sum_{e in (o,t)} n_e x[s_e] (.) ee[e]      (forward stream)
+      d_x[o]      += sum_t rel[t] (.) Q[o,t],   Q[o,t] = sum_{e in (o,t)} n_e g_out[s_e] (.) ee[e]  (src stream)
+      d_rel[t]     = sum_o g_in[o] (.) P[o,t]  (in types),   sum_o x[o] (.) Q[o,t]  (out types)
+    fwd: the dst-sorted records, each row's out-half records first (output row Nd + row), then its in-half records as one
+      run per (row, type) group (output row 2 Nd + group); their type field is the index of a row of ones appended to the
+      relation rows, so kgc_agg_fwd writes P.  rec_f, fwd (StreamPlan), n_in groups: grp_in_row / grp_in_type.
+    src: the src-sorted records, each row's in-half records first (output row = row), then its out-half records as one run
+      per (row, type) group (output row N + group): kgc_agg_bwd_src_grouped writes d_x without the out half, and Q.
+      rec_s, xrow_s (source row per record), src (StreamPlan), n_out groups: grp_out_row / grp_out_type.
+    Device memory: two record arrays (16 B per edge each), two rowflags arrays and xrow_s (4 B per edge each) - 44 B per
+    directed edge, 1.8 GB at the Wikidata5M shape - next to the plain streams, which bench.py and the partitioned layer keep."""
+
+    def __init__(self, plan, edge_index, n_in_groups_max, n_out_groups_max):
+        dev, Nd, N, T = plan.device, plan.num_dst_rows, plan.num_nodes, plan.num_types
+        n2, n_in = plan.num_edges2, plan.num_edges_in
+        self.ones_row = T - 1          # kgc_agg_fwd reads cat(rels, ones): row T - 1 of it is the row of ones
+        self.qualifies = False
+        # ---- forward stream: dst-sorted, in half grouped
+        eid = plan.rec_dst[:, 0].to(torch.int64)
+        g = build_grouped_stream_device(edge_index[1][eid], eid < n_in, plan.rec_dst[:, 2].to(torch.int64),
+                                        plan.rowptr_dst, T, Nd, 2 * Nd)
+        self.n_in = int(g['grp_row'].numel())
+        if self.n_in > n_in_groups_max:
+            return
+        rec = plan.rec_dst[g['order']]
+        rec[:, 2] = torch.where(rec[:, 0] < n_in, torch.full_like(rec[:, 2], self.ones_row), rec[:, 2])
+        self.rec_f = rec
+        del g['order'], rec, eid
+        i32 = lambda t: t.to(torch.int32).contiguous()
+        sp = build_stream_plan_device(i32(g['seg_beg']), i32(g['seg_end']), i32(g['seg_row']), n2)
+        self.fwd = StreamPlan(sp, n2, dev, prefill_ranges=[(Nd, 2 * Nd)])
+        grp_in_row, grp_in_type = g['grp_row'].cpu().numpy(), g['grp_type'].cpu().numpy()
+        del g, sp
+        # ---- src stream: src-sorted, out half grouped
+        eid = plan.rec_src[:, 0].to(torch.int64)
+        src = edge_index[0][eid]
+        g = build_grouped_stream_device(src, eid >= n_in, plan.rec_src[:, 2].to(torch.int64), plan.rowptr_src, T, 0, N)
+        self.n_out = int(g['grp_row'].numel())
+        if self.n_out > n_out_groups_max:
+            del self.rec_f, self.fwd
+            return
+        self.rec_s = plan.rec_src[g['order']].contiguous()
+        self.xrow_s = src[g['order']].to(torch.int32)
+        del src, eid
+        sp = build_stream_plan_device(i32(g['seg_beg']), i32(g['seg_end']), i32(g['seg_row']), n2)
+        self.src = StreamPlan(sp, n2, dev)
+        grp_out_row, grp_out_type = g['grp_row'].cpu().numpy(), g['grp_type'].cpu().numpy()
+        del g, sp
+        self.grp_in_row, self.grp_in_type, self.grp_out_row, self.grp_out_type = grp_in_row, grp_in_type, grp_out_row, grp_out_type
+        # ---- group reductions
+        # agg_in from P: one segment per occupied in-half row (plan.rows[0], ascending = the groups' row order), written to
+        # the compacted rows (row j) or to the plane (row rows[0][j])
+        b, e, r = group_segments(grp_in_row)
+        self.agg_in_c = GroupReduce(b, e, np.arange(r.shape[0]), grp_in_type, None, dev)
+        self.agg_in = GroupReduce(b, e, r, grp_in_type, None, dev)
+        self.n_in_rows = int(r.shape[0])
+        # d_x += rel (.) Q, on the rows that have out-half groups
+        b, e, r = group_segments(grp_out_row)
+        self.dx = GroupReduce(b, e, r, grp_out_type, None, dev)
+        # d_rel: every type row from P (types without in-half groups, the self-loop type among them, become 0), then the
+        # types of the out-half groups add their sum from Q; the groups of a type in their (row) order
+        o_in = np.argsort(grp_in_type, kind='stable')
+        b, e, r = group_segments(grp_in_type[o_in], T)
+        self.drel_in = GroupReduce(b, e, r, grp_in_row[o_in], o_in, dev)
+        o_out = np.argsort(grp_out_type, kind='stable')
+        b, e, r = group_segments(grp_out_type[o_out])
+        self.drel_out = GroupReduce(b, e, r, grp_out_row[o_out], o_out, dev)
+        self.qualifies = True
 
 
 def build_stream_plan(seg_beg, seg_end, seg_row, n_rec, chunk=CHUNK_EDGES, fan_in=CHUNK1):
@@ -189,12 +381,7 @@ class StreamPlan(object):
             else:
                 levels = [(empty, 0)]
             self.n_fill = 0
-        for it, n_part in levels:
-            # hub rows first (a block each), then the many rows that merely straddle a chunk boundary (a lane group each)
-            large = (it[:, 1] - it[:, 0]) > SMALL_ITEM
-            order = np.concatenate([np.nonzero(large)[0], np.nonzero(~large)[0]])
-            self.levels.append((torch.from_numpy(np.ascontiguousarray(it[order])).to(device), int(it.shape[0]), n_part,
-                                int(large.sum())))
+        self.levels = _fixup_levels(levels, device)
 
 
 class GraphPlan(object):
@@ -288,6 +475,11 @@ class GraphPlan(object):
                 self.rows.append(rows.to(torch.int32))
                 self.slot.append(slot)
                 self.n_c.append(int(rows.numel()))
+        # the d_rel pass factorized by (object, type) group (GroupedPlan): single GPU, large graph, both halves hub-heavy enough
+        self.grouped = None
+        if self.rows is not None and n2 >= GROUP_MIN_EDGES:
+            g = GroupedPlan(self, edge_index, GROUP_MAX_SHARE * self.num_edges_in, GROUP_MAX_SHARE * (n2 - self.num_edges_in))
+            self.grouped = g if g.qualifies else None
 
     def compact_halves(self, row_bytes):
         """(in, out): whether the single-GPU layer runs that half on its occupied rows, for planes of ``row_bytes`` per row
@@ -304,12 +496,12 @@ class GraphPlan(object):
             self._side = torch.cuda.Stream(device=self.device)
         return self._side
 
-    def scratch(self, name, shape, dtype=torch.float32):
-        """Reusable device workspace (caller-allocated, as the C ABI requires)."""
+    def scratch(self, name, shape, dtype=torch.float32, zeros=False):
+        """Reusable device workspace (caller-allocated, as the C ABI requires); ``zeros``: zero-filled when it is allocated."""
         key = (name, tuple(shape), dtype)
         t = self._scratch.get(key)
         if t is None:
-            t = torch.empty(shape, dtype=dtype, device=self.device)
+            t = (torch.zeros if zeros else torch.empty)(shape, dtype=dtype, device=self.device)
             self._scratch[key] = t
         return t
 
