@@ -585,6 +585,24 @@ int kgc_sampled_adv_fwd(const float* x, int64_t B, int32_t D, const float* ent, 
                         const float* bias, const int32_t* cand, int32_t C, int32_t n_pos, float pos, float add,
                         float temperature, float* g, float* d_x, int32_t* counts, double* loss_partial, float* loss,
                         void* stream);
+/* kgc_sampled_ce_fwd: the same pass with the softmax cross-entropy of each positive against its query's negatives
+ * (InfoNCE; LibKGE's `kl`, PyKEEN's CrossEntropyLoss) at label smoothing eps = `label_smoothing` (in [0, 1]; pos and add
+ * do not enter).  With P_b / Q_b the valid positive / negative slots of query b, z its logits, K_b = 1 + |Q_b| and, for
+ * each p in P_b, the classes {p} u Q_b (duplicates count as separate classes; the other positives are not in p's
+ * denominator), LSE_p = log(exp(z_p) + sum_{Q_b} exp(z_q)):
+ *   l_p = (1 - eps) (LSE_p - z_p) + eps (LSE_p - (z_p + sum_{Q_b} z_q) / K_b),  loss[0] = (1/P) sum_b sum_{P_b} l_p
+ * with P = count[0] = the number of valid positive slots (loss 0 when P = 0): cross_entropy(label_smoothing=eps) of
+ * the row [z_p, z_{Q_b}] with target 0, averaged over the valid positive slots.  g [B, C] = the logit gradient for a
+ * unit upstream gradient: (softmax_p(p) - (1 - eps) - eps / K_b) / P on a positive slot, sum_{P_b} (softmax_p(q) -
+ * eps / K_b) / P on a negative one (softmax_p(q) = exp(z_q) / (exp(z_p) + sum_{Q_b} exp(z_q))), 0 on empty slots; a
+ * positive without a valid negative adds 0 loss and 0 gradient.  d_x [B, D] = sum_c g[b, c] * ent[cand[b, c]] (up to
+ * rounding: the negative part is summed online against the running max of z).  The log-sum-exp is taken against that
+ * max, so no logit overflows.  loss_partial: kgc_sampled_bce_fwd_blocks(B) doubles.  Every negative row is read once,
+ * the positive rows twice.  The table gradient is kgc_sampled_bce_bwd_table on this g.  Deterministic, no host
+ * synchronisation (graph-capturable). */
+int kgc_sampled_ce_fwd(const float* x, int64_t B, int32_t D, const float* ent, int64_t n_ent, int64_t ld_ent,
+                       const float* bias, const int32_t* cand, int32_t C, int32_t n_pos, float label_smoothing,
+                       float* g, float* d_x, int32_t* count, double* loss_partial, float* loss, void* stream);
 size_t kgc_sampled_bce_bwd_table_workspace_bytes(int64_t n_slots, int64_t n_ent);
 int kgc_sampled_bce_bwd_table(const float* x, int64_t B, int32_t D, const int32_t* cand, int32_t C, const float* g,
                               const float* scale, int64_t n_ent, float* d_ent, int64_t ld_d, float* d_bias,

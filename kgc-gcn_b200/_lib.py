@@ -105,6 +105,8 @@ SIGNATURES = {
                                            _vp, _vp]),
     'kgc_sampled_adv_fwd': (ctypes.c_int, [_vp, _i64, _i32, _vp, _i64, _i64, _vp, _vp, _i32, _i32, _f32, _f32, _f32, _vp, _vp, _vp,
                                            _vp, _vp, _vp]),
+    'kgc_sampled_ce_fwd': (ctypes.c_int, [_vp, _i64, _i32, _vp, _i64, _i64, _vp, _vp, _i32, _i32, _f32, _vp, _vp, _vp, _vp, _vp,
+                                          _vp]),
     'kgc_sampled_bce_bwd_table_workspace_bytes': (_sz, [_i64, _i64]),
     'kgc_sampled_bce_bwd_table': (ctypes.c_int, [_vp, _i64, _i32, _vp, _i32, _vp, _vp, _i64, _vp, _i64, _vp, _vp, _sz, _vp]),
 }
@@ -128,7 +130,7 @@ def lib():
 
 
 LAUNCHES = 0     # kernels launched through the C ABI since import (bench.py reports it as gpu_launches)
-_KERNELS_PER_CALL = {'kgc_csr_build': 16, 'kgc_bce_1n_bwd_logit_t': 2, 'kgc_label_mask_t_build': 2, 'kgc_score_pairs': 3, 'kgc_rank_finalize': 2, 'kgc_score_topk': 2, 'kgc_topk_dense': 2, 'kgc_sampled_bce_fwd': 4, 'kgc_sampled_adv_fwd': 4, 'kgc_sampled_bce_bwd_table': 7, 'kgc_gemm_tn': 2, 'kgc_gemm_tn_tc_batch': 2}   # (kgc_p2p_allreduce: 1 or 3)
+_KERNELS_PER_CALL = {'kgc_csr_build': 16, 'kgc_bce_1n_bwd_logit_t': 2, 'kgc_label_mask_t_build': 2, 'kgc_score_pairs': 3, 'kgc_rank_finalize': 2, 'kgc_score_topk': 2, 'kgc_topk_dense': 2, 'kgc_sampled_bce_fwd': 4, 'kgc_sampled_adv_fwd': 4, 'kgc_sampled_ce_fwd': 3, 'kgc_sampled_bce_bwd_table': 7, 'kgc_gemm_tn': 2, 'kgc_gemm_tn_tc_batch': 2}   # (kgc_p2p_allreduce: 1 or 3)
 
 
 def call(name, *args):

@@ -17,7 +17,9 @@
 //
 // kgc_sampled_adv_fwd is the self-adversarial forward (Sun et al. 2019): each query's negatives are weighted by a softmax
 // of their own logits at a temperature, computed online in the same single pass (sampled_adv_fwd_kernel).  Its g is a
-// logit gradient like any other, so the table backward above serves both.
+// logit gradient like any other, so the table backward above serves both.  kgc_sampled_ce_fwd is the softmax
+// cross-entropy of each positive against its query's negatives (sampled_ce_fwd_kernel), in the same pass over the rows
+// and through the same table backward.
 #include <cmath>
 
 #include <cub/device/device_radix_sort.cuh>
@@ -319,6 +321,193 @@ sampled_adv_finalize_kernel(const double* __restrict__ partial, int64_t n_partia
   }
 }
 
+// Softmax cross-entropy variant.  P = the number of valid positive slots (integer sum: the order of the atomics does not
+// matter); slot i of the grid-stride walk is column i % n_pos of query i / n_pos.
+__global__ void __launch_bounds__(kThreadsSS)
+count_pos_kernel(const int32_t* __restrict__ cand, int64_t B, int C, int n_pos, int64_t n_ent, int32_t* __restrict__ count) {
+  int c = 0;
+  for (int64_t i = (int64_t)blockIdx.x * kThreadsSS + threadIdx.x; i < B * n_pos; i += (int64_t)gridDim.x * kThreadsSS)
+    c += slot_valid(cand[(i / n_pos) * C + i % n_pos], n_ent) ? 1 : 0;
+#pragma unroll
+  for (int o = 16; o > 0; o >>= 1) c += __shfl_xor_sync(kFull, c, o);
+  if ((threadIdx.x & 31) == 0 && c != 0) atomicAdd(count, c);
+}
+
+// Each valid positive slot p of query b against the valid negative slots Q_b of that query, K_b = 1 + |Q_b| classes
+// (other positives are not in p's denominator):
+//   l_p = (1 - eps) (LSE_p - z_p) + eps (LSE_p - (z_p + sum_{Q_b} z_q) / K_b),  LSE_p = log(e^{z_p} + sum_{Q_b} e^{z_q})
+// and L = (1 / P) sum l_p.  Same row traffic as sampled_adv_fwd_kernel for the negatives (each read once, kRowsInFlight in
+// flight): a warp-uniform running max m over the negative logits, S = sum e^{z_q - m} and acc_w = sum e^{z_q - m} E[q],
+// the latter two rescaled when a batch raises m; with eps > 0 also the plain sum acc_1 = sum E[q].  The main loop parks
+// each slot's logit in g.  After the query's last row a pass over its negative slots gives |Q_b| and Z = sum z_q from the
+// parked logits, and one over its positive slots gives, from the final S, the negatives' softmax mass under p,
+// 1 - softmax_p(p), the loss term and r_p = softmax_p(q) e^{m - z_q} (the same for every q), all against max(m, z_p) so
+// that no exponent is positive; then
+//   g_p = (eps |Q_b| / K_b - (1 - softmax_p(p))) / P,   g_q = (e^{z_q - m} R - |P_b| eps / K_b) / P,  R = sum_{P_b} r_p
+// and d_x = (R acc_w - |P_b| eps / K_b acc_1) / P + sum_{P_b} g_p E[p]: the positive rows (n_pos of the C) are read a
+// second time.  A positive without a valid negative has softmax_p(p) = 1 and |Q_b| = 0, so 0 loss and 0 gradient; a
+// query without a valid positive has R = |P_b| = 0.  loss_partial: [gridDim.x] per-CTA sums of l_p; the division by P
+// is sampled_bce_finalize_kernel's.
+// (two CTAs an SM: ptxas then keeps NV = 1 at 109 registers without spills instead of squeezing it into the 80 of three
+// CTAs with a spilled row offset)
+template <int NV>    // float4 columns per lane: D <= 128 * NV
+__global__ void __launch_bounds__(kThreadsSS, 2)
+sampled_ce_fwd_kernel(const float* __restrict__ x, int64_t B, int D4, const float* __restrict__ ent, int64_t ld_ent,
+                      int64_t n_ent, const float* __restrict__ bias, const int32_t* __restrict__ cand, int C, int n_pos,
+                      float eps, const int32_t* __restrict__ count, float* g_out, float* __restrict__ d_x,
+                      double* __restrict__ loss_partial) {
+  __shared__ double warp_loss[kWarpsSS];
+  const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5;
+  const int64_t b = (int64_t)blockIdx.x * kWarpsSS + warp;
+  double loss = 0.0;                                             // this query's sum of l_p, the same value in every lane
+  if (b < B) {
+    const float4 zero = make_float4(0.f, 0.f, 0.f, 0.f);
+    float4 xr[NV], acc_w[NV], acc_1[NV];
+#pragma unroll
+    for (int v = 0; v < NV; ++v) {
+      const int c4 = lane + 32 * v;
+      xr[v] = c4 < D4 ? ldg4(x + b * 4 * D4 + 4 * c4) : zero;
+      acc_w[v] = zero;
+      acc_1[v] = zero;
+    }
+    const int32_t* cb = cand + b * C;
+    float* gb = g_out + b * C;
+    float m = -INFINITY, S = 0.f;                                // warp-uniform
+    for (int c0 = 0; c0 < C; c0 += kRowsInFlight) {
+      const int32_t mine = (lane < kRowsInFlight && c0 + lane < C) ? cb[c0 + lane] : -1;
+      int32_t e[kRowsInFlight];
+      float4 r[kRowsInFlight][NV];
+      float bi[kRowsInFlight];
+#pragma unroll
+      for (int u = 0; u < kRowsInFlight; ++u) {
+        e[u] = __shfl_sync(kFull, mine, u);
+        if (!slot_valid(e[u], n_ent)) e[u] = -1;
+      }
+#pragma unroll
+      for (int u = 0; u < kRowsInFlight; ++u) {                  // every row load of the batch before any is consumed
+#pragma unroll
+        for (int v = 0; v < NV; ++v) {
+          const int c4 = lane + 32 * v;
+          r[u][v] = (e[u] >= 0 && c4 < D4) ? ldg4(ent + (int64_t)e[u] * ld_ent + 4 * c4) : zero;
+        }
+        bi[u] = e[u] >= 0 ? __ldg(bias + e[u]) : 0.f;
+      }
+      float z[kRowsInFlight];
+      float m_new = m;
+#pragma unroll
+      for (int u = 0; u < kRowsInFlight; ++u) {
+        z[u] = warp_dot(xr, r[u]) + bi[u];
+        if (e[u] >= 0 && c0 + u >= n_pos) m_new = fmaxf(m_new, z[u]);
+      }
+      if (m_new > m) {                                           // rescale what was summed under the old max
+        const float sc = expf(m - m_new);
+        S *= sc;
+#pragma unroll
+        for (int v = 0; v < NV; ++v) {
+          acc_w[v].x *= sc;
+          acc_w[v].y *= sc;
+          acc_w[v].z *= sc;
+          acc_w[v].w *= sc;
+        }
+        m = m_new;
+      }
+      float z_mine = 0.f;
+#pragma unroll
+      for (int u = 0; u < kRowsInFlight; ++u) {
+        if (e[u] >= 0) {
+          if (c0 + u >= n_pos) {
+            const float w = expf(z[u] - m);
+            S += w;
+#pragma unroll
+            for (int v = 0; v < NV; ++v) fma4(w, r[u][v], acc_w[v]);
+            if (eps > 0.f) {
+#pragma unroll
+              for (int v = 0; v < NV; ++v) fma4(1.f, r[u][v], acc_1[v]);
+            }
+          }
+        }
+        if (lane == u) z_mine = z[u];
+      }
+      if (lane < kRowsInFlight && c0 + lane < C) gb[c0 + lane] = z_mine;
+    }
+    __syncwarp();                                                // the parked logits are visible to every lane
+    int n_q = 0;                                                 // |Q_b| and the sum Z of its logits, from the parked ones
+    double Z = 0.0;
+    for (int c = n_pos + lane; c < C; c += 32) {
+      if (slot_valid(cb[c], n_ent)) {
+        ++n_q;
+        Z += (double)gb[c];
+      }
+    }
+    n_q = __reduce_add_sync(kFull, n_q);
+    Z = warp_sum(Z);
+    const int n_valid = *count;                                  // read here: one register less across the row loop
+    const float inv_p = n_valid > 0 ? (float)(1.0 / (double)n_valid) : 0.f;
+    const float inv_k = 1.f / (float)(1 + n_q);
+    const float eps_pos = eps * (float)n_q * inv_k;              // eps (1 - 1 / K_b)
+    float R = 0.f;
+    double l = 0.0;
+    int n_p = 0;                                                 // |P_b|
+    for (int c = lane; c < n_pos; c += 32) {
+      float gv = 0.f;                                            // 0 on empty slots
+      if (slot_valid(cb[c], n_ent)) {
+        const float zp = gb[c];
+        float q_mass, rp, lse_z;                                 // 1 - softmax_p(p), r_p, LSE_p - z_p
+        if (zp >= m) {                                           // also every positive of a query without negatives
+          const float em = expf(m - zp);
+          const float t = S * em;
+          q_mass = t / (1.f + t);
+          rp = em / (1.f + t);
+          lse_z = log1pf(t);
+        } else {
+          const float ep = expf(zp - m);
+          q_mass = S / (ep + S);
+          rp = 1.f / (ep + S);
+          lse_z = (m - zp) + logf(ep + S);
+        }
+        ++n_p;
+        R += rp;
+        l += (double)lse_z + (double)eps * ((double)n_q * (double)zp - Z) / (double)(1 + n_q);
+        gv = (eps_pos - q_mass) * inv_p;
+      }
+      gb[c] = gv;
+    }
+    R = (float)warp_sum((double)R);
+    loss = warp_sum(l);
+    n_p = __reduce_add_sync(kFull, n_p);
+    const float eps_neg = (float)n_p * eps * inv_k;              // |P_b| eps / K_b
+    for (int c = n_pos + lane; c < C; c += 32) {
+      float gv = 0.f;
+      if (slot_valid(cb[c], n_ent)) gv = (expf(gb[c] - m) * R - eps_neg) * inv_p;
+      gb[c] = gv;
+    }
+    const float cw = R * inv_p, c1 = -eps_neg * inv_p;
+    float4 o[NV];
+#pragma unroll
+    for (int v = 0; v < NV; ++v)
+      o[v] = make_float4(fmaf(cw, acc_w[v].x, c1 * acc_1[v].x), fmaf(cw, acc_w[v].y, c1 * acc_1[v].y),
+                         fmaf(cw, acc_w[v].z, c1 * acc_1[v].z), fmaf(cw, acc_w[v].w, c1 * acc_1[v].w));
+    __syncwarp();                                                // the positives' final g is visible to every lane
+    for (int c = 0; c < n_pos; ++c) {                            // the positive rows again, in slot order
+      const int32_t ep = cb[c];
+      if (!slot_valid(ep, n_ent)) continue;
+      const float gp = gb[c];
+#pragma unroll
+      for (int v = 0; v < NV; ++v) {
+        const int c4 = lane + 32 * v;
+        if (c4 < D4) fma4(gp, ldg4(ent + (int64_t)ep * ld_ent + 4 * c4), o[v]);
+      }
+    }
+#pragma unroll
+    for (int v = 0; v < NV; ++v) {
+      const int c4 = lane + 32 * v;
+      if (c4 < D4) *reinterpret_cast<float4*>(d_x + b * 4 * D4 + 4 * c4) = o[v];
+    }
+  }
+  const double s = cta_sum(loss, warp_loss, lane, warp);
+  if (threadIdx.x == 0) loss_partial[blockIdx.x] = s;
+}
+
 // sort keys: the entity, or N for an empty slot (sorts after every entity); values: the slot
 __global__ void __launch_bounds__(kThreadsSS)
 slot_keys_kernel(const int32_t* __restrict__ cand, int64_t n_slots, int64_t n_ent, int32_t* __restrict__ keys,
@@ -482,6 +671,29 @@ extern "C" int kgc_sampled_adv_fwd(const float* x, int64_t B, int32_t D, const f
                                               g, d_x, loss_partial);
   KGC_LAUNCH_CHECK();
   sampled_adv_finalize_kernel<<<1, kThreadsSS, 0, s>>>(loss_partial, blocks, counts, loss);
+  KGC_LAUNCH_CHECK();
+  return 0;
+}
+
+extern "C" int kgc_sampled_ce_fwd(const float* x, int64_t B, int32_t D, const float* ent, int64_t n_ent, int64_t ld_ent,
+                                  const float* bias, const int32_t* cand, int32_t C, int32_t n_pos, float label_smoothing,
+                                  float* g, float* d_x, int32_t* count, double* loss_partial, float* loss, void* stream) {
+  if (const char* err = check_fwd_args(x, B, D, ent, n_ent, ld_ent, bias, cand, C, n_pos, g, d_x, count, loss_partial, loss))
+    return fail(__func__, err);
+  KGC_REQUIRE(label_smoothing >= 0.f && label_smoothing <= 1.f, "the label smoothing must be a number in [0, 1]");
+  cudaStream_t s = as_stream(stream);
+  KGC_CUDA_TRY(cudaMemsetAsync(count, 0, sizeof(int32_t), s));
+  const int64_t pblocks = ceil_div(B * n_pos, kThreadsSS);       // 0 when n_pos = 0: then one CTA that counts nothing
+  const int64_t cblocks = pblocks < 1 ? 1 : pblocks < 4 * kNumSMs ? pblocks : 4 * kNumSMs;
+  count_pos_kernel<<<(unsigned)cblocks, kThreadsSS, 0, s>>>(cand, B, C, n_pos, n_ent, count);
+  KGC_LAUNCH_CHECK();
+  const int64_t blocks = kgc_sampled_bce_fwd_blocks(B);
+  const int D4 = D / 4;
+  const auto fwd = for_width(D4, sampled_ce_fwd_kernel<1>, sampled_ce_fwd_kernel<2>);
+  fwd<<<(unsigned)blocks, kThreadsSS, 0, s>>>(x, B, D4, ent, ld_ent, n_ent, bias, cand, C, n_pos, label_smoothing, count, g,
+                                              d_x, loss_partial);
+  KGC_LAUNCH_CHECK();
+  sampled_bce_finalize_kernel<<<1, kThreadsSS, 0, s>>>(loss_partial, blocks, count, loss);
   KGC_LAUNCH_CHECK();
   return 0;
 }

@@ -305,7 +305,8 @@ class MGCN(nn.Module):
         pos, add = dataset.label_values()
         return score_1n_bce(x, all_ent, self.conv2.bias, qid, ptr, idx, pos, add)
 
-    def loss_sampled(self, qid, dataset, data, k, n_pos=1, tries=4, draws=None, generator=None, adversarial_temperature=None):
+    def loss_sampled(self, qid, dataset, data, k, n_pos=1, tries=4, draws=None, generator=None, adversarial_temperature=None,
+                     criterion='bce', label_smoothing=0.0):
         """Negative-sampled (1-vs-k) training loss for the training queries ``qid`` of ``dataset`` (a KBDataset): each query
         scores ``n_pos`` of its known objects (``dataset.positives``) and ``k`` entities that are not (``dataset.negatives``,
         ``tries`` draws per slot) - candidates [pos | neg] - through ``scoring.score_sampled_bce`` with the dataset's
@@ -313,9 +314,12 @@ class MGCN(nn.Module):
         ``draws = (pos_draws [B, n_pos], neg_draws [B, k, tries])`` (uint32 values) makes the call a pure function of them;
         otherwise they come from torch's generator (``generator`` or the global one), positives first.
         ``adversarial_temperature=alpha`` weights each query's negatives by softmax(alpha * logit) (self-adversarial
-        negative sampling, see ``scoring.score_sampled_bce``); None: the plain mean over the valid slots."""
-        from .scoring import check_adversarial_temperature, score_sampled_bce
-        check_adversarial_temperature(adversarial_temperature)
+        negative sampling, see ``scoring.score_sampled_bce``); None: the plain mean over the valid slots.
+        ``criterion='ce'`` trains each positive's softmax cross-entropy against its query's negatives instead
+        (``scoring.score_sampled_ce``, with ``label_smoothing`` eps in [0, 1]; the dataset's label values do not enter).
+        A temperature with 'ce', a label smoothing with 'bce' or another criterion is a ValueError."""
+        from .scoring import check_sampled_criterion, score_sampled_bce, score_sampled_ce
+        _, eps = check_sampled_criterion(criterion, adversarial_temperature, label_smoothing)
         dev = self.entity_embedding.device
         triples, _, _ = dataset.device_csr(dev)
         qid = torch.as_tensor(qid, dtype=torch.int64).to(dev, non_blocking=True)
@@ -324,6 +328,8 @@ class MGCN(nn.Module):
         cand = torch.cat([dataset.positives(qid, n_pos, draws=pos_draws, device=dev, generator=generator),
                           dataset.negatives(qid, k, draws=neg_draws, tries=tries, device=dev, generator=generator)], 1)
         _, x, all_ent = self._train_queries(qid, triples, data)
+        if criterion == 'ce':
+            return score_sampled_ce(x, all_ent, self.conv2.bias, cand, n_pos, eps)
         pos, add = dataset.label_values()
         return score_sampled_bce(x, all_ent, self.conv2.bias, cand, n_pos, pos, add,
                                  adversarial_temperature=adversarial_temperature)

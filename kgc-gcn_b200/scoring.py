@@ -143,6 +143,23 @@ def score_1n_bce(x, all_ent, bias, qid, ptr, idx, pos=1.0, add=0.0):
     return total
 
 
+def _sampled_operands(x, all_ent, bias, cand):
+    """The sampled forwards' device operands: x, the entity rows (a row pitch is taken, so rows may sit in a wider table),
+    bias and cand, checked, and the g [B, C] and d_x [B, D] outputs."""
+    x = _lib.require_cuda(x.detach(), torch.float32, 'x')
+    ent = all_ent.detach()
+    if ent.dtype != torch.float32:
+        raise TypeError('all_ent must be torch.float32, got {}'.format(ent.dtype))
+    if ent.stride(1) != 1 or ent.stride(0) % 4 != 0 or ent.data_ptr() % 16 != 0:
+        ent = ent.clone(memory_format=torch.contiguous_format)
+    bias_ = _lib.require_cuda(bias.detach(), torch.float32, 'bias')
+    cand = _lib.require_cuda(cand, torch.int32, 'cand')
+    B, D, C = int(x.shape[0]), int(x.shape[1]), int(cand.shape[1])
+    g = torch.empty((B, C), dtype=torch.float32, device=x.device)
+    d_x = torch.empty((B, D), dtype=torch.float32, device=x.device)
+    return x, ent, bias_, cand, g, d_x
+
+
 class _ScoreSampledBCE(torch.autograd.Function):
     """loss = mean BCE of sigmoid(<x[b], all_ent[cand[b, c]]> + bias[cand[b, c]]) over the valid slots (K6s), or with a
     ``temperature`` the self-adversarial loss of ``score_sampled_bce``.  The forward makes one pass that yields the loss, the
@@ -151,19 +168,9 @@ class _ScoreSampledBCE(torch.autograd.Function):
 
     @staticmethod
     def forward(ctx, x, all_ent, bias, cand, n_pos, pos, add, temperature=None):
-        x = _lib.require_cuda(x.detach(), torch.float32, 'x')
-        ent = all_ent.detach()                           # rows may sit in a wider table: the kernel takes a row pitch
-        if ent.dtype != torch.float32:
-            raise TypeError('all_ent must be torch.float32, got {}'.format(ent.dtype))
-        if ent.stride(1) != 1 or ent.stride(0) % 4 != 0 or ent.data_ptr() % 16 != 0:
-            ent = ent.clone(memory_format=torch.contiguous_format)
-        bias_ = _lib.require_cuda(bias.detach(), torch.float32, 'bias')
-        cand = _lib.require_cuda(cand, torch.int32, 'cand')
-        B, D = int(x.shape[0]), int(x.shape[1])
-        C, N = int(cand.shape[1]), int(ent.shape[0])
+        x, ent, bias_, cand, g, d_x = _sampled_operands(x, all_ent, bias, cand)
+        B, D, C, N = int(x.shape[0]), int(x.shape[1]), int(cand.shape[1]), int(ent.shape[0])
         dev, p = x.device, _lib.ptr
-        g = torch.empty((B, C), dtype=torch.float32, device=dev)
-        d_x = torch.empty((B, D), dtype=torch.float32, device=dev)
         if temperature is None:
             count = torch.empty((1,), dtype=torch.int32, device=dev)
             partial = torch.empty((int(_lib.lib().kgc_sampled_bce_fwd_blocks(B)),), dtype=torch.float64, device=dev)
@@ -182,6 +189,7 @@ class _ScoreSampledBCE(torch.autograd.Function):
 
     @staticmethod
     def backward(ctx, d_loss):
+        # (also _ScoreSampledCE's: autograd drops the trailing None gradients of inputs that objective does not have)
         x, cand, g, d_x = ctx.saved_tensors
         B, D, C, N = int(x.shape[0]), int(x.shape[1]), int(cand.shape[1]), ctx.n_ent
         d_ent = d_bias = None
@@ -196,6 +204,26 @@ class _ScoreSampledBCE(torch.autograd.Function):
                       ws_bytes, _lib.stream())
         return (d_x * d_loss if ctx.needs_input_grad[0] else None, d_ent if ctx.needs_input_grad[1] else None,
                 d_bias if ctx.needs_input_grad[2] else None, None, None, None, None, None)
+
+
+class _ScoreSampledCE(_ScoreSampledBCE):
+    """loss = the softmax cross-entropy of ``score_sampled_ce`` (K6s, kgc_sampled_ce_fwd): the same single pass yields the
+    loss, the logit gradient g [B, C] and d_x for a unit upstream gradient, and _ScoreSampledBCE's backward turns g into
+    the table gradient."""
+
+    @staticmethod
+    def forward(ctx, x, all_ent, bias, cand, n_pos, label_smoothing):
+        x, ent, bias_, cand, g, d_x = _sampled_operands(x, all_ent, bias, cand)
+        B, D, C, N = int(x.shape[0]), int(x.shape[1]), int(cand.shape[1]), int(ent.shape[0])
+        dev, p = x.device, _lib.ptr
+        count = torch.empty((1,), dtype=torch.int32, device=dev)
+        partial = torch.empty((int(_lib.lib().kgc_sampled_bce_fwd_blocks(B)),), dtype=torch.float64, device=dev)
+        loss = torch.empty((1,), dtype=torch.float32, device=dev)
+        _lib.call('kgc_sampled_ce_fwd', p(x), B, D, p(ent), N, ent.stride(0), p(bias_), p(cand), C, int(n_pos),
+                  float(label_smoothing), p(g), p(d_x), p(count), p(partial), p(loss), _lib.stream())
+        ctx.save_for_backward(x, cand, g, d_x)
+        ctx.n_ent = N
+        return loss[0]
 
 
 def check_adversarial_temperature(temperature):
@@ -223,29 +251,76 @@ def score_sampled_bce(x, all_ent, bias, cand, n_pos, pos=1.0, add=0.0, adversari
     negative.  Same single pass, same row traffic and the same backward as the plain objective.  None (default): the plain
     mean over the valid slots."""
     temperature = check_adversarial_temperature(adversarial_temperature)
+    _check_sampled_args('score_sampled_bce', x, all_ent, bias, cand, n_pos)
+    return _ScoreSampledBCE.apply(x, all_ent, bias, cand, int(n_pos), pos, add, temperature)
+
+
+def check_label_smoothing(label_smoothing):
+    """``label_smoothing`` as a float: anything but a finite real number in [0, 1] is a ValueError."""
+    if isinstance(label_smoothing, bool) or not isinstance(label_smoothing, numbers.Real) \
+            or not (0.0 <= label_smoothing <= 1.0):
+        raise ValueError('label_smoothing must be a finite number in [0, 1], got {!r}'.format(label_smoothing))
+    return float(label_smoothing)
+
+
+def check_sampled_criterion(criterion, adversarial_temperature, label_smoothing):
+    """The loss options of the sampled objective (``MGCN.loss_sampled``, ``GraphedTrainStep``), checked together:
+    ``criterion`` 'bce' (``score_sampled_bce``, optionally self-adversarial) or 'ce' (``score_sampled_ce``, optionally
+    label-smoothed).  Returns (temperature or None, label smoothing as a float); a combination that one criterion does not
+    take is a ValueError."""
+    if criterion not in ('bce', 'ce'):
+        raise ValueError("criterion must be 'bce' or 'ce', got {!r}".format(criterion))
+    temperature = check_adversarial_temperature(adversarial_temperature)
+    eps = check_label_smoothing(label_smoothing)
+    if criterion == 'ce' and temperature is not None:
+        raise ValueError("adversarial_temperature weights the BCE negatives: it does not combine with criterion='ce'")
+    if criterion == 'bce' and eps != 0.0:
+        raise ValueError("label_smoothing is the cross-entropy's (criterion='ce'); the BCE criterion takes the dataset's "
+                         "label values")
+    return temperature, eps
+
+
+def score_sampled_ce(x, all_ent, bias, cand, n_pos, label_smoothing=0.0):
+    """Negative-sampled (1-vs-k) softmax cross-entropy (InfoNCE; LibKGE's ``kl``, PyKEEN's ``CrossEntropyLoss``): query b
+    of ``x`` [B, D] scores its candidates ``cand`` [B, C] (int32 entity ids, the first ``n_pos`` columns positives, the
+    rest negatives; an id outside [0, N) is an empty slot), z = <x[b], all_ent[c]> + bias[c].  Each valid positive p is
+    classified against the query's valid negatives Q_b: the row [z_p, z_{Q_b}] with target 0 (the other positives are not
+    in its denominator; duplicate entities count as separate classes), and the loss is
+    ``F.cross_entropy(row, 0, label_smoothing=eps)`` averaged over the valid positive slots of the batch (0 when there are
+    none).  A positive without a valid negative adds 0 loss and 0 gradient.  ``label_smoothing`` eps in [0, 1] is the
+    cross-entropy's own; the dataset's BCE label values do not enter.  Differentiable in ``x``, ``all_ent`` and
+    ``bias``; the log-sum-exp runs against a running max, so logits of any size are safe.  Same argument rules, single
+    pass over the candidate rows (the positive rows are read twice) and table backward as ``score_sampled_bce``;
+    deterministic and graph-capturable."""
+    eps = check_label_smoothing(label_smoothing)
+    _check_sampled_args('score_sampled_ce', x, all_ent, bias, cand, n_pos)
+    return _ScoreSampledCE.apply(x, all_ent, bias, cand, int(n_pos), eps)
+
+
+def _check_sampled_args(fn, x, all_ent, bias, cand, n_pos):
+    """The shapes, dtypes and devices the sampled forwards take (``fn`` names the caller in the messages)."""
     if x.dim() != 2 or all_ent.dim() != 2 or bias.dim() != 1 or cand.dim() != 2:
-        raise ValueError('score_sampled_bce takes x [B, D], all_ent [N, D], bias [N] and cand [B, C]')
+        raise ValueError('{} takes x [B, D], all_ent [N, D], bias [N] and cand [B, C]'.format(fn))
     B, D = int(x.shape[0]), int(x.shape[1])
     N, C = int(all_ent.shape[0]), int(cand.shape[1])
     if int(all_ent.shape[1]) != D or int(bias.shape[0]) != N or int(cand.shape[0]) != B:
         raise ValueError('shape mismatch: x {}, all_ent {}, bias {}, cand {}'.format(
             tuple(x.shape), tuple(all_ent.shape), tuple(bias.shape), tuple(cand.shape)))
     if B < 1 or C < 1 or N < 1 or D < 4 or D > 256 or D % 4 != 0:
-        raise ValueError('score_sampled_bce needs B, C, N >= 1 and D % 4 == 0, D <= 256 (got B={}, C={}, N={}, D={})'.format(
-            B, C, N, D))
+        raise ValueError('{} needs B, C, N >= 1 and D % 4 == 0, D <= 256 (got B={}, C={}, N={}, D={})'.format(
+            fn, B, C, N, D))
     if isinstance(n_pos, bool) or int(n_pos) != n_pos or not 0 <= n_pos <= C:
         raise ValueError('n_pos must be an integer in [0, C = {}], got {!r}'.format(C, n_pos))
     if cand.dtype != torch.int32:
         raise ValueError('cand must be torch.int32, got {}'.format(cand.dtype))
     if B * C >= 2 ** 31 or N >= 2 ** 31 - 1:
-        raise ValueError('score_sampled_bce takes B * C < 2^31 slots and N < 2^31 - 1 entities')
+        raise ValueError('{} takes B * C < 2^31 slots and N < 2^31 - 1 entities'.format(fn))
     for t, name in ((x, 'x'), (all_ent, 'all_ent'), (bias, 'bias'), (cand, 'cand')):
         if not t.is_cuda:
             raise RuntimeError('{} must be a CUDA tensor: the M-GCN hot path runs on the GPU only (no CPU fallback)'.format(name))
     if not torch.cuda.is_current_stream_capturing() and bool((cand >= N).any()):
         # (not checked while a CUDA graph is captured: the check reads back; the kernels treat such ids as empty slots)
         raise ValueError('cand holds entity ids >= N = {}'.format(N))
-    return _ScoreSampledBCE.apply(x, all_ent, bias, cand, int(n_pos), pos, add, temperature)
 
 
 def score_kpad(d):

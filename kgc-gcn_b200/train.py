@@ -24,14 +24,19 @@ class GraphedTrainStep(object):
     buffers (``pos_draws`` [B, n_pos], ``neg_draws`` [B, k, tries]) before the replay; the graph itself holds no RNG, so
     a replay equals the eager ``loss_sampled`` step on the same draws.  ``adversarial_temperature=alpha`` (with
     ``negatives=k`` only) trains with self-adversarial negative weights (``MGCN.loss_sampled``); the graph holds alpha as
-    a constant."""
+    a constant.  ``criterion='ce'`` (with ``negatives=k`` only) trains the sampled softmax cross-entropy instead, at
+    ``label_smoothing=eps`` (``MGCN.loss_sampled``); the graph holds eps as a constant."""
 
     def __init__(self, model, optimizer, graph, dataset, batch_size, clip_grad=1.0, warmup=3, fused_loss=False,
-                 negatives=None, n_pos=1, tries=4, generator=None, adversarial_temperature=None):
-        from .scoring import check_adversarial_temperature
-        adversarial_temperature = check_adversarial_temperature(adversarial_temperature)
+                 negatives=None, n_pos=1, tries=4, generator=None, adversarial_temperature=None, criterion='bce',
+                 label_smoothing=0.0):
+        from .scoring import check_sampled_criterion
+        adversarial_temperature, label_smoothing = check_sampled_criterion(criterion, adversarial_temperature,
+                                                                           label_smoothing)
         if adversarial_temperature is not None and negatives is None:
             raise ValueError('adversarial_temperature weights the sampled negatives: it needs negatives=k')
+        if criterion == 'ce' and negatives is None:
+            raise ValueError("criterion='ce' is a loss of the sampled objective: it needs negatives=k")
         if negatives is not None:
             if fused_loss:
                 raise ValueError('negatives= and fused_loss=True are two different objectives: pass one of them')
@@ -50,6 +55,7 @@ class GraphedTrainStep(object):
         self.negatives = None if negatives is None else int(negatives)
         self.n_pos, self.tries, self.generator = int(n_pos), int(tries), generator
         self.adversarial_temperature = adversarial_temperature
+        self.criterion, self.label_smoothing = criterion, label_smoothing
         self.pos_draws = self.neg_draws = self.label = None
         if self.objective == 'sampled':
             self.pos_draws = torch.zeros((self.B, self.n_pos), dtype=torch.int64, device=dev)
@@ -96,7 +102,8 @@ class GraphedTrainStep(object):
         if self.objective == 'sampled':
             loss = self.model.loss_sampled(qid, self.ds, self.graph_data, self.negatives, n_pos=self.n_pos, tries=self.tries,
                                            draws=draws, generator=self.generator,
-                                           adversarial_temperature=self.adversarial_temperature)
+                                           adversarial_temperature=self.adversarial_temperature, criterion=self.criterion,
+                                           label_smoothing=self.label_smoothing)
         elif self.objective == 'sparse':
             loss = self.model.loss_sparse(qid, self.ds, self.graph_data)
         else:
