@@ -1,25 +1,25 @@
-// K6s: sampled (1-vs-k) scoring fused with the BCE loss - the negative-sampled training objective (extension: the reference
-// trains 1-N only).  Each query b scores C chosen candidates cand[b, 0..C): the first n_pos are its positives (label pos),
-// the rest negatives (label add); an id outside [0, N) is an empty slot (no loss, no gradient).  The cost is B x C
-// gathered rows, independent of N, so the batch can grow far beyond what the 1-N objective's [N, B] tiles allow.
+// K6s: sampled (1-vs-k) scoring fused with the training loss - the negative-sampled objective (extension: the reference
+// trains 1-N only).  Each query b scores C chosen candidates cand[b, 0..C): the first n_pos are its positives, the rest
+// negatives; an id outside [0, N) is an empty slot (no loss, no gradient).  The cost is B x C gathered rows, independent
+// of N, so the batch can grow far beyond what the 1-N objective's [N, B] tiles allow.
 //
-// Forward (one pass): logit = <x[b], E[cand]> + bias[cand] in fp32 (warp_dot), p = sigmoid, then ATen's BCE as
-// kgc_bce_1n_bwd_logit_t (bce.cuh) with the VALID-slot count as the mean's divisor: g = bce_logit_grad(p, y, 1 / count)
-// (unit upstream gradient) and, while the candidate row is still in registers, d_x[b] += g * E[cand] in slot order.  A
-// warp owns one query: the x row lives in registers, a candidate row is one coalesced request of 4 D bytes (800 at
-// D = 200), and the rows of a batch of kRowsInFlight slots are all loaded before the first is consumed (the lesson of
-// agg_kernel, DESIGN section 4).
+// Forward (one pass, sampled_fwd_kernel): a warp owns one query, the x row lives in registers, a candidate row is one
+// coalesced request of 4 D bytes (800 at D = 200), and the rows of a batch of kRowsInFlight slots are all loaded before
+// the first is consumed (the lesson of agg_kernel, DESIGN section 4).  logit = <x[b], E[cand]> + bias[cand] in fp32
+// (warp_dot).  What the loss does with a batch of logits and rows, and after the query's last row, is a policy type:
+//   BceLoss  ATen's BCE (kgc_sampled_bce_fwd): p = sigmoid, labels pos / add, the valid-slot count as the mean's divisor,
+//            g = bce_logit_grad(p, y, 1 / count) and d_x[b] += g * E[cand] in slot order while the row is in registers;
+//   AdvLoss  self-adversarial BCE (kgc_sampled_adv_fwd, Sun et al. 2019): the negatives weighted by a softmax of their
+//            own logits at a temperature, computed online;
+//   CeLoss   softmax cross-entropy of each positive against its query's negatives (kgc_sampled_ce_fwd).
+// The three entries run one launcher: zero the counts, count_kernel (what the loss divides by), the forward, and
+// sampled_finalize_kernel (the per-CTA loss partials added in a fixed order).
 //
 // Table backward: d_E[n] = sum over the slots s with cand[s] = n of g[s] * (scale x[b(s)]) and d_bias[n] = scale sum g[s],
-// dense [N, D] / [N] with zeros elsewhere (the encoder's backward takes a dense upstream).  Duplicate candidates are the
-// normal case (across queries and within one), so instead of float atomics the (entity, slot) pairs are stable-sorted by
-// entity (CUB radix sort, as K1) and one warp per distinct entity adds its slots in slot order: deterministic.
-//
-// kgc_sampled_adv_fwd is the self-adversarial forward (Sun et al. 2019): each query's negatives are weighted by a softmax
-// of their own logits at a temperature, computed online in the same single pass (sampled_adv_fwd_kernel).  Its g is a
-// logit gradient like any other, so the table backward above serves both.  kgc_sampled_ce_fwd is the softmax
-// cross-entropy of each positive against its query's negatives (sampled_ce_fwd_kernel), in the same pass over the rows
-// and through the same table backward.
+// dense [N, D] / [N] with zeros elsewhere (the encoder's backward takes a dense upstream).  Every loss's g is a logit
+// gradient, so one backward serves all three.  Duplicate candidates are the normal case (across queries and within one),
+// so instead of float atomics the (entity, slot) pairs are stable-sorted by entity (CUB radix sort, as K1) and one warp
+// per distinct entity adds its slots in slot order: deterministic.
 #include <cmath>
 
 #include <cub/device/device_radix_sort.cuh>
@@ -63,449 +63,416 @@ __device__ __forceinline__ float warp_dot(const float4 (&xr)[NV], const float4 (
   return s;
 }
 
-// number of valid slots (integer sum: the order of the atomics does not matter)
-__global__ void __launch_bounds__(kThreadsSS)
-count_valid_kernel(const int32_t* __restrict__ cand, int64_t n_slots, int64_t n_ent, int32_t* __restrict__ count) {
-  int c = 0;
-  for (int64_t i = (int64_t)blockIdx.x * kThreadsSS + threadIdx.x; i < n_slots; i += (int64_t)gridDim.x * kThreadsSS)
-    c += slot_valid(cand[i], n_ent) ? 1 : 0;
-#pragma unroll
-  for (int o = 16; o > 0; o >>= 1) c += __shfl_xor_sync(kFull, c, o);
-  if ((threadIdx.x & 31) == 0 && c != 0) atomicAdd(count, c);
-}
-
-template <int NV>    // float4 columns per lane: D <= 128 * NV
-__global__ void __launch_bounds__(kThreadsSS)
-sampled_bce_fwd_kernel(const float* __restrict__ x, int64_t B, int D4, const float* __restrict__ ent, int64_t ld_ent,
-                       int64_t n_ent, const float* __restrict__ bias, const int32_t* __restrict__ cand, int C, int n_pos,
-                       float pos, float add, const int32_t* __restrict__ count, float* __restrict__ g_out,
-                       float* __restrict__ d_x, double* __restrict__ loss_partial) {
-  __shared__ double warp_loss[kWarpsSS];
-  const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5;
-  const int64_t b = (int64_t)blockIdx.x * kWarpsSS + warp;
-  const int n_valid = *count;
-  const float inv_count = n_valid > 0 ? (float)(1.0 / (double)n_valid) : 0.f;
-  double loss = 0.0;                                             // the same value in every lane
-  if (b < B) {
-    const float4 zero = make_float4(0.f, 0.f, 0.f, 0.f);
-    float4 xr[NV], acc[NV];
+// Online softmax: when a batch raises the warp-uniform running max m to m_new, rescale the sum S and the accumulator
+// summed under the old max
+template <int NV>
+__device__ __forceinline__ void raise_max(float m_new, float& m, float& S, float4 (&acc)[NV]) {
+  if (m_new > m) {
+    const float sc = expf(m - m_new);
+    S *= sc;
 #pragma unroll
     for (int v = 0; v < NV; ++v) {
-      const int c4 = lane + 32 * v;
-      xr[v] = c4 < D4 ? ldg4(x + b * 4 * D4 + 4 * c4) : zero;
-      acc[v] = zero;
+      acc[v].x *= sc;
+      acc[v].y *= sc;
+      acc[v].z *= sc;
+      acc[v].w *= sc;
     }
-    const int32_t* cb = cand + b * C;
-    for (int c0 = 0; c0 < C; c0 += kRowsInFlight) {
-      const int32_t mine = (lane < kRowsInFlight && c0 + lane < C) ? cb[c0 + lane] : -1;
-      int32_t e[kRowsInFlight];
-      float4 r[kRowsInFlight][NV];
-      float bi[kRowsInFlight];
+    m = m_new;
+  }
+}
+
+// The forward's operands, the same for the three losses.  counts: what the loss divides by (count_kernel);
+// loss_partial: Loss::kHalves x gridDim.x per-CTA sums.
+struct SampledArgs {
+  const float* x;             // [B, 4 * D4]
+  int64_t B;
+  int D4;
+  const float* ent;           // [n_ent] rows of pitch ld_ent
+  int64_t ld_ent;
+  int64_t n_ent;
+  const float* bias;          // [n_ent]
+  const int32_t* cand;        // [B, C]
+  int C;
+  int n_pos;
+  float pos, add;             // BceLoss, AdvLoss: the labels
+  float alpha;                // AdvLoss: the temperature
+  float eps;                  // CeLoss: the label smoothing
+  int32_t* counts;
+  float* g;                   // [B, C]
+  float* d_x;                 // [B, 4 * D4]
+  double* loss_partial;
+};
+
+// A loss policy supplies, for sampled_fwd_kernel and the launcher:
+//   kHalves      the number of counts and of per-CTA loss sums (1, or 2 for the self-adversarial loss's two halves);
+//   kMinBlocks   the CTAs an SM the forward is compiled for (__launch_bounds__), at NV = 1 and 2: without a bound
+//                ptxas gives the NV = 2 loops 148 to 168 registers (one CTA an SM) and the NV = 1 BCE loop 108 (two);
+//   tally        what count_kernel adds for a query with n_p valid positive and n_q valid negative slots;
+//   State<NV>    the per-query state: batch() takes a batch's logits z and rows and leaves in z the values to park in
+//                g; finish() runs after the query's last row and gives d_x[b] and the query's loss halves.
+
+// Plain BCE: L = mean over the valid slots of ATen's BCE; counts[0] = the valid slots
+struct BceLoss {
+  static constexpr int kHalves = 1, kMinBlocks[2] = {3, 2};   // 80 and 128 registers, no spills
+  __device__ static void tally(int n_p, int n_q, int (&t)[2]) { t[0] += n_p + n_q; }
+
+  template <int NV>
+  struct State {
+    float4 acc[NV];
+    float inv_count;
+    double loss = 0.0;                                           // the same value in every lane
+
+    __device__ explicit State(const SampledArgs& a) {
+      const int n_valid = *a.counts;
+      inv_count = n_valid > 0 ? (float)(1.0 / (double)n_valid) : 0.f;
+#pragma unroll
+      for (int v = 0; v < NV; ++v) acc[v] = make_float4(0.f, 0.f, 0.f, 0.f);
+    }
+
+    __device__ void batch(const SampledArgs& a, int c0, const int32_t (&e)[kRowsInFlight],
+                          const float4 (&r)[kRowsInFlight][NV], float (&z)[kRowsInFlight]) {
 #pragma unroll
       for (int u = 0; u < kRowsInFlight; ++u) {
-        e[u] = __shfl_sync(kFull, mine, u);
-        if (!slot_valid(e[u], n_ent)) e[u] = -1;
-      }
-#pragma unroll
-      for (int u = 0; u < kRowsInFlight; ++u) {                  // every row load of the batch before any is consumed
-#pragma unroll
-        for (int v = 0; v < NV; ++v) {
-          const int c4 = lane + 32 * v;
-          r[u][v] = (e[u] >= 0 && c4 < D4) ? ldg4(ent + (int64_t)e[u] * ld_ent + 4 * c4) : zero;
-        }
-        bi[u] = e[u] >= 0 ? __ldg(bias + e[u]) : 0.f;
-      }
-      float g_mine = 0.f;
-#pragma unroll
-      for (int u = 0; u < kRowsInFlight; ++u) {
-        const float s = warp_dot(xr, r[u]);
-        float g = 0.f;
+        float g = 0.f;                                           // 0 on empty slots
         if (e[u] >= 0) {
-          const float z = s + bi[u];
-          const float p = 1.f / (1.f + expf(-z));                 // the 1-N scorer's epilogue sigmoid
-          const float y = c0 + u < n_pos ? pos : add;
+          const float p = 1.f / (1.f + expf(-z[u]));              // the 1-N scorer's epilogue sigmoid
+          const float y = c0 + u < a.n_pos ? a.pos : a.add;
           loss += (double)bce_loss_term(p, y);
           g = bce_logit_grad(p, y, inv_count);
 #pragma unroll
           for (int v = 0; v < NV; ++v) fma4(g, r[u][v], acc[v]);
         }
-        if (lane == u) g_mine = g;
+        z[u] = g;
       }
-      if (lane < kRowsInFlight && c0 + lane < C) g_out[b * C + c0 + lane] = g_mine;   // 0 on empty slots
     }
+
+    __device__ void finish(const SampledArgs&, const int32_t*, float*, int, float4 (&o)[NV], double (&l)[kHalves]) {
 #pragma unroll
-    for (int v = 0; v < NV; ++v) {
-      const int c4 = lane + 32 * v;
-      if (c4 < D4) *reinterpret_cast<float4*>(d_x + b * 4 * D4 + 4 * c4) = acc[v];
+      for (int v = 0; v < NV; ++v) o[v] = acc[v];
+      l[0] = loss;
     }
-  }
-  const double s = cta_sum(loss, warp_loss, lane, warp);
-  if (threadIdx.x == 0) loss_partial[blockIdx.x] = s;
-}
+  };
+};
 
-// mean over the valid slots: one CTA adds the per-CTA partials in a fixed order (0 when no slot is valid)
-__global__ void __launch_bounds__(kThreadsSS)
-sampled_bce_finalize_kernel(const double* __restrict__ partial, int64_t n_partial, const int32_t* __restrict__ count,
-                            float* __restrict__ loss) {
-  __shared__ double sh[kThreadsSS];
-  const double s = cta_sum_partials(partial, n_partial, sh);
-  if (threadIdx.x == 0) loss[0] = *count > 0 ? (float)(s / (double)*count) : 0.f;
-}
-
-// Self-adversarial variant (RotatE's negative weighting).  Q+ / Q- = the queries with at least one valid positive /
-// negative slot (integer sums: the order of the atomics does not matter).  One warp per query, grid-stride.
-__global__ void __launch_bounds__(kThreadsSS)
-count_adv_kernel(const int32_t* __restrict__ cand, int64_t B, int C, int n_pos, int64_t n_ent, int32_t* __restrict__ counts) {
-  const int lane = threadIdx.x & 31;
-  int qp = 0, qn = 0;
-  for (int64_t b = ((int64_t)blockIdx.x * kThreadsSS + threadIdx.x) >> 5; b < B; b += ((int64_t)gridDim.x * kThreadsSS) >> 5) {
-    bool hp = false, hn = false;
-    for (int c = lane; c < C; c += 32)
-      if (slot_valid(cand[b * C + c], n_ent)) (c < n_pos ? hp : hn) = true;
-    qp += __any_sync(kFull, hp) ? 1 : 0;
-    qn += __any_sync(kFull, hn) ? 1 : 0;
-  }
-  if (lane == 0 && qp != 0) atomicAdd(counts, qp);
-  if (lane == 0 && qn != 0) atomicAdd(counts + 1, qn);
-}
-
-// The loss of sampled_bce_fwd_kernel with the negatives of query b weighted by w = softmax over its valid negative slots
-// of (alpha z) (constants: no gradient through them), the two halves averaged over the queries that have them:
+// Self-adversarial BCE (RotatE's negative weighting): the negatives of query b weighted by w = softmax over its valid
+// negative slots of (alpha z) (constants: no gradient through them), the two halves averaged over the queries that have
+// them:
 //   L = 1/2 (1/Q+) sum_b (1/|P_b|) sum_{P_b} l(z, pos) + 1/2 (1/Q-) sum_b sum_{Q_b} w l(z, add)
-// Same row traffic as sampled_bce_fwd_kernel (every candidate row read once, kRowsInFlight in flight).  The softmax is
-// taken online: a warp-uniform running max m of alpha z, sum S of exp(alpha z - m) and negative d_x accumulator, the
-// latter two rescaled when a batch raises m.  The main loop parks each slot's logit in g; once the query's last row is
-// done one pass over its C slots turns the logits into the final coefficients and the loss terms (recomputed from the
-// parked logit with the same formulas).  d_x = acc_pos / (2 Q+ |P_b|) + acc_neg / (2 Q- S).
-// loss_partial: [gridDim.x] positive-half sums, then [gridDim.x] negative-half sums (per query already divided by
-// |P_b| / S); sampled_adv_finalize_kernel divides by 2 Q+ / 2 Q-.
-template <int NV>    // float4 columns per lane: D <= 128 * NV
-__global__ void __launch_bounds__(kThreadsSS)
-sampled_adv_fwd_kernel(const float* __restrict__ x, int64_t B, int D4, const float* __restrict__ ent, int64_t ld_ent,
-                       int64_t n_ent, const float* __restrict__ bias, const int32_t* __restrict__ cand, int C, int n_pos,
-                       float pos, float add, float alpha, const int32_t* __restrict__ counts, float* g_out,
-                       float* __restrict__ d_x, double* __restrict__ loss_partial) {
-  __shared__ double warp_loss[2][kWarpsSS];
-  const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5;
-  const int64_t b = (int64_t)blockIdx.x * kWarpsSS + warp;
-  const int q_pos = counts[0], q_neg = counts[1];
-  double loss_p = 0.0, loss_n = 0.0;                             // this query's two halves, the same value in every lane
-  if (b < B) {
-    const float4 zero = make_float4(0.f, 0.f, 0.f, 0.f);
-    float4 xr[NV], acc_p[NV], acc_n[NV];
-#pragma unroll
-    for (int v = 0; v < NV; ++v) {
-      const int c4 = lane + 32 * v;
-      xr[v] = c4 < D4 ? ldg4(x + b * 4 * D4 + 4 * c4) : zero;
-      acc_p[v] = zero;
-      acc_n[v] = zero;
-    }
-    const int32_t* cb = cand + b * C;
-    float* gb = g_out + b * C;
+// counts = Q+, Q- (the queries with at least one valid positive / negative slot).  The softmax is taken online: a
+// warp-uniform running max m of alpha z, sum S of exp(alpha z - m) and negative d_x accumulator.  The logits are parked
+// in g; after the query's last row one pass over its C slots turns them into the final coefficients and the loss terms
+// (recomputed from the parked logit with the same formulas).  d_x = acc_pos / (2 Q+ |P_b|) + acc_neg / (2 Q- S).  The
+// loss halves are per query already divided by |P_b| / S; sampled_finalize_kernel divides by 2 Q+ / 2 Q-.
+struct AdvLoss {
+  static constexpr int kHalves = 2, kMinBlocks[2] = {2, 2};
+  __device__ static void tally(int n_p, int n_q, int (&t)[2]) {
+    t[0] += n_p > 0 ? 1 : 0;
+    t[1] += n_q > 0 ? 1 : 0;
+  }
+
+  template <int NV>
+  struct State {
+    float4 acc_p[NV], acc_n[NV];
     float m = -INFINITY, S = 0.f;                                // warp-uniform running max of alpha z and sum
     int n_p = 0;                                                 // |P_b|
-    for (int c0 = 0; c0 < C; c0 += kRowsInFlight) {
-      const int32_t mine = (lane < kRowsInFlight && c0 + lane < C) ? cb[c0 + lane] : -1;
-      int32_t e[kRowsInFlight];
-      float4 r[kRowsInFlight][NV];
-      float bi[kRowsInFlight];
+
+    __device__ explicit State(const SampledArgs&) {
 #pragma unroll
-      for (int u = 0; u < kRowsInFlight; ++u) {
-        e[u] = __shfl_sync(kFull, mine, u);
-        if (!slot_valid(e[u], n_ent)) e[u] = -1;
-      }
-#pragma unroll
-      for (int u = 0; u < kRowsInFlight; ++u) {                  // every row load of the batch before any is consumed
-#pragma unroll
-        for (int v = 0; v < NV; ++v) {
-          const int c4 = lane + 32 * v;
-          r[u][v] = (e[u] >= 0 && c4 < D4) ? ldg4(ent + (int64_t)e[u] * ld_ent + 4 * c4) : zero;
-        }
-        bi[u] = e[u] >= 0 ? __ldg(bias + e[u]) : 0.f;
-      }
-      float z[kRowsInFlight];
+      for (int v = 0; v < NV; ++v) acc_p[v] = acc_n[v] = make_float4(0.f, 0.f, 0.f, 0.f);
+    }
+
+    __device__ void batch(const SampledArgs& a, int c0, const int32_t (&e)[kRowsInFlight],
+                          const float4 (&r)[kRowsInFlight][NV], float (&z)[kRowsInFlight]) {
       float m_new = m;
 #pragma unroll
-      for (int u = 0; u < kRowsInFlight; ++u) {
-        z[u] = warp_dot(xr, r[u]) + bi[u];
-        if (e[u] >= 0 && c0 + u >= n_pos) m_new = fmaxf(m_new, alpha * z[u]);
-      }
-      if (m_new > m) {                                           // rescale what was summed under the old max
-        const float sc = expf(m - m_new);
-        S *= sc;
-#pragma unroll
-        for (int v = 0; v < NV; ++v) {
-          acc_n[v].x *= sc;
-          acc_n[v].y *= sc;
-          acc_n[v].z *= sc;
-          acc_n[v].w *= sc;
-        }
-        m = m_new;
-      }
-      float z_mine = 0.f;
+      for (int u = 0; u < kRowsInFlight; ++u)
+        if (e[u] >= 0 && c0 + u >= a.n_pos) m_new = fmaxf(m_new, a.alpha * z[u]);
+      raise_max(m_new, m, S, acc_n);
 #pragma unroll
       for (int u = 0; u < kRowsInFlight; ++u) {
         if (e[u] >= 0) {
           const float p = 1.f / (1.f + expf(-z[u]));
-          if (c0 + u < n_pos) {
+          if (c0 + u < a.n_pos) {
             ++n_p;
 #pragma unroll
-            for (int v = 0; v < NV; ++v) fma4(bce_logit_grad(p, pos, 1.f), r[u][v], acc_p[v]);
+            for (int v = 0; v < NV; ++v) fma4(bce_logit_grad(p, a.pos, 1.f), r[u][v], acc_p[v]);
           } else {
-            const float w = expf(alpha * z[u] - m);
+            const float w = expf(a.alpha * z[u] - m);
             S += w;
 #pragma unroll
-            for (int v = 0; v < NV; ++v) fma4(bce_logit_grad(p, add, w), r[u][v], acc_n[v]);
+            for (int v = 0; v < NV; ++v) fma4(bce_logit_grad(p, a.add, w), r[u][v], acc_n[v]);
           }
         }
-        if (lane == u) z_mine = z[u];
       }
-      if (lane < kRowsInFlight && c0 + lane < C) gb[c0 + lane] = z_mine;
     }
-    __syncwarp();                                                // the parked logits are visible to every lane
-    const float cp = n_p > 0 ? (float)(1.0 / (2.0 * (double)q_pos * (double)n_p)) : 0.f;
-    const float cn = S > 0.f ? (float)(1.0 / (2.0 * (double)q_neg * (double)S)) : 0.f;
-    double lp = 0.0, ln = 0.0;
-    for (int c = lane; c < C; c += 32) {
-      float gv = 0.f;                                            // 0 on empty slots
-      if (slot_valid(cb[c], n_ent)) {
-        const float zc = gb[c];
-        const float p = 1.f / (1.f + expf(-zc));
-        const float y = c < n_pos ? pos : add;
-        const float term = bce_loss_term(p, y);
-        if (c < n_pos) {
-          lp += (double)term;
-          gv = bce_logit_grad(p, y, cp);
-        } else {
-          const float w = expf(alpha * zc - m);
-          ln += (double)w * (double)term;
-          gv = bce_logit_grad(p, y, w * cn);
+
+    __device__ void finish(const SampledArgs& a, const int32_t* cb, float* gb, int lane, float4 (&o)[NV],
+                           double (&l)[kHalves]) {
+      __syncwarp();                                              // the parked logits are visible to every lane
+      const int q_pos = a.counts[0], q_neg = a.counts[1];
+      const float cp = n_p > 0 ? (float)(1.0 / (2.0 * (double)q_pos * (double)n_p)) : 0.f;
+      const float cn = S > 0.f ? (float)(1.0 / (2.0 * (double)q_neg * (double)S)) : 0.f;
+      double lp = 0.0, ln = 0.0;
+      for (int c = lane; c < a.C; c += 32) {
+        float gv = 0.f;                                          // 0 on empty slots
+        if (slot_valid(cb[c], a.n_ent)) {
+          const float zc = gb[c];
+          const float p = 1.f / (1.f + expf(-zc));
+          const float y = c < a.n_pos ? a.pos : a.add;
+          const float term = bce_loss_term(p, y);
+          if (c < a.n_pos) {
+            lp += (double)term;
+            gv = bce_logit_grad(p, y, cp);
+          } else {
+            const float w = expf(a.alpha * zc - m);
+            ln += (double)w * (double)term;
+            gv = bce_logit_grad(p, y, w * cn);
+          }
         }
+        gb[c] = gv;
       }
-      gb[c] = gv;
-    }
-    lp = warp_sum(lp);
-    ln = warp_sum(ln);
-    loss_p = n_p > 0 ? lp / (double)n_p : 0.0;
-    loss_n = S > 0.f ? ln / (double)S : 0.0;
+      lp = warp_sum(lp);
+      ln = warp_sum(ln);
+      l[0] = n_p > 0 ? lp / (double)n_p : 0.0;
+      l[1] = S > 0.f ? ln / (double)S : 0.0;
 #pragma unroll
-    for (int v = 0; v < NV; ++v) {
-      const int c4 = lane + 32 * v;
-      if (c4 < D4) {
-        const float4 o = make_float4(fmaf(cn, acc_n[v].x, cp * acc_p[v].x), fmaf(cn, acc_n[v].y, cp * acc_p[v].y),
-                                     fmaf(cn, acc_n[v].z, cp * acc_p[v].z), fmaf(cn, acc_n[v].w, cp * acc_p[v].w));
-        *reinterpret_cast<float4*>(d_x + b * 4 * D4 + 4 * c4) = o;
-      }
+      for (int v = 0; v < NV; ++v)
+        o[v] = make_float4(fmaf(cn, acc_n[v].x, cp * acc_p[v].x), fmaf(cn, acc_n[v].y, cp * acc_p[v].y),
+                           fmaf(cn, acc_n[v].z, cp * acc_p[v].z), fmaf(cn, acc_n[v].w, cp * acc_p[v].w));
     }
-  }
-  const double sp = cta_sum(loss_p, warp_loss[0], lane, warp);
-  const double sn = cta_sum(loss_n, warp_loss[1], lane, warp);
-  if (threadIdx.x == 0) {
-    loss_partial[blockIdx.x] = sp;
-    loss_partial[gridDim.x + blockIdx.x] = sn;
-  }
-}
+  };
+};
 
-// L = sum_pos / (2 Q+) + sum_neg / (2 Q-): each half's per-CTA partials added by one CTA in a fixed order (a half whose
-// count is 0 adds 0)
-__global__ void __launch_bounds__(kThreadsSS)
-sampled_adv_finalize_kernel(const double* __restrict__ partial, int64_t n_partial, const int32_t* __restrict__ counts,
-                            float* __restrict__ loss) {
-  __shared__ double sh[2][kThreadsSS];
-  const double sp = cta_sum_partials(partial, n_partial, sh[0]);
-  const double sn = cta_sum_partials(partial + n_partial, n_partial, sh[1]);
-  if (threadIdx.x == 0) {
-    const double lp = counts[0] > 0 ? sp / (2.0 * (double)counts[0]) : 0.0;
-    const double ln = counts[1] > 0 ? sn / (2.0 * (double)counts[1]) : 0.0;
-    loss[0] = (float)(lp + ln);
-  }
-}
-
-// Softmax cross-entropy variant.  P = the number of valid positive slots (integer sum: the order of the atomics does not
-// matter); slot i of the grid-stride walk is column i % n_pos of query i / n_pos.
-__global__ void __launch_bounds__(kThreadsSS)
-count_pos_kernel(const int32_t* __restrict__ cand, int64_t B, int C, int n_pos, int64_t n_ent, int32_t* __restrict__ count) {
-  int c = 0;
-  for (int64_t i = (int64_t)blockIdx.x * kThreadsSS + threadIdx.x; i < B * n_pos; i += (int64_t)gridDim.x * kThreadsSS)
-    c += slot_valid(cand[(i / n_pos) * C + i % n_pos], n_ent) ? 1 : 0;
-#pragma unroll
-  for (int o = 16; o > 0; o >>= 1) c += __shfl_xor_sync(kFull, c, o);
-  if ((threadIdx.x & 31) == 0 && c != 0) atomicAdd(count, c);
-}
-
-// Each valid positive slot p of query b against the valid negative slots Q_b of that query, K_b = 1 + |Q_b| classes
-// (other positives are not in p's denominator):
+// Softmax cross-entropy: each valid positive slot p of query b against the valid negative slots Q_b of that query,
+// K_b = 1 + |Q_b| classes (other positives are not in p's denominator):
 //   l_p = (1 - eps) (LSE_p - z_p) + eps (LSE_p - (z_p + sum_{Q_b} z_q) / K_b),  LSE_p = log(e^{z_p} + sum_{Q_b} e^{z_q})
-// and L = (1 / P) sum l_p.  Same row traffic as sampled_adv_fwd_kernel for the negatives (each read once, kRowsInFlight in
-// flight): a warp-uniform running max m over the negative logits, S = sum e^{z_q - m} and acc_w = sum e^{z_q - m} E[q],
-// the latter two rescaled when a batch raises m; with eps > 0 also the plain sum acc_1 = sum E[q].  The main loop parks
-// each slot's logit in g.  After the query's last row a pass over its negative slots gives |Q_b| and Z = sum z_q from the
-// parked logits, and one over its positive slots gives, from the final S, the negatives' softmax mass under p,
-// 1 - softmax_p(p), the loss term and r_p = softmax_p(q) e^{m - z_q} (the same for every q), all against max(m, z_p) so
-// that no exponent is positive; then
+// and L = (1 / P) sum l_p, counts[0] = P the valid positive slots.  Online over the negatives: a warp-uniform running
+// max m over their logits, S = sum e^{z_q - m} and acc_w = sum e^{z_q - m} E[q]; with eps > 0 also the plain sum
+// acc_1 = sum E[q].  The logits are parked in g.  After the query's last row a pass over its negative slots gives |Q_b|
+// and Z = sum z_q from the parked logits, and one over its positive slots gives, from the final S, the negatives'
+// softmax mass under p, 1 - softmax_p(p), the loss term and r_p = softmax_p(q) e^{m - z_q} (the same for every q), all
+// against max(m, z_p) so that no exponent is positive; then
 //   g_p = (eps |Q_b| / K_b - (1 - softmax_p(p))) / P,   g_q = (e^{z_q - m} R - |P_b| eps / K_b) / P,  R = sum_{P_b} r_p
 // and d_x = (R acc_w - |P_b| eps / K_b acc_1) / P + sum_{P_b} g_p E[p]: the positive rows (n_pos of the C) are read a
 // second time.  A positive without a valid negative has softmax_p(p) = 1 and |Q_b| = 0, so 0 loss and 0 gradient; a
-// query without a valid positive has R = |P_b| = 0.  loss_partial: [gridDim.x] per-CTA sums of l_p; the division by P
-// is sampled_bce_finalize_kernel's.
-// (two CTAs an SM: ptxas then keeps NV = 1 at 109 registers without spills instead of squeezing it into the 80 of three
-// CTAs with a spilled row offset)
-template <int NV>    // float4 columns per lane: D <= 128 * NV
-__global__ void __launch_bounds__(kThreadsSS, 2)
-sampled_ce_fwd_kernel(const float* __restrict__ x, int64_t B, int D4, const float* __restrict__ ent, int64_t ld_ent,
-                      int64_t n_ent, const float* __restrict__ bias, const int32_t* __restrict__ cand, int C, int n_pos,
-                      float eps, const int32_t* __restrict__ count, float* g_out, float* __restrict__ d_x,
-                      double* __restrict__ loss_partial) {
-  __shared__ double warp_loss[kWarpsSS];
+// query without a valid positive has R = |P_b| = 0.  (Two CTAs an SM at NV = 1 too: in the 80 registers of three ptxas
+// spills a row offset.)
+struct CeLoss {
+  static constexpr int kHalves = 1, kMinBlocks[2] = {2, 2};
+  __device__ static void tally(int n_p, int, int (&t)[2]) { t[0] += n_p; }
+
+  template <int NV>
+  struct State {
+    float4 acc_w[NV], acc_1[NV];
+    float m = -INFINITY, S = 0.f;                                // warp-uniform
+
+    __device__ explicit State(const SampledArgs&) {
+#pragma unroll
+      for (int v = 0; v < NV; ++v) acc_w[v] = acc_1[v] = make_float4(0.f, 0.f, 0.f, 0.f);
+    }
+
+    __device__ void batch(const SampledArgs& a, int c0, const int32_t (&e)[kRowsInFlight],
+                          const float4 (&r)[kRowsInFlight][NV], float (&z)[kRowsInFlight]) {
+      float m_new = m;
+#pragma unroll
+      for (int u = 0; u < kRowsInFlight; ++u)
+        if (e[u] >= 0 && c0 + u >= a.n_pos) m_new = fmaxf(m_new, z[u]);
+      raise_max(m_new, m, S, acc_w);
+#pragma unroll
+      for (int u = 0; u < kRowsInFlight; ++u) {
+        if (e[u] >= 0 && c0 + u >= a.n_pos) {
+          const float w = expf(z[u] - m);
+          S += w;
+#pragma unroll
+          for (int v = 0; v < NV; ++v) fma4(w, r[u][v], acc_w[v]);
+          if (a.eps > 0.f) {
+#pragma unroll
+            for (int v = 0; v < NV; ++v) fma4(1.f, r[u][v], acc_1[v]);
+          }
+        }
+      }
+    }
+
+    __device__ void finish(const SampledArgs& a, const int32_t* cb, float* gb, int lane, float4 (&o)[NV],
+                           double (&l)[kHalves]) {
+      __syncwarp();                                              // the parked logits are visible to every lane
+      const float eps = a.eps;
+      int n_q = 0;                                               // |Q_b| and the sum Z of its logits, from the parked ones
+      double Z = 0.0;
+      for (int c = a.n_pos + lane; c < a.C; c += 32) {
+        if (slot_valid(cb[c], a.n_ent)) {
+          ++n_q;
+          Z += (double)gb[c];
+        }
+      }
+      n_q = __reduce_add_sync(kFull, n_q);
+      Z = warp_sum(Z);
+      const int n_valid = *a.counts;                             // read here: one register less across the row loop
+      const float inv_p = n_valid > 0 ? (float)(1.0 / (double)n_valid) : 0.f;
+      const float inv_k = 1.f / (float)(1 + n_q);
+      const float eps_pos = eps * (float)n_q * inv_k;            // eps (1 - 1 / K_b)
+      float R = 0.f;
+      double lsum = 0.0;
+      int n_p = 0;                                               // |P_b|
+      for (int c = lane; c < a.n_pos; c += 32) {
+        float gv = 0.f;                                          // 0 on empty slots
+        if (slot_valid(cb[c], a.n_ent)) {
+          const float zp = gb[c];
+          float q_mass, rp, lse_z;                               // 1 - softmax_p(p), r_p, LSE_p - z_p
+          if (zp >= m) {                                         // also every positive of a query without negatives
+            const float em = expf(m - zp);
+            const float t = S * em;
+            q_mass = t / (1.f + t);
+            rp = em / (1.f + t);
+            lse_z = log1pf(t);
+          } else {
+            const float ep = expf(zp - m);
+            q_mass = S / (ep + S);
+            rp = 1.f / (ep + S);
+            lse_z = (m - zp) + logf(ep + S);
+          }
+          ++n_p;
+          R += rp;
+          lsum += (double)lse_z + (double)eps * ((double)n_q * (double)zp - Z) / (double)(1 + n_q);
+          gv = (eps_pos - q_mass) * inv_p;
+        }
+        gb[c] = gv;
+      }
+      R = (float)warp_sum((double)R);
+      l[0] = warp_sum(lsum);
+      n_p = __reduce_add_sync(kFull, n_p);
+      const float eps_neg = (float)n_p * eps * inv_k;            // |P_b| eps / K_b
+      for (int c = a.n_pos + lane; c < a.C; c += 32) {
+        float gv = 0.f;
+        if (slot_valid(cb[c], a.n_ent)) gv = (expf(gb[c] - m) * R - eps_neg) * inv_p;
+        gb[c] = gv;
+      }
+      const float cw = R * inv_p, c1 = -eps_neg * inv_p;
+#pragma unroll
+      for (int v = 0; v < NV; ++v)
+        o[v] = make_float4(fmaf(cw, acc_w[v].x, c1 * acc_1[v].x), fmaf(cw, acc_w[v].y, c1 * acc_1[v].y),
+                           fmaf(cw, acc_w[v].z, c1 * acc_1[v].z), fmaf(cw, acc_w[v].w, c1 * acc_1[v].w));
+      __syncwarp();                                              // the positives' final g is visible to every lane
+      for (int c = 0; c < a.n_pos; ++c) {                        // the positive rows again, in slot order
+        const int32_t ep = cb[c];
+        if (!slot_valid(ep, a.n_ent)) continue;
+        const float gp = gb[c];
+#pragma unroll
+        for (int v = 0; v < NV; ++v) {
+          const int c4 = lane + 32 * v;
+          if (c4 < a.D4) fma4(gp, ldg4(a.ent + (int64_t)ep * a.ld_ent + 4 * c4), o[v]);
+        }
+      }
+    }
+  };
+};
+
+// |P_b| and |Q_b|, query b's valid positive and negative slots (one warp per query, grid-stride), added into the counts
+// the loss divides by (integer sums: the order of the atomics does not matter)
+template <class Loss>
+__global__ void __launch_bounds__(kThreadsSS)
+count_kernel(const int32_t* __restrict__ cand, int64_t B, int C, int n_pos, int64_t n_ent, int32_t* __restrict__ counts) {
+  const int lane = threadIdx.x & 31;
+  int t[2] = {0, 0};
+  for (int64_t b = ((int64_t)blockIdx.x * kThreadsSS + threadIdx.x) >> 5; b < B; b += ((int64_t)gridDim.x * kThreadsSS) >> 5) {
+    int n_p = 0, n_q = 0;
+    for (int c = lane; c < C; c += 32)
+      if (slot_valid(cand[b * C + c], n_ent)) ++(c < n_pos ? n_p : n_q);
+    Loss::tally(__reduce_add_sync(kFull, n_p), __reduce_add_sync(kFull, n_q), t);
+  }
+#pragma unroll
+  for (int h = 0; h < Loss::kHalves; ++h)
+    if (lane == 0 && t[h] != 0) atomicAdd(counts + h, t[h]);
+}
+
+// One warp per query b: the x row, the candidate loop (a batch of kRowsInFlight ids, their rows and biases loaded before
+// any is consumed, the logits, the Loss's batch step, the values it parks stored to g), the Loss's finish, d_x[b], and
+// the CTA's loss partials (Loss::kHalves sums, each in warp order).
+template <class Loss, int NV>    // float4 columns per lane: D <= 128 * NV
+__global__ void __launch_bounds__(kThreadsSS, Loss::kMinBlocks[NV - 1])
+sampled_fwd_kernel(const SampledArgs a) {
+  constexpr int H = Loss::kHalves;
+  __shared__ double warp_loss[H][kWarpsSS];
   const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5;
   const int64_t b = (int64_t)blockIdx.x * kWarpsSS + warp;
-  double loss = 0.0;                                             // this query's sum of l_p, the same value in every lane
-  if (b < B) {
+  double loss[H] = {};                                           // this query's loss halves, the same value in every lane
+  if (b < a.B) {
+    const int D4 = a.D4;
     const float4 zero = make_float4(0.f, 0.f, 0.f, 0.f);
-    float4 xr[NV], acc_w[NV], acc_1[NV];
+    float4 xr[NV];
 #pragma unroll
     for (int v = 0; v < NV; ++v) {
       const int c4 = lane + 32 * v;
-      xr[v] = c4 < D4 ? ldg4(x + b * 4 * D4 + 4 * c4) : zero;
-      acc_w[v] = zero;
-      acc_1[v] = zero;
+      xr[v] = c4 < D4 ? ldg4(a.x + b * 4 * D4 + 4 * c4) : zero;
     }
-    const int32_t* cb = cand + b * C;
-    float* gb = g_out + b * C;
-    float m = -INFINITY, S = 0.f;                                // warp-uniform
-    for (int c0 = 0; c0 < C; c0 += kRowsInFlight) {
-      const int32_t mine = (lane < kRowsInFlight && c0 + lane < C) ? cb[c0 + lane] : -1;
+    typename Loss::template State<NV> st(a);
+    const int32_t* cb = a.cand + b * a.C;
+    float* gb = a.g + b * a.C;
+    for (int c0 = 0; c0 < a.C; c0 += kRowsInFlight) {
+      const int32_t mine = (lane < kRowsInFlight && c0 + lane < a.C) ? cb[c0 + lane] : -1;
       int32_t e[kRowsInFlight];
       float4 r[kRowsInFlight][NV];
       float bi[kRowsInFlight];
 #pragma unroll
       for (int u = 0; u < kRowsInFlight; ++u) {
         e[u] = __shfl_sync(kFull, mine, u);
-        if (!slot_valid(e[u], n_ent)) e[u] = -1;
+        if (!slot_valid(e[u], a.n_ent)) e[u] = -1;
       }
 #pragma unroll
       for (int u = 0; u < kRowsInFlight; ++u) {                  // every row load of the batch before any is consumed
 #pragma unroll
         for (int v = 0; v < NV; ++v) {
           const int c4 = lane + 32 * v;
-          r[u][v] = (e[u] >= 0 && c4 < D4) ? ldg4(ent + (int64_t)e[u] * ld_ent + 4 * c4) : zero;
+          r[u][v] = (e[u] >= 0 && c4 < D4) ? ldg4(a.ent + (int64_t)e[u] * a.ld_ent + 4 * c4) : zero;
         }
-        bi[u] = e[u] >= 0 ? __ldg(bias + e[u]) : 0.f;
+        bi[u] = e[u] >= 0 ? __ldg(a.bias + e[u]) : 0.f;
       }
       float z[kRowsInFlight];
-      float m_new = m;
 #pragma unroll
-      for (int u = 0; u < kRowsInFlight; ++u) {
-        z[u] = warp_dot(xr, r[u]) + bi[u];
-        if (e[u] >= 0 && c0 + u >= n_pos) m_new = fmaxf(m_new, z[u]);
-      }
-      if (m_new > m) {                                           // rescale what was summed under the old max
-        const float sc = expf(m - m_new);
-        S *= sc;
+      for (int u = 0; u < kRowsInFlight; ++u) z[u] = warp_dot(xr, r[u]) + bi[u];
+      st.batch(a, c0, e, r, z);
+      float park = 0.f;
 #pragma unroll
-        for (int v = 0; v < NV; ++v) {
-          acc_w[v].x *= sc;
-          acc_w[v].y *= sc;
-          acc_w[v].z *= sc;
-          acc_w[v].w *= sc;
-        }
-        m = m_new;
-      }
-      float z_mine = 0.f;
-#pragma unroll
-      for (int u = 0; u < kRowsInFlight; ++u) {
-        if (e[u] >= 0) {
-          if (c0 + u >= n_pos) {
-            const float w = expf(z[u] - m);
-            S += w;
-#pragma unroll
-            for (int v = 0; v < NV; ++v) fma4(w, r[u][v], acc_w[v]);
-            if (eps > 0.f) {
-#pragma unroll
-              for (int v = 0; v < NV; ++v) fma4(1.f, r[u][v], acc_1[v]);
-            }
-          }
-        }
-        if (lane == u) z_mine = z[u];
-      }
-      if (lane < kRowsInFlight && c0 + lane < C) gb[c0 + lane] = z_mine;
+      for (int u = 0; u < kRowsInFlight; ++u)
+        if (lane == u) park = z[u];
+      if (lane < kRowsInFlight && c0 + lane < a.C) gb[c0 + lane] = park;
     }
-    __syncwarp();                                                // the parked logits are visible to every lane
-    int n_q = 0;                                                 // |Q_b| and the sum Z of its logits, from the parked ones
-    double Z = 0.0;
-    for (int c = n_pos + lane; c < C; c += 32) {
-      if (slot_valid(cb[c], n_ent)) {
-        ++n_q;
-        Z += (double)gb[c];
-      }
-    }
-    n_q = __reduce_add_sync(kFull, n_q);
-    Z = warp_sum(Z);
-    const int n_valid = *count;                                  // read here: one register less across the row loop
-    const float inv_p = n_valid > 0 ? (float)(1.0 / (double)n_valid) : 0.f;
-    const float inv_k = 1.f / (float)(1 + n_q);
-    const float eps_pos = eps * (float)n_q * inv_k;              // eps (1 - 1 / K_b)
-    float R = 0.f;
-    double l = 0.0;
-    int n_p = 0;                                                 // |P_b|
-    for (int c = lane; c < n_pos; c += 32) {
-      float gv = 0.f;                                            // 0 on empty slots
-      if (slot_valid(cb[c], n_ent)) {
-        const float zp = gb[c];
-        float q_mass, rp, lse_z;                                 // 1 - softmax_p(p), r_p, LSE_p - z_p
-        if (zp >= m) {                                           // also every positive of a query without negatives
-          const float em = expf(m - zp);
-          const float t = S * em;
-          q_mass = t / (1.f + t);
-          rp = em / (1.f + t);
-          lse_z = log1pf(t);
-        } else {
-          const float ep = expf(zp - m);
-          q_mass = S / (ep + S);
-          rp = 1.f / (ep + S);
-          lse_z = (m - zp) + logf(ep + S);
-        }
-        ++n_p;
-        R += rp;
-        l += (double)lse_z + (double)eps * ((double)n_q * (double)zp - Z) / (double)(1 + n_q);
-        gv = (eps_pos - q_mass) * inv_p;
-      }
-      gb[c] = gv;
-    }
-    R = (float)warp_sum((double)R);
-    loss = warp_sum(l);
-    n_p = __reduce_add_sync(kFull, n_p);
-    const float eps_neg = (float)n_p * eps * inv_k;              // |P_b| eps / K_b
-    for (int c = n_pos + lane; c < C; c += 32) {
-      float gv = 0.f;
-      if (slot_valid(cb[c], n_ent)) gv = (expf(gb[c] - m) * R - eps_neg) * inv_p;
-      gb[c] = gv;
-    }
-    const float cw = R * inv_p, c1 = -eps_neg * inv_p;
     float4 o[NV];
-#pragma unroll
-    for (int v = 0; v < NV; ++v)
-      o[v] = make_float4(fmaf(cw, acc_w[v].x, c1 * acc_1[v].x), fmaf(cw, acc_w[v].y, c1 * acc_1[v].y),
-                         fmaf(cw, acc_w[v].z, c1 * acc_1[v].z), fmaf(cw, acc_w[v].w, c1 * acc_1[v].w));
-    __syncwarp();                                                // the positives' final g is visible to every lane
-    for (int c = 0; c < n_pos; ++c) {                            // the positive rows again, in slot order
-      const int32_t ep = cb[c];
-      if (!slot_valid(ep, n_ent)) continue;
-      const float gp = gb[c];
-#pragma unroll
-      for (int v = 0; v < NV; ++v) {
-        const int c4 = lane + 32 * v;
-        if (c4 < D4) fma4(gp, ldg4(ent + (int64_t)ep * ld_ent + 4 * c4), o[v]);
-      }
-    }
+    st.finish(a, cb, gb, lane, o, loss);
 #pragma unroll
     for (int v = 0; v < NV; ++v) {
       const int c4 = lane + 32 * v;
-      if (c4 < D4) *reinterpret_cast<float4*>(d_x + b * 4 * D4 + 4 * c4) = o[v];
+      if (c4 < D4) *reinterpret_cast<float4*>(a.d_x + b * 4 * D4 + 4 * c4) = o[v];
     }
   }
-  const double s = cta_sum(loss, warp_loss, lane, warp);
-  if (threadIdx.x == 0) loss_partial[blockIdx.x] = s;
+  double s[H];
+#pragma unroll
+  for (int h = 0; h < H; ++h) s[h] = cta_sum(loss[h], warp_loss[h], lane, warp);
+  if (threadIdx.x == 0) {
+#pragma unroll
+    for (int h = 0; h < H; ++h) a.loss_partial[h * gridDim.x + blockIdx.x] = s[h];
+  }
+}
+
+// The loss from the per-CTA partials, each half added by one CTA in a fixed order; a zero count gives 0.
+//   one half: sum / counts[0];   two halves (self-adversarial): sum_pos / (2 Q+) + sum_neg / (2 Q-)
+template <int H>
+__global__ void __launch_bounds__(kThreadsSS)
+sampled_finalize_kernel(const double* __restrict__ partial, int64_t n_partial, const int32_t* __restrict__ counts,
+                        float* __restrict__ loss) {
+  __shared__ double sh[H][kThreadsSS];
+  double s[H];
+#pragma unroll
+  for (int h = 0; h < H; ++h) s[h] = cta_sum_partials(partial + h * n_partial, n_partial, sh[h]);
+  if (threadIdx.x == 0) {
+    if constexpr (H == 1) {
+      loss[0] = counts[0] > 0 ? (float)(s[0] / (double)counts[0]) : 0.f;
+    } else {
+      const double lp = counts[0] > 0 ? s[0] / (2.0 * (double)counts[0]) : 0.0;
+      const double ln = counts[1] > 0 ? s[1] / (2.0 * (double)counts[1]) : 0.0;
+      loss[0] = (float)(lp + ln);
+    }
+  }
 }
 
 // sort keys: the entity, or N for an empty slot (sorts after every entity); values: the slot
@@ -588,6 +555,7 @@ table_grad_kernel(const int32_t* __restrict__ keys, const int32_t* __restrict__ 
   }
 }
 
+
 size_t align_up(size_t v) { return (v + 255) / 256 * 256; }
 
 int key_bits(int64_t n_ent) {        // bits that hold 0 .. n_ent (the empty-slot key)
@@ -606,15 +574,13 @@ bool shapes_ok(int64_t B, int32_t D, int32_t C, int64_t n_ent) {
          B * (int64_t)C < (int64_t{1} << 31);
 }
 
-// the requirements kgc_sampled_bce_fwd and kgc_sampled_adv_fwd share: the failed one's message, or nullptr
-const char* check_fwd_args(const float* x, int64_t B, int32_t D, const float* ent, int64_t n_ent, int64_t ld_ent,
-                           const float* bias, const int32_t* cand, int32_t C, int32_t n_pos, const float* g, const float* d_x,
-                           const int32_t* counts, const double* loss_partial, const float* loss) {
-  if (!shapes_ok(B, D, C, n_ent)) return "bad sizes (B, C > 0, B * C < 2^31, 0 < D <= 256, D % 4 == 0, 0 < N < 2^31 - 1)";
-  if (n_pos < 0 || n_pos > C) return "n_pos must lie in [0, C]";
-  if (ld_ent < D || ld_ent % 4 != 0) return "entity rows need ld_ent >= D and a 16-byte pitch";
-  if (!(x && ent && bias && cand && g && d_x && counts && loss_partial && loss)) return "null buffer";
-  if (((reinterpret_cast<uintptr_t>(x) | reinterpret_cast<uintptr_t>(ent) | reinterpret_cast<uintptr_t>(d_x)) & 15) != 0)
+// the requirements the three sampled forwards share: the failed one's message, or nullptr
+const char* check_fwd_args(const SampledArgs& a, int32_t D, const float* loss) {
+  if (!shapes_ok(a.B, D, a.C, a.n_ent)) return "bad sizes (B, C > 0, B * C < 2^31, 0 < D <= 256, D % 4 == 0, 0 < N < 2^31 - 1)";
+  if (a.n_pos < 0 || a.n_pos > a.C) return "n_pos must lie in [0, C]";
+  if (a.ld_ent < D || a.ld_ent % 4 != 0) return "entity rows need ld_ent >= D and a 16-byte pitch";
+  if (!(a.x && a.ent && a.bias && a.cand && a.g && a.d_x && a.counts && a.loss_partial && loss)) return "null buffer";
+  if (((reinterpret_cast<uintptr_t>(a.x) | reinterpret_cast<uintptr_t>(a.ent) | reinterpret_cast<uintptr_t>(a.d_x)) & 15) != 0)
     return "x, all_ent and d_x must be 16-byte aligned";
   return nullptr;
 }
@@ -622,6 +588,23 @@ const char* check_fwd_args(const float* x, int64_t B, int32_t D, const float* en
 // the instantiation of a row kernel for D = 4 * D4: one float4 column per lane up to D = 128, two up to 256
 template <typename Kernel>
 Kernel for_width(int D4, Kernel nv1, Kernel nv2) { return D4 <= 32 ? nv1 : nv2; }
+
+// the sampled forward of one loss: zero its counts, count them, one pass over the rows, the loss from the partials
+template <class Loss>
+cudaError_t launch_sampled_fwd(const SampledArgs& a, float* loss, cudaStream_t s) {
+  cudaError_t err = cudaMemsetAsync(a.counts, 0, Loss::kHalves * sizeof(int32_t), s);
+  if (err != cudaSuccess) return err;
+  const int64_t blocks = kgc_sampled_bce_fwd_blocks(a.B);
+  const int64_t cblocks = blocks < 4 * kNumSMs ? blocks : 4 * kNumSMs;
+  count_kernel<Loss><<<(unsigned)cblocks, kThreadsSS, 0, s>>>(a.cand, a.B, a.C, a.n_pos, a.n_ent,
+                                                              a.counts);
+  if ((err = cudaGetLastError()) != cudaSuccess) return err;
+  const auto fwd = for_width(a.D4, sampled_fwd_kernel<Loss, 1>, sampled_fwd_kernel<Loss, 2>);
+  fwd<<<(unsigned)blocks, kThreadsSS, 0, s>>>(a);
+  if ((err = cudaGetLastError()) != cudaSuccess) return err;
+  sampled_finalize_kernel<Loss::kHalves><<<1, kThreadsSS, 0, s>>>(a.loss_partial, blocks, a.counts, loss);
+  return cudaGetLastError();
+}
 
 }  // namespace
 }  // namespace kgc
@@ -633,22 +616,9 @@ extern "C" int64_t kgc_sampled_bce_fwd_blocks(int64_t B) { return ceil_div(B > 0
 extern "C" int kgc_sampled_bce_fwd(const float* x, int64_t B, int32_t D, const float* ent, int64_t n_ent, int64_t ld_ent,
                                    const float* bias, const int32_t* cand, int32_t C, int32_t n_pos, float pos, float add,
                                    float* g, float* d_x, int32_t* count, double* loss_partial, float* loss, void* stream) {
-  if (const char* err = check_fwd_args(x, B, D, ent, n_ent, ld_ent, bias, cand, C, n_pos, g, d_x, count, loss_partial, loss))
-    return fail(__func__, err);
-  cudaStream_t s = as_stream(stream);
-  const int64_t n_slots = B * C;
-  KGC_CUDA_TRY(cudaMemsetAsync(count, 0, sizeof(int32_t), s));
-  const int64_t cblocks = ceil_div(n_slots, kThreadsSS) < 4 * kNumSMs ? ceil_div(n_slots, kThreadsSS) : 4 * kNumSMs;
-  count_valid_kernel<<<(unsigned)cblocks, kThreadsSS, 0, s>>>(cand, n_slots, n_ent, count);
-  KGC_LAUNCH_CHECK();
-  const int64_t blocks = kgc_sampled_bce_fwd_blocks(B);
-  const int D4 = D / 4;
-  const auto fwd = for_width(D4, sampled_bce_fwd_kernel<1>, sampled_bce_fwd_kernel<2>);
-  fwd<<<(unsigned)blocks, kThreadsSS, 0, s>>>(x, B, D4, ent, ld_ent, n_ent, bias, cand, C, n_pos, pos, add, count, g, d_x,
-                                              loss_partial);
-  KGC_LAUNCH_CHECK();
-  sampled_bce_finalize_kernel<<<1, kThreadsSS, 0, s>>>(loss_partial, blocks, count, loss);
-  KGC_LAUNCH_CHECK();
+  const SampledArgs a{x, B, D / 4, ent, ld_ent, n_ent, bias, cand, C, n_pos, pos, add, 0.f, 0.f, count, g, d_x, loss_partial};
+  if (const char* err = check_fwd_args(a, D, loss)) return fail(__func__, err);
+  KGC_CUDA_TRY(launch_sampled_fwd<BceLoss>(a, loss, as_stream(stream)));
   return 0;
 }
 
@@ -656,45 +626,22 @@ extern "C" int kgc_sampled_adv_fwd(const float* x, int64_t B, int32_t D, const f
                                    const float* bias, const int32_t* cand, int32_t C, int32_t n_pos, float pos, float add,
                                    float temperature, float* g, float* d_x, int32_t* counts, double* loss_partial, float* loss,
                                    void* stream) {
-  if (const char* err = check_fwd_args(x, B, D, ent, n_ent, ld_ent, bias, cand, C, n_pos, g, d_x, counts, loss_partial, loss))
-    return fail(__func__, err);
+  const SampledArgs a{x, B, D / 4, ent, ld_ent, n_ent, bias, cand, C, n_pos, pos, add, temperature, 0.f, counts, g, d_x,
+                      loss_partial};
+  if (const char* err = check_fwd_args(a, D, loss)) return fail(__func__, err);
   KGC_REQUIRE(std::isfinite(temperature) && temperature >= 0.f, "the adversarial temperature must be finite and >= 0");
-  cudaStream_t s = as_stream(stream);
-  KGC_CUDA_TRY(cudaMemsetAsync(counts, 0, 2 * sizeof(int32_t), s));
-  const int64_t blocks = kgc_sampled_bce_fwd_blocks(B);
-  const int64_t cblocks = blocks < 4 * kNumSMs ? blocks : 4 * kNumSMs;
-  count_adv_kernel<<<(unsigned)cblocks, kThreadsSS, 0, s>>>(cand, B, C, n_pos, n_ent, counts);
-  KGC_LAUNCH_CHECK();
-  const int D4 = D / 4;
-  const auto fwd = for_width(D4, sampled_adv_fwd_kernel<1>, sampled_adv_fwd_kernel<2>);
-  fwd<<<(unsigned)blocks, kThreadsSS, 0, s>>>(x, B, D4, ent, ld_ent, n_ent, bias, cand, C, n_pos, pos, add, temperature, counts,
-                                              g, d_x, loss_partial);
-  KGC_LAUNCH_CHECK();
-  sampled_adv_finalize_kernel<<<1, kThreadsSS, 0, s>>>(loss_partial, blocks, counts, loss);
-  KGC_LAUNCH_CHECK();
+  KGC_CUDA_TRY(launch_sampled_fwd<AdvLoss>(a, loss, as_stream(stream)));
   return 0;
 }
 
 extern "C" int kgc_sampled_ce_fwd(const float* x, int64_t B, int32_t D, const float* ent, int64_t n_ent, int64_t ld_ent,
                                   const float* bias, const int32_t* cand, int32_t C, int32_t n_pos, float label_smoothing,
                                   float* g, float* d_x, int32_t* count, double* loss_partial, float* loss, void* stream) {
-  if (const char* err = check_fwd_args(x, B, D, ent, n_ent, ld_ent, bias, cand, C, n_pos, g, d_x, count, loss_partial, loss))
-    return fail(__func__, err);
+  const SampledArgs a{x, B, D / 4, ent, ld_ent, n_ent, bias, cand, C, n_pos, 0.f, 0.f, 0.f, label_smoothing, count, g, d_x,
+                      loss_partial};
+  if (const char* err = check_fwd_args(a, D, loss)) return fail(__func__, err);
   KGC_REQUIRE(label_smoothing >= 0.f && label_smoothing <= 1.f, "the label smoothing must be a number in [0, 1]");
-  cudaStream_t s = as_stream(stream);
-  KGC_CUDA_TRY(cudaMemsetAsync(count, 0, sizeof(int32_t), s));
-  const int64_t pblocks = ceil_div(B * n_pos, kThreadsSS);       // 0 when n_pos = 0: then one CTA that counts nothing
-  const int64_t cblocks = pblocks < 1 ? 1 : pblocks < 4 * kNumSMs ? pblocks : 4 * kNumSMs;
-  count_pos_kernel<<<(unsigned)cblocks, kThreadsSS, 0, s>>>(cand, B, C, n_pos, n_ent, count);
-  KGC_LAUNCH_CHECK();
-  const int64_t blocks = kgc_sampled_bce_fwd_blocks(B);
-  const int D4 = D / 4;
-  const auto fwd = for_width(D4, sampled_ce_fwd_kernel<1>, sampled_ce_fwd_kernel<2>);
-  fwd<<<(unsigned)blocks, kThreadsSS, 0, s>>>(x, B, D4, ent, ld_ent, n_ent, bias, cand, C, n_pos, label_smoothing, count, g,
-                                              d_x, loss_partial);
-  KGC_LAUNCH_CHECK();
-  sampled_bce_finalize_kernel<<<1, kThreadsSS, 0, s>>>(loss_partial, blocks, count, loss);
-  KGC_LAUNCH_CHECK();
+  KGC_CUDA_TRY(launch_sampled_fwd<CeLoss>(a, loss, as_stream(stream)));
   return 0;
 }
 

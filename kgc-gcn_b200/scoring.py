@@ -143,53 +143,45 @@ def score_1n_bce(x, all_ent, bias, qid, ptr, idx, pos=1.0, add=0.0):
     return total
 
 
-def _sampled_operands(x, all_ent, bias, cand):
-    """The sampled forwards' device operands: x, the entity rows (a row pitch is taken, so rows may sit in a wider table),
-    bias and cand, checked, and the g [B, C] and d_x [B, D] outputs."""
-    x = _lib.require_cuda(x.detach(), torch.float32, 'x')
-    ent = all_ent.detach()
-    if ent.dtype != torch.float32:
-        raise TypeError('all_ent must be torch.float32, got {}'.format(ent.dtype))
-    if ent.stride(1) != 1 or ent.stride(0) % 4 != 0 or ent.data_ptr() % 16 != 0:
-        ent = ent.clone(memory_format=torch.contiguous_format)
-    bias_ = _lib.require_cuda(bias.detach(), torch.float32, 'bias')
-    cand = _lib.require_cuda(cand, torch.int32, 'cand')
-    B, D, C = int(x.shape[0]), int(x.shape[1]), int(cand.shape[1])
-    g = torch.empty((B, C), dtype=torch.float32, device=x.device)
-    d_x = torch.empty((B, D), dtype=torch.float32, device=x.device)
-    return x, ent, bias_, cand, g, d_x
+# each sampled loss: its C forward and its number of halves (int32 counts, and fp64 loss partials per forward CTA)
+_SAMPLED_FWD = {'bce': ('kgc_sampled_bce_fwd', 1), 'adv': ('kgc_sampled_adv_fwd', 2), 'ce': ('kgc_sampled_ce_fwd', 1)}
 
 
-class _ScoreSampledBCE(torch.autograd.Function):
-    """loss = mean BCE of sigmoid(<x[b], all_ent[cand[b, c]]> + bias[cand[b, c]]) over the valid slots (K6s), or with a
-    ``temperature`` the self-adversarial loss of ``score_sampled_bce``.  The forward makes one pass that yields the loss, the
-    logit gradient g [B, C] and d_x for a unit upstream gradient; the backward (shared by both objectives) scales d_x and
-    builds the dense table gradient by sorting the (entity, slot) pairs (no float atomics)."""
+class _ScoreSampled(torch.autograd.Function):
+    """loss = the sampled 1-vs-k loss ``kind`` (K6s): 'bce' the mean BCE of sigmoid(<x[b], all_ent[cand[b, c]]> +
+    bias[cand[b, c]]) over the valid slots, 'adv' the self-adversarial loss of ``score_sampled_bce`` and 'ce' the softmax
+    cross-entropy of ``score_sampled_ce``; ``scalars`` are that entry's own ((pos, add), (pos, add, temperature) or
+    (label_smoothing,)).  The forward makes one pass that yields the loss, the logit gradient g [B, C] and d_x for a unit
+    upstream gradient; the backward, the same for every loss, scales d_x and builds the dense table gradient by sorting
+    the (entity, slot) pairs (no float atomics).  The entity rows are taken with their row pitch, so they may sit in a
+    wider table."""
 
     @staticmethod
-    def forward(ctx, x, all_ent, bias, cand, n_pos, pos, add, temperature=None):
-        x, ent, bias_, cand, g, d_x = _sampled_operands(x, all_ent, bias, cand)
+    def forward(ctx, x, all_ent, bias, cand, n_pos, kind, scalars):
+        x = _lib.require_cuda(x.detach(), torch.float32, 'x')
+        ent = all_ent.detach()
+        if ent.dtype != torch.float32:
+            raise TypeError('all_ent must be torch.float32, got {}'.format(ent.dtype))
+        if ent.stride(1) != 1 or ent.stride(0) % 4 != 0 or ent.data_ptr() % 16 != 0:
+            ent = ent.clone(memory_format=torch.contiguous_format)
+        bias_ = _lib.require_cuda(bias.detach(), torch.float32, 'bias')
+        cand = _lib.require_cuda(cand, torch.int32, 'cand')
         B, D, C, N = int(x.shape[0]), int(x.shape[1]), int(cand.shape[1]), int(ent.shape[0])
         dev, p = x.device, _lib.ptr
-        if temperature is None:
-            count = torch.empty((1,), dtype=torch.int32, device=dev)
-            partial = torch.empty((int(_lib.lib().kgc_sampled_bce_fwd_blocks(B)),), dtype=torch.float64, device=dev)
-            loss = torch.empty((1,), dtype=torch.float32, device=dev)
-            _lib.call('kgc_sampled_bce_fwd', p(x), B, D, p(ent), N, ent.stride(0), p(bias_), p(cand), C, int(n_pos), float(pos),
-                      float(add), p(g), p(d_x), p(count), p(partial), p(loss), _lib.stream())
-        else:
-            counts = torch.empty((2,), dtype=torch.int32, device=dev)
-            partial = torch.empty((2 * int(_lib.lib().kgc_sampled_bce_fwd_blocks(B)),), dtype=torch.float64, device=dev)
-            loss = torch.empty((1,), dtype=torch.float32, device=dev)
-            _lib.call('kgc_sampled_adv_fwd', p(x), B, D, p(ent), N, ent.stride(0), p(bias_), p(cand), C, int(n_pos), float(pos),
-                      float(add), float(temperature), p(g), p(d_x), p(counts), p(partial), p(loss), _lib.stream())
+        fn, halves = _SAMPLED_FWD[kind]
+        g = torch.empty((B, C), dtype=torch.float32, device=dev)
+        d_x = torch.empty((B, D), dtype=torch.float32, device=dev)
+        counts = torch.empty((halves,), dtype=torch.int32, device=dev)
+        partial = torch.empty((halves * int(_lib.lib().kgc_sampled_bce_fwd_blocks(B)),), dtype=torch.float64, device=dev)
+        loss = torch.empty((1,), dtype=torch.float32, device=dev)
+        _lib.call(fn, p(x), B, D, p(ent), N, ent.stride(0), p(bias_), p(cand), C, int(n_pos), *(float(v) for v in scalars),
+                  p(g), p(d_x), p(counts), p(partial), p(loss), _lib.stream())
         ctx.save_for_backward(x, cand, g, d_x)
         ctx.n_ent = N
         return loss[0]
 
     @staticmethod
     def backward(ctx, d_loss):
-        # (also _ScoreSampledCE's: autograd drops the trailing None gradients of inputs that objective does not have)
         x, cand, g, d_x = ctx.saved_tensors
         B, D, C, N = int(x.shape[0]), int(x.shape[1]), int(cand.shape[1]), ctx.n_ent
         d_ent = d_bias = None
@@ -203,27 +195,7 @@ class _ScoreSampledBCE(torch.autograd.Function):
             _lib.call('kgc_sampled_bce_bwd_table', p(x), B, D, p(cand), C, p(g), p(scale), N, p(d_ent), D, p(d_bias), p(ws),
                       ws_bytes, _lib.stream())
         return (d_x * d_loss if ctx.needs_input_grad[0] else None, d_ent if ctx.needs_input_grad[1] else None,
-                d_bias if ctx.needs_input_grad[2] else None, None, None, None, None, None)
-
-
-class _ScoreSampledCE(_ScoreSampledBCE):
-    """loss = the softmax cross-entropy of ``score_sampled_ce`` (K6s, kgc_sampled_ce_fwd): the same single pass yields the
-    loss, the logit gradient g [B, C] and d_x for a unit upstream gradient, and _ScoreSampledBCE's backward turns g into
-    the table gradient."""
-
-    @staticmethod
-    def forward(ctx, x, all_ent, bias, cand, n_pos, label_smoothing):
-        x, ent, bias_, cand, g, d_x = _sampled_operands(x, all_ent, bias, cand)
-        B, D, C, N = int(x.shape[0]), int(x.shape[1]), int(cand.shape[1]), int(ent.shape[0])
-        dev, p = x.device, _lib.ptr
-        count = torch.empty((1,), dtype=torch.int32, device=dev)
-        partial = torch.empty((int(_lib.lib().kgc_sampled_bce_fwd_blocks(B)),), dtype=torch.float64, device=dev)
-        loss = torch.empty((1,), dtype=torch.float32, device=dev)
-        _lib.call('kgc_sampled_ce_fwd', p(x), B, D, p(ent), N, ent.stride(0), p(bias_), p(cand), C, int(n_pos),
-                  float(label_smoothing), p(g), p(d_x), p(count), p(partial), p(loss), _lib.stream())
-        ctx.save_for_backward(x, cand, g, d_x)
-        ctx.n_ent = N
-        return loss[0]
+                d_bias if ctx.needs_input_grad[2] else None, None, None, None, None)
 
 
 def check_adversarial_temperature(temperature):
@@ -252,7 +224,9 @@ def score_sampled_bce(x, all_ent, bias, cand, n_pos, pos=1.0, add=0.0, adversari
     mean over the valid slots."""
     temperature = check_adversarial_temperature(adversarial_temperature)
     _check_sampled_args('score_sampled_bce', x, all_ent, bias, cand, n_pos)
-    return _ScoreSampledBCE.apply(x, all_ent, bias, cand, int(n_pos), pos, add, temperature)
+    if temperature is None:
+        return _ScoreSampled.apply(x, all_ent, bias, cand, int(n_pos), 'bce', (pos, add))
+    return _ScoreSampled.apply(x, all_ent, bias, cand, int(n_pos), 'adv', (pos, add, temperature))
 
 
 def check_label_smoothing(label_smoothing):
@@ -294,7 +268,7 @@ def score_sampled_ce(x, all_ent, bias, cand, n_pos, label_smoothing=0.0):
     deterministic and graph-capturable."""
     eps = check_label_smoothing(label_smoothing)
     _check_sampled_args('score_sampled_ce', x, all_ent, bias, cand, n_pos)
-    return _ScoreSampledCE.apply(x, all_ent, bias, cand, int(n_pos), eps)
+    return _ScoreSampled.apply(x, all_ent, bias, cand, int(n_pos), 'ce', (eps,))
 
 
 def _check_sampled_args(fn, x, all_ent, bias, cand, n_pos):

@@ -24,7 +24,7 @@ sys.path.insert(0, HERE)
 import numpy as np       # noqa: E402
 import torch             # noqa: E402
 
-from sampled_loss_time import gpu_info, k          # noqa: E402  (puts the repository and oracle/ on sys.path)
+from sampled_time import gpu_info, k               # noqa: E402  (puts the repository and oracle/ on sys.path)
 from bench import D_IN, Flusher, LayerCase, oracle, synth_rows      # noqa: E402
 from compact_planes_time import timed               # noqa: E402
 

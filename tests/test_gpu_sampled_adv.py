@@ -1,5 +1,5 @@
 """Self-adversarial negative sampling on the GPU: kgc_sampled_adv_fwd + the shared table backward against the float64
-restatement of tests/sampled_adv_oracle.py, its bridge to the plain sampled objective at alpha = 0, the hardest-negative
+restatement of tests/sampled_oracle.py, its bridge to the plain sampled objective at alpha = 0, the hardest-negative
 limit, MGCN.loss_sampled(adversarial_temperature=...) and GraphedTrainStep(negatives=k, adversarial_temperature=...)
 on data/Toy."""
 import copy
@@ -11,7 +11,6 @@ import pytest
 import torch
 
 import mgcn_oracle as orc
-import sampled_adv_oracle as sa
 import sampled_oracle as so
 
 pytestmark = pytest.mark.gpu
@@ -78,7 +77,7 @@ def test_sampled_adv_matches_float64(k, B, C, N, D, n_pos, strided, smooth, alph
     for a, b in zip(*outs):
         assert torch.equal(a, b)
     loss, d_x, d_ent, d_bias = outs[0]
-    r_loss, _, r_x, r_ent, r_bias = sa.sampled_adv(x, ent, bias, cand, n_pos, alpha, pos, add)
+    r_loss, _, r_x, r_ent, r_bias = so.sampled_adv(x, ent, bias, cand, n_pos, alpha, pos, add)
     assert abs(float(loss) - float(r_loss)) <= 1e-6 * abs(float(r_loss)), (float(loss), float(r_loss))
     for got, ref, name in ((d_x, 2.5 * r_x, 'd_x'), (d_ent, 2.5 * r_ent, 'd_ent'), (d_bias, 2.5 * r_bias, 'd_bias')):
         err = float((got.double() - ref).abs().max()) / float(ref.abs().max())
@@ -106,7 +105,7 @@ def test_sampled_adv_logit_gradient_and_counts_through_the_c_abi(k, alpha):
     torch.cuda.synchronize()
     valid = cand >= 0
     assert counts.cpu().tolist() == [int(valid[:, :n_pos].any(1).sum()), int(valid[:, n_pos:].any(1).sum())]
-    r_loss, r_g, r_x, _, _ = sa.sampled_adv(x, ent, bias, cand, n_pos, alpha)
+    r_loss, r_g, r_x, _, _ = so.sampled_adv(x, ent, bias, cand, n_pos, alpha)
     assert float((g.cpu().double() - r_g).abs().max()) <= 1e-5 * float(r_g.abs().max())
     assert float(g.cpu()[~valid].abs().sum()) == 0.0
     assert float((d_x.cpu().double() - r_x).abs().max()) <= 1e-5 * float(r_x.abs().max())
@@ -174,7 +173,7 @@ def test_sampled_adv_hardest_negative(k):
     top = z[:, 1:].max(1).values
     ref = 0.5 * float((-torch.nn.functional.logsigmoid(z[:, 0])).mean() + (-torch.nn.functional.logsigmoid(-top)).mean())
     assert abs(float(loss) - ref) <= 1e-6 * abs(ref), (float(loss), ref)
-    _, r_g, _, _, _ = sa.sampled_adv(x, ent, bias, cand, 1, 50.0)
+    _, r_g, _, _, _ = so.sampled_adv(x, ent, bias, cand, 1, 50.0)
     L, p = k._lib, k._lib.ptr
     g = torch.empty((B, C), device='cuda')
     counts = torch.empty((2,), dtype=torch.int32, device='cuda')

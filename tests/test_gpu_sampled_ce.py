@@ -1,5 +1,5 @@
 """Negative-sampled softmax cross-entropy on the GPU: kgc_sampled_ce_fwd + the shared table backward against the float64
-restatement of tests/sampled_ce_oracle.py, at ordinary and at large logits, its bridge to the 1vsAll cross-entropy,
+restatement of tests/sampled_oracle.py, at ordinary and at large logits, its bridge to the 1vsAll cross-entropy,
 MGCN.loss_sampled(criterion='ce') and GraphedTrainStep(negatives=k, criterion='ce') on data/Toy."""
 import copy
 import os
@@ -11,7 +11,6 @@ import torch
 import torch.nn.functional as F
 
 import mgcn_oracle as orc
-import sampled_ce_oracle as sc
 import sampled_oracle as so
 
 pytestmark = pytest.mark.gpu
@@ -98,7 +97,7 @@ def _check(k, x, ent, bias, cand, n_pos, eps, strided):
     loss, d_x, d_ent, d_bias = outs[0]
     for t in outs[0]:
         assert bool(torch.isfinite(t).all())
-    r_loss, _, r_x, r_ent, r_bias = sc.sampled_ce(x, ent, bias, cand, n_pos, eps)
+    r_loss, _, r_x, r_ent, r_bias = so.sampled_ce(x, ent, bias, cand, n_pos, eps)
     assert abs(float(loss) - float(r_loss)) <= 1e-6 * abs(float(r_loss)), (float(loss), float(r_loss))
     for got, ref, name in ((d_x, 2.5 * r_x, 'd_x'), (d_ent, 2.5 * r_ent, 'd_ent'), (d_bias, 2.5 * r_bias, 'd_bias')):
         err = float((got.double() - ref).abs().max()) / float(ref.abs().max())
@@ -145,7 +144,7 @@ def test_sampled_ce_logit_gradient_through_the_c_abi(k, eps):
     torch.cuda.synchronize()
     valid = cand >= 0
     assert int(count) == int(valid[:, :n_pos].sum())
-    r_loss, r_g, r_x, _, _ = sc.sampled_ce(x, ent, bias, cand, n_pos, eps)
+    r_loss, r_g, r_x, _, _ = so.sampled_ce(x, ent, bias, cand, n_pos, eps)
     assert float((g.cpu().double() - r_g).abs().max()) <= 1e-5 * float(r_g.abs().max())
     assert float(g.cpu()[~valid].abs().sum()) == 0.0
     assert float(g.cpu()[2].abs().sum()) == 0.0           # positives without negatives

@@ -1,11 +1,10 @@
-"""Self-adversarial negative sampling, host side: the float64 restatement of tests/sampled_adv_oracle.py against
+"""Self-adversarial negative sampling, host side: the float64 restatement of tests/sampled_oracle.py against
 torch.nn.BCELoss(weight=...) + autograd on the gathered probabilities and against RotatE's logsigmoid formula, its bridge
 to the plain sampled objective at alpha = 0, and the argument checks of the Python surface (no GPU needed)."""
 import numpy as np
 import pytest
 import torch
 
-import sampled_adv_oracle as sa
 import sampled_oracle as so
 
 
@@ -61,7 +60,7 @@ def _case(B, C, N, D, n_pos, seed):
 def test_sampled_adv_oracle_matches_weighted_bceloss(B, C, N, D, n_pos, smooth, seed, alpha):
     x, ent, bias, cand = _case(B, C, N, D, n_pos, seed)
     pos, add = (float(np.float32(1.0 - smooth) + np.float32(1.0 / N)), float(np.float32(1.0 / N))) if smooth else (1.0, 0.0)
-    loss, gl, d_x, d_ent, d_bias = sa.sampled_adv(x, ent, bias, cand, n_pos, alpha, pos, add)
+    loss, gl, d_x, d_ent, d_bias = so.sampled_adv(x, ent, bias, cand, n_pos, alpha, pos, add)
     r_loss, r_x, r_ent, r_bias = _weighted_bce_autograd(x, ent, bias, cand, n_pos, alpha, pos, add)
     assert abs(float(loss) - float(r_loss)) <= 1e-12 * abs(float(r_loss))
     for got, ref in ((d_x, r_x), (d_ent, r_ent), (d_bias, r_bias)):
@@ -82,7 +81,7 @@ def test_sampled_adv_oracle_is_rotate_formula(alpha):
     ent = torch.randn(N, D, generator=g) * (1.0 / D ** 0.5)
     bias = torch.randn(N, generator=g) * 0.1
     cand = torch.randint(0, N, (B, C), generator=g)
-    loss, _, d_x, d_ent, d_bias = sa.sampled_adv(x, ent, bias, cand, 1, alpha)
+    loss, _, d_x, d_ent, d_bias = so.sampled_adv(x, ent, bias, cand, 1, alpha)
     xd, ed, bd = (t.clone().double().requires_grad_(True) for t in (x, ent, bias))
     z = (xd[:, None, :] * ed[cand]).sum(-1) + bd[cand]
     assert float(z.detach().abs().max()) < 10.0
@@ -96,7 +95,7 @@ def test_sampled_adv_oracle_is_rotate_formula(alpha):
 
 
 def test_sampled_adv_oracle_without_valid_slots():
-    loss, gl, d_x, d_ent, d_bias = sa.sampled_adv(torch.ones(2, 4), torch.ones(3, 4), torch.zeros(3),
+    loss, gl, d_x, d_ent, d_bias = so.sampled_adv(torch.ones(2, 4), torch.ones(3, 4), torch.zeros(3),
                                                   torch.full((2, 5), -1), 1, 1.0)
     assert float(loss) == 0.0 and float(gl.abs().sum()) == 0.0
     assert float(d_x.abs().sum()) == 0.0 and float(d_ent.abs().sum()) == 0.0 and float(d_bias.abs().sum()) == 0.0
@@ -115,7 +114,7 @@ def test_sampled_adv_oracle_alpha_zero_bridge(n_pos):
     cand[:, n_pos - 1] = -1                               # one empty positive and one empty negative slot per query
     cand[:, C - 2] = -1
     pos, add = 0.93, 0.01
-    got = sa.sampled_adv(x, ent, bias, cand, n_pos, 0.0, pos, add)
+    got = so.sampled_adv(x, ent, bias, cand, n_pos, 0.0, pos, add)
     a = so.sampled_bce(x, ent, bias, cand[:, :n_pos], n_pos, pos, add)
     b = so.sampled_bce(x, ent, bias, cand[:, n_pos:], 0, pos, add)
     assert abs(float(got[0]) - 0.5 * float(a[0] + b[0])) <= 1e-12 * abs(float(got[0]))

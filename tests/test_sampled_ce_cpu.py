@@ -1,4 +1,4 @@
-"""Negative-sampled softmax cross-entropy, host side: the float64 restatement of tests/sampled_ce_oracle.py against
+"""Negative-sampled softmax cross-entropy, host side: the float64 restatement of tests/sampled_oracle.py against
 torch.nn.functional.cross_entropy(label_smoothing=eps) + autograd on explicitly built per-positive logit rows, and the
 argument checks of the Python surface (no GPU needed)."""
 import numpy as np
@@ -6,7 +6,7 @@ import pytest
 import torch
 import torch.nn.functional as F
 
-import sampled_ce_oracle as sc
+import sampled_oracle as so
 
 
 def _cross_entropy_autograd(x, ent, bias, cand, n_pos, eps):
@@ -58,7 +58,7 @@ def _case(B, C, N, D, n_pos, seed, scale=1.0):
 ])
 def test_sampled_ce_oracle_matches_cross_entropy(B, C, N, D, n_pos, seed, scale, eps):
     x, ent, bias, cand = _case(B, C, N, D, n_pos, seed, scale)
-    loss, gl, d_x, d_ent, d_bias = sc.sampled_ce(x, ent, bias, cand, n_pos, eps)
+    loss, gl, d_x, d_ent, d_bias = so.sampled_ce(x, ent, bias, cand, n_pos, eps)
     r_loss, r_x, r_ent, r_bias = _cross_entropy_autograd(x, ent, bias, cand, n_pos, eps)
     assert abs(float(loss) - float(r_loss)) <= 1e-12 * abs(float(r_loss))
     for got, ref in ((d_x, r_x), (d_ent, r_ent), (d_bias, r_bias)):
@@ -77,15 +77,15 @@ def test_sampled_ce_oracle_positive_without_negatives_adds_nothing():
     x, ent, bias = torch.randn(2, 4), torch.randn(6, 4), torch.randn(6)
     cand = torch.tensor([[1, -1, -1], [2, 3, 4]])
     for eps in (0.0, 0.1):
-        loss, gl, d_x, _, _ = sc.sampled_ce(x[:1], ent, bias, cand[:1], 1, eps)
+        loss, gl, d_x, _, _ = so.sampled_ce(x[:1], ent, bias, cand[:1], 1, eps)
         assert float(loss) == 0.0 and float(gl.abs().sum()) == 0.0 and float(d_x.abs().sum()) == 0.0
-        both = sc.sampled_ce(x, ent, bias, cand, 1, eps)[0]
-        one = sc.sampled_ce(x[1:], ent, bias, cand[1:], 1, eps)[0]
+        both = so.sampled_ce(x, ent, bias, cand, 1, eps)[0]
+        one = so.sampled_ce(x[1:], ent, bias, cand[1:], 1, eps)[0]
         assert abs(float(both) - 0.5 * float(one)) <= 1e-15 * abs(float(one))
 
 
 def test_sampled_ce_oracle_without_valid_slots():
-    loss, gl, d_x, d_ent, d_bias = sc.sampled_ce(torch.ones(2, 4), torch.ones(3, 4), torch.zeros(3),
+    loss, gl, d_x, d_ent, d_bias = so.sampled_ce(torch.ones(2, 4), torch.ones(3, 4), torch.zeros(3),
                                                  torch.full((2, 5), -1), 1, 0.1)
     assert float(loss) == 0.0 and float(gl.abs().sum()) == 0.0
     assert float(d_x.abs().sum()) == 0.0 and float(d_ent.abs().sum()) == 0.0 and float(d_bias.abs().sum()) == 0.0
