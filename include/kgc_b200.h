@@ -608,6 +608,57 @@ int kgc_sampled_bce_bwd_table(const float* x, int64_t B, int32_t D, const int32_
                               const float* scale, int64_t n_ent, float* d_ent, int64_t ld_d, float* d_bias,
                               void* workspace, size_t workspace_bytes, void* stream);
 
+/* K6s, shared negatives: every query of the batch scores the same k negatives shared [k] (int32) besides its own n_pos
+ * positives pos_cand [B, n_pos] (n_pos >= 1).  The loss is the per-query loss above (kgc_sampled_*_fwd) on the broadcast
+ * candidate matrix cand[b] = [pos_cand[b] | shared, with every entry that is a known object of query qid[b] (the
+ * query->objects CSR of kgc_label_mask_t_build) set to -1]: the same value, gradients, divisors and empty-slot rules.
+ * Duplicates in shared are separate slots; a filtered entry is an empty slot of that query only; an id outside
+ * [0, n_ent) is an empty slot of every query.
+ *   kgc_score_1n_logits_t: logitT[n, b] = E[n,:] . X[b,:] + bias[n] (fp32-grade, 3xTF32), kgc_score_1n_fwd_t without
+ *     the sigmoid; here on E = the gathered shared rows.
+ *   kgc_shared_rows: rows [k, D] contiguous = ent[shared], row_bias [k] = bias[shared] (zeros for an invalid id).
+ *   kgc_shared_mask_build: mask_t [k, ceil(B / 32)] uint32, bit (b & 31) of word (b >> 5) of row j set iff shared[j] is
+ *     a known object of query qid[b] (zeroed by the call); sorted_ids / sorted_slots [k]: the (id, slot) pairs
+ *     stable-sorted by id (an invalid id sorts as n_ent), which kgc_shared_bwd_table takes.  CUB radix sort and a binary
+ *     search per known object, integer operations only.  workspace: kgc_shared_mask_workspace_bytes(k, n_ent).
+ *   kgc_shared_{bce,adv,ce}_loss: over logit_t [k, ldt] (ldt >= B; the shared logits of query b in column b), the mask
+ *     and the positives: loss[0]; the logit gradient for a unit upstream gradient OVER logit_t (0 on filtered and empty
+ *     slots and in columns [B, ldt) of the CTAs' 32-query groups); g_pos [B, n_pos], the positive slots' gradient;
+ *     d_x [B, D] = sum_c g_pos[b, c] ent[pos_cand[b, c]] in slot order (the negatives' part is the caller's product of
+ *     the gradient tile with the shared rows); d_bias_s [k] = sum_b of the gradient tile's row j, the CTAs' partials
+ *     added in a fixed order.  The adversarial weights and the cross-entropy's log-sum-exp are per query over its k
+ *     shared slots against their max.  workspace: kgc_shared_loss_workspace_bytes(B, k).
+ *   kgc_shared_bwd_table: d_ent[n] += *scale * sum over the slots j with shared[j] = n of d_rows[j] (rows of pitch
+ *     ld_rows), d_bias[n] += *scale * sum d_row_bias[j], added in slot order through the sorted pairs (no float atomics);
+ *     the positives' part and the zero fill come first from kgc_sampled_bce_bwd_table on (pos_cand, g_pos).
+ * All deterministic, no host synchronisation (graph-capturable). */
+int kgc_score_1n_logits_t(const float* ent, int64_t n_ent, int32_t D, int64_t ld_ent, const float* packed_x, int32_t B,
+                          const float* bias, float* logit_t, int64_t ld_t, void* stream);
+int kgc_shared_rows(const float* ent, int64_t n_ent, int32_t D, int64_t ld_ent, const float* bias, const int32_t* shared,
+                    int32_t k, float* rows, float* row_bias, void* stream);
+size_t kgc_shared_mask_workspace_bytes(int32_t k, int64_t n_ent);
+int kgc_shared_mask_build(const int32_t* shared, int32_t k, const int64_t* qid, int64_t B, const int64_t* ptr,
+                          const int32_t* idx, int64_t n_ent, uint32_t* mask_t, int32_t* sorted_ids, int32_t* sorted_slots,
+                          void* workspace, size_t workspace_bytes, void* stream);
+int64_t kgc_shared_loss_blocks(int64_t B);
+size_t kgc_shared_loss_workspace_bytes(int64_t B, int32_t k);
+int kgc_shared_bce_loss(float* logit_t, int64_t ldt, const uint32_t* mask_t, const int32_t* shared, int32_t k,
+                        const float* x, int64_t B, int32_t D, const float* ent, int64_t n_ent, int64_t ld_ent,
+                        const float* bias, const int32_t* pos_cand, int32_t n_pos, float pos, float add, float* g_pos,
+                        float* d_x, float* d_bias_s, float* loss, void* workspace, size_t workspace_bytes, void* stream);
+int kgc_shared_adv_loss(float* logit_t, int64_t ldt, const uint32_t* mask_t, const int32_t* shared, int32_t k,
+                        const float* x, int64_t B, int32_t D, const float* ent, int64_t n_ent, int64_t ld_ent,
+                        const float* bias, const int32_t* pos_cand, int32_t n_pos, float pos, float add, float temperature,
+                        float* g_pos, float* d_x, float* d_bias_s, float* loss, void* workspace, size_t workspace_bytes,
+                        void* stream);
+int kgc_shared_ce_loss(float* logit_t, int64_t ldt, const uint32_t* mask_t, const int32_t* shared, int32_t k,
+                       const float* x, int64_t B, int32_t D, const float* ent, int64_t n_ent, int64_t ld_ent,
+                       const float* bias, const int32_t* pos_cand, int32_t n_pos, float label_smoothing, float* g_pos,
+                       float* d_x, float* d_bias_s, float* loss, void* workspace, size_t workspace_bytes, void* stream);
+int kgc_shared_bwd_table(const int32_t* sorted_ids, const int32_t* sorted_slots, int32_t k, int64_t n_ent, int32_t D,
+                         const float* d_rows, int64_t ld_rows, const float* d_row_bias, const float* scale, float* d_ent,
+                         int64_t ld_d, float* d_bias, void* stream);
+
 #if defined(__GNUC__)
 #pragma GCC visibility pop
 #endif

@@ -109,6 +109,19 @@ SIGNATURES = {
                                           _vp]),
     'kgc_sampled_bce_bwd_table_workspace_bytes': (_sz, [_i64, _i64]),
     'kgc_sampled_bce_bwd_table': (ctypes.c_int, [_vp, _i64, _i32, _vp, _i32, _vp, _vp, _i64, _vp, _i64, _vp, _vp, _sz, _vp]),
+    'kgc_score_1n_logits_t': (ctypes.c_int, [_vp, _i64, _i32, _i64, _vp, _i32, _vp, _vp, _i64, _vp]),
+    'kgc_shared_rows': (ctypes.c_int, [_vp, _i64, _i32, _i64, _vp, _vp, _i32, _vp, _vp, _vp]),
+    'kgc_shared_mask_workspace_bytes': (_sz, [_i32, _i64]),
+    'kgc_shared_mask_build': (ctypes.c_int, [_vp, _i32, _vp, _i64, _vp, _vp, _i64, _vp, _vp, _vp, _vp, _sz, _vp]),
+    'kgc_shared_loss_blocks': (_i64, [_i64]),
+    'kgc_shared_loss_workspace_bytes': (_sz, [_i64, _i32]),
+    'kgc_shared_bce_loss': (ctypes.c_int, [_vp, _i64, _vp, _vp, _i32, _vp, _i64, _i32, _vp, _i64, _i64, _vp, _vp, _i32, _f32, _f32,
+                                           _vp, _vp, _vp, _vp, _vp, _sz, _vp]),
+    'kgc_shared_adv_loss': (ctypes.c_int, [_vp, _i64, _vp, _vp, _i32, _vp, _i64, _i32, _vp, _i64, _i64, _vp, _vp, _i32, _f32, _f32,
+                                           _f32, _vp, _vp, _vp, _vp, _vp, _sz, _vp]),
+    'kgc_shared_ce_loss': (ctypes.c_int, [_vp, _i64, _vp, _vp, _i32, _vp, _i64, _i32, _vp, _i64, _i64, _vp, _vp, _i32, _f32,
+                                          _vp, _vp, _vp, _vp, _vp, _sz, _vp]),
+    'kgc_shared_bwd_table': (ctypes.c_int, [_vp, _vp, _i32, _i64, _i32, _vp, _i64, _vp, _vp, _vp, _i64, _vp, _vp]),
 }
 
 
@@ -130,7 +143,7 @@ def lib():
 
 
 LAUNCHES = 0     # kernels launched through the C ABI since import (bench.py reports it as gpu_launches)
-_KERNELS_PER_CALL = {'kgc_csr_build': 16, 'kgc_bce_1n_bwd_logit_t': 2, 'kgc_label_mask_t_build': 2, 'kgc_score_pairs': 3, 'kgc_rank_finalize': 2, 'kgc_score_topk': 2, 'kgc_topk_dense': 2, 'kgc_sampled_bce_fwd': 4, 'kgc_sampled_adv_fwd': 4, 'kgc_sampled_ce_fwd': 3, 'kgc_sampled_bce_bwd_table': 7, 'kgc_gemm_tn': 2, 'kgc_gemm_tn_tc_batch': 2}   # (kgc_p2p_allreduce: 1 or 3)
+_KERNELS_PER_CALL = {'kgc_csr_build': 16, 'kgc_bce_1n_bwd_logit_t': 2, 'kgc_label_mask_t_build': 2, 'kgc_score_pairs': 3, 'kgc_rank_finalize': 2, 'kgc_score_topk': 2, 'kgc_topk_dense': 2, 'kgc_sampled_bce_fwd': 4, 'kgc_sampled_adv_fwd': 4, 'kgc_sampled_ce_fwd': 3, 'kgc_sampled_bce_bwd_table': 7, 'kgc_gemm_tn': 2, 'kgc_gemm_tn_tc_batch': 2, 'kgc_shared_mask_build': 3, 'kgc_shared_bce_loss': 4, 'kgc_shared_adv_loss': 4, 'kgc_shared_ce_loss': 4}   # (kgc_p2p_allreduce: 1 or 3)
 
 
 def call(name, *args):

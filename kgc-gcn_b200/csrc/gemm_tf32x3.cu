@@ -1164,3 +1164,11 @@ extern "C" int kgc_gemm_nt_splitk(const float* A, int64_t lda, const float* Bt, 
                                   float* C, void* workspace, size_t workspace_bytes, void* stream) {
   return launch_gemm_tn_tc(1, &A, lda, &Bt, ldb, K, Ma, Nb, &C, workspace, workspace_bytes, 1, stream);
 }
+
+// Entity-major raw logits: logitT[n, b] = E[n, :] . X[b, :] + bias[n], rows of ld_t >= B floats - kgc_score_1n_fwd_t
+// without the sigmoid, for the losses that need the logit itself (the shared-negative cross-entropy's log-sum-exp)
+extern "C" int kgc_score_1n_logits_t(const float* ent, int64_t n_ent, int32_t D, int64_t ld_ent, const float* packed_x,
+                                     int32_t B, const float* bias, float* logit_t, int64_t ld_t, void* stream) {
+  KGC_REQUIRE(bias != nullptr, "bias is required");
+  return launch_gemm_nt(1, &ent, n_ent, D, ld_ent, &packed_x, B, &logit_t, ld_t, bias, 0, 0, 0, stream);
+}

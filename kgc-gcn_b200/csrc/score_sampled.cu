@@ -21,6 +21,7 @@
 // so instead of float atomics the (entity, slot) pairs are stable-sorted by entity (CUB radix sort, as K1) and one warp
 // per distinct entity adds its slots in slot order: deterministic.
 #include <cmath>
+#include <type_traits>
 
 #include <cub/device/device_radix_sort.cuh>
 
@@ -606,6 +607,413 @@ cudaError_t launch_sampled_fwd(const SampledArgs& a, float* loss, cudaStream_t s
   return cudaGetLastError();
 }
 
+// ---- Shared negatives: every query of the batch scores the same k rows E_S = ent[shared] ----------------------------
+// The candidate layout is cand[b] = [pos_cand[b] | shared with query b's known objects set to -1], the loss is the
+// per-query one above on that matrix.  The k x B logits of the shared part come from the tensor-core scorer
+// (kgc_score_1n_logits_t, entity-major logitT[j, b]); the filter is a bit per (slot, query) in the same orientation; the
+// n_pos positive rows of each query are gathered by a warp as in sampled_fwd_kernel.  A CTA of the loss pass owns 32
+// queries (lane = query, so a row of the tile is one coalesced 128-byte piece and a mask word serves the whole warp)
+// and its 16 warps share the k rows.
+
+constexpr int kWarpsSh = 16;                      // warps of a shared loss CTA (32 queries: two each for the positives)
+constexpr int kThreadsSh = 32 * kWarpsSh;
+constexpr int kRowsSh = 8;                        // tile rows a warp loads before consuming the first
+
+// The operands of the shared pass.  nq [B]: query b's valid unfiltered shared slots (shared_count_kernel);
+// loss_partial: Loss::kHalves x gridDim.x sums; bias_partial [gridDim.x, k]: each CTA's sum of g over its 32 queries.
+struct SharedArgs {
+  float* logit_t;             // [k, ldt]: logits in, the logit gradient out
+  int64_t ldt;
+  const uint32_t* mask_t;     // [k, W]
+  int64_t W;
+  const int32_t* shared;      // [k]
+  int k;
+  const float* x;             // [B, 4 * D4]
+  int64_t B;
+  int D4;
+  const float* ent;           // rows of pitch ld_ent
+  int64_t ld_ent;
+  int64_t n_ent;
+  const float* bias;
+  const int32_t* pos_cand;    // [B, n_pos]
+  int n_pos;
+  float pos, add, alpha, eps;
+  float* g_pos;               // [B, n_pos]
+  float* d_x;                 // [B, 4 * D4]: the positives' part
+  int32_t* counts;
+  int32_t* nq;
+  double* loss_partial;
+  float* bias_partial;
+};
+
+// is slot j of the shared tile a valid negative of lane `lane`'s query (b < B)
+__device__ __forceinline__ bool shared_ok(const SharedArgs& a, int j, bool in_batch, int lane) {
+  return in_batch && slot_valid(__ldg(a.shared + j), a.n_ent) &&
+         ((__ldg(a.mask_t + (int64_t)j * a.W + blockIdx.x) >> lane) & 1u) == 0u;
+}
+
+// The filter bits: one warp per query b, its lanes over the query's known objects; each object is looked up in the
+// shared ids sorted by id and every slot of its run gets bit (b & 31) of word (b >> 5).  Integer ORs only.
+__global__ void __launch_bounds__(kThreadsSS)
+shared_mask_kernel(const int32_t* __restrict__ ids, int k, const int64_t* __restrict__ qid, int64_t B,
+                   const int64_t* __restrict__ ptr, const int32_t* __restrict__ idx, int64_t n_ent, const int32_t* __restrict__ slots,
+                   uint32_t* __restrict__ mask_t, int64_t W) {
+  const int lane = threadIdx.x & 31;
+  const int64_t b = (int64_t)blockIdx.x * kWarpsSS + (threadIdx.x >> 5);
+  if (b >= B) return;
+  const int64_t q = qid[b];
+  const uint32_t bit = 1u << (b & 31);
+  for (int64_t i = ptr[q] + lane; i < ptr[q + 1]; i += 32) {
+    const int32_t o = idx[i];
+    if (!slot_valid(o, n_ent)) continue;
+    int lo = 0, hi = k;                                          // the first position with ids[pos] >= o
+    while (lo < hi) {
+      const int mid = (lo + hi) >> 1;
+      if (ids[mid] < o) lo = mid + 1; else hi = mid;
+    }
+    for (int j = lo; j < k && ids[j] == o; ++j) atomicOr(mask_t + (int64_t)slots[j] * W + (b >> 5), bit);
+  }
+}
+
+// ent rows and biases of the shared ids (zeros for an id outside [0, n_ent)): E_S [k, D] contiguous, b_S [k]
+__global__ void __launch_bounds__(kThreadsSS)
+shared_rows_kernel(const float* __restrict__ ent, int64_t ld_ent, const float* __restrict__ bias, int64_t n_ent,
+                   const int32_t* __restrict__ shared, int k, int D4, float* __restrict__ rows, float* __restrict__ row_bias) {
+  const int64_t i = (int64_t)blockIdx.x * kThreadsSS + threadIdx.x;
+  if (i >= (int64_t)k * D4) return;
+  const int j = (int)(i / D4), c4 = (int)(i % D4);
+  const int32_t e = shared[j];
+  const bool ok = slot_valid(e, n_ent);
+  *reinterpret_cast<float4*>(rows + 4 * i) = ok ? ldg4(ent + (int64_t)e * ld_ent + 4 * c4) : make_float4(0.f, 0.f, 0.f, 0.f);
+  if (c4 == 0) row_bias[j] = ok ? bias[e] : 0.f;
+}
+
+// |P_b| and |Q_b| of the broadcast matrix: a CTA owns the 32 queries of one mask word column, its warps share the k
+// rows (lane = query), the warps' counts are added in shared memory; nq[b] = |Q_b| for the pass, the Loss's tally into
+// the counts (integer sums)
+template <class Loss>
+__global__ void __launch_bounds__(kThreadsSS)
+shared_count_kernel(const SharedArgs a) {
+  __shared__ int sh[kWarpsSS][32];
+  const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5;
+  const int64_t b = (int64_t)blockIdx.x * 32 + lane;
+  int n = 0;
+  for (int j = warp; j < a.k; j += kWarpsSS) n += shared_ok(a, j, b < a.B, lane) ? 1 : 0;
+  sh[warp][lane] = n;
+  __syncthreads();
+  if (warp != 0) return;
+  int n_q = 0, n_p = 0;
+  for (int w = 0; w < kWarpsSS; ++w) n_q += sh[w][lane];
+  int t[2] = {0, 0};
+  if (b < a.B) {
+    for (int c = 0; c < a.n_pos; ++c) n_p += slot_valid(a.pos_cand[b * a.n_pos + c], a.n_ent) ? 1 : 0;
+    a.nq[b] = n_q;
+    Loss::tally(n_p, n_q, t);
+  }
+#pragma unroll
+  for (int h = 0; h < Loss::kHalves; ++h) {
+    const int s = __reduce_add_sync(kFull, t[h]);
+    if (lane == 0 && s != 0) atomicAdd(a.counts + h, s);
+  }
+}
+
+// The shared loss pass, one CTA per 32 queries b0 + lane:
+//   A (AdvLoss, CeLoss)  per query the online max m and sum S of exp(v - m) over its valid negatives (v = alpha z / z),
+//                        and for CeLoss the sum Z of their logits, each warp over its rows, the warps merged in order;
+//   B                    warp w gathers the positive rows of queries b0 + w and b0 + w + 16: their logits, gradients g_pos, loss terms and
+//                        d_x[b] = sum g_pos E[p] in slot order (CeLoss: also R = sum r_p, as CeLoss::State::finish);
+//   C                    each warp over its rows again: the negatives' gradient (over the logit in place), loss terms,
+//                        and the row's sum of g over the 32 queries into bias_partial.
+// The per-slot arithmetic is that of the per-query policies above.
+template <class Loss, int NV>
+__global__ void __launch_bounds__(kThreadsSh, 1)
+shared_loss_kernel(const SharedArgs a) {
+  constexpr int H = Loss::kHalves;
+  constexpr bool kAdv = std::is_same<Loss, AdvLoss>::value, kCe = std::is_same<Loss, CeLoss>::value;
+  __shared__ float sh_m[kWarpsSh][32], sh_s[kWarpsSh][32];
+  __shared__ double sh_z[kWarpsSh][32];
+  __shared__ float q_m[32], q_s[32], q_c[32], q_r[32];          // per query: max, sum, negative coefficient, R
+  __shared__ double warp_loss[H][kWarpsSh];
+  const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5;
+  const int64_t b0 = (int64_t)blockIdx.x * 32, b = b0 + lane;
+  const bool in_batch = b < a.B, in_tile = b < a.ldt;
+  double loss[H] = {};
+  if constexpr (kAdv || kCe) {
+    float m = -INFINITY, S = 0.f;
+    double Z = 0.0;
+    for (int j0 = warp; j0 < a.k; j0 += kWarpsSh * kRowsSh) {
+      float z[kRowsSh];
+      bool ok[kRowsSh];
+#pragma unroll
+      for (int u = 0; u < kRowsSh; ++u) {                        // every load of the batch before any is consumed
+        const int j = j0 + u * kWarpsSh;
+        ok[u] = j < a.k && shared_ok(a, j, in_batch, lane);
+        z[u] = ok[u] ? a.logit_t[(int64_t)j * a.ldt + b] : 0.f;
+      }
+#pragma unroll
+      for (int u = 0; u < kRowsSh; ++u) {
+        if (!ok[u]) continue;
+        const float v = kAdv ? a.alpha * z[u] : z[u];
+        if (v > m) {
+          S = S * expf(m - v) + 1.f;
+          m = v;
+        } else {
+          S += expf(v - m);
+        }
+        if (kCe) Z += (double)z[u];
+      }
+    }
+    sh_m[warp][lane] = m;
+    sh_s[warp][lane] = S;
+    sh_z[warp][lane] = Z;
+    __syncthreads();
+    if (warp == 0) {
+      float M = -INFINITY;
+      for (int w = 0; w < kWarpsSh; ++w) M = fmaxf(M, sh_m[w][lane]);
+      float St = 0.f;
+      double Zt = 0.0;
+      for (int w = 0; w < kWarpsSh; ++w) {
+        if (sh_s[w][lane] > 0.f) St += sh_s[w][lane] * expf(sh_m[w][lane] - M);
+        Zt += sh_z[w][lane];
+      }
+      q_m[lane] = M;
+      q_s[lane] = St;
+      sh_z[0][lane] = Zt;
+    }
+    __syncthreads();
+  }
+  for (int qw = warp; qw < 32; qw += kWarpsSh) {                 // B: the positives of query b0 + qw
+    const int64_t bq = b0 + qw;
+    if (bq < a.B) {
+      const int D4 = a.D4;
+      const float4 zero = make_float4(0.f, 0.f, 0.f, 0.f);
+      float4 acc[NV];
+#pragma unroll
+      for (int v = 0; v < NV; ++v) acc[v] = zero;
+      const int32_t* pc = a.pos_cand + bq * a.n_pos;
+      int n_p = 0;
+      for (int c = lane; c < a.n_pos; c += 32) n_p += slot_valid(pc[c], a.n_ent) ? 1 : 0;
+      n_p = __reduce_add_sync(kFull, n_p);
+      const int n_q = a.nq[bq];
+      // CeLoss's per-query constants (CeLoss::State::finish)
+      const float inv_p = a.counts[0] > 0 ? (float)(1.0 / (double)a.counts[0]) : 0.f;
+      float cp = 0.f;                                            // the positives' coefficient of BCE / AdvLoss
+      if (kAdv) cp = n_p > 0 ? (float)(1.0 / (2.0 * (double)a.counts[0] * (double)n_p)) : 0.f;
+      else if (!kCe) cp = inv_p;                                 // BceLoss: 1 / the valid slots
+      float R = 0.f;
+      double lsum = 0.0;
+      for (int c = 0; c < a.n_pos; ++c) {
+        const int32_t e = pc[c];
+        float gv = 0.f;
+        if (slot_valid(e, a.n_ent)) {
+          float4 r[NV];
+          float dot = 0.f;                                       // warp_dot with the x columns held one at a time
+#pragma unroll
+          for (int v = 0; v < NV; ++v) {
+            const int c4 = lane + 32 * v;
+            r[v] = c4 < D4 ? ldg4(a.ent + (int64_t)e * a.ld_ent + 4 * c4) : zero;
+            const float4 xv = c4 < D4 ? ldg4(a.x + bq * 4 * D4 + 4 * c4) : zero;
+            dot = fmaf(xv.x, r[v].x, dot);
+            dot = fmaf(xv.y, r[v].y, dot);
+            dot = fmaf(xv.z, r[v].z, dot);
+            dot = fmaf(xv.w, r[v].w, dot);
+          }
+#pragma unroll
+          for (int o = 16; o > 0; o >>= 1) dot += __shfl_xor_sync(kFull, dot, o);
+          const float zp = dot + __ldg(a.bias + e);
+          if constexpr (kCe) {
+            const float m = q_m[qw], S = q_s[qw];
+            float q_mass, rp, lse_z;
+            if (zp >= m) {
+              const float em = expf(m - zp);
+              const float t = S * em;
+              q_mass = t / (1.f + t);
+              rp = em / (1.f + t);
+              lse_z = log1pf(t);
+            } else {
+              const float ep = expf(zp - m);
+              q_mass = S / (ep + S);
+              rp = 1.f / (ep + S);
+              lse_z = (m - zp) + logf(ep + S);
+            }
+            R += rp;
+            lsum += (double)lse_z + (double)a.eps * ((double)n_q * (double)zp - sh_z[0][qw]) / (double)(1 + n_q);
+            gv = (a.eps * (float)n_q * (1.f / (float)(1 + n_q)) - q_mass) * inv_p;    // eps (1 - 1 / K_b) - ...
+          } else {
+            const float p = 1.f / (1.f + expf(-zp));
+            lsum += (double)bce_loss_term(p, a.pos);
+            gv = bce_logit_grad(p, a.pos, cp);
+          }
+#pragma unroll
+          for (int v = 0; v < NV; ++v) fma4(gv, r[v], acc[v]);
+        }
+        if (lane == 0) a.g_pos[bq * a.n_pos + c] = gv;
+      }
+#pragma unroll
+      for (int v = 0; v < NV; ++v) {
+        const int c4 = lane + 32 * v;
+        if (c4 < D4) *reinterpret_cast<float4*>(a.d_x + bq * 4 * D4 + 4 * c4) = acc[v];
+      }
+      if (lane == 0) loss[0] += kAdv ? (n_p > 0 ? lsum / (double)n_p : 0.0) : lsum;
+      if (lane == 0) {                                           // the negatives' coefficients of this query
+        if (kAdv) {
+          q_c[qw] = q_s[qw] > 0.f ? (float)(1.0 / (2.0 * (double)a.counts[1] * (double)q_s[qw])) : 0.f;
+        } else if (kCe) {
+          q_r[qw] = R * inv_p;
+          q_c[qw] = (float)n_p * a.eps * (1.f / (float)(1 + n_q)) * inv_p;    // |P_b| eps / K_b / P
+        } else {
+          q_c[qw] = inv_p;
+        }
+      }
+    }
+  }
+  __syncthreads();
+  {                                                              // C: the negatives' gradient over the logit tile
+    const float c_neg = in_batch ? q_c[lane] : 0.f;
+    const float m = (kAdv || kCe) && in_batch ? q_m[lane] : 0.f;
+    const float r_q = kCe && in_batch ? q_r[lane] : 0.f;
+    double ln = 0.0;
+    for (int j0 = warp; j0 < a.k; j0 += kWarpsSh * kRowsSh) {
+      float z[kRowsSh];
+      bool ok[kRowsSh];
+#pragma unroll
+      for (int u = 0; u < kRowsSh; ++u) {
+        const int j = j0 + u * kWarpsSh;
+        ok[u] = j < a.k && shared_ok(a, j, in_batch, lane);
+        z[u] = ok[u] ? a.logit_t[(int64_t)j * a.ldt + b] : 0.f;
+      }
+#pragma unroll
+      for (int u = 0; u < kRowsSh; ++u) {
+        const int j = j0 + u * kWarpsSh;
+        if (j >= a.k) break;
+        float gv = 0.f;                                          // 0 on filtered and empty slots
+        if (ok[u]) {
+          if constexpr (kCe) {
+            gv = expf(z[u] - m) * r_q - c_neg;
+          } else {
+            const float p = 1.f / (1.f + expf(-z[u]));
+            const float term = bce_loss_term(p, a.add);
+            if constexpr (kAdv) {
+              const float w = expf(a.alpha * z[u] - m);
+              ln += (double)w * (double)term;
+              gv = bce_logit_grad(p, a.add, w * c_neg);
+            } else {
+              loss[0] += (double)term;
+              gv = bce_logit_grad(p, a.add, c_neg);
+            }
+          }
+        }
+        if (in_tile) a.logit_t[(int64_t)j * a.ldt + b] = gv;
+        const float gs = (float)warp_sum((double)gv);
+        if (lane == 0) a.bias_partial[(int64_t)blockIdx.x * a.k + j] = gs;
+      }
+    }
+    if constexpr (kAdv) loss[1] = in_batch && q_s[lane] > 0.f ? ln / (double)q_s[lane] : 0.0;
+  }
+  double s[H];
+#pragma unroll
+  for (int h = 0; h < H; ++h) s[h] = cta_sum(warp_sum(loss[h]), warp_loss[h], lane, warp);
+  if (threadIdx.x == 0) {
+#pragma unroll
+    for (int h = 0; h < H; ++h) a.loss_partial[h * gridDim.x + blockIdx.x] = s[h];
+  }
+}
+
+// d_bias_s[j] = sum over the CTAs of the pass of bias_partial[c, j], in CTA order
+__global__ void __launch_bounds__(kThreadsSS)
+shared_bias_kernel(const float* __restrict__ bias_partial, int64_t n_cta, int k, float* __restrict__ d_bias_s) {
+  const int64_t j = (int64_t)blockIdx.x * kThreadsSS + threadIdx.x;
+  if (j >= k) return;
+  float s = 0.f;
+  for (int64_t c = 0; c < n_cta; ++c) s += bias_partial[c * k + j];
+  d_bias_s[j] = s;
+}
+
+// d_ent[n] += scale * sum over the shared slots j with shared[j] = n of d_rows[j], d_bias[n] likewise: a warp per 32
+// sorted positions takes every run of one id that starts there and adds its slots in slot order
+template <int NV>
+__global__ void __launch_bounds__(kThreadsSS)
+shared_table_kernel(const int32_t* __restrict__ ids, const int32_t* __restrict__ slots, int k, int64_t n_ent,
+                    const float* __restrict__ d_rows, int64_t ld_rows, const float* __restrict__ d_row_bias, int D4,
+                    const float* __restrict__ scale, float* __restrict__ d_ent, int64_t ld_d, float* __restrict__ d_bias) {
+  const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5;
+  const int64_t base = ((int64_t)blockIdx.x * kWarpsSS + warp) * 32;
+  if (base >= k) return;
+  const int64_t i = base + lane;
+  const int32_t key = i < k ? ids[i] : (int32_t)n_ent;
+  const int32_t prev = (i > 0 && i < k) ? ids[i - 1] : -1;
+  uint32_t heads = __ballot_sync(kFull, slot_valid(key, n_ent) && key != prev);
+  const float sc = *scale;
+  while (heads) {
+    const int h = __ffs(heads) - 1;
+    heads &= heads - 1;
+    const int32_t n = __shfl_sync(kFull, key, h);
+    float4 acc[NV];
+#pragma unroll
+    for (int v = 0; v < NV; ++v) acc[v] = make_float4(0.f, 0.f, 0.f, 0.f);
+    float bsum = 0.f;
+    for (int64_t j = base + h; j < k && ids[j] == n; ++j) {
+      const int32_t sl = slots[j];
+#pragma unroll
+      for (int v = 0; v < NV; ++v) {
+        const int c4 = lane + 32 * v;
+        if (c4 < D4) {
+          const float4 r = ldg4(d_rows + (int64_t)sl * ld_rows + 4 * c4);
+          acc[v].x += r.x;
+          acc[v].y += r.y;
+          acc[v].z += r.z;
+          acc[v].w += r.w;
+        }
+      }
+      bsum += d_row_bias[sl];
+    }
+#pragma unroll
+    for (int v = 0; v < NV; ++v) {
+      const int c4 = lane + 32 * v;
+      if (c4 < D4) {
+        float4* o = reinterpret_cast<float4*>(d_ent + (int64_t)n * ld_d + 4 * c4);
+        float4 t = *o;
+        t.x = fmaf(sc, acc[v].x, t.x);
+        t.y = fmaf(sc, acc[v].y, t.y);
+        t.z = fmaf(sc, acc[v].z, t.z);
+        t.w = fmaf(sc, acc[v].w, t.w);
+        *o = t;
+      }
+    }
+    if (lane == 0) d_bias[n] = fmaf(sc, bsum, d_bias[n]);
+  }
+}
+
+// the shared loss of one policy: zero its counts, count them, the pass, the shared slots' d_bias, the loss
+template <class Loss>
+cudaError_t launch_shared_loss(const SharedArgs& a, float* d_bias_s, float* loss, cudaStream_t s) {
+  cudaError_t err = cudaMemsetAsync(a.counts, 0, Loss::kHalves * sizeof(int32_t), s);
+  if (err != cudaSuccess) return err;
+  const int64_t blocks = kgc_shared_loss_blocks(a.B);
+  shared_count_kernel<Loss><<<(unsigned)blocks, kThreadsSS, 0, s>>>(a);
+  if ((err = cudaGetLastError()) != cudaSuccess) return err;
+  const auto pass = for_width(a.D4, shared_loss_kernel<Loss, 1>, shared_loss_kernel<Loss, 2>);
+  pass<<<(unsigned)blocks, kThreadsSh, 0, s>>>(a);
+  if ((err = cudaGetLastError()) != cudaSuccess) return err;
+  shared_bias_kernel<<<(unsigned)ceil_div(a.k, kThreadsSS), kThreadsSS, 0, s>>>(a.bias_partial, blocks, a.k, d_bias_s);
+  if ((err = cudaGetLastError()) != cudaSuccess) return err;
+  sampled_finalize_kernel<Loss::kHalves><<<1, kThreadsSS, 0, s>>>(a.loss_partial, blocks, a.counts, loss);
+  return cudaGetLastError();
+}
+
+// workspace of the shared loss: counts (2), nq [B], loss partials (2 x blocks doubles), bias partials [blocks, k]
+struct SharedWs {
+  size_t counts, nq, loss_partial, bias_partial, total;
+  SharedWs(int64_t B, int64_t k) {
+    const int64_t blocks = ceil_div(B, 32);
+    counts = 0;
+    nq = align_up(2 * sizeof(int32_t));
+    loss_partial = nq + align_up((size_t)B * sizeof(int32_t));
+    bias_partial = loss_partial + align_up((size_t)2 * blocks * sizeof(double));
+    total = bias_partial + align_up((size_t)blocks * k * sizeof(float));
+  }
+};
+
 }  // namespace
 }  // namespace kgc
 
@@ -683,6 +1091,139 @@ extern "C" int kgc_sampled_bce_bwd_table(const float* x, int64_t B, int32_t D, c
   const int D4 = D / 4;
   const auto grad = for_width(D4, table_grad_kernel<1>, table_grad_kernel<2>);
   grad<<<blocks, kThreadsSS, 0, s>>>(keys_out, slots_out, n_slots, n_ent, x, D4, C, g, scale, d_ent, ld_d, d_bias);
+  KGC_LAUNCH_CHECK();
+  return 0;
+}
+
+extern "C" size_t kgc_shared_mask_workspace_bytes(int32_t k, int64_t n_ent) {
+  if (k <= 0 || n_ent <= 0 || n_ent >= (int64_t{1} << 31) - 1) return 0;
+  size_t temp = 0;
+  if (sort_temp_bytes(k, n_ent, &temp) != cudaSuccess) return 0;
+  return 2 * align_up((size_t)k * sizeof(int32_t)) + align_up(temp);
+}
+
+extern "C" int kgc_shared_mask_build(const int32_t* shared, int32_t k, const int64_t* qid, int64_t B, const int64_t* ptr,
+                                     const int32_t* idx, int64_t n_ent, uint32_t* mask_t, int32_t* sorted_ids,
+                                     int32_t* sorted_slots, void* workspace, size_t workspace_bytes, void* stream) {
+  KGC_REQUIRE(k > 0 && B > 0 && n_ent > 0 && n_ent < (int64_t{1} << 31) - 1, "bad sizes (k, B > 0, 0 < N < 2^31 - 1)");
+  KGC_REQUIRE(shared && qid && ptr && idx && mask_t && sorted_ids && sorted_slots && workspace, "null buffer");
+  const size_t need = kgc_shared_mask_workspace_bytes(k, n_ent);
+  KGC_REQUIRE(need > 0 && workspace_bytes >= need, "workspace too small (kgc_shared_mask_workspace_bytes)");
+  cudaStream_t s = as_stream(stream);
+  const size_t arr = align_up((size_t)k * sizeof(int32_t));
+  uint8_t* w = static_cast<uint8_t*>(workspace);
+  int32_t* keys_in = reinterpret_cast<int32_t*>(w);
+  int32_t* slots_in = reinterpret_cast<int32_t*>(w + arr);
+  const int64_t W = ceil_div(B, 32);
+  KGC_CUDA_TRY(cudaMemsetAsync(mask_t, 0, (size_t)k * W * sizeof(uint32_t), s));
+  slot_keys_kernel<<<(unsigned)ceil_div(k, kThreadsSS), kThreadsSS, 0, s>>>(shared, k, n_ent, keys_in, slots_in);
+  KGC_LAUNCH_CHECK();
+  size_t temp_bytes = workspace_bytes - 2 * arr;
+  KGC_CUDA_TRY(cub::DeviceRadixSort::SortPairs(w + 2 * arr, temp_bytes, keys_in, sorted_ids, slots_in, sorted_slots, (int)k,
+                                               0, key_bits(n_ent), s));
+  shared_mask_kernel<<<(unsigned)ceil_div(B, kWarpsSS), kThreadsSS, 0, s>>>(sorted_ids, k, qid, B, ptr, idx, n_ent,
+                                                                            sorted_slots, mask_t, W);
+  KGC_LAUNCH_CHECK();
+  return 0;
+}
+
+extern "C" int kgc_shared_rows(const float* ent, int64_t n_ent, int32_t D, int64_t ld_ent, const float* bias,
+                               const int32_t* shared, int32_t k, float* rows, float* row_bias, void* stream) {
+  KGC_REQUIRE(k > 0 && n_ent > 0 && D > 0 && D % 4 == 0 && ld_ent >= D && ld_ent % 4 == 0, "bad sizes");
+  KGC_REQUIRE(ent && bias && shared && rows && row_bias, "null buffer");
+  KGC_REQUIRE(((reinterpret_cast<uintptr_t>(ent) | reinterpret_cast<uintptr_t>(rows)) & 15) == 0,
+              "all_ent and rows must be 16-byte aligned");
+  const int64_t n4 = (int64_t)k * (D / 4);
+  shared_rows_kernel<<<(unsigned)ceil_div(n4, kThreadsSS), kThreadsSS, 0, as_stream(stream)>>>(
+      ent, ld_ent, bias, n_ent, shared, k, D / 4, rows, row_bias);
+  KGC_LAUNCH_CHECK();
+  return 0;
+}
+
+extern "C" int64_t kgc_shared_loss_blocks(int64_t B) { return ceil_div(B > 0 ? B : 1, 32); }
+
+extern "C" size_t kgc_shared_loss_workspace_bytes(int64_t B, int32_t k) {
+  if (B <= 0 || k <= 0) return 0;
+  return SharedWs(B, k).total;
+}
+
+namespace kgc {
+namespace {
+
+template <class Loss>
+int shared_loss_entry(const char* fn, float* logit_t, int64_t ldt, const uint32_t* mask_t, const int32_t* shared, int32_t k,
+                      const float* x, int64_t B, int32_t D, const float* ent, int64_t n_ent, int64_t ld_ent,
+                      const float* bias, const int32_t* pos_cand, int32_t n_pos, float pos, float add, float alpha,
+                      float eps, float* g_pos, float* d_x, float* d_bias_s, float* loss, void* workspace,
+                      size_t workspace_bytes, void* stream) {
+  if (!(k > 0 && n_pos > 0 && B > 0 && B * (int64_t)k < (int64_t{1} << 31) && D > 0 && D <= 256 && D % 4 == 0 &&
+        n_ent > 0 && n_ent < (int64_t{1} << 31) - 1 && ldt >= B && ld_ent >= D && ld_ent % 4 == 0))
+    return fail(fn, "bad sizes (k, n_pos, B > 0, B * k < 2^31, 0 < D <= 256, D % 4 == 0, ldt >= B, ld_ent >= D, "
+                    "ld_ent % 4 == 0)");
+  if (!(logit_t && mask_t && shared && x && ent && bias && pos_cand && g_pos && d_x && d_bias_s && loss && workspace))
+    return fail(fn, "null buffer");
+  if (((reinterpret_cast<uintptr_t>(x) | reinterpret_cast<uintptr_t>(ent) | reinterpret_cast<uintptr_t>(d_x)) & 15) != 0)
+    return fail(fn, "x, all_ent and d_x must be 16-byte aligned");
+  const SharedWs ws(B, k);
+  if (workspace_bytes < ws.total) return fail(fn, "workspace too small (kgc_shared_loss_workspace_bytes)");
+  uint8_t* w = static_cast<uint8_t*>(workspace);
+  const SharedArgs a{logit_t, ldt, mask_t, ceil_div(B, 32), shared, k, x, B, D / 4, ent, ld_ent, n_ent, bias, pos_cand,
+                     n_pos, pos, add, alpha, eps, g_pos, d_x,
+                     reinterpret_cast<int32_t*>(w + ws.counts), reinterpret_cast<int32_t*>(w + ws.nq),
+                     reinterpret_cast<double*>(w + ws.loss_partial), reinterpret_cast<float*>(w + ws.bias_partial)};
+  const cudaError_t err = launch_shared_loss<Loss>(a, d_bias_s, loss, as_stream(stream));
+  if (err != cudaSuccess) return fail(fn, std::string("launch -> ") + cudaGetErrorString(err));
+  return 0;
+}
+
+}  // namespace
+}  // namespace kgc
+
+extern "C" int kgc_shared_bce_loss(float* logit_t, int64_t ldt, const uint32_t* mask_t, const int32_t* shared, int32_t k,
+                                   const float* x, int64_t B, int32_t D, const float* ent, int64_t n_ent, int64_t ld_ent,
+                                   const float* bias, const int32_t* pos_cand, int32_t n_pos, float pos, float add,
+                                   float* g_pos, float* d_x, float* d_bias_s, float* loss, void* workspace,
+                                   size_t workspace_bytes, void* stream) {
+  return shared_loss_entry<BceLoss>(__func__, logit_t, ldt, mask_t, shared, k, x, B, D, ent, n_ent, ld_ent, bias, pos_cand,
+                                    n_pos, pos, add, 0.f, 0.f, g_pos, d_x, d_bias_s, loss, workspace, workspace_bytes,
+                                    stream);
+}
+
+extern "C" int kgc_shared_adv_loss(float* logit_t, int64_t ldt, const uint32_t* mask_t, const int32_t* shared, int32_t k,
+                                   const float* x, int64_t B, int32_t D, const float* ent, int64_t n_ent, int64_t ld_ent,
+                                   const float* bias, const int32_t* pos_cand, int32_t n_pos, float pos, float add,
+                                   float temperature, float* g_pos, float* d_x, float* d_bias_s, float* loss,
+                                   void* workspace, size_t workspace_bytes, void* stream) {
+  KGC_REQUIRE(std::isfinite(temperature) && temperature >= 0.f, "the adversarial temperature must be finite and >= 0");
+  return shared_loss_entry<AdvLoss>(__func__, logit_t, ldt, mask_t, shared, k, x, B, D, ent, n_ent, ld_ent, bias, pos_cand,
+                                    n_pos, pos, add, temperature, 0.f, g_pos, d_x, d_bias_s, loss, workspace,
+                                    workspace_bytes, stream);
+}
+
+extern "C" int kgc_shared_ce_loss(float* logit_t, int64_t ldt, const uint32_t* mask_t, const int32_t* shared, int32_t k,
+                                  const float* x, int64_t B, int32_t D, const float* ent, int64_t n_ent, int64_t ld_ent,
+                                  const float* bias, const int32_t* pos_cand, int32_t n_pos, float label_smoothing,
+                                  float* g_pos, float* d_x, float* d_bias_s, float* loss, void* workspace,
+                                  size_t workspace_bytes, void* stream) {
+  KGC_REQUIRE(label_smoothing >= 0.f && label_smoothing <= 1.f, "the label smoothing must be a number in [0, 1]");
+  return shared_loss_entry<CeLoss>(__func__, logit_t, ldt, mask_t, shared, k, x, B, D, ent, n_ent, ld_ent, bias, pos_cand,
+                                   n_pos, 0.f, 0.f, 0.f, label_smoothing, g_pos, d_x, d_bias_s, loss, workspace,
+                                   workspace_bytes, stream);
+}
+
+extern "C" int kgc_shared_bwd_table(const int32_t* sorted_ids, const int32_t* sorted_slots, int32_t k, int64_t n_ent,
+                                    int32_t D, const float* d_rows, int64_t ld_rows, const float* d_row_bias,
+                                    const float* scale, float* d_ent, int64_t ld_d, float* d_bias, void* stream) {
+  KGC_REQUIRE(k > 0 && n_ent > 0 && n_ent < (int64_t{1} << 31) - 1 && D > 0 && D <= 256 && D % 4 == 0, "bad sizes");
+  KGC_REQUIRE(ld_rows >= D && ld_rows % 4 == 0 && ld_d >= D && ld_d % 4 == 0, "rows need a 16-byte pitch of >= D floats");
+  KGC_REQUIRE(sorted_ids && sorted_slots && d_rows && d_row_bias && scale && d_ent && d_bias, "null buffer");
+  KGC_REQUIRE(((reinterpret_cast<uintptr_t>(d_rows) | reinterpret_cast<uintptr_t>(d_ent)) & 15) == 0,
+              "d_rows and d_ent must be 16-byte aligned");
+  const unsigned blocks = (unsigned)ceil_div(ceil_div(k, 32), kWarpsSS);
+  const int D4 = D / 4;
+  const auto add = for_width(D4, shared_table_kernel<1>, shared_table_kernel<2>);
+  add<<<blocks, kThreadsSS, 0, as_stream(stream)>>>(sorted_ids, sorted_slots, k, n_ent, d_rows, ld_rows, d_row_bias, D4,
+                                                    scale, d_ent, ld_d, d_bias);
   KGC_LAUNCH_CHECK();
   return 0;
 }

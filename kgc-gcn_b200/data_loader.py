@@ -266,6 +266,24 @@ class KBDataset(object):
             _lib.call('kgc_neg_sample', p(qid), b, p(ptr), p(idx), self.num_entity, p(d32), int(k), int(tries), p(neg), _lib.stream())
         return neg
 
+    def shared_negatives(self, k, draws=None, device='cuda', generator=None):
+        """Batch-shared negatives for ``scoring.score_shared_bce`` / ``score_shared_ce``: ``k`` entity ids drawn uniformly
+        with replacement -> int32 [k] on ``device``, id = (u * N) >> 32.  Nothing is filtered here (the loss leaves out each
+        query's known objects).  A pure function of ``draws`` (uint32 [k]); when omitted they come from torch's generator
+        (``generator`` or the global one on the device)."""
+        if isinstance(k, bool) or int(k) != k or k < 1:
+            raise ValueError('k must be a positive integer, got {!r}'.format(k))
+        device = torch.device(device)
+        if device.type != 'cuda':
+            raise RuntimeError('the shared negative sampler runs on the GPU only (no CPU fallback)')
+        if draws is None:
+            draws = torch.randint(0, 1 << 32, (int(k),), dtype=torch.int64, device=device, generator=generator)
+        draws = torch.as_tensor(draws).to(device)
+        if tuple(draws.shape) != (int(k),):
+            raise ValueError('draws must be [k]')
+        u = _u32_bits(draws).to(torch.int64) & 0xFFFFFFFF
+        return ((u * self.num_entity) >> 32).to(torch.int32)
+
     def positives(self, qid, p, draws=None, device='cuda', generator=None):
         """GPU positive sampler, the companion of ``negatives``: ``p`` of each query's known objects, drawn with replacement
         from its object list (the training queries are (s, r, -1): the objects come from the lists, not the triple) ->

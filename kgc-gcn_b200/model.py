@@ -306,7 +306,7 @@ class MGCN(nn.Module):
         return score_1n_bce(x, all_ent, self.conv2.bias, qid, ptr, idx, pos, add)
 
     def loss_sampled(self, qid, dataset, data, k, n_pos=1, tries=4, draws=None, generator=None, adversarial_temperature=None,
-                     criterion='bce', label_smoothing=0.0):
+                     criterion='bce', label_smoothing=0.0, shared_negatives=False):
         """Negative-sampled (1-vs-k) training loss for the training queries ``qid`` of ``dataset`` (a KBDataset): each query
         scores ``n_pos`` of its known objects (``dataset.positives``) and ``k`` entities that are not (``dataset.negatives``,
         ``tries`` draws per slot) - candidates [pos | neg] - through ``scoring.score_sampled_bce`` with the dataset's
@@ -317,13 +317,31 @@ class MGCN(nn.Module):
         negative sampling, see ``scoring.score_sampled_bce``); None: the plain mean over the valid slots.
         ``criterion='ce'`` trains each positive's softmax cross-entropy against its query's negatives instead
         (``scoring.score_sampled_ce``, with ``label_smoothing`` eps in [0, 1]; the dataset's label values do not enter).
-        A temperature with 'ce', a label smoothing with 'bce' or another criterion is a ValueError."""
-        from .scoring import check_sampled_criterion, score_sampled_bce, score_sampled_ce
+        A temperature with 'ce', a label smoothing with 'bce' or another criterion is a ValueError.
+        ``shared_negatives=True`` draws ONE set of k negatives for the whole batch (``dataset.shared_negatives``, draws
+        ``(pos_draws [B, n_pos], neg_draws [k])``) and scores every query against it, each query's known objects left out
+        (``scoring.score_shared_bce`` / ``score_shared_ce``, with the same criteria and options): the shared rows are read
+        once per batch, so k can be in the thousands.  ``tries`` does not apply to it (a value other than 4 is a
+        ValueError)."""
+        from .scoring import check_sampled_criterion, score_sampled_bce, score_sampled_ce, score_shared_bce, score_shared_ce
         _, eps = check_sampled_criterion(criterion, adversarial_temperature, label_smoothing)
+        if shared_negatives and tries != 4:
+            raise ValueError('tries redraws the per-query negatives that hit a known object; shared negatives are filtered '
+                             'instead (leave tries at its default)')
         dev = self.entity_embedding.device
-        triples, _, _ = dataset.device_csr(dev)
+        triples, ptr, idx = dataset.device_csr(dev)
         qid = torch.as_tensor(qid, dtype=torch.int64).to(dev, non_blocking=True)
         pos_draws, neg_draws = draws if draws is not None else (None, None)
+        if shared_negatives:
+            # drawn before encode, positives first, as below
+            pos_cand = dataset.positives(qid, n_pos, draws=pos_draws, device=dev, generator=generator)
+            shared = dataset.shared_negatives(k, draws=neg_draws, device=dev, generator=generator)
+            _, x, all_ent = self._train_queries(qid, triples, data)
+            if criterion == 'ce':
+                return score_shared_ce(x, all_ent, self.conv2.bias, pos_cand, shared, qid, ptr, idx, eps)
+            pos, add = dataset.label_values()
+            return score_shared_bce(x, all_ent, self.conv2.bias, pos_cand, shared, qid, ptr, idx, pos, add,
+                                    adversarial_temperature=adversarial_temperature)
         # drawn before encode, which may also draw from torch's generator: this order fixes the random stream
         cand = torch.cat([dataset.positives(qid, n_pos, draws=pos_draws, device=dev, generator=generator),
                           dataset.negatives(qid, k, draws=neg_draws, tries=tries, device=dev, generator=generator)], 1)

@@ -297,6 +297,177 @@ def _check_sampled_args(fn, x, all_ent, bias, cand, n_pos):
         raise ValueError('cand holds entity ids >= N = {}'.format(N))
 
 
+# each shared loss: its C pass
+_SHARED_LOSS = {'bce': 'kgc_shared_bce_loss', 'adv': 'kgc_shared_adv_loss', 'ce': 'kgc_shared_ce_loss'}
+
+
+class _ScoreShared(torch.autograd.Function):
+    """The sampled loss ``kind`` of ``_ScoreSampled`` on the broadcast candidates [pos_cand[b] | shared, filtered by query
+    b's known objects], with the shared part on the tensor cores: the k gathered rows E_S are scored against the batch
+    tile by tile (entity-major logitT [k, ldb], kgc_score_1n_logits_t), the loss pass overwrites the tile with the logit
+    gradient and yields the positives' gradient g_pos and d_x part.  The backward scales by the upstream scalar: d_x =
+    g_T^T E_S + the positives' part, d_E_S = the per-tile g_T x products added in tile order, and the table gradient is
+    the positives' (kgc_sampled_bce_bwd_table, which zero-fills) plus the shared rows added through the sorted ids."""
+
+    @staticmethod
+    def forward(ctx, x, all_ent, bias, pos_cand, shared, qid, ptr, idx, kind, scalars):
+        x = _lib.require_cuda(x.detach(), torch.float32, 'x').contiguous()
+        ent = all_ent.detach()
+        if ent.dtype != torch.float32:
+            raise TypeError('all_ent must be torch.float32, got {}'.format(ent.dtype))
+        if ent.stride(1) != 1 or ent.stride(0) % 4 != 0 or ent.data_ptr() % 16 != 0:
+            ent = ent.clone(memory_format=torch.contiguous_format)
+        bias_ = _lib.require_cuda(bias.detach(), torch.float32, 'bias').contiguous()
+        pos_cand = _lib.require_cuda(pos_cand, torch.int32, 'pos_cand').contiguous()
+        shared = _lib.require_cuda(shared, torch.int32, 'shared').contiguous()
+        qid = _lib.require_cuda(qid, torch.int64, 'qid').contiguous()
+        ptr = _lib.require_cuda(ptr, torch.int64, 'ptr')
+        idx = _lib.require_cuda(idx, torch.int32, 'idx')
+        B, D, N = int(x.shape[0]), int(x.shape[1]), int(ent.shape[0])
+        n_pos, k = int(pos_cand.shape[1]), int(shared.numel())
+        dev, p, lib = x.device, _lib.ptr, _lib.lib()
+        ldb = (B + 31) // 32 * 32                       # a whole 32-query group per column block of the loss pass
+        rows = torch.empty((k, D), dtype=torch.float32, device=dev)
+        row_bias = torch.empty((k,), dtype=torch.float32, device=dev)
+        _lib.call('kgc_shared_rows', p(ent), N, D, ent.stride(0), p(bias_), p(shared), k, p(rows), p(row_bias), _lib.stream())
+        logit_t = torch.empty((k, ldb), dtype=torch.float32, device=dev)
+        for i in range(0, B, B_TILE):
+            bt = min(B_TILE, B - i)
+            _lib.call('kgc_score_1n_logits_t', p(rows), k, D, D, p(_pack_b(x[i:i + bt].t())), bt, p(row_bias),
+                      p(logit_t[:, i:]), ldb, _lib.stream())
+        mask_t = torch.empty((k, ldb // 32), dtype=torch.int32, device=dev)
+        ids = torch.empty((k,), dtype=torch.int32, device=dev)
+        slots = torch.empty((k,), dtype=torch.int32, device=dev)
+        ws_bytes = int(lib.kgc_shared_mask_workspace_bytes(k, N))
+        ws = torch.empty((ws_bytes,), dtype=torch.uint8, device=dev)
+        _lib.call('kgc_shared_mask_build', p(shared), k, p(qid), B, p(ptr), p(idx), N, p(mask_t), p(ids), p(slots), p(ws),
+                  ws_bytes, _lib.stream())
+        g_pos = torch.empty((B, n_pos), dtype=torch.float32, device=dev)
+        d_x = torch.empty((B, D), dtype=torch.float32, device=dev)
+        d_bias_s = torch.empty((k,), dtype=torch.float32, device=dev)
+        loss = torch.empty((1,), dtype=torch.float32, device=dev)
+        ws_bytes = int(lib.kgc_shared_loss_workspace_bytes(B, k))
+        ws = torch.empty((ws_bytes,), dtype=torch.uint8, device=dev)
+        _lib.call(_SHARED_LOSS[kind], p(logit_t), ldb, p(mask_t), p(shared), k, p(x), B, D, p(ent), N, ent.stride(0),
+                  p(bias_), p(pos_cand), n_pos, *(float(v) for v in scalars), p(g_pos), p(d_x), p(d_bias_s), p(loss), p(ws),
+                  ws_bytes, _lib.stream())
+        ctx.save_for_backward(x, rows, logit_t, pos_cand, g_pos, d_x, d_bias_s, ids, slots)
+        ctx.n_ent = N
+        return loss[0]
+
+    @staticmethod
+    def backward(ctx, d_loss):
+        from .conv import gemm_nt, gemm_tn
+        x, rows, g_t, pos_cand, g_pos, d_x_pos, d_bias_s, ids, slots = ctx.saved_tensors
+        B, D, N = int(x.shape[0]), int(x.shape[1]), ctx.n_ent
+        k, ldb, n_pos = int(rows.shape[0]), int(g_t.shape[1]), int(pos_cand.shape[1])
+        dev, p = x.device, _lib.ptr
+        d_x = d_ent = d_bias = None
+        if ctx.needs_input_grad[0]:
+            d_x = (gemm_tn(g_t, rows, torch.empty((ldb, D), dtype=torch.float32, device=dev))[:B] + d_x_pos) * d_loss
+        if ctx.needs_input_grad[1] or ctx.needs_input_grad[2]:
+            scale = d_loss.reshape(1).to(torch.float32).contiguous()
+            d_rows = torch.empty((k, D), dtype=torch.float32, device=dev)
+            part = torch.empty((k, D), dtype=torch.float32, device=dev) if B > B_TILE else None
+            for i in range(0, B, B_TILE):               # the tiles' products added in tile order
+                bt = min(B_TILE, B - i)
+                gemm_nt(g_t[:, i:i + bt], x[i:i + bt], d_rows if i == 0 else part)
+                if i > 0:
+                    d_rows += part
+            d_ent = torch.empty((N, D), dtype=torch.float32, device=dev)
+            d_bias = torch.empty((N,), dtype=torch.float32, device=dev)
+            ws_bytes = int(_lib.lib().kgc_sampled_bce_bwd_table_workspace_bytes(B * n_pos, N))
+            ws = torch.empty((ws_bytes,), dtype=torch.uint8, device=dev)
+            _lib.call('kgc_sampled_bce_bwd_table', p(x), B, D, p(pos_cand), n_pos, p(g_pos), p(scale), N, p(d_ent), D,
+                      p(d_bias), p(ws), ws_bytes, _lib.stream())
+            _lib.call('kgc_shared_bwd_table', p(ids), p(slots), k, N, D, p(d_rows), D, p(d_bias_s), p(scale), p(d_ent), D,
+                      p(d_bias), _lib.stream())
+        return (d_x, d_ent if ctx.needs_input_grad[1] else None, d_bias if ctx.needs_input_grad[2] else None,
+                None, None, None, None, None, None, None)
+
+
+def score_shared_bce(x, all_ent, bias, pos_cand, shared, qid, ptr, idx, pos=1.0, add=0.0, adversarial_temperature=None):
+    """``score_sampled_bce`` with batch-shared negatives: query b of ``x`` [B, D] scores its positives ``pos_cand``
+    [B, n_pos] (int32, -1 an empty slot, e.g. ``KBDataset.positives``) and the ``k`` entities ``shared`` (int32 [k], e.g.
+    ``KBDataset.shared_negatives``) that every query shares, each with the entries that are known objects of query
+    ``qid[b]`` (the query -> objects CSR ``ptr`` int64 / ``idx`` int32 that ``score_1n_bce`` takes) left out.  The value
+    and the gradients are exactly those of ``score_sampled_bce`` on the candidates [pos_cand[b] | shared with the known
+    objects of qid[b] set to -1] (duplicates in ``shared`` count as separate slots; a filtered entry is an empty slot of
+    that query only).  The k x B logits are one dense product on the tensor cores, so each shared row is read once per
+    batch instead of once per query: thousands of negatives per query cost about what the per-query path pays for
+    hundreds.  D % 4 == 0, D <= 224; deterministic and graph-capturable."""
+    temperature = check_adversarial_temperature(adversarial_temperature)
+    _check_shared_args('score_shared_bce', x, all_ent, bias, pos_cand, shared, qid, ptr, idx)
+    if temperature is None:
+        return _ScoreShared.apply(x, all_ent, bias, pos_cand, shared, qid, ptr, idx, 'bce', (pos, add))
+    return _ScoreShared.apply(x, all_ent, bias, pos_cand, shared, qid, ptr, idx, 'adv', (pos, add, temperature))
+
+
+def score_shared_ce(x, all_ent, bias, pos_cand, shared, qid, ptr, idx, label_smoothing=0.0):
+    """``score_sampled_ce`` with batch-shared negatives: each valid positive of ``pos_cand`` [B, n_pos] is classified
+    against the ``shared`` [k] entities that are not known objects of its query (see ``score_shared_bce`` for the
+    candidate layout and the arguments).  The value and gradients are those of ``score_sampled_ce`` on the broadcast
+    candidates; the log-sum-exp runs against each query's max, so logits of any size are safe."""
+    eps = check_label_smoothing(label_smoothing)
+    _check_shared_args('score_shared_ce', x, all_ent, bias, pos_cand, shared, qid, ptr, idx)
+    return _ScoreShared.apply(x, all_ent, bias, pos_cand, shared, qid, ptr, idx, 'ce', (eps,))
+
+
+def shared_candidates(pos_cand, shared, qid, ptr, idx):
+    """The broadcast candidate matrix that defines the shared losses: int32 [B, n_pos + k], row b = [pos_cand[b] | shared
+    with every entry that is a known object of query qid[b] set to -1] (torch ops, any device: a reference, not the
+    training path)."""
+    pos_cand = torch.as_tensor(pos_cand).to(torch.int32)
+    shared = torch.as_tensor(shared, device=pos_cand.device).to(torch.int32).reshape(-1)
+    qid = torch.as_tensor(qid, device=pos_cand.device).to(torch.int64).reshape(-1)
+    ptr = torch.as_tensor(ptr, device=pos_cand.device).to(torch.int64)
+    idx = torch.as_tensor(idx, device=pos_cand.device).to(torch.int64)
+    B, k = int(pos_cand.shape[0]), int(shared.numel())
+    lens = ptr[qid + 1] - ptr[qid]
+    rows = torch.repeat_interleave(torch.arange(B, device=pos_cand.device), lens)
+    starts = torch.repeat_interleave(ptr[qid], lens)
+    offs = torch.arange(int(lens.sum()), device=pos_cand.device) - torch.repeat_interleave(torch.cumsum(lens, 0) - lens, lens)
+    known = torch.zeros((B, k), dtype=torch.int32, device=pos_cand.device)
+    objs = idx[starts + offs]
+    known.index_add_(0, rows, (objs[:, None] == shared[None, :].to(torch.int64)).to(torch.int32))    # [nnz, k] hits
+    neg = torch.where(known > 0, torch.full_like(shared, -1)[None, :].expand(B, k), shared[None, :].expand(B, k))
+    return torch.cat([pos_cand, neg], 1)
+
+
+def _check_shared_args(fn, x, all_ent, bias, pos_cand, shared, qid, ptr, idx):
+    """The shapes, dtypes and devices the shared-negative losses take (``fn`` names the caller in the messages)."""
+    if x.dim() != 2 or all_ent.dim() != 2 or bias.dim() != 1 or pos_cand.dim() != 2 or shared.dim() != 1:
+        raise ValueError('{} takes x [B, D], all_ent [N, D], bias [N], pos_cand [B, n_pos] and shared [k]'.format(fn))
+    B, D = int(x.shape[0]), int(x.shape[1])
+    N, n_pos, k = int(all_ent.shape[0]), int(pos_cand.shape[1]), int(shared.shape[0])
+    if int(all_ent.shape[1]) != D or int(bias.shape[0]) != N or int(pos_cand.shape[0]) != B or qid.dim() != 1 \
+            or int(qid.shape[0]) != B:
+        raise ValueError('shape mismatch: x {}, all_ent {}, bias {}, pos_cand {}, qid {}'.format(
+            tuple(x.shape), tuple(all_ent.shape), tuple(bias.shape), tuple(pos_cand.shape), tuple(qid.shape)))
+    if B < 1 or N < 1 or D < 4 or D > 224 or D % 4 != 0:
+        raise ValueError('{} needs B, N >= 1 and D % 4 == 0, D <= 224 (got B={}, N={}, D={})'.format(fn, B, N, D))
+    if k < 1 or n_pos < 1:
+        raise ValueError('{} needs k >= 1 shared negatives and n_pos >= 1 positive columns (got k={}, n_pos={})'.format(
+            fn, k, n_pos))
+    if pos_cand.dtype != torch.int32 or shared.dtype != torch.int32 or idx.dtype != torch.int32:
+        raise ValueError('pos_cand, shared and idx must be torch.int32, got {}, {}, {}'.format(
+            pos_cand.dtype, shared.dtype, idx.dtype))
+    if qid.dtype != torch.int64 or ptr.dtype != torch.int64:
+        raise ValueError('qid and ptr must be torch.int64, got {}, {}'.format(qid.dtype, ptr.dtype))
+    if B * k >= 2 ** 31 or B * n_pos >= 2 ** 31 or N >= 2 ** 31 - 1:
+        raise ValueError('{} takes B * k < 2^31 slots and N < 2^31 - 1 entities'.format(fn))
+    for t, name in ((x, 'x'), (all_ent, 'all_ent'), (bias, 'bias'), (pos_cand, 'pos_cand'), (shared, 'shared'),
+                    (qid, 'qid'), (ptr, 'ptr'), (idx, 'idx')):
+        if not t.is_cuda:
+            raise RuntimeError('{} must be a CUDA tensor: the M-GCN hot path runs on the GPU only (no CPU fallback)'.format(name))
+    if not torch.cuda.is_current_stream_capturing():
+        # (not checked while a CUDA graph is captured: the checks read back; the kernels treat such ids as empty slots)
+        if bool(((shared < 0) | (shared >= N)).any()):
+            raise ValueError('shared holds entity ids outside [0, N = {})'.format(N))
+        if bool((pos_cand >= N).any()):
+            raise ValueError('pos_cand holds entity ids >= N = {}'.format(N))
+
+
 def score_kpad(d):
     kpad = int(_lib.lib().kgc_score_kpad(int(d)))
     if kpad < 0:

@@ -25,11 +25,13 @@ class GraphedTrainStep(object):
     a replay equals the eager ``loss_sampled`` step on the same draws.  ``adversarial_temperature=alpha`` (with
     ``negatives=k`` only) trains with self-adversarial negative weights (``MGCN.loss_sampled``); the graph holds alpha as
     a constant.  ``criterion='ce'`` (with ``negatives=k`` only) trains the sampled softmax cross-entropy instead, at
-    ``label_smoothing=eps`` (``MGCN.loss_sampled``); the graph holds eps as a constant."""
+    ``label_smoothing=eps`` (``MGCN.loss_sampled``); the graph holds eps as a constant.  ``shared_negatives=True`` (with
+    ``negatives=k`` only) scores every query against one set of k negatives per batch (``MGCN.loss_sampled``); the
+    static draw buffer of the negatives is then ``neg_draws`` [k], and ``tries`` stays at its default."""
 
     def __init__(self, model, optimizer, graph, dataset, batch_size, clip_grad=1.0, warmup=3, fused_loss=False,
                  negatives=None, n_pos=1, tries=4, generator=None, adversarial_temperature=None, criterion='bce',
-                 label_smoothing=0.0):
+                 label_smoothing=0.0, shared_negatives=False):
         from .scoring import check_sampled_criterion
         adversarial_temperature, label_smoothing = check_sampled_criterion(criterion, adversarial_temperature,
                                                                            label_smoothing)
@@ -37,6 +39,11 @@ class GraphedTrainStep(object):
             raise ValueError('adversarial_temperature weights the sampled negatives: it needs negatives=k')
         if criterion == 'ce' and negatives is None:
             raise ValueError("criterion='ce' is a loss of the sampled objective: it needs negatives=k")
+        if shared_negatives and negatives is None:
+            raise ValueError('shared_negatives shares the sampled negatives across the batch: it needs negatives=k')
+        if shared_negatives and tries != 4:
+            raise ValueError('tries redraws the per-query negatives; shared negatives are filtered instead (leave tries '
+                             'at its default)')
         if negatives is not None:
             if fused_loss:
                 raise ValueError('negatives= and fused_loss=True are two different objectives: pass one of them')
@@ -56,10 +63,12 @@ class GraphedTrainStep(object):
         self.n_pos, self.tries, self.generator = int(n_pos), int(tries), generator
         self.adversarial_temperature = adversarial_temperature
         self.criterion, self.label_smoothing = criterion, label_smoothing
+        self.shared_negatives = bool(shared_negatives)
         self.pos_draws = self.neg_draws = self.label = None
         if self.objective == 'sampled':
             self.pos_draws = torch.zeros((self.B, self.n_pos), dtype=torch.int64, device=dev)
-            self.neg_draws = torch.zeros((self.B, self.negatives, self.tries), dtype=torch.int64, device=dev)
+            neg_shape = (self.negatives,) if self.shared_negatives else (self.B, self.negatives, self.tries)
+            self.neg_draws = torch.zeros(neg_shape, dtype=torch.int64, device=dev)
         elif self.objective == 'dense':
             self.label = torch.zeros((self.B, dataset.num_entity), dtype=torch.float32, device=dev)
         self.qid = torch.zeros((self.B,), dtype=torch.int64, device=dev)
@@ -103,7 +112,7 @@ class GraphedTrainStep(object):
             loss = self.model.loss_sampled(qid, self.ds, self.graph_data, self.negatives, n_pos=self.n_pos, tries=self.tries,
                                            draws=draws, generator=self.generator,
                                            adversarial_temperature=self.adversarial_temperature, criterion=self.criterion,
-                                           label_smoothing=self.label_smoothing)
+                                           label_smoothing=self.label_smoothing, shared_negatives=self.shared_negatives)
         elif self.objective == 'sparse':
             loss = self.model.loss_sparse(qid, self.ds, self.graph_data)
         else:
