@@ -393,6 +393,15 @@ typedef struct { float* param; const float* grad; float* exp_avg; float* exp_avg
 int32_t kgc_opt_chunk_elems(void);
 int kgc_clip_adam_step(const kgc_opt_tensor_t* tensors, const int32_t* items, int64_t n_items, const float* hyper,
                        double* state, double* partials, void* stream);
+/* The same step split in two for a model sharded over several GPUs (each rank holds some tensors, or some rows of them):
+ * kgc_clip_adam_sqnorm writes sqnorm[0] (device fp64) = the squared norm of this rank's items, where an item whose 4th
+ * field is non-zero adds 0 (a replicated tensor that another rank counts); the caller sums sqnorm over the ranks and
+ * kgc_clip_adam_apply runs the step's coefficient and update kernels with the norm sqrt(sqnorm[0]).  On one rank without
+ * flags the two calls equal kgc_clip_adam_step bit for bit.  partials[n_items] as above; the step ignores the 4th field. */
+int kgc_clip_adam_sqnorm(const kgc_opt_tensor_t* tensors, const int32_t* items, int64_t n_items, double* partials,
+                         double* sqnorm, void* stream);
+int kgc_clip_adam_apply(const kgc_opt_tensor_t* tensors, const int32_t* items, int64_t n_items, const float* hyper,
+                        double* state, const double* sqnorm, void* stream);
 
 /* ---- K10: halo exchange of the dst-partitioned layer over NVLink peer memory (SURVEY.md 8(e)) -----------------
  * Replaces the library all-gather of x / reduce-scatter of d_x of the partitioned layer: every rank keeps the gathered
@@ -489,6 +498,19 @@ int kgc_label_mask_t_build(const int64_t* qid, int64_t B, const int64_t* ptr, co
                            uint32_t* mask_t, void* stream);
 int kgc_bce_1n_bwd_logit_t(float* pred_t, const uint32_t* mask_t, int64_t n_ent, int32_t B, int32_t ldt, float pos, float add,
                            float* d_bias, double* loss_partial, float* loss, void* stream);
+/* The same loss on an entity-sharded table (MGCN.shard: each GPU holds the rows of the entities it owns, in its own order).
+ * kgc_label_mask_t_build_rows: kgc_label_mask_t_build with positive j's bit set in row row_of[j] of mask_t [n_rows,
+ * ceil(B / 32)] (zeroed by the call); row_of [n_entity] int32 maps a global id to its local row, -1 when another rank owns
+ * it (every id in idx must index row_of).  kgc_bce_1n_bwd_logit_t_shard: kgc_bce_1n_bwd_logit_t's pass over the n_rows
+ * local rows with the divisor of the whole table, B * n_total (formed as the unsharded call forms B * n_ent), so every
+ * gradient row and d_bias entry is bit-identical to that entity's row of the unsharded call; instead of the mean it writes
+ * the shard's fp64 sum of the loss terms, in a fixed order, to loss_sum[0] (device).  loss_partial:
+ * kgc_bce_1n_t_blocks(n_rows) doubles. */
+int kgc_label_mask_t_build_rows(const int64_t* qid, int64_t B, const int64_t* ptr, const int32_t* idx, const int32_t* row_of,
+                                int64_t n_rows, uint32_t* mask_t, void* stream);
+int kgc_bce_1n_bwd_logit_t_shard(float* pred_t, const uint32_t* mask_t, int64_t n_rows, int32_t B, int32_t ldt, float pos,
+                                 float add, int64_t n_total, float* d_bias, double* loss_partial, double* loss_sum,
+                                 void* stream);
 
 /* ---- K6: fused 1-N scoring + filter + rank (tcgen05 / TMA) --------------------------------------------
  * Replaces model.py:177-178 (X @ all_ent^T + bias) and main.py:122-126 (filter, rank) without

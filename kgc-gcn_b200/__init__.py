@@ -7,12 +7,12 @@ there is no CPU fallback.
 """
 from .conv import (MGCNConv, get_param, gemm_nt, gemm_tn, gemm_nt_trans, gemm_nt_splitk,   # noqa: F401
                    linear_tc, linear_tc_supported)
-from .model import MGCN, ConvE                   # noqa: F401
+from .model import MGCN, ConvE, ShardedMGCN      # noqa: F401
 from .data_loader import DataLoader, KBDataset, GraphData, BatchIterator, epoch_permutation   # noqa: F401
 from .plan import GraphPlan, get_plan, build_levels, build_stream_plan   # noqa: F401
 from .scoring import (EntityTable, filtered_rank, pack_queries, pair_scores, predict, evaluate,   # noqa: F401
                       score_kpad, topk, merge_topk, score_sampled_bce, score_sampled_ce, score_shared_bce,
-                      score_shared_ce)
+                      score_shared_ce, score_1n_bce_shard)
 from .partition import GraphPartition, partition_edges   # noqa: F401
 from .train import GraphedTrainStep             # noqa: F401
 from .optim import ClipAdam                      # noqa: F401

@@ -71,6 +71,8 @@ SIGNATURES = {
     'kgc_conv1ch_bwd': (ctypes.c_int, [_vp, _vp, _vp, _i64, _i32, _i32, _i32, _i32, _vp, _vp, _vp, _vp]),
     'kgc_opt_chunk_elems': (_i32, []),
     'kgc_clip_adam_step': (ctypes.c_int, [_vp, _vp, _i64, _vp, _vp, _vp, _vp]),
+    'kgc_clip_adam_sqnorm': (ctypes.c_int, [_vp, _vp, _i64, _vp, _vp, _vp]),
+    'kgc_clip_adam_apply': (ctypes.c_int, [_vp, _vp, _i64, _vp, _vp, _vp, _vp]),
     'kgc_p2p_allreduce': (ctypes.c_int, [_vp, _i64, _vp, _i32, _i32, _vp, _vp, _vp, _vp, _i64, _i32, _vp]),
     'kgc_p2p_barrier': (ctypes.c_int, [_vp, _i32, _i32, _vp, _vp, _vp]),
     'kgc_p2p_halo_gather': (ctypes.c_int, [_vp, _i32, _vp, _vp, _i64, _i64, _i32, _vp]),
@@ -88,6 +90,8 @@ SIGNATURES = {
     'kgc_bce_1n_t_blocks': (_i64, [_i64]),
     'kgc_label_mask_t_build': (ctypes.c_int, [_vp, _i64, _vp, _vp, _i64, _vp, _vp]),
     'kgc_bce_1n_bwd_logit_t': (ctypes.c_int, [_vp, _vp, _i64, _i32, _i32, _f32, _f32, _vp, _vp, _vp, _vp]),
+    'kgc_label_mask_t_build_rows': (ctypes.c_int, [_vp, _i64, _vp, _vp, _vp, _i64, _vp, _vp]),
+    'kgc_bce_1n_bwd_logit_t_shard': (ctypes.c_int, [_vp, _vp, _i64, _i32, _i32, _f32, _f32, _i64, _vp, _vp, _vp, _vp]),
     'kgc_score_kpad': (_i32, [_i32]),
     'kgc_score_pack_entities': (ctypes.c_int, [_vp, _vp, _i64, _i32, _vp, _vp]),
     'kgc_score_pack_queries': (ctypes.c_int, [_vp, _i64, _i32, _vp, _vp]),
@@ -143,7 +147,7 @@ def lib():
 
 
 LAUNCHES = 0     # kernels launched through the C ABI since import (bench.py reports it as gpu_launches)
-_KERNELS_PER_CALL = {'kgc_csr_build': 16, 'kgc_bce_1n_bwd_logit_t': 2, 'kgc_label_mask_t_build': 2, 'kgc_score_pairs': 3, 'kgc_rank_finalize': 2, 'kgc_score_topk': 2, 'kgc_topk_dense': 2, 'kgc_sampled_bce_fwd': 4, 'kgc_sampled_adv_fwd': 4, 'kgc_sampled_ce_fwd': 3, 'kgc_sampled_bce_bwd_table': 7, 'kgc_gemm_tn': 2, 'kgc_gemm_tn_tc_batch': 2, 'kgc_shared_mask_build': 3, 'kgc_shared_bce_loss': 4, 'kgc_shared_adv_loss': 4, 'kgc_shared_ce_loss': 4}   # (kgc_p2p_allreduce: 1 or 3)
+_KERNELS_PER_CALL = {'kgc_csr_build': 16, 'kgc_bce_1n_bwd_logit_t': 2, 'kgc_label_mask_t_build': 2, 'kgc_label_mask_t_build_rows': 2, 'kgc_bce_1n_bwd_logit_t_shard': 2, 'kgc_clip_adam_sqnorm': 2, 'kgc_clip_adam_apply': 2, 'kgc_score_pairs': 3, 'kgc_rank_finalize': 2, 'kgc_score_topk': 2, 'kgc_topk_dense': 2, 'kgc_sampled_bce_fwd': 4, 'kgc_sampled_adv_fwd': 4, 'kgc_sampled_ce_fwd': 3, 'kgc_sampled_bce_bwd_table': 7, 'kgc_gemm_tn': 2, 'kgc_gemm_tn_tc_batch': 2, 'kgc_shared_mask_build': 3, 'kgc_shared_bce_loss': 4, 'kgc_shared_adv_loss': 4, 'kgc_shared_ce_loss': 4}   # (kgc_p2p_allreduce: 1 or 3)
 
 
 def call(name, *args):

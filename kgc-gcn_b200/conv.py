@@ -819,23 +819,26 @@ class MGCNConv(nn.Module):
                 bn.running_mean.mul_(1.0 - mom).add_(stats[0], alpha=mom)
                 bn.running_var.mul_(1.0 - mom).add_(stats[1], alpha=mom * unbias)
 
-    def forward_partitioned(self, x_local, part, edge_embs_local, rels_embs):
+    def forward_partitioned(self, x_local, part, edge_embs_local, rels_embs, _out_drop=0.0):
         """The same layer on a dst-partitioned graph (SURVEY.md 8(e)): ``x_local`` = this rank's node rows,
         ``edge_embs_local`` = the rows of the edges it owns (``part.owned_eids`` order), ``part`` = a
         GraphPartition.  Exchanges: all-gather of x (forward), reduce-scatter of d_x (backward), all-reduce of the
-        BatchNorm column sums (2 x Dout doubles, both ways) and of the replicated-parameter gradients."""
+        BatchNorm column sums (2 x Dout doubles, both ways) and of the replicated-parameter gradients.
+        ``_out_drop`` as in ``forward`` (used by the sharded MGCN's encoder)."""
         m_in, m_out, keep_scale, seed, drop_p = self._masks(x_local.size(0), x_local.device)
         if seed is not None:
             seed = seed + part.rank          # decorrelate the row blocks of different ranks
         self._last_seed = seed
+        out_drop = self._out_drop_cfg(_out_drop, seed)
+        if out_drop is not None and seed is None:
+            out_drop = (out_drop[0], out_drop[1] + part.rank)       # its own stream: decorrelated as above
         bn = self.ent_bn
         use_batch_stats = self.training or bn.running_mean is None
-        coll = _Collectives(part.group, part.world, part.num_nodes, part.n_hub, part.hub_idx_mine, part.hub_rows_mine,
-                            part.p2p(x_local.shape[1]), part.rank, getattr(part, 'halo_rows64', None), part.n_loc)
+        coll = part.collectives(x_local.shape[1])
         all_ent, all_rel, stats = _ConvFn.apply(
             x_local, rels_embs, edge_embs_local, self.in_weight, self.out_weight, self.loop_weight, self.rels_weight,
             self.loop_rel, self.loop_edge, bn.weight, bn.bias, self.bias, part.plan, m_in, m_out, keep_scale,
-            use_batch_stats, bn.running_mean, bn.running_var, bn.eps, coll, seed, drop_p)
+            use_batch_stats, bn.running_mean, bn.running_var, bn.eps, coll, seed, drop_p, None, out_drop)
         self._update_running_stats(stats, part.num_nodes)
         return all_ent, all_rel
 

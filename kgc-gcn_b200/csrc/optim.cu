@@ -49,13 +49,8 @@ adam_prepare_kernel(const double* __restrict__ partials, int64_t n_partials, con
   state[4] = norm;
 }
 
-// work item i covers elements [items[i].y, items[i].y + items[i].z) of tensor items[i].x
-__global__ void __launch_bounds__(kThreadsOpt)
-grad_sqnorm_kernel(const kgc_opt_tensor_t* __restrict__ tensors, const int4* __restrict__ items, double* __restrict__ partials) {
-  __shared__ double sm[kThreadsOpt / 32];
-  const int4 it = __ldg(items + blockIdx.x);
-  const float* g = tensors[it.x].grad + (int64_t)it.y * kChunkOpt;
-  const int n = it.z;
+// The fp64 sum of the squares of g[0, n) in a fixed order (per-thread fp32, warp tree, warps in order): thread 0 returns it.
+__device__ __forceinline__ double chunk_sqnorm(const float* g, int n, double (&sm)[kThreadsOpt / 32]) {
   float acc = 0.f;                                   // <= 64 squares per thread before the fp64 tree
   if ((reinterpret_cast<uintptr_t>(g) & 15) == 0) {
     const float4* g4 = reinterpret_cast<const float4*>(g);
@@ -72,11 +67,50 @@ grad_sqnorm_kernel(const kgc_opt_tensor_t* __restrict__ tensors, const int4* __r
   for (int o = 16; o > 0; o >>= 1) d += __shfl_xor_sync(0xffffffffu, d, o);
   if (threadIdx.x % 32 == 0) sm[threadIdx.x / 32] = d;
   __syncthreads();
-  if (threadIdx.x == 0) {
-    double s = 0.0;
+  double s = 0.0;
+  if (threadIdx.x == 0)
     for (int w = 0; w < kThreadsOpt / 32; ++w) s += sm[w];
-    partials[blockIdx.x] = s;
+  return s;
+}
+
+// work item i covers elements [items[i].y, items[i].y + items[i].z) of tensor items[i].x
+__global__ void __launch_bounds__(kThreadsOpt)
+grad_sqnorm_kernel(const kgc_opt_tensor_t* __restrict__ tensors, const int4* __restrict__ items, double* __restrict__ partials) {
+  __shared__ double sm[kThreadsOpt / 32];
+  const int4 it = __ldg(items + blockIdx.x);
+  const double s = chunk_sqnorm(tensors[it.x].grad + (int64_t)it.y * kChunkOpt, it.z, sm);
+  if (threadIdx.x == 0) partials[blockIdx.x] = s;
+}
+
+// the same, except that an item with items[i].w != 0 adds 0: a tensor another rank counts (sharded models, kgc_clip_adam_sqnorm)
+__global__ void __launch_bounds__(kThreadsOpt)
+grad_sqnorm_flagged_kernel(const kgc_opt_tensor_t* __restrict__ tensors, const int4* __restrict__ items,
+                           double* __restrict__ partials) {
+  __shared__ double sm[kThreadsOpt / 32];
+  const int4 it = __ldg(items + blockIdx.x);
+  if (it.w != 0) {
+    if (threadIdx.x == 0) partials[blockIdx.x] = 0.0;
+    return;
   }
+  const double s = chunk_sqnorm(tensors[it.x].grad + (int64_t)it.y * kChunkOpt, it.z, sm);
+  if (threadIdx.x == 0) partials[blockIdx.x] = s;
+}
+
+// sqnorm[0] = the partials added in adam_prepare_kernel's order: on one rank without flags, sqrt(sqnorm[0]) is the norm
+// kgc_clip_adam_step computes, bit for bit
+__global__ void __launch_bounds__(kThreadsOpt)
+sqnorm_sum_kernel(const double* __restrict__ partials, int64_t n_partials, double* __restrict__ sqnorm) {
+  __shared__ double sm[kThreadsOpt / 32];
+  double d = 0.0;
+  for (int64_t i = threadIdx.x; i < n_partials; i += kThreadsOpt) d += partials[i];     // fixed order per thread
+#pragma unroll
+  for (int o = 16; o > 0; o >>= 1) d += __shfl_xor_sync(0xffffffffu, d, o);
+  if (threadIdx.x % 32 == 0) sm[threadIdx.x / 32] = d;
+  __syncthreads();
+  if (threadIdx.x != 0) return;
+  double s = 0.0;
+  for (int w = 0; w < kThreadsOpt / 32; ++w) s += sm[w];
+  sqnorm[0] = s;
 }
 
 __device__ __forceinline__ void adam1(float& p, float g, float& m, float& v, float coef, float wd, float b1c, float b2,
@@ -145,6 +179,37 @@ extern "C" int kgc_clip_adam_step(const kgc_opt_tensor_t* tensors, const int32_t
   grad_sqnorm_kernel<<<(unsigned)n_items, kThreadsOpt, 0, st>>>(tensors, it4, partials);
   KGC_LAUNCH_CHECK();
   adam_prepare_kernel<<<1, kThreadsOpt, 0, st>>>(partials, n_items, hyper, state);
+  KGC_LAUNCH_CHECK();
+  adam_update_kernel<<<(unsigned)n_items, kThreadsOpt, 0, st>>>(tensors, it4, hyper, state);
+  KGC_LAUNCH_CHECK();
+  return 0;
+}
+
+extern "C" int kgc_clip_adam_sqnorm(const kgc_opt_tensor_t* tensors, const int32_t* items, int64_t n_items, double* partials,
+                                    double* sqnorm, void* stream) {
+  KGC_REQUIRE(tensors != nullptr && items != nullptr && partials != nullptr && sqnorm != nullptr, "null argument");
+  KGC_REQUIRE(n_items >= 0 && n_items < (1ll << 31), "bad number of work items");
+  cudaStream_t st = as_stream(stream);
+  if (n_items == 0) {
+    KGC_CUDA_TRY(cudaMemsetAsync(sqnorm, 0, sizeof(double), st));
+    return 0;
+  }
+  grad_sqnorm_flagged_kernel<<<(unsigned)n_items, kThreadsOpt, 0, st>>>(tensors, reinterpret_cast<const int4*>(items), partials);
+  KGC_LAUNCH_CHECK();
+  sqnorm_sum_kernel<<<1, kThreadsOpt, 0, st>>>(partials, n_items, sqnorm);
+  KGC_LAUNCH_CHECK();
+  return 0;
+}
+
+extern "C" int kgc_clip_adam_apply(const kgc_opt_tensor_t* tensors, const int32_t* items, int64_t n_items, const float* hyper,
+                                   double* state, const double* sqnorm, void* stream) {
+  KGC_REQUIRE(tensors != nullptr && items != nullptr && hyper != nullptr && state != nullptr && sqnorm != nullptr,
+              "null argument");
+  if (n_items == 0) return 0;
+  KGC_REQUIRE(n_items < (1ll << 31), "too many work items");
+  cudaStream_t st = as_stream(stream);
+  const int4* it4 = reinterpret_cast<const int4*>(items);
+  adam_prepare_kernel<<<1, kThreadsOpt, 0, st>>>(sqnorm, 1, hyper, state);      // the norm of ONE partial: sqrt(*sqnorm)
   KGC_LAUNCH_CHECK();
   adam_update_kernel<<<(unsigned)n_items, kThreadsOpt, 0, st>>>(tensors, it4, hyper, state);
   KGC_LAUNCH_CHECK();

@@ -127,6 +127,32 @@ bce_1n_finalize_kernel(const double* __restrict__ partial, int64_t n_partial, do
   if (threadIdx.x == 0) loss[0] = (float)(s * inv_count);
 }
 
+// ---- the same loss on an ENTITY-SHARDED table (several GPUs, MGCN.shard): rank r holds the rows of the entities it owns,
+// in its own row order.  The label bits of a shard are those of kgc_label_mask_t_build with entity j moved to its local
+// row row_of[j] (-1: another rank owns j).  The loss pass is bce_1n_t_kernel itself, with the divisor of the whole table
+// (B * n_total): each of the shard's gradient rows is bit-identical to that row of the unsharded pass.  The shard's loss is
+// returned as a plain fp64 sum (the ranks add their sums; the caller divides).
+__global__ void __launch_bounds__(kThreadsST)
+label_mask_t_rows_kernel(const int64_t* __restrict__ qid, const int64_t* __restrict__ ptr, const int32_t* __restrict__ idx,
+                         const int32_t* __restrict__ row_of, int64_t n_rows, int wb, uint32_t* __restrict__ mask_t) {
+  const int64_t b = blockIdx.x;
+  const int64_t q = qid[b];
+  for (int64_t k = ptr[q] + threadIdx.x; k < ptr[q + 1]; k += kThreadsST) {
+    const int64_t j = idx[k];
+    if (j < 0) continue;
+    const int64_t r = row_of[j];
+    if (r >= 0 && r < n_rows) atomicOr(mask_t + r * wb + (b >> 5), 1u << (b & 31));
+  }
+}
+
+// the shard's loss: the per-CTA partials added in bce_1n_finalize_kernel's order, not scaled
+__global__ void __launch_bounds__(kThreadsST)
+bce_1n_sum_kernel(const double* __restrict__ partial, int64_t n_partial, double* __restrict__ loss_sum) {
+  __shared__ double sh[kThreadsST];
+  const double s = cta_sum_partials(partial, n_partial, sh);
+  if (threadIdx.x == 0) loss_sum[0] = s;
+}
+
 }  // namespace
 }  // namespace kgc
 
@@ -170,6 +196,36 @@ extern "C" int kgc_bce_1n_bwd_logit_t(float* pred_t, const uint32_t* mask_t, int
                                                                        add, (float)(1.0 / count), d_bias, loss_partial);
   KGC_LAUNCH_CHECK();
   bce_1n_finalize_kernel<<<1, kThreadsST, 0, as_stream(stream)>>>(loss_partial, blocks, 1.0 / count, loss);
+  KGC_LAUNCH_CHECK();
+  return 0;
+}
+
+extern "C" int kgc_label_mask_t_build_rows(const int64_t* qid, int64_t B, const int64_t* ptr, const int32_t* idx,
+                                           const int32_t* row_of, int64_t n_rows, uint32_t* mask_t, void* stream) {
+  KGC_REQUIRE(B >= 0 && n_rows >= 0, "bad sizes");
+  if (B == 0 || n_rows == 0) return 0;
+  KGC_REQUIRE(qid && ptr && idx && row_of && mask_t, "null buffer");
+  const int wb = (int)ceil_div(B, 32);
+  KGC_CUDA_TRY(cudaMemsetAsync(mask_t, 0, (size_t)(n_rows * wb) * sizeof(uint32_t), as_stream(stream)));
+  label_mask_t_rows_kernel<<<(unsigned)B, kThreadsST, 0, as_stream(stream)>>>(qid, ptr, idx, row_of, n_rows, wb, mask_t);
+  KGC_LAUNCH_CHECK();
+  return 0;
+}
+
+extern "C" int kgc_bce_1n_bwd_logit_t_shard(float* pred_t, const uint32_t* mask_t, int64_t n_rows, int32_t B, int32_t ldt,
+                                            float pos, float add, int64_t n_total, float* d_bias, double* loss_partial,
+                                            double* loss_sum, void* stream) {
+  KGC_REQUIRE(n_rows >= 0 && n_total > 0 && n_rows <= n_total && B > 0 && ldt >= B && ldt % 4 == 0,
+              "bad sizes (0 <= n_rows <= n_total, ldt a multiple of 4)");
+  KGC_REQUIRE(loss_partial && loss_sum, "null buffer");
+  KGC_REQUIRE(n_rows == 0 || (pred_t && mask_t && d_bias), "null buffer");
+  KGC_REQUIRE((reinterpret_cast<uintptr_t>(pred_t) & 15) == 0, "pred_t must be 16-byte aligned");
+  const int64_t blocks = kgc_bce_1n_t_blocks(n_rows);
+  const double count = (double)B * (double)n_total;                 // the unsharded call's divisor, formed the same way
+  bce_1n_t_kernel<<<(unsigned)blocks, kThreadsST, 0, as_stream(stream)>>>(pred_t, mask_t, (int)ceil_div(B, 32), n_rows, B, ldt,
+                                                                       pos, add, (float)(1.0 / count), d_bias, loss_partial);
+  KGC_LAUNCH_CHECK();
+  bce_1n_sum_kernel<<<1, kThreadsST, 0, as_stream(stream)>>>(loss_partial, blocks, loss_sum);
   KGC_LAUNCH_CHECK();
   return 0;
 }

@@ -7,6 +7,7 @@ the convolution (K8) and the fc layer (3xTF32 tensor-core GEMMs) run on our kern
 call-compatible) and its autograd run on the 3xTF32 tensor-core kernels (K6t, scoring.score_1n); ``rank`` uses the
 fused tensor-core scoring + ranking kernel (K6).
 """
+import copy
 import weakref
 
 import torch
@@ -211,6 +212,39 @@ class _RowsAndTable(torch.autograd.Function):
         return d_table, None
 
 
+class _ShardRows(torch.autograd.Function):
+    """_RowsAndTable for an entity-sharded table (MGCN.shard): (the batch's subject rows [B, D], table) where ``rows`` [B]
+    holds each subject's local row, -1 when another rank owns it.  Forward: every rank writes the rows it owns and zeros
+    elsewhere, and the ranks add the [B, D] buffers - each row is non-zero on one rank only, so the sum is exact and the
+    same on every rank.  Backward: the rows' gradient is the same on every rank (ConvE is replicated); the owner adds it
+    into its table gradient, duplicates summed by a [B, B] equality product as _RowsAndTable does.  No exchange, static
+    shapes, no host sync."""
+
+    @staticmethod
+    def forward(ctx, table, rows, coll):
+        mine = rows >= 0
+        key = torch.where(mine, rows, torch.zeros_like(rows))          # row 0 stands in for the other ranks' subjects
+        out = torch.where(mine[:, None], table.index_select(0, key), table.new_zeros(())).contiguous()
+        coll.all_reduce(out, 'shard_rows')
+        ctx.save_for_backward(key, mine)
+        ctx.shape = table.shape
+        return out, table.detach().view_as(table)
+
+    @staticmethod
+    def backward(ctx, d_rows, d_table):
+        key, mine = ctx.saved_tensors
+        if d_table is None:
+            d_table = torch.zeros(ctx.shape, dtype=d_rows.dtype, device=d_rows.device)
+        elif not d_table.is_contiguous():
+            d_table = d_table.contiguous()
+        if d_rows is not None:
+            # the stand-in rows add nothing, so every entry with key k writes the same total: deterministic
+            c = torch.where(mine[:, None], d_rows, d_rows.new_zeros(()))
+            total = (key[:, None] == key[None, :]).to(d_rows.dtype) @ c
+            d_table.index_copy_(0, key, d_table.index_select(0, key) + total)
+        return d_table, None, None
+
+
 class MGCN(nn.Module):
 
     def __init__(self, num_entities, num_relations, num_edges, params):
@@ -352,6 +386,13 @@ class MGCN(nn.Module):
         return score_sampled_bce(x, all_ent, self.conv2.bias, cand, n_pos, pos, add,
                                  adversarial_temperature=adversarial_temperature)
 
+    def shard(self, part):
+        """This model split over the ranks of ``part`` (a GraphPartition of its graph) for multi-GPU training: a
+        ShardedMGCN on ``part.device`` that holds ``entity_embedding[owned_nodes]``, ``edge_embeddings[owned_eids]`` and
+        ``conv2.bias[owned_nodes]`` and a copy of every other parameter and buffer.  This model may live on the host: only
+        the shards and the replicated parts are copied to the device.  Every rank calls it on the same model."""
+        return ShardedMGCN(self, part)
+
     def rank(self, src, rel, obj, filt_ptr, filt_idx, data, count_eq=False):
         """Filtered rank of obj among all entities for the queries (src, rel) without materialising the
         [B, N] scores (K6): what main.py:121-126 computes from model(sub, rel, graph)."""
@@ -388,3 +429,114 @@ class MGCN(nn.Module):
             n_offset = lo
             ent, bias = all_ent[lo:hi], (bias[lo:hi] if bias is not None else None)
         return topk(xq, ent, bias, k, ptr, idx, table=table, precision=precision, n_offset=n_offset, group=group)
+
+
+class ShardedMGCN(nn.Module):
+    """An MGCN split over the ranks of a GraphPartition (``MGCN.shard(part)``), one process per GPU.
+
+    The entity table, the edge table and ConvE's per-entity bias are sharded as the partition shards the layer
+    (``owned_nodes``, ``owned_eids``); every other parameter is replicated.  Every rank handles the same batch of queries:
+    the encoder runs partitioned (``MGCNConv.forward_partitioned``), the subjects' rows are gathered across the ranks,
+    ConvE runs replicated on identical inputs and scores the rank's own entities (``scoring.score_1n_bce_shard``).  The
+    replicated parameters therefore receive identical gradients on every rank without an exchange.  ConvE's dropouts draw
+    from torch's generator: seed it identically on every rank (``torch.manual_seed``).  Parameter names are MGCN's;
+    ``full_state_dict()`` reassembles the unsharded state dict."""
+
+    def __init__(self, model, part):
+        super(ShardedMGCN, self).__init__()
+        if not isinstance(model.conv1, MGCNConv):
+            raise ValueError('MGCN.shard: the encoder must be the CUDA MGCNConv')
+        if not 0.0 <= float(model.params.gcn_drop) < 1.0:
+            raise ValueError('MGCN.shard: gcn_drop must be in [0, 1)')
+        n, e2 = model.entity_embedding.shape[0], model.edge_embeddings.shape[0]
+        if part.num_nodes != n or int(part.plan.num_types) != model.relation_embedding.shape[0] + 1:
+            raise ValueError('MGCN.shard: the partition is not one of this model\'s graph')
+        dev = part.device
+        self.params = model.params
+        self.partition = part
+        self.num_edges2 = int(e2)
+
+        def rows(t, ids):
+            return nn.Parameter(t.detach().index_select(0, ids.to(t.device)).to(dev, copy=True))
+        self.entity_embedding = rows(model.entity_embedding, part.owned_nodes)
+        self.relation_embedding = nn.Parameter(model.relation_embedding.detach().to(dev, copy=True))
+        self.edge_embeddings = rows(model.edge_embeddings, part.owned_eids)
+        self.conv1 = copy.deepcopy(model.conv1).to(dev)
+        bias = model.conv2.bias
+        model.conv2.bias = None                  # not copied whole: only this rank's rows go to the device
+        try:
+            self.conv2 = copy.deepcopy(model.conv2).to(dev)
+        finally:
+            model.conv2.bias = bias
+        self.conv2.bias = rows(bias, part.owned_nodes)
+
+    def sharded_parameters(self):
+        """The parameters that hold only this rank's rows (``ClipAdam(..., sharded=)``)."""
+        return [self.entity_embedding, self.edge_embeddings, self.conv2.bias]
+
+    def encode(self):
+        """The partitioned encoder: (this rank's rows of all_ent after gcn_drop, all_rel) - gcn_drop inside the layer's
+        last kernel, as MGCN.encode on one GPU."""
+        return self.conv1.forward_partitioned(self.entity_embedding, self.partition, self.edge_embeddings,
+                                              self.relation_embedding, _out_drop=float(self.params.gcn_drop))
+
+    def loss_sparse(self, qid, dataset, data=None):
+        """``MGCN.loss_sparse`` on the sharded model: the mean BCE over the batch's queries ``qid`` against ALL entities,
+        the same value on every rank.  Every rank must pass the same qid.  ``data`` is not used (the partition holds the
+        graph); it is accepted so that the call matches MGCN's."""
+        from .scoring import score_1n_bce_shard
+        part = self.partition
+        dev = self.entity_embedding.device
+        triples, ptr, idx = dataset.device_csr(dev)
+        qid = torch.as_tensor(qid, dtype=torch.int64).to(dev, non_blocking=True)
+        trip = torch.index_select(triples, 0, qid)
+        all_ent, all_rel = self.encode()
+        coll = part.collectives(self.entity_embedding.shape[1])
+        row_of = part.row_of()
+        src_emb, all_ent = _ShardRows.apply(all_ent, row_of.index_select(0, trip[:, 0]).to(torch.int64), coll)
+        x = self.conv2.query(src_emb, torch.index_select(all_rel, 0, trip[:, 1]))
+        pos, add = dataset.label_values()
+        return score_1n_bce_shard(x, all_ent, self.conv2.bias, qid, ptr, idx, row_of, part.num_nodes, coll, pos, add)
+
+    def loss_sampled(self, *args, **kwargs):
+        raise ValueError('the sampled objectives (negatives=k) score rows of arbitrary candidates, which a sharded model '
+                         'does not hold; train a sharded model with loss_sparse')
+
+    def full_state_dict(self):
+        """The unsharded state dict (MGCN's key names and layout) as host tensors on rank 0, None on the other ranks: the
+        sharded rows are sent to rank 0 and put back in their global order.  Every rank must call it."""
+        import torch.distributed as dist
+        part = self.partition
+        group = part.group
+        rank = part.rank
+        root = 0 if group is None else dist.get_global_rank(group, 0)
+        glob = lambda r: r if group is None else dist.get_global_rank(group, r)        # noqa: E731
+        full_rows = {'entity_embedding': (part.owned_nodes, part.num_nodes), 'conv2.bias': (part.owned_nodes, part.num_nodes),
+                     'edge_embeddings': (part.owned_eids, self.num_edges2)}
+        out = {} if rank == 0 else None
+        for name, t in self.state_dict().items():
+            if name not in full_rows:
+                if out is not None:
+                    out[name] = t.detach().cpu().clone()
+                continue
+            ids, n = full_rows[name]
+            t = t.detach().contiguous()
+            ids = ids.to(device=t.device, dtype=torch.int64).contiguous()
+            cnt = torch.tensor([ids.numel()], dtype=torch.int64, device=t.device)
+            counts = [torch.zeros_like(cnt) for _ in range(part.world)]
+            dist.all_gather(counts, cnt, group=group)
+            if rank != 0:
+                dist.send(ids, dst=root, group=group)
+                dist.send(t, dst=root, group=group)
+                continue
+            full = torch.empty((n,) + tuple(t.shape[1:]), dtype=t.dtype)
+            full[ids.cpu()] = t.cpu()
+            for r in range(1, part.world):
+                m = int(counts[r])
+                r_ids = torch.empty((m,), dtype=torch.int64, device=t.device)
+                r_rows = torch.empty((m,) + tuple(t.shape[1:]), dtype=t.dtype, device=t.device)
+                dist.recv(r_ids, src=glob(r), group=group)
+                dist.recv(r_rows, src=glob(r), group=group)
+                full[r_ids.cpu()] = r_rows.cpu()
+            out[name] = full
+        return out

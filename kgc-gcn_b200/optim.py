@@ -9,6 +9,11 @@ The learning rate, step counter and bias corrections live in device memory: a CU
 scheduler changes ``param_group['lr']`` (call ``sync_hyper()`` - ``step()`` does outside graph capture).
 GPU only, fp32 parameters, one parameter group when clipping (the norm is taken over the group, as the reference's is
 over all parameters).
+
+A model sharded over several GPUs (``MGCN.shard``) passes ``partition=`` (its GraphPartition) and ``sharded=`` (its
+sharded parameters, ``model.sharded_parameters()``): the norm is then that of the whole model - every rank's sharded
+parameters plus the replicated ones counted on rank 0, summed over the ranks in one all-reduce of the partition's
+exchange (peer memory when it has it, NCCL otherwise) - and every rank applies the same coefficient.
 """
 import torch
 
@@ -17,7 +22,8 @@ from . import _lib
 
 class ClipAdam(torch.optim.Optimizer):
 
-    def __init__(self, params, lr=1e-3, betas=(0.9, 0.999), eps=1e-8, weight_decay=0.0, max_norm=None):
+    def __init__(self, params, lr=1e-3, betas=(0.9, 0.999), eps=1e-8, weight_decay=0.0, max_norm=None, partition=None,
+                 sharded=()):
         if lr < 0.0 or eps < 0.0 or not 0.0 <= betas[0] < 1.0 or not 0.0 <= betas[1] < 1.0 or weight_decay < 0.0:
             raise ValueError('invalid Adam hyper-parameters')
         defaults = dict(lr=lr, betas=tuple(betas), eps=eps, weight_decay=weight_decay, max_norm=max_norm,
@@ -26,6 +32,13 @@ class ClipAdam(torch.optim.Optimizer):
         super(ClipAdam, self).__init__(params, defaults)
         if len(self.param_groups) > 1 and any(g.get('max_norm') for g in self.param_groups):
             raise ValueError('ClipAdam clips over one parameter group (the reference passes model.parameters())')
+        if partition is None and len(tuple(sharded)):
+            raise ValueError('sharded= names the parameters a partition splits: pass partition= as well')
+        if partition is not None and len(self.param_groups) > 1:
+            raise ValueError('ClipAdam over a sharded model takes one parameter group')
+        self.partition = partition
+        self._sharded = set(id(p) for p in sharded)
+        self._coll = None
         self._dev = {}            # group index -> device-side buffers
         self.last_grad_norm = None
 
@@ -40,8 +53,10 @@ class ClipAdam(torch.optim.Optimizer):
         items = []
         for t, p in enumerate(params):
             n = p.numel()
+            # a replicated tensor of a sharded model enters the norm on rank 0 only
+            skip = int(self.partition is not None and self.partition.rank != 0 and id(p) not in self._sharded)
             for c in range((n + chunk - 1) // chunk):
-                items.append((t, c, min(chunk, n - c * chunk), 0))
+                items.append((t, c, min(chunk, n - c * chunk), skip))
         step0 = 0.0
         for p in params:
             s = self.state[p]
@@ -57,6 +72,7 @@ class ClipAdam(torch.optim.Optimizer):
             'items': torch.tensor(items, dtype=torch.int32, device=dev).reshape(-1, 4),
             'n_items': len(items),
             'partials': torch.empty((max(len(items), 1),), dtype=torch.float64, device=dev),
+            'sqnorm': torch.zeros((2,), dtype=torch.float64, device=dev),      # [0]: squared norm; 16-byte all-reduce payload
             'state': torch.tensor([step0, 1.0, 0.0, 0.0, 0.0], dtype=torch.float64, device=dev),
             'hyper': torch.zeros((6,), dtype=torch.float32, device=dev),
             'hyper_host': None,
@@ -143,8 +159,17 @@ class ClipAdam(torch.optim.Optimizer):
                 st['table'].copy_(pinned, non_blocking=True)
             else:                             # gradients are re-allocated by every backward: refresh the table (32 B / tensor)
                 st['table'].copy_(host)
-            _lib.call('kgc_clip_adam_step', _lib.ptr(st['table']), _lib.ptr(st['items']), st['n_items'], _lib.ptr(st['hyper']),
-                      _lib.ptr(st['state']), _lib.ptr(st['partials']), _lib.stream())
+            if self.partition is None:
+                _lib.call('kgc_clip_adam_step', _lib.ptr(st['table']), _lib.ptr(st['items']), st['n_items'],
+                          _lib.ptr(st['hyper']), _lib.ptr(st['state']), _lib.ptr(st['partials']), _lib.stream())
+            else:
+                _lib.call('kgc_clip_adam_sqnorm', _lib.ptr(st['table']), _lib.ptr(st['items']), st['n_items'],
+                          _lib.ptr(st['partials']), _lib.ptr(st['sqnorm']), _lib.stream())
+                if self._coll is None:                # the exchange of the model's forward (it ran before this step)
+                    self._coll = self.partition.collectives()
+                self._coll.all_reduce(st['sqnorm'], 'clip_sqnorm')
+                _lib.call('kgc_clip_adam_apply', _lib.ptr(st['table']), _lib.ptr(st['items']), st['n_items'],
+                          _lib.ptr(st['hyper']), _lib.ptr(st['state']), _lib.ptr(st['sqnorm']), _lib.stream())
             self.last_grad_norm = st['state'][4]
         return loss
 

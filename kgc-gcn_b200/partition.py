@@ -470,6 +470,23 @@ class GraphPartition(object):
                               n_dst_rows=ext_nodes if self.hybrid else self.block, dst_offset=offset,
                               deg=as_t(info['deg']))
 
+    def collectives(self, D=None):
+        """The exchanges of this partition (conv._Collectives) for feature width ``D``.  ``D=None``: those of a width
+        already in use (the first peer-memory context created, e.g. by the layer's forward), NCCL when there is none."""
+        from .conv import _Collectives
+        ctx = next((c for c in self._p2p.values() if c is not None), None) if D is None else self.p2p(D)
+        return _Collectives(self.group, self.world, self.num_nodes, self.n_hub, self.hub_idx_mine, self.hub_rows_mine, ctx,
+                            self.rank, getattr(self, 'halo_rows64', None), self.n_loc)
+
+    def row_of(self):
+        """[num_nodes] int32 on the device: the local row of every node this rank owns (``owned_nodes`` order), -1 for
+        the nodes of other ranks."""
+        if getattr(self, '_row_of', None) is None:
+            r = torch.full((self.num_nodes,), -1, dtype=torch.int32, device=self.device)
+            r[self.owned_nodes] = torch.arange(self.owned_nodes.numel(), dtype=torch.int32, device=self.device)
+            self._row_of = r
+        return self._row_of
+
     # ------------------------------------------------------------------ peer-memory halo exchange (K10)
     def p2p(self, D):
         """Symmetric buffers + peer pointer tables of the halo exchange for feature width ``D`` (allocated and rendezvoused

@@ -143,6 +143,91 @@ def score_1n_bce(x, all_ent, bias, qid, ptr, idx, pos=1.0, add=0.0):
     return total
 
 
+class _Score1NBCEShard(torch.autograd.Function):
+    """``score_1n_bce`` on an entity-sharded table (``MGCN.shard``): this rank holds the rows ``ent`` / ``bias`` of the
+    entities it owns, and every rank scores the same B queries x.  Per tile of B_TILE queries the scorer runs on the local
+    rows, the positives set their bits in the local rows (``row_of``) and the shard loss pass writes the logit gradient with
+    the divisor of the whole table (B_tile * n_total) and the shard's fp64 loss sum.  The ranks add the loss sums (ONE
+    all-reduce); in the backward they add the partial d_x [B, D] (ONE all-reduce), while d_ent and d_bias stay local."""
+
+    @staticmethod
+    def forward(ctx, x, all_ent, bias, qid, ptr, idx, row_of, n_total, coll, pos, add):
+        x = _lib.require_cuda(x.detach(), torch.float32, 'x')
+        ent = _lib.require_cuda(all_ent.detach(), torch.float32, 'all_ent')
+        bias_ = _lib.require_cuda(bias.detach(), torch.float32, 'bias')
+        qid = _lib.require_cuda(qid, torch.int64, 'qid')
+        ptr = _lib.require_cuda(ptr, torch.int64, 'ptr')
+        idx = _lib.require_cuda(idx, torch.int32, 'idx')
+        row_of = _lib.require_cuda(row_of, torch.int32, 'row_of')
+        B, D = int(x.shape[0]), int(x.shape[1])
+        Nl = int(ent.shape[0])
+        if int(qid.numel()) != B:
+            raise ValueError('qid has {} entries for {} queries'.format(int(qid.numel()), B))
+        p, dev = _lib.ptr, x.device
+        tiles = [(i, min(B_TILE, B - i)) for i in range(0, B, B_TILE)]
+        sums = torch.zeros(((len(tiles) + 1) // 2 * 2,), dtype=torch.float64, device=dev)     # 16-byte all-reduce payload
+        d_logit, d_bias = [], []
+        for t, (i, bt) in enumerate(tiles):
+            ldt = (bt + 3) // 4 * 4
+            d_logit_t = torch.empty((Nl, ldt), dtype=torch.float32, device=dev)
+            _lib.call('kgc_score_1n_fwd_t', p(ent), Nl, D, ent.stride(0), p(_pack_b(x[i:i + bt].t())), bt, p(bias_), p(d_logit_t),
+                      ldt, _lib.stream())
+            mask_t = torch.empty((Nl, (bt + 31) // 32), dtype=torch.int32, device=dev)
+            _lib.call('kgc_label_mask_t_build_rows', p(qid[i:i + bt]), bt, p(ptr), p(idx), p(row_of), Nl, p(mask_t), _lib.stream())
+            db = torch.empty((Nl,), dtype=torch.float32, device=dev)
+            partial = torch.empty((int(_lib.lib().kgc_bce_1n_t_blocks(Nl)),), dtype=torch.float64, device=dev)
+            _lib.call('kgc_bce_1n_bwd_logit_t_shard', p(d_logit_t), p(mask_t), Nl, bt, ldt, float(pos), float(add), int(n_total),
+                      p(db), p(partial), p(sums[t:t + 1]), _lib.stream())
+            d_logit.append(d_logit_t)
+            d_bias.append(db)
+        coll.all_reduce(sums, 'bce_1n_loss')
+        # score_1n_bce's value: per tile the mean over bt * N, weighted by the tile's share of the batch
+        loss = None
+        for t, (i, bt) in enumerate(tiles):
+            part = sums[t] * (1.0 / (float(bt) * float(n_total)))
+            if len(tiles) > 1:
+                part = part * (float(bt) / B)
+            loss = part if loss is None else loss + part
+        ctx.save_for_backward(x, ent, *d_logit, *d_bias)
+        ctx.tiles, ctx.coll = tiles, coll
+        return loss.to(torch.float32)
+
+    @staticmethod
+    def backward(ctx, g):
+        from .conv import gemm_nt, gemm_tn
+        x, ent = ctx.saved_tensors[:2]
+        T = len(ctx.tiles)
+        d_logit, d_bias_t = ctx.saved_tensors[2:2 + T], ctx.saved_tensors[2 + T:]
+        B, D = int(x.shape[0]), int(x.shape[1])
+        Nl = int(ent.shape[0])
+        gs = [g if T == 1 else g * (float(bt) / B) for _, bt in ctx.tiles]
+        d_x = torch.empty((B, D), dtype=torch.float32, device=x.device)
+        for (i, bt), dl, gt in zip(ctx.tiles, d_logit, gs):
+            d_x[i:i + bt] = gemm_tn(dl, ent, torch.empty((dl.shape[1], D), dtype=torch.float32, device=x.device))[:bt] * gt
+        ctx.coll.all_reduce(d_x, 'bce_1n_dx')                 # every rank's entities contribute to every query's d_x
+        d_ent = d_bias = None
+        if ctx.needs_input_grad[1]:
+            for (i, bt), dl, gt in zip(ctx.tiles, d_logit, gs):
+                part = gemm_nt(dl[:, :bt], (x[i:i + bt] * gt).contiguous(), torch.empty((Nl, D), dtype=torch.float32,
+                                                                                       device=x.device))
+                d_ent = part if d_ent is None else d_ent + part
+        if ctx.needs_input_grad[2]:
+            for db, gt in zip(d_bias_t, gs):
+                d_bias = db * gt if d_bias is None else d_bias + db * gt
+        return d_x, d_ent, d_bias, None, None, None, None, None, None, None, None
+
+
+def score_1n_bce_shard(x, all_ent, bias, qid, ptr, idx, row_of, n_total, coll, pos=1.0, add=0.0):
+    """``score_1n_bce`` over all ``n_total`` entities when this rank holds only the rows of the entities it owns:
+    ``all_ent`` / ``bias`` are those rows, ``row_of`` [n_total] int32 maps a global entity id to its local row (-1: another
+    rank's), ``coll`` is the partition's exchange (``GraphPartition.collectives``).  Every rank passes the same x and qid and
+    gets the same loss; the gradients of x are summed over the ranks, those of all_ent and bias are the local rows'.
+    Batches above B_TILE queries are scored tile by tile as ``score_1n_bce`` does."""
+    if not score_1n_supported(x, all_ent):
+        raise RuntimeError('score_1n_bce_shard: shape not taken by the tensor-core scorer (Dout <= 224, Dout % 4 == 0)')
+    return _Score1NBCEShard.apply(x, all_ent, bias, qid, ptr, idx, row_of, int(n_total), coll, pos, add)
+
+
 # each sampled loss: its C forward and its number of halves (int32 counts, and fp64 loss partials per forward CTA)
 _SAMPLED_FWD = {'bce': ('kgc_sampled_bce_fwd', 1), 'adv': ('kgc_sampled_adv_fwd', 2), 'ce': ('kgc_sampled_ce_fwd', 1)}
 

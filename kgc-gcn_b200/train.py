@@ -27,7 +27,14 @@ class GraphedTrainStep(object):
     a constant.  ``criterion='ce'`` (with ``negatives=k`` only) trains the sampled softmax cross-entropy instead, at
     ``label_smoothing=eps`` (``MGCN.loss_sampled``); the graph holds eps as a constant.  ``shared_negatives=True`` (with
     ``negatives=k`` only) scores every query against one set of k negatives per batch (``MGCN.loss_sampled``); the
-    static draw buffer of the negatives is then ``neg_draws`` [k], and ``tries`` stays at its default."""
+    static draw buffer of the negatives is then ``neg_draws`` [k], and ``tries`` stays at its default.
+
+    A sharded model (``MGCN.shard``, one process per GPU) trains with ``fused_loss=True`` and ``ClipAdam(...,
+    max_norm=clip_grad, partition=, sharded=)``; ``graph`` is not used then (the partition holds it) and may be None.  The
+    graph holds the whole step: encoder, subject rows, scorer, loss, the loss and d_x all-reduces, ConvE, backward and
+    ClipAdam.  Capture needs the partition's peer-memory exchange; on NCCL the constructor raises a ValueError, and the
+    eager ``loss_sparse`` / ``backward`` / ``step`` loop trains the model instead.  Every rank passes the same query ids
+    (e.g. ``BatchIterator`` with the same seed): the eager calls before the capture and the ragged batches check it."""
 
     def __init__(self, model, optimizer, graph, dataset, batch_size, clip_grad=1.0, warmup=3, fused_loss=False,
                  negatives=None, n_pos=1, tries=4, generator=None, adversarial_temperature=None, criterion='bce',
@@ -44,6 +51,20 @@ class GraphedTrainStep(object):
         if shared_negatives and tries != 4:
             raise ValueError('tries redraws the per-query negatives; shared negatives are filtered instead (leave tries '
                              'at its default)')
+        self.sharded = getattr(model, 'partition', None) is not None
+        if self.sharded:
+            if negatives is not None:
+                raise ValueError('the sampled objectives (negatives=k) score rows of arbitrary candidates, which a sharded '
+                                 'model does not hold: train a sharded model with fused_loss=True')
+            if not fused_loss:
+                raise ValueError('a sharded model trains through loss_sparse: pass fused_loss=True')
+            if getattr(optimizer, 'partition', None) is not model.partition or \
+                    not all(g.get('max_norm') for g in optimizer.param_groups):
+                raise ValueError('a sharded model needs ClipAdam(..., max_norm=clip_grad, partition=model.partition, '
+                                 'sharded=model.sharded_parameters()): the gradient norm is taken over all ranks')
+            if model.partition.p2p(model.entity_embedding.shape[1]) is None:
+                raise ValueError('a sharded model on the NCCL exchange (no peer memory) cannot be captured into a CUDA '
+                                 'graph: train it eagerly (loss_sparse, backward, ClipAdam.step)')
         if negatives is not None:
             if fused_loss:
                 raise ValueError('negatives= and fused_loss=True are two different objectives: pass one of them')
@@ -51,7 +72,7 @@ class GraphedTrainStep(object):
                 raise ValueError('negatives, n_pos and tries must be positive')
         self.model, self.opt, self.graph_data, self.ds = model, optimizer, graph, dataset
         self.clip, self.B = float(clip_grad), int(batch_size)
-        dev = graph.edge_index.device
+        dev = model.entity_embedding.device if self.sharded else graph.edge_index.device
         if dev.type != 'cuda':
             raise RuntimeError('GraphedTrainStep runs on the GPU only')
         self.dev = dev
@@ -181,7 +202,26 @@ class GraphedTrainStep(object):
             return self.qid, (self.pos_draws, self.neg_draws)
         return (self.qid if self.objective == 'sparse' else None), None
 
+    def _check_same_queries(self, qid):
+        """A sharded model replicates the batch: every rank must pass the same query ids (eager calls only)."""
+        import torch.distributed as dist
+        part = self.model.partition
+        q = torch.as_tensor(qid, dtype=torch.int64).to(self.dev)
+        n = torch.tensor([q.numel()], dtype=torch.int64, device=self.dev)
+        ns = [torch.empty_like(n) for _ in range(part.world)]
+        dist.all_gather(ns, n, group=part.group)
+        same = all(int(v) == q.numel() for v in ns)
+        if same:
+            every = torch.empty((part.world * q.numel(),), dtype=torch.int64, device=self.dev)
+            dist.all_gather_into_tensor(every, q, group=part.group)
+            same = bool((every.view(part.world, -1) == q[None]).all())
+        if not same:                                 # every rank sees the same ids, so all of them raise
+            raise ValueError('a sharded model needs the same query ids on every rank (e.g. BatchIterator with the same '
+                             'seed); the ranks passed different ones')
+
     def __call__(self, qid):
+        if self.sharded and (self.cuda_graph is None or len(qid) != self.B):
+            self._check_same_queries(qid)
         if len(qid) != self.B:                       # ragged last batch: the eager path (same arithmetic)
             self.opt.zero_grad(set_to_none=True)
             if self.objective != 'dense':
